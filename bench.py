@@ -21,6 +21,10 @@ integrator, 8 agents, 2 landmarks per agent, HJ safety filter on with the synthe
 
 `--impl reference` times the CPU oracle port alone (the reference itself is Python and does not exist
 on the GPU box); rank 0 only.
+
+`--steps K` is the number of timed steps of the headline measurement (of every arm). `--dump-outputs DIR` writes, after
+the timed steps, what the last timed step returned to its caller as DIR/<name>.npy (see dump_outputs); the inputs are
+seeded, so two builds run with the same arguments can be compared array by array.
 """
 from __future__ import annotations
 
@@ -32,6 +36,7 @@ import subprocess
 import sys
 import time
 
+sys.dont_write_bytecode = True      # the benchmark leaves the tree it runs from as it found it
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
 sys.path.insert(0, os.path.join(REPO, 'tests'))
@@ -81,6 +86,30 @@ def measured_peak():
         except Exception:
             pass
     return 6650.0, 'fallback (B200_PROFILING.md 6.65 TB/s)'
+
+
+DUMP_BYTES = 64 * 1000 * 1000     # upper bound of the files --dump-outputs writes, headers included
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """`--dump-outputs`: save {name: array with the environments on axis 0} (torch or numpy) as <out_dir>/<name>.npy,
+    float64 arrays as float64 and everything else (float32 observations, int agent ids, bool / uint8 dones) as float32.
+    When the whole batch would exceed DUMP_BYTES, every array keeps the same fixed sample of environments: the sorted
+    indices of a default_rng(seed) draw without replacement, as many as fit."""
+    import torch
+    arrays = {k: (v if torch.is_tensor(v) else np.asarray(v)) for k, v in arrays.items()}
+    wide = {k: v.dtype in (torch.float64, np.float64) for k, v in arrays.items()}
+    n = int(next(iter(arrays.values())).shape[0])
+    per_env = sum(int(np.prod(v.shape[1:])) * (8 if wide[k] else 4) for k, v in arrays.items())
+    keep = min(n, (DUMP_BYTES - 1024 * len(arrays)) // per_env)
+    idx = np.sort(np.random.default_rng(seed).choice(n, keep, replace=False)) if keep < n else None
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        if idx is not None:       # sample before the copy: a whole cfg4 adjacency is 9.7 GB
+            v = v[torch.as_tensor(idx, device=v.device)] if torch.is_tensor(v) else v[idx]
+        a = v.detach().cpu().numpy() if torch.is_tensor(v) else v
+        np.save(os.path.join(out_dir, k + '.npy'), np.ascontiguousarray(a, dtype=np.float64 if wide[k] else np.float32))
+    return {"dir": out_dir, "envs": int(keep), "of_envs": n, "arrays": sorted(arrays)}
 
 
 class ClockSampler:
@@ -151,21 +180,24 @@ def oracle_throughput(workload, n_envs, steps, warmup, nthreads, seed=0):
     for t in range(warmup, warmup + steps):
         env.step(acts[t], episode=episode, auto_reset=True)
     dt = time.perf_counter() - t0
-    return n_envs * params.num_agents * steps / dt, dt, params
+    return n_envs * params.num_agents * steps / dt, dt, params, env
 
 
 def run_reference(a):
-    """`--impl reference`: the CPU oracle port with every host thread; rank 0 only. Whatever --steps says, the timed
-    loop runs for at least ~5 s (a 0.05 s sample moved by +-20 %); both step counts are reported."""
+    """`--impl reference`: the CPU oracle port with every host thread; rank 0 only. The timed loop runs --steps steps
+    (a 0.05 s sample moves by +-20 %: ask for a few seconds' worth)."""
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
     cores = os.cpu_count() or 1
     n_sample = 1024
-    _, dtp, _ = oracle_throughput(a.workload, n_sample, 60, 10, cores)     # calibration (thread pool warm)
-    steps_run = int(max(a.steps, min(100000, 6.0 / max(dtp / 60, 1e-6))))
-    val, dt, params = oracle_throughput(a.workload, n_sample, steps_run, a.warmup, cores)
-    sample = (f"{n_sample} envs x {steps_run} steps ({dt:.1f} s; --steps asked for {a.steps}) of {a.workload} on {cores} host threads "
+    steps_run = a.steps
+    val, dt, params, ora = oracle_throughput(a.workload, n_sample, steps_run, a.warmup, cores)
+    if a.dump_outputs:
+        info = dump_outputs(a.dump_outputs, dict(obs=ora.obs, node_obs=ora.node_obs, adj=ora.adj, rewards=ora.reward,
+                                                 dones=ora.done))
+        print(f"outputs of the last timed step: {info}", file=sys.stderr, flush=True)
+    sample = (f"{n_sample} envs x {steps_run} steps ({dt:.1f} s) of {a.workload} on {cores} host threads "
               f"(C oracle port of the reference's Python path)")
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps,
             "steps_run": steps_run, "warmup": a.warmup, "ms_per_step": 1000.0 * dt / steps_run, "higher_is_better": True,
@@ -285,11 +317,17 @@ def run_ours(a):
         x = step_actions(W + t)               # this step's actions (not timed: resident in HBM when the step starts)
         flush.fill_(0.0)                      # L2 flush between timed iterations (not timed)
         starts[t].record()
-        env.step(x, episode)                  # agent -> emit -> pair kernels (launch_info.launches_per_step)
+        last = env.step(x, episode)           # agent -> emit -> pair kernels (launch_info.launches_per_step)
         stops[t].record()
     torch.cuda.synchronize()
     gc.enable()
     t_wall = time.perf_counter() - t_wall0
+    if a.dump_outputs and rank == 0:
+        # the returned tensors alias the env's output buffers: save them before any later step overwrites them
+        obs, agent_id, node_obs, adj, rewards, dones, _ = last
+        info = dump_outputs(a.dump_outputs, dict(obs=obs, agent_id=agent_id, node_obs=node_obs, adj=adj, rewards=rewards,
+                                                 dones=dones))
+        print(f"outputs of the last timed step: {info}", file=sys.stderr, flush=True)
     step_ms = np.array([s.elapsed_time(e) for s, e in zip(starts, stops)])
     total_ms = float(step_ms.sum())
     if os.environ.get('LSM_BENCH_DUMP'):
@@ -467,9 +505,9 @@ def run_ours(a):
     if not a.no_cpu_baseline:
         cores = os.cpu_count() or 1
         n_s = 1024
-        probe, dtp, _ = oracle_throughput(a.workload, n_s, 3, 1, cores)
+        probe, dtp, _, _ = oracle_throughput(a.workload, n_s, 3, 1, cores)
         steps_s = int(max(5, min(20000, 12.0 / max(dtp / 3, 1e-6))))      # ~12 s of CPU work on every host thread
-        val, dts, _ = oracle_throughput(a.workload, n_s, steps_s, 2, cores)
+        val, dts, _, _ = oracle_throughput(a.workload, n_s, steps_s, 2, cores)
         cpu = {"value": val, "unit": UNIT, "cores": cores, "kind": "port",
                "sample": f"{n_s} envs x {steps_s} steps of {a.workload} ({dts:.1f} s) with the C oracle port of the "
                          f"reference's Python path on {cores} host threads; the Python reference itself measured "
@@ -506,7 +544,7 @@ def run_ours(a):
         dist.destroy_process_group()
 
 
-def measure_rollout(device, rank, world, n_envs, K, W):
+def measure_rollout(device, rank, world, n_envs, K, W, dump_dir=None):
     """BASELINE configs[4] shape - rollout collection of the onpolicy GraphMPE runner (8 agents, 8192 envs per GPU) with
     the device-resident rollout buffer: env.step writes observations / graphs / rewards straight into the buffer slot
     (zero copy), insert() builds masks / share_obs on the device. The policy forward is NOT part of this repo: actions
@@ -524,20 +562,28 @@ def measure_rollout(device, rank, world, n_envs, K, W):
     buf.warmup(num_current_episode=episode)
 
     def collect(steps):
+        out = None
         for _ in range(steps):
             actions = torch.randint(0, 25, (n_envs, N), generator=gen, device=device, dtype=torch.int32)
             out = env.step(actions, episode)
             buf.insert(out, actions=actions)
             if buf.step == 0:
                 buf.after_update()
+        return out
     collect(W)
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record(); collect(K); e1.record()
+    e0.record(); last = collect(K); e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
+    if dump_dir and rank == 0:
+        # zero copy: the returned tensors are views of the buffer slot the last step wrote; no step runs before the dump
+        obs, agent_id, node_obs, adj, rewards, dones, _ = last
+        info = dump_outputs(dump_dir, dict(obs=obs, agent_id=agent_id, node_obs=node_obs, adj=adj, rewards=rewards,
+                                           dones=dones))
+        print(f"outputs of the last timed step: {info}", file=sys.stderr, flush=True)
     if world > 1:
         tt = torch.tensor([ms], dtype=torch.float64, device=device); dist.all_reduce(tt, op=dist.ReduceOp.MAX); ms = float(tt[0])
     peak, peak_src = measured_peak()
@@ -570,7 +616,7 @@ def run_rollout(a):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    r = measure_rollout(device, rank, world, a.envs or 8192, a.steps, a.warmup)
+    r = measure_rollout(device, rank, world, a.envs or 8192, a.steps, a.warmup, dump_dir=a.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
     if rank == 0:
         peak, _ = measured_peak()
@@ -605,7 +651,12 @@ def main():
     ap.add_argument('--use-graph', type=int, default=-1, choices=[-1, 0, 1],
                     help='lsm_tuning.use_graph of the device-timed env: -1 automatic (= plain launches), 0 plain launches, 1 graph replay from a static action buffer')
     ap.add_argument('--no-extra-workloads', action='store_true', help='skip the cfg3 / cfg4 / cfg5 sub-blocks of the default line')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, save what the last one returned as DIR/<name>.npy (float32 / float64, '
+                         'at most 64 MB: a fixed sample of the environments when the batch is larger; rank 0)')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     if a.warmup < 3:
         a.warmup = 3
     if a.impl == 'reference':

@@ -5,10 +5,10 @@
     GraphReplayBuffer        /root/reference/onpolicy/utils/graph_buffer.py:45-373 (insert, after_update, compute_returns)
 
 on seeded inputs and records inputs + the buffer's resulting arrays in tests/golden/aux/rollout_buffer.npz. The reference
-is imported from /root/reference (only here, in the build container); gym comes from oracle/ref_stubs, the logging
+is imported from the checkout LSM_REFERENCE_PATH names (only here); gym comes from oracle/ref_stubs, the logging
 packages the runner module imports at the top (tensorboardX, wandb, imageio) are empty stand-ins.
 
-usage: python oracle/gen_rollout_golden.py
+usage: LSM_REFERENCE_PATH=<checkout of the original project> python oracle/gen_rollout_golden.py
 """
 import os
 import sys
@@ -17,7 +17,9 @@ import types
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = '/root/reference'
+REF = os.environ.get('LSM_REFERENCE_PATH', '')
+if not REF or not os.path.isdir(os.path.join(REF, 'onpolicy')):
+    sys.exit("set LSM_REFERENCE_PATH to a checkout of the original project")
 sys.path.insert(0, os.path.join(HERE, 'ref_stubs'))
 sys.path.insert(0, REF)
 for _name in ('tensorboardX', 'wandb', 'imageio'):

@@ -12,6 +12,16 @@ from layered_safe_marl_b200 import config as cfg
 from layered_safe_marl_b200 import hj_grid
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+# a checkout of the original project (DINaMo-MIT/Layered-Safe-MARL), which the fixture generators under oracle/ drive; only
+# the tests that regenerate fixtures need it and they skip without it
+REFERENCE = os.environ.get('LSM_REFERENCE_PATH', '')
+REFERENCE_SKIP = "needs a checkout of the original project: set LSM_REFERENCE_PATH"
+
+
+def have_reference(subdir):
+    return bool(REFERENCE) and os.path.isdir(os.path.join(REFERENCE, subdir))
+
+
 STATE_KEYS = ('agent_values', 'p_dist', 'state_time', 'done', 'safety_filtered', 'deconflicting_agent_index',
               'min_relative_distance', 'goal_min_time', 'action_diff', 'reached_goal', 'landmark_pos',
               'landmark_heading', 'landmark_speed', 'times_required', 'dists_to_goal', 'dist_left_to_goal',

@@ -135,9 +135,9 @@ def test_rollout_rotation_form(name):
         print(f"{name} (rotation form): roundoff ties at {ties}")
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/multiagent'), reason="the reference tree only exists in the build container")
+@pytest.mark.skipif(not G.have_reference('multiagent'), reason=G.REFERENCE_SKIP)
 def test_golden_fixtures_are_reproducible_from_the_reference(tmp_path):
-    """Regenerate a few fixtures from /root/reference with the committed generator (pure reference code, filter on, the declared
+    """Regenerate a few fixtures from the original project with the committed generator (pure reference code, filter on, the declared
     obstacle extension, 3 landmarks per agent) and compare every array with the committed .npz, bit for bit."""
     import subprocess
     names = ['di3_nofilter_ep0', 'di8_filter', 'di3_obst2', 'at3_landmarks3']

@@ -80,9 +80,9 @@ def test_rollout_buffer_matches_the_reference_buffer(use_gae, proper, centralize
     assert np.array_equal(oh.numpy(), np.squeeze(np.eye(25)[z['in_actions'][0].astype(np.int64)], 2).astype(np.float32))   # graph_mpe_runner.py:431-433
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/onpolicy'), reason="the reference tree only exists in the build container")
+@pytest.mark.skipif(not G.have_reference('onpolicy'), reason=G.REFERENCE_SKIP)
 def test_rollout_golden_fixture_is_reproducible_from_the_reference(tmp_path):
-    """Regenerate the fixture from /root/reference and compare with the committed one (build container only)."""
+    """Regenerate the fixture from the original project and compare with the committed one."""
     import subprocess
     repo = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     src = open(os.path.join(repo, 'oracle', 'gen_rollout_golden.py')).read().replace(
