@@ -119,6 +119,10 @@ struct lsm_handle {
     double* d_pairval = nullptr;        // library-owned scratch of the specialised pipeline
     unsigned char* d_emit_rec = nullptr;
     unsigned long long* d_timeline = nullptr;   // diagnostics only (lsm_debug_timeline)
+#ifdef LSM_EXPERIMENTS
+    unsigned long long* d_phase = nullptr;      // lab build: agent-kernel phase stamps (lsm_debug_phase_stamps)
+    size_t phase_bytes = 0;
+#endif
     float* d_vpacked = nullptr;          // corner-packed copy of the value grid (GridDev::packed)
     // chunked launches: big batches are split into `chunks` env ranges on library-owned streams so that the latency-bound
     // agent kernel of one range runs beside the HBM-bound emit kernel of another (fork / join with events, no host sync)
@@ -373,6 +377,9 @@ int lsm_destroy(lsm_handle* h) {
     if (h->d_pairval) cudaFree(h->d_pairval);
     if (h->d_emit_rec) cudaFree(h->d_emit_rec);
     if (h->d_timeline) cudaFree(h->d_timeline);
+#ifdef LSM_EXPERIMENTS
+    if (h->d_phase) cudaFree(h->d_phase);
+#endif
     if (h->d_vpacked) cudaFree(h->d_vpacked);
     if (h->d_grads8) cudaFree(h->d_grads8);
     if (h->d_edge_local) cudaFree(h->d_edge_local);
@@ -1149,5 +1156,39 @@ int lsm_debug_timeline(lsm_handle* h, int arm, uint64_t* out_ns) {
     }
     return 0;
 }
+
+#ifdef LSM_EXPERIMENTS
+// Lab build only: per env group (%globaltimer ns, clock64) at each phase boundary of the specialised agent kernel,
+// [ngroups][lsm::kPhaseSlots][2] uint64 (tools/agent_phases.py). `out` (capacity `cap` uint64) receives the stamps of the
+// steps since the last arm; returns the number of uint64 written through *n_out. arm = 1 clears and keeps stamping.
+int lsm_debug_phase_stamps(lsm_handle* h, int arm, uint64_t* out, long long cap, long long* n_out) {
+    if (h == nullptr) return fail(1, "lsm_debug_phase_stamps: null handle");
+    if (!h->have_buffers) return fail(5, "lsm_debug_phase_stamps: lsm_bind_buffers has not been called");
+    DeviceGuard guard(h->device);
+    cudaError_t e;
+    const size_t words = (size_t)((h->kp.b.num_envs + h->kp.EPW - 1) / h->kp.EPW) * lsm::kPhaseSlots * 2;
+    if (n_out != nullptr) *n_out = 0;
+    if (out != nullptr && h->d_phase != nullptr) {
+        if ((long long)words > cap) return fail(2, "lsm_debug_phase_stamps: output too small");
+        if ((e = cudaDeviceSynchronize()) != cudaSuccess) return cuda_fail(e, "lsm_debug_phase_stamps");
+        if ((e = cudaMemcpy(out, h->d_phase, words * sizeof(uint64_t), cudaMemcpyDeviceToHost)) != cudaSuccess)
+            return cuda_fail(e, "lsm_debug_phase_stamps");
+        if (n_out != nullptr) *n_out = (long long)words;
+    }
+    if (arm) {
+        if (h->phase_bytes < words * sizeof(uint64_t)) {
+            if (h->d_phase) cudaFree(h->d_phase);
+            h->d_phase = nullptr; h->phase_bytes = 0;
+            if ((e = cudaMalloc(&h->d_phase, words * sizeof(uint64_t))) != cudaSuccess) return cuda_fail(e, "lsm_debug_phase_stamps");
+            h->phase_bytes = words * sizeof(uint64_t);
+        }
+        if ((e = cudaMemset(h->d_phase, 0, words * sizeof(uint64_t))) != cudaSuccess) return cuda_fail(e, "lsm_debug_phase_stamps");
+        h->kp.phase_stamps = h->d_phase;
+    } else {
+        h->kp.phase_stamps = nullptr;
+    }
+    return 0;
+}
+#endif
 
 }  // extern "C"

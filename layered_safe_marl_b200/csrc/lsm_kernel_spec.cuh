@@ -324,8 +324,13 @@ __device__ __forceinline__ bool packed_value(const GridDev& g, const double (&x)
     return true;
 }
 
+// the relative state arrives as scalars (r4 unused for ND == 4): an array reference would put the caller's `rel` in
+// local memory
 template <int ND>
-__device__ __noinline__ double pair_value_scattered(const GridDev& vg, const double (&rel)[ND]) {
+__device__ __noinline__ double pair_value_scattered(const GridDev& vg, double r0, double r1, double r2, double r3, double r4) {
+    double rel[ND];
+    rel[0] = r0; rel[1] = r1; rel[2] = r2; rel[3] = r3;
+    if constexpr (ND == 5) rel[4] = r4;
     Stencil32<ND> st;
     stencil32_setup<ND>(vg, rel, st);
     if (!st.valid) return INFINITY;
@@ -346,7 +351,7 @@ __device__ __forceinline__ double pair_value_raw(const GridDev& vg, double ex, d
         double v;
         if (packed_value<ND>(vg, rel, v)) return isnan(v) ? INFINITY : v;
     }
-    return pair_value_scattered<ND>(vg, rel);
+    return pair_value_scattered<ND>(vg, rel[0], rel[1], rel[2], rel[3], ND == 5 ? rel[ND - 1] : 0.0);
 }
 
 // value shift of HjDataHandle.update_separation_distance (safety_filter.py:170-174); inf stays inf
@@ -407,7 +412,7 @@ __global__ void __launch_bounds__(kPairThreads) lsm_pair_kernel(const __grid_con
 template <int DYN, int N, int L, int O>
 __device__ __noinline__ void pair_phase(const GridDev* __restrict__ vg, EmitRec<DYN, N, L, O>* Rw, AgentScratch<DYN, N, L>* Pw,
                                        int nenv, int lane) {
-    const GridDev g = *vg;
+    const GridDev& g = *vg;
     for (int t = lane; t < nenv * N * N; t += 32) {
         const int el = t / (N * N), r = t - el * (N * N);
         const int i = r / N, j = r - i * N;
@@ -428,7 +433,7 @@ __device__ __noinline__ void pair_phase(const GridDev* __restrict__ vg, EmitRec<
 template <int DYN, int N, int L, int O>
 __device__ __noinline__ void pair_tail_phase(const GridDev* __restrict__ vg, const EmitRec<DYN, N, L, O>* Rw, double* __restrict__ pairval,
                                             int env0, int nenv, unsigned on_mask, int lane) {
-    const GridDev g = *vg;
+    const GridDev& g = *vg;
     for (int t = lane; t < nenv * N * N; t += 32) {
         const int el = t / (N * N), r = t - el * (N * N);
         const int i = r / N, j = r - i * N;
@@ -582,7 +587,7 @@ __device__ __noinline__ void sample_scenario(const KParams& kp, EmitRec<DYN, N, 
     }
     for (int m = 0; m < M; ++m) {
         double sv, cv;
-        lsm_sincos(P.lh[m], &sv, &cv);
+        lsm_sincos_inl(P.lh[m], &sv, &cv);     // the out-of-line lsm_sincos would put sv / cv in local memory
         P.lsin[m] = sv; P.lcos[m] = cv;
         R.cst[m] = make_float4((float)sv, (float)cv, (float)P.lsp[m], 1.0f);
     }
@@ -619,10 +624,11 @@ __device__ __noinline__ double magnetic_penalty(double x, double y, double s2, d
     return hap;
 }
 
-// navigation_graph_safe.py:700-720: heading * speed * cross-track factor of the goal reward (only on the step a goal is reached)
-__device__ __noinline__ double goal_reward_factor(double theta, double pdx, double pdy, double hpr, double sen) {
+// navigation_graph_safe.py:700-720: heading * speed * cross-track factor of the goal reward (only on the step a goal is
+// reached); (sth, cth) = lsm_sincos(theta)
+__device__ __forceinline__ double goal_reward_factor(double sth, double cth, double pdx, double pdy, double hpr, double sen) {
     const double spr = 1.0 - sen;
-    double cte = pdx * lsm_sin(theta) - pdy * lsm_cos(theta);
+    double cte = pdx * sth - pdy * cth;
     const double nrm = norm2(pdx, pdy);
     cte = fabs(cte) / (nrm > 1e-6 ? nrm : 1e-6);
     cte = clipd(cte, 0.0, 1.0);
@@ -662,7 +668,7 @@ __device__ __noinline__ double potential_conflict_penalty(const EmitRec<DYN, N, 
 template <int DYN, int N, int L, int O>
 __device__ __noinline__ double hj_value_reward(const GridDev* __restrict__ vg, const EmitRec<DYN, N, L, O>& R,
                                               const AgentScratch<DYN, N, L>& P, int ai, double x, double y, double sep, double cvalue_rew) {
-    const GridDev g = *vg;
+    const GridDev& g = *vg;
     double r = 0.0;
     for (int a = 0; a < N; ++a) {
         if (a == ai) continue;
@@ -675,15 +681,6 @@ __device__ __noinline__ double hj_value_reward(const GridDev* __restrict__ vg, c
         r += cvalue_rew * cvp;
     }
     return r;
-}
-
-template <int DYN>
-__device__ __noinline__ bool goal_reached_cold(double x, double y, double s2, double s3, double gx, double gy, double gh, double gs,
-                                              double dist_thresh, double heading_thresh, double speed_thresh) {
-    const double th2 = theta_of<DYN>(s2, s3), sp2 = speed_of<DYN>(s2, s3);
-    Curriculum q;
-    q.dist_thresh = dist_thresh; q.heading_thresh = heading_thresh; q.speed_thresh = speed_thresh;
-    return goal_reached<DYN>(x, y, th2, sp2, gx, gy, gh, gs, q);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -763,6 +760,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
         if (kp.mode == MODE_RESET && kp.env_mask != nullptr && env_on) env_on = kp.env_mask[env] != 0;
         const bool agent_on = env_on && ai < N;
         if (__ballot_sync(0xffffffffu, env_on) == 0u) continue;
+        LSM_PHASE_STAMP(PH_GROUP_START);
         const int nenv = (n - env0) < EPW ? (n - env0) : EPW;   // envs of this group
 
         // ---------------- P0: load ----------------
@@ -839,6 +837,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
             if constexpr (O > 0) nobst = aip[LSM_AI_NUM_OBST_COLLISIONS * fstride]; \
         }
         if (kp.mode != MODE_STEP) { LSM_LOAD_MOTION() LSM_LOAD_BOOKKEEPING(false) }
+        LSM_PHASE_STAMP(PH_LOADS);
         // landmark tables of the group's environments: contiguous runs per field
         {
             const int total = nenv * M;
@@ -871,6 +870,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
             if (ai == 0) { P.cur_sep = q.sep; P.cur_filter = q.world_filter ? 1 : 0; R.vel[2 * N] = make_double2(0.0, 0.0); }
         }
         __syncwarp();
+        LSM_PHASE_STAMP(PH_LANDMARKS);
 
         bool all_done_env = false;
         const unsigned any_filter = __ballot_sync(0xffffffffu, env_on && q.world_filter);
@@ -952,6 +952,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 }
                 __syncwarp();
             }
+            LSM_PHASE_STAMP(PH_FILTER);
             // ---------------- P2: goal / reward / done ----------------
             int goal_pre = 0, goal_post = 0, reached_post = reached, done_post = done;
             double rew = 0.0;
@@ -959,6 +960,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
             double theta = 0, speed = 0;
             double cth = 1.0, sth = 0.0;
             bool reached_now = false;
+            bool frozen = false;                  // reached its last goal this step: velocity / speed zeroed
             if (agent_on) {
                 // the two / three trigonometric evaluations on this kernel's critical path are the force-inlined flavours
                 // of the shared implementation (same arithmetic as lsm_atan2 / lsm_cos / lsm_sincos, include/lsm_math.h)
@@ -977,8 +979,12 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 double cra = ratio_sloped(ratio, 0.25, 0.75);
                 if (use_filter_arg) cra = 1.0;
                 reached_now = goal_reached_he<DYN>(x, y, he, speed, gx, gy, gs, q);
+                // The goal branches below run in a few warps of every step, and the kernel ends with its slowest warp.
+                // Their trigonometry is inlined so that those warps do not wait on the fetch of cold out-of-line code.
                 if (reached_now) {
-                    const double pr = goal_reward_factor(theta, gx - x, gy - y, hpr, sen);
+                    double st = sth, ct = cth;          // airtaxi: lsm_sincos(theta) already
+                    if constexpr (DYN == LSM_DYN_DOUBLE_INTEGRATOR) lsm_sincos_inl(theta, &st, &ct);
+                    const double pr = goal_reward_factor(st, ct, gx - x, gy - y, hpr, sen);
                     double goal_rew;
                     if (DYN == LSM_DYN_DOUBLE_INTEGRATOR) goal_rew = c.goal_rew * pr;
                     else goal_rew = c.goal_rew * (pr * cra + (1.0 - cra));
@@ -1006,7 +1012,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 vqx = vpx; vqy = vpy;
                 double s2q = s2, s3q = s3;
                 if (reached_post >= L) {
-                    done_post = 1;
+                    done_post = 1; frozen = true;
                     if (DYN == LSM_DYN_DOUBLE_INTEGRATOR) { s2q = 0.0; s3q = 0.0; vqx = 0.0; vqy = 0.0; }
                     else { s3q = 0.0; vqx = s3q * cth; vqy = s3q * sth; }
                 }
@@ -1024,6 +1030,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 s2 = s2q; s3 = s3q;
             }
             __syncwarp();
+            LSM_PHASE_STAMP(PH_GOAL);
             LSM_LOAD_BOOKKEEPING(true)
             if (agent_on) {
                 // one pass over the other agents: min distance, collisions, episode statistics, proximity rewards.
@@ -1098,9 +1105,15 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                     const double dx = x - gq.x, dy = y - gq.y;
                     // same goal and same (unfrozen) state as before the update -> same answer as `reached_now`
                     bool r2 = reached_now;
-                    if (goal_post != goal_pre || done_post != done)
-                        r2 = goal_reached_cold<DYN>(x, y, s2, s3, gq.x, gq.y, P.lh[goal_post], P.lsp[goal_post], q.dist_thresh, q.heading_thresh,
-                                                    q.speed_thresh);
+                    if (goal_post != goal_pre || done_post != done) {
+                        // theta_of / speed_of of the post-update state: unchanged unless the double integrator was frozen
+                        // to zero velocity (lsm_atan2(+0, +0) = +0, sqrt(0) = 0); the airtaxi keeps its heading
+                        const bool zero = DYN == LSM_DYN_DOUBLE_INTEGRATOR && frozen;
+                        const double th2 = zero ? 0.0 : theta;
+                        const double sp2 = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? (zero ? 0.0 : speed) : s3;
+                        const double he2 = 0.5 - 0.5 * lsm_cos_inl(th2 - P.lh[goal_post]);   // direction_alignment_error
+                        r2 = goal_reached_he<DYN>(x, y, he2, sp2, gq.x, gq.y, P.lsp[goal_post], q);
+                    }
                     if (r2) times_req = (double)current_step * c.dt;
                     dists_goal = p_dist; dist_left = sqrt(dx * dx + dy * dy);
                 }
@@ -1122,6 +1135,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
             }
             reached = reached_post; done = done_post;
             parity ^= 1;
+            LSM_PHASE_STAMP(PH_OTHERS);
         } else {
             if (agent_on) {
                 double vx, vy;
@@ -1215,6 +1229,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
         } else if (kp.mode == MODE_OBSERVE && agent_on) {
             emit_obs_row<DYN, N, L, O>(R, P, ai, goal_obs, x, y, s2, s3, kp.b.obs + ((size_t)env * N + ai) * Dobs);
         }
+        LSM_PHASE_STAMP(PH_RESET);
 
         // ---------------- state write-back ----------------
         if (kp.mode != MODE_OBSERVE) {
@@ -1245,6 +1260,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 if constexpr (O > 0) aip[LSM_AI_NUM_OBST_COLLISIONS * fstride] = nobst;
             }
         }
+        LSM_PHASE_STAMP(PH_WRITEBACK);
         // ---------------- emit records -> global memory (consumed by lsm_emit_kernel; L2 resident) ----------------
         if (env_on && ai == 0) R.next_filter = q.world_filter ? 1 : 0;     // q follows a reset's new curriculum ratio
         if constexpr (DYN != LSM_DYN_DOUBLE_INTEGRATOR) {
@@ -1274,6 +1290,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
             if (kp.pair_tail) pair_tail_phase<DYN, N, L, O>(&kp.vg, Rw, kp.pairval, env0, nenv, on_mask, lane);
         }
         __syncwarp();
+        LSM_PHASE_STAMP(PH_EMIT_REC);
     }
     tl_end(kp.timeline, TL_AGENT_END);
 }
