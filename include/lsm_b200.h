@@ -207,7 +207,9 @@ int lsm_step(lsm_handle *h, const int32_t *action_idx, const float *action_oneho
              uint64_t seed, int auto_reset, void *stream);
 
 /* env.reset(episode) for every env with env_mask[e] != 0 (DEVICE uint8, NULL = all). sample != 0
- * draws a new random scenario on device; sample == 0 keeps the injected agents / landmarks. */
+ * draws a new random scenario on device; sample == 0 keeps the injected agents / landmarks. The other envs keep their
+ * state and outputs; with the fused edge output on (lsm_set_edge_output) their edges are written again, because the
+ * offsets of every later graph move. */
 int lsm_reset(lsm_handle *h, const uint8_t *env_mask, int64_t episode, uint64_t seed, int sample,
               void *stream);
 
@@ -286,8 +288,10 @@ int lsm_edge_list(lsm_handle *h, const float *adj, int64_t *edge_index, float *e
  * ballot, ranks by popcount, per-graph start offsets from a counting pre-pass over the per-env records) - the dense
  * tensor is not read back, and with dense_adj == 0 it is not written at all (the 4*N*E*E term of SURVEY 8d disappears;
  * per edge 20 bytes are written instead, which pays when the mean degree is below ~E/5). Nothing is synchronised:
- * offsets[graphs] holds nnz ON THE DEVICE; entries past `capacity` are dropped. All four pointers NULL switches it
- * off. Specialised (dynamics, N, L) configurations only (returns 6 otherwise).
+ * offsets[graphs] holds nnz ON THE DEVICE; entries past `capacity` are dropped (counts, offsets and nnz stay exact).
+ * A masked lsm_reset writes the list of ALL environments, the ones outside the mask from their unchanged state; this
+ * holds for the first launch after this call too (the arrays need no prior contents). All four pointers NULL switches
+ * it off. Specialised (dynamics, N, L) configurations only (returns 6 otherwise).
  *   edge_index DEVICE int64 [2][capacity], edge_attr DEVICE float [capacity], counts DEVICE int32 [graphs],
  *   offsets DEVICE int64 [graphs + 1]                                         graphs = num_envs * N */
 int lsm_set_edge_output(lsm_handle *h, int64_t *edge_index, float *edge_attr, int32_t *counts, int64_t *offsets,

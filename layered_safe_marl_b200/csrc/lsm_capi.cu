@@ -237,6 +237,13 @@ int lsm_create(const lsm_config* cfg, lsm_handle** out) {
         };
         const double R = cfg->coordination_range;
         kp.r2_lt = lt(R); kp.r2_gt = gt(R);
+        // the reference's float32 adjacency drops an entity pair whose distance rounds to 0 in float32 (d <= 2^-150)
+        {
+            double t = std::ldexp(1.0, -300);
+            while ((float)std::sqrt(t) != 0.0f) t = std::nextafter(t, 0.0);
+            while ((float)std::sqrt(std::nextafter(t, INFINITY)) == 0.0f) t = std::nextafter(t, INFINITY);
+            kp.r2_nz = t;
+        }
         kp.col2_lt = lt(1.05 * (0.050 + 0.050));
         kp.engref2_lt = lt(cfg->engagement_distance_ref);
         kp.septgt2_lt = lt(cfg->separation_distance_target);

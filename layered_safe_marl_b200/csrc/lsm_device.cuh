@@ -93,6 +93,7 @@ struct KParams {
     // exact squared thresholds (host): lt(T) = min{t : sqrt_rn(t) >= T} so that d < T <=> d2 < lt(T);
     //                                  gt(T) = min{t : sqrt_rn(t) >  T} so that d > T <=> d2 >= gt(T)
     double r2_lt, r2_gt;       // coordination_range (adjacency radius / filter range)
+    double r2_nz;              // max{t : (float)sqrt_rn(t) == 0}: the float32 adjacency has an entry <=> r2_nz < d2 < r2_lt
     double col2_lt;            // 1.05 * (size + size) agent collision distance
     double engref2_lt;         // world.engagement_distance (episode statistics)
     double septgt2_lt;         // world.separation_distance_target (episode statistics)

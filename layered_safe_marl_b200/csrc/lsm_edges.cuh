@@ -134,19 +134,17 @@ __global__ void __launch_bounds__(32 * kEdgeCountWarps) lsm_edge_count_kernel(co
     __shared__ long long s_w[kEdgeCountWarps + 1];
     __shared__ bool s_last;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const double r2_lt = kp.r2_lt;
+    const double r2_lt = kp.r2_lt, r2_nz = kp.r2_nz;
     pdl_launch_dependents();
     pdl_wait();
-    const bool masked_reset = kp.mode == MODE_RESET && kp.env_mask != nullptr;
     // this block's CONTIGUOUS run of environments (so that its graph counts are one contiguous run of the prefix)
     const int c = kp.edge_envs_per_block;
     const int e0 = kp.env_begin + blockIdx.x * c;
     const int e1 = (e0 + c) < kp.env_end ? (e0 + c) : kp.env_end;
+    // Every environment is counted from its emit record, also the ones a masked reset leaves alone: the emit kernel
+    // re-emits those from the same (unchanged) record, while counts stored by an earlier launch may not describe it
+    // (fresh buffers after lsm_set_edge_output are zero-filled).
     for (int ee = e0 + warp; ee < e1; ee += kEdgeCountWarps) {
-        if (masked_reset && kp.env_mask[ee] == 0) {                  // state unchanged: the counts of its last emission
-            for (int i = lane; i < N; i += 32) s_cnt[(ee - e0) * N + i] = kp.edge_counts[(size_t)ee * N + i];
-            continue;
-        }
         const REC& R = *reinterpret_cast<const REC*>(kp.emit_rec + (size_t)ee * sizeof(REC));
         unsigned* rowmask = s_rowmask[warp];
         unsigned* keep = s_keep[warp];
@@ -171,7 +169,8 @@ __global__ void __launch_bounds__(32 * kEdgeCountWarps) lsm_edge_count_kernel(co
             for (int q = 0; q < W; ++q) if (q == w) { pr = dpre[q]; po = dpost[q]; }
             keep[k] = ~((po & sel) | (pr & ~sel));
         }
-        // non-zero pattern of the thresholded distance matrix: d2 in float64 against the exact squared radius
+        // non-zero pattern of the thresholded distance matrix: d2 in float64 against the exact squared radius, and above
+        // the largest d2 whose float32 distance is 0 (the emit kernel's test)
         double2 pb[W];
 #pragma unroll
         for (int w = 0; w < W; ++w) pb[w] = (w * 32 + lane) < E ? R.pos[w * 32 + lane] : make_double2(0.0, 0.0);
@@ -181,7 +180,7 @@ __global__ void __launch_bounds__(32 * kEdgeCountWarps) lsm_edge_count_kernel(co
             for (int w = 0; w < W; ++w) {
                 const double dx = pa.x - pb[w].x, dy = pa.y - pb[w].y;
                 const double d2 = dx * dx + dy * dy;
-                const unsigned m = __ballot_sync(0xffffffffu, (w * 32 + lane) < E && d2 < r2_lt && d2 > 0.0);
+                const unsigned m = __ballot_sync(0xffffffffu, (w * 32 + lane) < E && d2 < r2_lt && d2 > r2_nz);
                 if (lane == 0) rowmask[a * W + w] = m;
             }
         }

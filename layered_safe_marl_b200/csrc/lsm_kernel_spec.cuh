@@ -27,7 +27,8 @@
 //     {t : sqrt_rn(t) >= T} is an interval whose lower end the host finds with nextafter). Square roots
 //     are taken only where a distance VALUE is stored (min distance, float32 adjacency).
 //   * the float32 adjacency value is d2f * rsqrt(d2f) (<= 4e-7 relative from the float64 reference, bar
-//     1e-5); which entries are non-zero is decided exactly in float64.
+//     1e-5; a distance below 1e-15 is stored as 1e-15); which entries are non-zero is decided exactly in float64,
+//     strictly inside the radius and above the largest d2 whose float32 root is 0 (r2_nz).
 //   * node features are branch-free rows over unified per-entity tables (landmarks carry zero velocity and
 //     their own position as "goal"), read with 16-byte shared-memory loads.
 #pragma once
@@ -1466,7 +1467,7 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
     extern __shared__ __align__(16) unsigned char smem_raw[];
     ES& S = *reinterpret_cast<ES*>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31;
-    const double r2_lt = kp.r2_lt;
+    const double r2_lt = kp.r2_lt, r2_nz = kp.r2_nz;
     // ablation switches exist only in the LSM_EXPERIMENTS build (liblsm_b200_exp.so); the product kernel has none
 #ifdef LSM_EXPERIMENTS
     const int debug = kp.debug;
@@ -1590,7 +1591,7 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
                     const float d2f = fmaxf((float)d2, 1.0e-30f);
                     float rs;
                     asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(rs) : "f"(d2f));
-                    const float v = (d2 < r2_lt && d2 > 0.0) ? d2f * rs : 0.0f;
+                    const float v = (d2 < r2_lt && d2 > r2_nz) ? d2f * rs : 0.0f;
                     dthr[a * E + b] = v; dthr[b * E + a] = v;
                 }
             }

@@ -1,6 +1,7 @@
 """CPU: host-side logic - config mirror, layout agreement with the oracle header, C-ABI exports,
 lazy infos against the golden info dicts, synthetic grids, sharding over gloo (world_size 2)."""
 import ctypes
+import math
 import os
 import re
 import sys
@@ -127,6 +128,42 @@ def test_grad_values_matches_declared_semantics():
     a = hj_grid.synthetic_airtaxi_grid(shape=(7, 7, 8, 3, 3))
     grid = hj.Grid(a.lo, a.hi, a.shape, (2,))
     np.testing.assert_array_equal(a.grads, grid.grad_values(a.values))
+
+
+def _fma(a, b, c):
+    """fma(a, b, c) in float64: exact product and sum, one rounding (float(Fraction) is correctly rounded)."""
+    from fractions import Fraction
+    return float(Fraction(a) * Fraction(b) + Fraction(c))
+
+
+@pytest.mark.parametrize('which', ['di', 'airtaxi', 'ttr'])
+def test_div_exact_equals_division_on_the_synthetic_grids(which):
+    """lsm_kernel_spec.cuh div_exact: the HJ stencil divides by the grid spacing b through y = RN(1/b) as
+    q0 = a*y; r = fma(-b, q0, a); q = fma(r, y, q0). Markstein's proof that q = RN(a/b) assumes y is within one ulp of
+    1/b in a sense RN(1/b) does not always meet, so check every dimension of the three synthetic grids: dividends
+    a = x - lo for the grid nodes +-8 ulps, the box faces and random positions within two box widths outside."""
+    g = dict(di=hj_grid.synthetic_di_grid, airtaxi=hj_grid.synthetic_airtaxi_grid, ttr=hj_grid.synthetic_ttr_grid)[which]()
+    rng = np.random.default_rng(11)
+    for d in range(g.ndim):
+        lo, hi, n = float(g.lo[d]), float(g.hi[d]), g.shape[d]
+        b = (hi - lo) / n if g.periodic[d] else (hi - lo) / (n - 1.0)      # lsm_capi.cu fill_grid
+        y = 1.0 / b
+        xs = [lo, hi]
+        for k in range(n):
+            x = lo + b * k
+            xs.append(x)
+            up = dn = x
+            for _ in range(8):
+                up, dn = math.nextafter(up, math.inf), math.nextafter(dn, -math.inf)
+                xs += [up, dn]
+        w = hi - lo
+        xs += [float(v) for v in rng.uniform(lo - 2.0 * w, hi + 2.0 * w, 2000)]
+        for x in xs:
+            a = x - lo
+            q0 = a * y
+            r = _fma(-b, q0, a)
+            q = _fma(r, y, q0)
+            assert q == a / b, f"{which} dim {d}: x={x!r} a={a!r} b={b!r}: div_exact {q!r} vs {a / b!r}"
 
 
 def test_oracle_interpolation_matches_stub():
