@@ -349,6 +349,13 @@ int lsm_emit_only(lsm_handle *h, void *stream);
  * launches, 0 disables it. */
 int lsm_debug_timeline(lsm_handle *h, int arm, uint64_t *out_ns);
 
+/* Diagnostics (never on the product path): copy the specialised pipeline's HJ pair-value scratch, the raw values
+ * V(x_i - x_j) the next lsm_step's filter starts from, to `out` (device or pinned host memory, num_envs * N * N
+ * doubles, [env][ego][other]) with one cudaMemcpyAsync on `stream`. Read-only. Only the entries the next step reads
+ * are defined: envs whose curriculum has the filter on, i != j, both agents not done. Returns 6 when the
+ * configuration keeps no pair values (generic kernel). */
+int lsm_debug_pair_values(lsm_handle *h, double *out, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

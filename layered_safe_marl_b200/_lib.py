@@ -68,7 +68,7 @@ EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_dest
                     'lsm_observe', 'lsm_emit_only', 'lsm_invalidate', 'lsm_set_output_buffers', 'lsm_edge_list',
                     'lsm_debug_timeline', 'lsm_rollout_insert', 'lsm_math_eval', 'lsm_math_eval_device', 'lsm_set_tuning',
                     'lsm_set_compact_adjacency', 'lsm_expand_adjacency_host', 'lsm_set_edge_output', 'lsm_world_graph', 'lsm_fetch_host', 'lsm_step_host',
-                    'lsm_episode_stats')
+                    'lsm_episode_stats', 'lsm_debug_pair_values')
 
 _lib = None
 
@@ -109,6 +109,7 @@ def load():
     lib.lsm_set_output_buffers.argtypes = [C.c_void_p] + [C.c_void_p] * 5
     lib.lsm_edge_list.argtypes = [C.c_void_p] * 6 + [C.c_int64, C.c_void_p]
     lib.lsm_debug_timeline.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+    lib.lsm_debug_pair_values.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     lib.lsm_rollout_insert.argtypes = [C.c_void_p] * 7
     lib.lsm_set_tuning.argtypes = [C.c_void_p, C.POINTER(LsmTuning)]
     lib.lsm_set_compact_adjacency.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]

@@ -607,6 +607,9 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
     const bool was_valid = h->pairval_valid;
 
     const bool edges = h->spec && kp.edge_index != nullptr;
+    // the agent kernel of this launch writes the emit record of every env of its range (a masked reset only those in
+    // the mask): the pair kernel behind it can then read its inputs from the records (see lsm_pair_kernel)
+    const bool rec_fresh = !(mode == lsm::MODE_RESET && env_mask != nullptr);
     // the launches of one env-group range [g0, g1) on stream `s` (range `q` of `nq`)
     auto launch_range = [&](long long g0, long long g1, cudaStream_t s, int q, int nq) -> cudaError_t {
         lsm::KParams k = kp;
@@ -626,6 +629,7 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
         k.pairval = nullptr;
         k.pair_late = 0;
         k.pair_tail = 0;
+        k.pair_rec = 0;
         if (pair_path && placement == 4) {
             // the agent kernel leaves the next step's pair values behind itself (all modes: a reset / observe launch makes
             // them valid for the step that follows)
@@ -649,7 +653,9 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
                 // K_a for the NEXT step between the agent and the emit kernel: alone on the GPU at full occupancy
                 k.pairval = h->d_pairval;
                 k.pair_late = 0;
+                k.pair_rec = rec_fresh ? 1 : 0;
                 e = lsm::spec_launch_pair(k, s, persist, h->persist_bytes);
+                k.pair_rec = 0;
                 if (e != cudaSuccess) return e;
             }
             if (edges) {
@@ -675,6 +681,7 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
                 // K_a for the NEXT step, beside the emit kernel's drain (see lsm_pair_kernel)
                 k.pairval = h->d_pairval;
                 k.pair_late = (k.debug & 1) ? 0 : 1;
+                k.pair_rec = rec_fresh ? 1 : 0;
                 e = lsm::spec_launch_pair(k, s, persist, h->persist_bytes);
                 if (e != cudaSuccess) return e;
             }
@@ -1138,6 +1145,18 @@ int lsm_emit_only(lsm_handle* h, void* stream) {
     kp.pairval = pie ? h->d_pairval : nullptr;
     cudaError_t e = lsm::spec_launch_emit(kp, (cudaStream_t)stream, nullptr, 0, pair_path && placement == 0, pie);
     if (e != cudaSuccess) return cuda_fail(e, "lsm_emit_only");
+    return 0;
+}
+
+int lsm_debug_pair_values(lsm_handle* h, double* out, void* stream) {
+    if (h == nullptr) return fail(1, "lsm_debug_pair_values: null handle");
+    if (!h->have_buffers) return fail(5, "lsm_debug_pair_values: lsm_bind_buffers has not been called");
+    if (h->d_pairval == nullptr) return fail(6, "lsm_debug_pair_values: this configuration keeps no pair values");
+    if (out == nullptr) return fail(2, "lsm_debug_pair_values: null output");
+    DeviceGuard guard(h->device);
+    const size_t bytes = (size_t)h->kp.b.num_envs * h->kp.N * h->kp.N * sizeof(double);
+    const cudaError_t e = cudaMemcpyAsync(out, h->d_pairval, bytes, cudaMemcpyDefault, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "lsm_debug_pair_values");
     return 0;
 }
 

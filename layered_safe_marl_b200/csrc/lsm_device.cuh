@@ -103,6 +103,7 @@ struct KParams {
     unsigned char* emit_rec;   // [num_envs][sizeof(EmitRec)] per-env record consumed by lsm_emit_kernel
     int pair_late;             // lsm_pair_kernel launched BEHIND the emit kernel of the same step (runs beside its drain)
     int pair_tail;             // the agent kernel itself computes the NEXT step's pair values at its tail (placement 4)
+    int pair_rec;              // lsm_pair_kernel reads the emit records this launch's agent kernel wrote, not the SoA state
     float* adj_base;           // compact adjacency (lsm_set_compact_adjacency): [num_envs][E][E], NULL = dense adj output
     unsigned* adj_keep;        //                                             [num_envs][N][W]
     // fused COO edge output (lsm_set_edge_output, SURVEY 8f N2); edge_index == nullptr = off

@@ -278,8 +278,22 @@ __global__ void __launch_bounds__(256) lsm_pack_grid_kernel(const float* __restr
     packed[t] = values[lin];
 }
 
+// Which dimensions of a lookup wrap. kPeriodicRuntime reads GridDev::periodic (any grid); any other value is a
+// compile-time mask (bit d = dimension d is periodic), so the per-dimension branch and the inline integer modulo of the
+// dimensions that cannot wrap are not in the code at all. The pair kernel is instantiated for the mask of the grids the
+// specialised shapes are built for (kPairPeriodic) and falls back to the run-time form for any other grid.
+constexpr int kPeriodicRuntime = -1;
+template <int PER>
+__device__ __forceinline__ bool dim_periodic(const GridDev& g, int d) {
+    if constexpr (PER == kPeriodicRuntime) return g.periodic[d] != 0;
+    else return ((PER >> d) & 1) != 0;
+}
+// double integrator: no periodic dimension; airtaxi: the relative heading, dimension 2 (hj_grid.py)
+template <int DYN>
+constexpr int kPairPeriodic = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 0 : 1 << 2;
+
 // reproduces stencil32_setup + stencil32_value bit for bit; false only for NaN positions
-template <int ND>
+template <int ND, int PER = kPeriodicRuntime>
 __device__ __forceinline__ bool packed_value(const GridDev& g, const double (&x)[ND], double& out) {
     constexpr int NC = 1 << ND;
     double wlo[ND], whi[ND];
@@ -294,7 +308,7 @@ __device__ __forceinline__ bool packed_value(const GridDev& g, const double (&x)
         const double w = pos - fl;
         wlo[d] = 1.0 - w; whi[d] = w;
         const int n = g.shape[d];
-        if (g.periodic[d]) {
+        if (dim_periodic<PER>(g, d)) {
             const int il = wrap_index<(ND == 5)>((int)fl, n);
             cell += il * mul; mul *= n;
         } else {
@@ -340,6 +354,16 @@ __device__ __noinline__ double pair_value_scattered(const GridDev& vg, double r0
     return v;
 }
 
+// raw (unshifted) HJ value of a relative state; +inf = outside the declared range / NaN
+template <int ND, int PER>
+__device__ __forceinline__ double pair_value_rel(const GridDev& vg, const double (&rel)[ND]) {
+    if (vg.packed != nullptr) {
+        double v;
+        if (packed_value<ND, PER>(vg, rel, v)) return isnan(v) ? INFINITY : v;
+    }
+    return pair_value_scattered<ND>(vg, rel[0], rel[1], rel[2], rel[3], ND == 5 ? rel[ND - 1] : 0.0);
+}
+
 // raw (unshifted) HJ value of the pair (ego, other); +inf = outside the declared range / NaN
 template <int DYN>
 __device__ __forceinline__ double pair_value_raw(const GridDev& vg, double ex, double ey, double e2, double e3,
@@ -348,11 +372,25 @@ __device__ __forceinline__ double pair_value_raw(const GridDev& vg, double ex, d
     constexpr int ND = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5;
     double rel[ND];
     relative_state_rot<DYN>(ex, ey, e2, e3, ox, oy, o2, o3, rel);
-    if (vg.packed != nullptr) {
-        double v;
-        if (packed_value<ND>(vg, rel, v)) return isnan(v) ? INFINITY : v;
+    return pair_value_rel<ND, kPeriodicRuntime>(vg, rel);
+}
+
+// Relative state of (ego i, other j) from an emit record, i.e. from the state the agent kernel left behind: positions
+// after the dynamics, velocity (double integrator) / heading and speed (airtaxi) after the own goal update - exactly
+// the state it writes back to the SoA tensors. The airtaxi ego frame uses the record's (sth, cth): every path that
+// writes a record takes them from lsm_sincos(theta) of the heading the record carries (integrate() after the
+// dynamics, the observe / reset branches), the same function relative_state_rot evaluates per pair.
+template <int DYN, int N, int L, int O>
+__device__ __forceinline__ void pair_rel_rec(const EmitRec<DYN, N, L, O>& R, int i, int j,
+                                             double (&rel)[DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5]) {
+    const double2 pi = R.pos[i], pj = R.pos[j];
+    if constexpr (DYN == LSM_DYN_DOUBLE_INTEGRATOR) {
+        const double2 vi = R.vel[N + i], vj = R.vel[N + j];
+        relative_state_rot_sc<DYN>(pi.x, pi.y, vi.x, vi.y, pj.x, pj.y, vj.x, vj.y, 0.0, 1.0, rel);
+    } else {
+        relative_state_rot_sc<DYN>(pi.x, pi.y, R.air.theta[i], R.air.spd_post[i], pj.x, pj.y, R.air.theta[j],
+                                   R.air.spd_post[j], R.air.sth[i], R.air.cth[i], rel);
     }
-    return pair_value_scattered<ND>(vg, rel[0], rel[1], rel[2], rel[3], ND == 5 ? rel[ND - 1] : 0.0);
 }
 
 // value shift of HjDataHandle.update_separation_distance (safety_filter.py:170-174); inf stays inf
@@ -369,40 +407,63 @@ __device__ __forceinline__ double shift_value(double raw, double sep, const Grid
 // releases its dependents only after its own wait, i.e. once the agent kernel is complete and flushed - so these
 // latency-bound L2 gathers run on the issue slots the store-bound emit kernel leaves idle, at full thread-per-pair
 // parallelism. Block 0 waits for the emit kernel before it retires, which keeps "this grid complete" => "emit grid
-// complete" for the next step's agent kernel. Fallback placement (pair_late == 0): in front of the agent kernel, when
-// the state was edited from outside (lsm_invalidate / set_state).
+// complete" for the next step's agent kernel. Middle placement (pair_late == 0): between the agent and the emit kernel.
+// Fallback placement: in front of the agent kernel, when the state was edited from outside (lsm_invalidate / set_state).
+//
+// One thread per ORDERED pair i != j: N(N-1) tasks per env (r -> i = r / (N-1), j = r % (N-1) skipping i), 32-bit task
+// indices (spec_launch_pair bounds the range), divisors known at compile time. pairval keeps its [env][N][N] layout;
+// the diagonal is never written or read.
+//
+// Where the inputs come from (kp.pair_rec, chosen per launch in lsm_capi.cu):
+//   * pair_rec = 1: the emit record this launch's agent kernel wrote for the env (pair_rel_rec): positions, velocity /
+//     heading + speed, the done flags after the step and next_filter (the curriculum decision for the state the record
+//     describes). Behind the agent kernel the record describes exactly the state it wrote back to the SoA tensors, in
+//     every launch that writes the record of every env of the range: step (with or without auto-reset; the reset
+//     branch rewrites the record), unmasked reset (sampled, or reset_from_state), observe.
+//   * pair_rec = 0: the SoA state tensors and the curriculum ratio. In front of the agent kernel (the state may have
+//     been edited after the last record was written), and behind a masked reset, which leaves the records of envs
+//     outside the mask untouched (they may predate a set_state or never have been written).
 // ---------------------------------------------------------------------------------------------
 constexpr int kPairThreads = 128;
-template <int DYN, int N>
+template <int DYN, int N, int L, int O, int PER>
 __global__ void __launch_bounds__(kPairThreads) lsm_pair_kernel(const __grid_constant__ KParams kp) {
+    using REC = EmitRec<DYN, N, L, O>;
+    constexpr int ND = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5;
+    constexpr unsigned T = N * (N - 1);
     pdl_launch_dependents();
     if (!kp.pair_late) pdl_wait();
     tl_start(kp.timeline, TL_PAIR_START);
-    const long long n = kp.b.num_envs;
+    const unsigned tasks = (unsigned)(kp.env_end - kp.env_begin) * T;
     // grid-stride: the late placement runs a bounded number of blocks per SM (lsm_kernels.cu) so that these fp64-heavy
     // warps take a fixed share of the issue slots next to the emit kernel's producers
-    for (long long t = (long long)kp.env_begin * (N * N) + (long long)blockIdx.x * blockDim.x + threadIdx.x; t < (long long)kp.env_end * (N * N);
-         t += (long long)gridDim.x * blockDim.x)
-    [&] {
-        const int env = (int)(t / (N * N)), r = (int)(t - (long long)env * (N * N));
-        const int i = r / N, j = r - i * N;
-        if (i == j) return;
-        // world.use_safety_filter of this env (curriculum, navigation_graph_safe.py:351-357)
-        const lsm_config& c = kp.c;
-        if (!(c.flags & LSM_FLAG_INITIAL_PHASE_USE_SAFETY_FILTER)) {
-            const double ratio = kp.b.env_f64[(size_t)LSM_EF_CURRICULUM_RATIO * n + env];
-            if (!(ratio_sloped(ratio, 0.25, 0.75) > 0.0)) return;
+    for (unsigned t = blockIdx.x * blockDim.x + threadIdx.x; t < tasks; t += gridDim.x * blockDim.x) {
+        const unsigned el = t / T, r = t - el * T;
+        const int i = (int)(r / (N - 1)), jj = (int)(r - (unsigned)i * (N - 1));
+        const int j = jj + (jj >= i);
+        const int env = kp.env_begin + (int)el;
+        double rel[ND];
+        if (kp.pair_rec) {
+            const REC& R = reinterpret_cast<const REC*>(kp.emit_rec)[env];
+            if (!R.next_filter || R.done[1][i] || R.done[1][j]) continue;
+            pair_rel_rec<DYN, N, L, O>(R, i, j, rel);
+        } else {
+            const size_t n = (size_t)kp.b.num_envs;
+            // world.use_safety_filter of this env (curriculum, navigation_graph_safe.py:351-357)
+            if (!(kp.c.flags & LSM_FLAG_INITIAL_PHASE_USE_SAFETY_FILTER)) {
+                const double ratio = kp.b.env_f64[(size_t)LSM_EF_CURRICULUM_RATIO * n + env];
+                if (!(ratio_sloped(ratio, 0.25, 0.75) > 0.0)) continue;
+            }
+            const size_t fs = n * N;
+            const size_t ia = (size_t)env * N + i, ja = (size_t)env * N + j;
+            const int* dn = kp.b.agent_i32 + LSM_AI_DONE * fs;
+            if (dn[ia] || dn[ja]) continue;
+            const double* af = kp.b.agent_f64;
+            relative_state_rot<DYN>(af[LSM_AF_X * fs + ia], af[LSM_AF_Y * fs + ia], af[LSM_AF_S2 * fs + ia],
+                                    af[LSM_AF_S3 * fs + ia], af[LSM_AF_X * fs + ja], af[LSM_AF_Y * fs + ja],
+                                    af[LSM_AF_S2 * fs + ja], af[LSM_AF_S3 * fs + ja], rel);
         }
-        const size_t fs = (size_t)n * N;
-        const size_t ia = (size_t)env * N + i, ja = (size_t)env * N + j;
-        const int* dn = kp.b.agent_i32 + LSM_AI_DONE * fs;
-        if (dn[ia] || dn[ja]) return;
-        const double* af = kp.b.agent_f64;
-        const double v = pair_value_raw<DYN>(kp.vg, af[LSM_AF_X * fs + ia], af[LSM_AF_Y * fs + ia], af[LSM_AF_S2 * fs + ia],
-                                             af[LSM_AF_S3 * fs + ia], af[LSM_AF_X * fs + ja], af[LSM_AF_Y * fs + ja],
-                                             af[LSM_AF_S2 * fs + ja], af[LSM_AF_S3 * fs + ja]);
-        kp.pairval[t] = v;
-    }();
+        kp.pairval[(size_t)env * (N * N) + (i * N + j)] = pair_value_rel<ND, PER>(kp.vg, rel);
+    }
     tl_end(kp.timeline, TL_PAIR_BODY_END);
     if (kp.pair_late && blockIdx.x == 0 && threadIdx.x == 0) pdl_wait();
     tl_end(kp.timeline, TL_PAIR_END);
@@ -440,15 +501,9 @@ __device__ __noinline__ void pair_tail_phase(const GridDev* __restrict__ vg, con
         const int i = r / N, j = r - i * N;
         const EmitRec<DYN, N, L, O>& R = Rw[el];
         if (!((on_mask >> ((el * N) & 31)) & 1u) || !R.next_filter || i == j || R.done[1][i] || R.done[1][j]) continue;
-        const double2 pi = R.pos[i], pj = R.pos[j];
-        double i2, i3, j2, j3;
-        if constexpr (DYN == LSM_DYN_DOUBLE_INTEGRATOR) {
-            const double2 vi = R.vel[N + i], vj = R.vel[N + j];
-            i2 = vi.x; i3 = vi.y; j2 = vj.x; j3 = vj.y;
-        } else {
-            i2 = R.air.theta[i]; i3 = R.air.spd_post[i]; j2 = R.air.theta[j]; j3 = R.air.spd_post[j];
-        }
-        pairval[(size_t)(env0 + el) * (N * N) + r] = pair_value_raw<DYN>(g, pi.x, pi.y, i2, i3, pj.x, pj.y, j2, j3);
+        double rel[DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5];
+        pair_rel_rec<DYN, N, L, O>(R, i, j, rel);
+        pairval[(size_t)(env0 + el) * (N * N) + r] = pair_value_rel<DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5, kPeriodicRuntime>(g, rel);
     }
 }
 
@@ -1777,15 +1832,9 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
                 for (int t = tid; t < N * N; t += T) {
                     const int i = t / N, j = t - i * N;
                     if (i == j || R.done[1][i] || R.done[1][j]) continue;
-                    const double2 pi = R.pos[i], pj = R.pos[j];
-                    double i2, i3, j2, j3;
-                    if constexpr (DYN == LSM_DYN_DOUBLE_INTEGRATOR) {
-                        const double2 vi = R.vel[N + i], vj = R.vel[N + j];
-                        i2 = vi.x; i3 = vi.y; j2 = vj.x; j3 = vj.y;
-                    } else {
-                        i2 = R.air.theta[i]; i3 = R.air.spd_post[i]; j2 = R.air.theta[j]; j3 = R.air.spd_post[j];
-                    }
-                    pv[t] = pair_value_raw<DYN>(kp.vg, pi.x, pi.y, i2, i3, pj.x, pj.y, j2, j3);
+                    double rel[DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5];
+                    pair_rel_rec<DYN, N, L, O>(R, i, j, rel);
+                    pv[t] = pair_value_rel<DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5, kPeriodicRuntime>(kp.vg, rel);
                 }
             }
         }

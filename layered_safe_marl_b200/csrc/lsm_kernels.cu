@@ -19,6 +19,7 @@
 #include "lsm_rollout.cuh"
 #include "lsm_host.h"
 
+#include <climits>
 #include <cstdlib>
 
 namespace lsm {
@@ -52,8 +53,13 @@ namespace lsm {
 constexpr int kAgentBlock = 128;
 constexpr int kAgentMinB = 2;
 constexpr int kPairBlock = kPairThreads;
-constexpr int kPairResident = 2;          // SM room the emit grid leaves for pair blocks (placement "late")
-constexpr int kPairLateBlocksPerSm = 8;   // grid bound of the late pair kernel (measured: >= 6 is best everywhere)
+// SM room the emit grid leaves for pair blocks (placement "late") and the late pair kernel's grid bound. Swept on B200
+// with the record-reading pair kernel (profiles/experiments/r03_pair_kernel_sweep.txt, r03_pair_kernel_ab.txt): with no
+// room reserved the cfg2 emit kernel gets 6 instead of 5 blocks per SM and ends ~2.5 us earlier; the pair blocks then
+// start as emit blocks retire and finish the lookups in the emit kernel's tail (cfg2 -1.1 us against one reserved
+// block, cfg4 and cfg5 slightly faster too). A grid bound of 16 blocks per SM lets them fill the SMs the emit kernel frees.
+constexpr int kPairResident = 0;
+constexpr int kPairLateBlocksPerSm = 16;
 
 // The product library (liblsm_b200.so) has ONE instantiation per kernel and configuration and reads no environment
 // variable. Alternative kernel shapes and ablation switches are compiled only with -DLSM_EXPERIMENTS
@@ -68,7 +74,10 @@ static int env_int(const char* name, int dflt) { const char* e = std::getenv(nam
 #endif
 
 struct SpecFns {
-    const void* pair; const void* agent; const void* emit;
+    const void* pair;         // lsm_pair_kernel for the periodic-dimension mask pair_periodic (kPairPeriodic)
+    const void* pair_rt;      // the same kernel reading the mask from the bound grid (any other grid)
+    int pair_periodic;
+    const void* agent; const void* emit;
     const void* emit_pie;     // emit kernel that also computes the next step's pair values (placement "emit")
     const void* edge_count;   // per-graph edge counts + range prefix for the fused COO output
     int rec_bytes, scratch_bytes, emit_smem, emit_threads;
@@ -111,7 +120,9 @@ static bool spec_fns(int dynamics, int N, int L, int O, SpecFns* f) {
 static bool spec_fns_base(int dynamics, int N, int L, int O, SpecFns* f) {
 #define X(DYN_, N_, L_, O_, WPE_, EMINB_)                                                         \
     if (dynamics == DYN_ && N == N_ && L == L_ && O == O_) {                                      \
-        f->pair = (const void*)lsm_pair_kernel<DYN_, N_>;                                         \
+        f->pair = (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPairPeriodic<DYN_>>;            \
+        f->pair_rt = (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPeriodicRuntime>;            \
+        f->pair_periodic = kPairPeriodic<DYN_>;                                                   \
         f->agent = LSM_AGENT_FN(DYN_, N_, L_, O_);                                                \
         f->emit = (const void*)lsm_emit_kernel<DYN_, N_, L_, O_, WPE_, EMINB_>;                   \
         f->emit_pie = LSM_EMIT_PIE_FN(DYN_, N_, L_, O_, WPE_, EMINB_);                            \
@@ -232,7 +243,12 @@ cudaError_t kernel_launch(const KParams& kp, bool spec, int grid_blocks, int blo
 cudaError_t spec_launch_pair(const KParams& kp, cudaStream_t stream, const void* persist_ptr, size_t persist_bytes) {
     SpecFns f;
     if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, &f)) return cudaErrorInvalidValue;
-    const long long tasks = (long long)(kp.env_end - kp.env_begin) * kp.N * kp.N;
+    // one thread per ordered pair i != j, 32-bit task indices in the kernel
+    const long long tasks = (long long)(kp.env_end - kp.env_begin) * kp.N * (kp.N - 1);
+    if (tasks > INT_MAX) return cudaErrorInvalidValue;
+    int periodic = 0;
+    for (int d = 0; d < kp.vg.ndim; ++d) periodic |= kp.vg.periodic[d] ? 1 << d : 0;
+    const void* fn = periodic == f.pair_periodic ? f.pair : f.pair_rt;
     long long blocks = (tasks + kPairBlock - 1) / kPairBlock;
     if (blocks < 1) blocks = 1;
     if (kp.pair_late) {
@@ -245,7 +261,7 @@ cudaError_t spec_launch_pair(const KParams& kp, cudaStream_t stream, const void*
 #endif
         if (blocks > (long long)sm_count * bps) blocks = (long long)sm_count * bps;
     }
-    return launch_one(f.pair, kp, (unsigned)blocks, kPairBlock, 0, stream, persist_ptr, persist_bytes, true);
+    return launch_one(fn, kp, (unsigned)blocks, kPairBlock, 0, stream, persist_ptr, persist_bytes, true);
 }
 
 // resident emit blocks per SM: what fits, minus (when the pair kernel runs beside the emit kernel) enough registers /
@@ -269,7 +285,11 @@ static cudaError_t emit_blocks_per_sm(const SpecFns& f, bool reserve_pair, bool 
         if ((e = cudaFuncGetAttributes(&fe, fn)) != cudaSuccess) return e;
         if ((e = cudaFuncGetAttributes(&fp, f.pair)) != cudaSuccess) return e;
         auto block_regs = [](int regs, int threads) { return ((regs * 32 + 255) / 256 * 256) * ((threads + 31) / 32); };
-        const int need_regs = kPairResident * block_regs(fp.numRegs, kPairBlock), need_thr = kPairResident * kPairBlock;
+        int resident = kPairResident;
+#ifdef LSM_EXPERIMENTS
+        { const int v = env_int("LSM_PAIR_RESIDENT", -1); if (v >= 0) resident = v; }
+#endif
+        const int need_regs = resident * block_regs(fp.numRegs, kPairBlock), need_thr = resident * kPairBlock;
         while (bps > 1 && (65536 - bps * block_regs(fe.numRegs, f.emit_threads) < need_regs || 2048 - bps * f.emit_threads < need_thr)) --bps;
     }
 #ifdef LSM_EXPERIMENTS
