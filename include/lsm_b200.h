@@ -56,7 +56,10 @@ enum {
     LSM_FLAG_INTERP_FLOAT32 = 1 << 10      /* grid interpolation (hj_reachability Grid.interpolate: safety_filter.py:195,245,
                                               348,418, core.py:463, navigation_graph_safe.py:751) in float32 - position,
                                               weights and corner sum - as jax computes it without jax_enable_x64 (the
-                                              reference never enables it); default: the same formula in float64 */
+                                              reference never enables it); default: the same formula in float64.
+                                              Both modes run the specialised pipeline on the shapes it is compiled for
+                                              (float32 agent / pair kernels of their own) and the generic kernel on the
+                                              others */
 };
 
 /* state layout: agent_f64[field][env][agent], agent_i32[field][env][agent],
@@ -230,7 +233,8 @@ int lsm_set_output_buffers(lsm_handle *h, float *obs, float *node_obs, float *ad
  *   adj_base  DEVICE float    [num_envs][E][E]     thresholded distances, unmasked
  *   adj_keep  DEVICE uint32   [num_envs][N][W]     W = ceil(E / 32): bit e of observer i's words = entity e is connected
  * so that 1/N of the adjacency bytes cross PCIe; lsm_expand_adjacency_host rebuilds the dense array byte for byte.
- * Both NULL restores the dense output. Specialised (dynamics, N, L) configurations only (returns 6 otherwise). */
+ * Both NULL restores the dense output. Specialised (dynamics, N, L) configurations only, in either interpolation mode
+ * (returns 6 otherwise). */
 int lsm_set_compact_adjacency(lsm_handle *h, float *adj_base, uint32_t *adj_keep);
 
 /* HOST function (no GPU work): adj[e][i][a][b] = keep_i[a] && keep_i[b] ? base[e][a][b] : 0 for e in [0, num_envs),
@@ -291,7 +295,7 @@ int lsm_edge_list(lsm_handle *h, const float *adj, int64_t *edge_index, float *e
  * offsets[graphs] holds nnz ON THE DEVICE; entries past `capacity` are dropped (counts, offsets and nnz stay exact).
  * A masked lsm_reset writes the list of ALL environments, the ones outside the mask from their unchanged state; this
  * holds for the first launch after this call too (the arrays need no prior contents). All four pointers NULL switches
- * it off. Specialised (dynamics, N, L) configurations only (returns 6 otherwise).
+ * it off. Specialised (dynamics, N, L) configurations only, in either interpolation mode (returns 6 otherwise).
  *   edge_index DEVICE int64 [2][capacity], edge_attr DEVICE float [capacity], counts DEVICE int32 [graphs],
  *   offsets DEVICE int64 [graphs + 1]                                         graphs = num_envs * N */
 int lsm_set_edge_output(lsm_handle *h, int64_t *edge_index, float *edge_attr, int32_t *counts, int64_t *offsets,

@@ -280,11 +280,12 @@ int lsm_create(const lsm_config* cfg, lsm_handle** out) {
     sl.bytes_per_env = align_up(off, 16);
     h->smem_optin = (int)prop.sharedMemPerBlockOptin;
 
-    // both node-feature types ('relative', which every shipped script uses, and 'global') run the specialised pipeline; the
-    // float32 interpolation arithmetic (LSM_FLAG_INTERP_FLOAT32, a parity mode) lives in the generic kernel only, so that
-    // the specialised kernels carry none of its code
+    // both node-feature types ('relative', which every shipped script uses, and 'global') and both interpolation
+    // arithmetics run the specialised pipeline; LSM_FLAG_INTERP_FLOAT32 selects agent / pair kernels compiled with float32
+    // grid lookups, so that the float64 kernels carry none of its code
     // (the obstacle extension is specialised for the shapes LSM_SPEC_LIST names with O > 0; other obstacle counts: generic)
-    h->spec = lsm::spec_available(cfg->dynamics, N, L, O, &h->geo) && !(cfg->flags & LSM_FLAG_INTERP_FLOAT32);
+    const bool f32 = (cfg->flags & LSM_FLAG_INTERP_FLOAT32) != 0;
+    h->spec = lsm::spec_available(cfg->dynamics, N, L, O, &h->geo);
 #ifdef LSM_EXPERIMENTS
     { const char* force_generic = std::getenv("LSM_FORCE_GENERIC"); if (force_generic != nullptr && force_generic[0] == '1') h->spec = false; }
 #endif
@@ -300,6 +301,8 @@ int lsm_create(const lsm_config* cfg, lsm_handle** out) {
         else if (!std::strcmp(pp, "front")) h->pair_placement = 2;
         else if (!std::strcmp(pp, "middle")) h->pair_placement = 3;
     }
+    // the in-emit pair values (placement 1) exist in float64 only: a float32 handle keeps its default placement
+    if (f32 && h->pair_placement == 1) h->pair_placement = cfg->dynamics == LSM_DYN_AIRTAXI ? 3 : 0;
     { const char* fe = std::getenv("LSM_EPW"); h->forced_epw = fe ? std::atoi(fe) : 0; }
 #endif
     if (h->spec) {
@@ -327,13 +330,13 @@ int lsm_create(const lsm_config* cfg, lsm_handle** out) {
         delete h;
         return fail(4, "lsm_create: one environment group does not fit in shared memory");
     }
-    e = lsm::kernel_prepare(cfg->dynamics, N, L, O, h->spec, h->smem_per_block, h->block_threads, &h->regs, &h->blocks_per_sm);
+    e = lsm::kernel_prepare(cfg->dynamics, N, L, O, f32, h->spec, h->smem_per_block, h->block_threads, &h->regs, &h->blocks_per_sm);
     if (e != cudaSuccess) { delete h; return cuda_fail(e, "kernel_prepare"); }
     if (h->blocks_per_sm < 1) { delete h; return fail(4, "lsm_create: kernel does not fit on an SM"); }
     h->grid_cap = h->sm_count * h->blocks_per_sm;
     if (h->spec) {
         if (h->geo.emit_smem > h->smem_optin) { delete h; return fail(4, "lsm_create: emit record does not fit in shared memory"); }
-        e = lsm::spec_prepare_aux(cfg->dynamics, N, L, O, &h->emit_regs, &h->emit_blocks_per_sm, &h->pair_regs);
+        e = lsm::spec_prepare_aux(cfg->dynamics, N, L, O, f32, &h->emit_regs, &h->emit_blocks_per_sm, &h->pair_regs);
         if (e != cudaSuccess) { delete h; return cuda_fail(e, "spec_prepare_aux"); }
         if (h->emit_blocks_per_sm < 1) { delete h; return fail(4, "lsm_create: emit kernel does not fit on an SM"); }
     }
@@ -436,10 +439,10 @@ int lsm_set_value_grid(lsm_handle* h, const lsm_grid_desc* g) {
     for (int k = 0; k < g->ndim; ++k) cells *= (size_t)g->shape[k];
     h->persist_bytes = cells * sizeof(float);
     if (h->persist_bytes > h->max_window) h->persist_bytes = h->max_window;
-    // corner-packed copy for the pair kernel (one aligned chunk per lookup); lsm_tuning.packed_grid = 0 keeps the scattered
-    // gathers; tables larger than 2 GiB are not built.
+    // corner-packed copy for the pair kernel (one aligned chunk per lookup; the same table serves the float64 and the
+    // float32 lookups); lsm_tuning.packed_grid = 0 keeps the scattered gathers; tables larger than 2 GiB are not built.
     DeviceGuard guard(h->device);
-    const bool want_packed = h->tuning.packed_grid != 0 && !(h->kp.c.flags & LSM_FLAG_INTERP_FLOAT32);
+    const bool want_packed = h->tuning.packed_grid != 0;
     if (h->d_vpacked) { cudaFree(h->d_vpacked); h->d_vpacked = nullptr; }
     h->kp.vg.packed = nullptr;
     if (h->spec && want_packed) {
@@ -489,7 +492,9 @@ int lsm_set_tuning(lsm_handle* h, const lsm_tuning* t) {
     if (t->use_graph < -1 || t->use_graph > 1) return fail(2, "lsm_set_tuning: use_graph must be -1, 0 or 1");
     if (h->have_buffers || h->kp.has_vg) return fail(5, "lsm_set_tuning: call it right after lsm_create (before lsm_set_value_grid / lsm_bind_buffers)");
     h->tuning = *t;
-    if (t->pair_placement >= 0) h->pair_placement = t->pair_placement;
+    // placement 1 (lab build) has no float32 form: a float32 handle keeps its placement (see lsm_create)
+    const bool f32 = (h->kp.c.flags & LSM_FLAG_INTERP_FLOAT32) != 0;
+    if (t->pair_placement >= 0 && !(f32 && t->pair_placement == 1)) h->pair_placement = t->pair_placement;
     return 0;
 }
 
@@ -564,7 +569,8 @@ int lsm_get_launch_info(lsm_handle* h, lsm_launch_info* out) {
     const bool pair_path_li = h->spec && (h->kp.c.flags & LSM_FLAG_USE_SAFETY_FILTER) && h->kp.has_vg;
     if (h->spec) {   // the emit kernel / grid lsm_step launches (room left for the pair kernel with placement "late")
         int bps = 0, regs = 0;
-        if (lsm::spec_emit_blocks_per_sm(h->kp.c.dynamics, h->kp.N, h->kp.L, h->kp.O, pair_path_li && h->pair_placement == 0,
+        if (lsm::spec_emit_blocks_per_sm(h->kp.c.dynamics, h->kp.N, h->kp.L, h->kp.O, (h->kp.c.flags & LSM_FLAG_INTERP_FLOAT32) != 0,
+                                         pair_path_li && h->pair_placement == 0,
                                          pair_path_li && h->pair_placement == 1, &bps, &regs) == cudaSuccess) {
             out->emit_blocks_per_sm = bps; out->emit_regs_per_thread = regs;
         }

@@ -11,15 +11,16 @@ struct SpecGeometry {
 };
 bool spec_available(int dynamics, int N, int L, int O, SpecGeometry* g);
 // agent kernel (specialised) or the fused generic kernel
-cudaError_t kernel_prepare(int dynamics, int N, int L, int O, bool spec, int smem_bytes, int block_threads, int* regs,
+// f32: the LSM_FLAG_INTERP_FLOAT32 instantiations of the agent / pair kernels (specialised path)
+cudaError_t kernel_prepare(int dynamics, int N, int L, int O, bool f32, bool spec, int smem_bytes, int block_threads, int* regs,
                            int* blocks_per_sm);
-cudaError_t spec_prepare_aux(int dynamics, int N, int L, int O, int* emit_regs, int* emit_blocks_per_sm, int* pair_regs);
+cudaError_t spec_prepare_aux(int dynamics, int N, int L, int O, bool f32, int* emit_regs, int* emit_blocks_per_sm, int* pair_regs);
 cudaError_t upload_magnetic_tables(const double* cos_tab, const double* sin_tab);
 cudaError_t kernel_launch(const KParams& kp, bool spec, int grid_blocks, int block_threads, int smem_bytes,
                           cudaStream_t stream, const void* persist_ptr, size_t persist_bytes);
 cudaError_t spec_launch_pair(const KParams& kp, cudaStream_t stream, const void* persist_ptr, size_t persist_bytes);
 cudaError_t spec_launch_emit(const KParams& kp, cudaStream_t stream, const void* persist_ptr, size_t persist_bytes, bool reserve_pair, bool pie);
-cudaError_t spec_emit_blocks_per_sm(int dynamics, int N, int L, int O, bool reserve_pair, bool pie, int* out, int* regs);
+cudaError_t spec_emit_blocks_per_sm(int dynamics, int N, int L, int O, bool f32, bool reserve_pair, bool pie, int* out, int* regs);
 int edge_count_envs_per_block(long long envs);
 cudaError_t spec_launch_edge_count(const KParams& kp, cudaStream_t stream);
 cudaError_t world_graph_launch(const KParams& kp, int32_t* counts, long long* offsets, long long* edge_index, double* edge_weight,

@@ -238,13 +238,126 @@ __global__ void __launch_bounds__(256) lsm_pad_grads_kernel(const float* __restr
     grads8[t] = d < 5 ? grads[cell * 5 + d] : 0.0f;
 }
 
+// ---------------------------------------------------------------------------------------------
+// float32 stencil (LSM_FLAG_INTERP_FLOAT32, compiled into the F32 instantiations only): the arithmetic of interp_f32
+// (lsm_device.cuh) and of the oracle's interpolate_f32, inline and without pointer arguments. State, lo and spacing
+// rounded to float32, IEEE float32 division (not the float64 reciprocal of div_exact), the declared clamp, float32
+// weights, weight products (dim 0 first) and sequential corner sums in binary counting order; no FMA (-fmad=false).
+// Same 32-bit index handling as stencil32_setup: (il + 1) mod n of the wrapped il equals interp_f32's ih mod n.
+// ---------------------------------------------------------------------------------------------
+template <int ND>
+struct Stencil32f {
+    int lo[ND], hi[ND];
+    float wlo[ND], whi[ND];
+    bool valid;
+};
+
+// float32 grid position of x[d] on dimension d; NaN = invalid
+__device__ __forceinline__ float grid_pos_f32(const GridDev& g, double x, int d) {
+    return __fdiv_rn((float)x - (float)g.lo[d], (float)g.spacing[d]);
+}
+
+template <int ND>
+__device__ __forceinline__ void stencil32f_setup(const GridDev& g, const double (&x)[ND], Stencil32f<ND>& s) {
+    s.valid = true;
+    int mul = 1;
+#pragma unroll
+    for (int d = ND - 1; d >= 0; --d) {
+        float pos = grid_pos_f32(g, x[d], d);
+        if (isnan(pos)) s.valid = false;
+        pos = fminf(fmaxf(pos, -1.0e9f), 1.0e9f);      // declared clamp
+        const float fl = floorf(pos);
+        const float whi = pos - fl;
+        s.wlo[d] = 1.0f - whi; s.whi[d] = whi;
+        const int n = g.shape[d];
+        int il = (int)fl, ih = il + 1;                 // |fl| <= 1e9 fits in int32
+        if (g.periodic[d]) {
+            il = wrap_index<(ND == 5)>(il, n);
+            ih = il + 1 == n ? 0 : il + 1;
+        } else {
+            il = min(max(il, 0), n - 1);
+            ih = min(max(ih, 0), n - 1);
+        }
+        s.lo[d] = il * mul; s.hi[d] = ih * mul;
+        mul *= n;
+    }
+}
+
+template <int ND>
+__device__ __forceinline__ float corner_weight_f32(const float (&wlo)[ND], const float (&whi)[ND], int corner) {
+    float weight = 0.0f;
+#pragma unroll
+    for (int d = 0; d < ND; ++d) {
+        const float wd = ((corner >> (ND - 1 - d)) & 1) ? whi[d] : wlo[d];
+        weight = (d == 0) ? wd : weight * wd;
+    }
+    return weight;
+}
+
+template <int ND>
+__device__ __forceinline__ double stencil32f_value(const GridDev& g, const Stencil32f<ND>& s) {
+    constexpr int NC = 1 << ND;
+    float v[NC];
+    const unsigned long long keep = l2_evict_last();
+#pragma unroll
+    for (int corner = 0; corner < NC; ++corner) {
+        int lin = 0;
+#pragma unroll
+        for (int d = 0; d < ND; ++d) lin += ((corner >> (ND - 1 - d)) & 1) ? s.hi[d] : s.lo[d];
+        v[corner] = ldg_hint(g.values + lin, keep);
+    }
+    float acc = 0.0f;
+#pragma unroll
+    for (int corner = 0; corner < NC; ++corner) acc = acc + corner_weight_f32<ND>(s.wlo, s.whi, corner) * v[corner];
+    return (double)acc;
+}
+
+// gradient rows as in stencil32_grad (float4 rows for 4-D, padded grads8 rows for 5-D), each component summed in
+// float32; a NaN position gives NaN components, as interp_f32_grad does
+template <int ND>
+__device__ __forceinline__ void stencil32f_grad(const GridDev& g, const Stencil32f<ND>& s, double (&out)[ND]) {
+    static_assert(ND == 4 || ND == 5, "the specialised grids are 4-D or 5-D");
+    float acc[ND];
+#pragma unroll
+    for (int d = 0; d < ND; ++d) acc[d] = 0.0f;
+    const unsigned long long keep = l2_evict_last();
+#pragma unroll
+    for (int corner = 0; corner < (1 << ND); ++corner) {
+        const float weight = corner_weight_f32<ND>(s.wlo, s.whi, corner);
+        int lin = 0;
+#pragma unroll
+        for (int d = 0; d < ND; ++d) lin += ((corner >> (ND - 1 - d)) & 1) ? s.hi[d] : s.lo[d];
+        if constexpr (ND == 4) {
+            const float4 v = ldg_hint(reinterpret_cast<const float4*>(g.grads) + lin, keep);
+            acc[0] = acc[0] + weight * v.x; acc[1] = acc[1] + weight * v.y;
+            acc[2] = acc[2] + weight * v.z; acc[3] = acc[3] + weight * v.w;
+        } else {
+            const float4 a = ldg_hint(reinterpret_cast<const float4*>(g.grads8) + 2 * (size_t)lin, keep);
+            const float4 b = ldg_hint(reinterpret_cast<const float4*>(g.grads8) + 2 * (size_t)lin + 1, keep);
+            acc[0] = acc[0] + weight * a.x; acc[1] = acc[1] + weight * a.y;
+            acc[2] = acc[2] + weight * a.z; acc[3] = acc[3] + weight * a.w;
+            acc[ND - 1] = acc[ND - 1] + weight * b.x;
+        }
+    }
+#pragma unroll
+    for (int d = 0; d < ND; ++d) out[d] = s.valid ? (double)acc[d] : NAN;
+}
+
+// gradient lookup of the specialised filter (filter_resolve); F32 = LSM_FLAG_INTERP_FLOAT32
+template <bool F32>
 struct LeanGrad {
     static constexpr bool kRotRel = true;     // relative_state_rot, like pair_value_raw below
     template <int ND>
     __device__ __forceinline__ static void eval(const GridDev& g, const double (&rel)[ND], double (&out)[ND]) {
-        Stencil32<ND> st;
-        stencil32_setup<ND>(g, rel, st);
-        stencil32_grad<ND>(g, st, out);
+        if constexpr (F32) {
+            Stencil32f<ND> st;
+            stencil32f_setup<ND>(g, rel, st);
+            stencil32f_grad<ND>(g, st, out);
+        } else {
+            Stencil32<ND> st;
+            stencil32_setup<ND>(g, rel, st);
+            stencil32_grad<ND>(g, st, out);
+        }
     }
 };
 
@@ -339,6 +452,47 @@ __device__ __forceinline__ bool packed_value(const GridDev& g, const double (&x)
     return true;
 }
 
+// float32 twin of packed_value: reproduces stencil32f_setup + stencil32f_value bit for bit from the same table. The
+// slot c = clamp((int)fl, -1, n - 1) + 1 stands for the index pair interp_f32's clamp gives (non-periodic dims), the
+// wrapped il for the pair (il, (il + 1) mod n) (periodic dims). False only for NaN positions.
+template <int ND, int PER = kPeriodicRuntime>
+__device__ __forceinline__ bool packed_value_f32(const GridDev& g, const double (&x)[ND], double& out) {
+    constexpr int NC = 1 << ND;
+    float wlo[ND], whi[ND];
+    bool ok = true;
+    int cell = 0, mul = 1;
+#pragma unroll
+    for (int d = ND - 1; d >= 0; --d) {
+        float pos = grid_pos_f32(g, x[d], d);
+        if (isnan(pos)) ok = false;
+        pos = fminf(fmaxf(pos, -1.0e9f), 1.0e9f);      // declared clamp, as in stencil32f_setup
+        const float fl = floorf(pos);
+        const float w = pos - fl;
+        wlo[d] = 1.0f - w; whi[d] = w;
+        const int n = g.shape[d];
+        if (dim_periodic<PER>(g, d)) {
+            const int il = wrap_index<(ND == 5)>((int)fl, n);
+            cell += il * mul; mul *= n;
+        } else {
+            const int c = min(max((int)fl, -1), n - 1) + 1;
+            cell += c * mul; mul *= n + 1;
+        }
+    }
+    if (!ok) return false;
+    const float4* src = reinterpret_cast<const float4*>(g.packed) + (size_t)cell * (NC / 4);
+    float v[NC];
+#pragma unroll
+    for (int k = 0; k < NC / 4; ++k) {
+        const float4 q = __ldg(src + k);
+        v[4 * k] = q.x; v[4 * k + 1] = q.y; v[4 * k + 2] = q.z; v[4 * k + 3] = q.w;
+    }
+    float acc = 0.0f;
+#pragma unroll
+    for (int corner = 0; corner < NC; ++corner) acc = acc + corner_weight_f32<ND>(wlo, whi, corner) * v[corner];
+    out = (double)acc;
+    return true;
+}
+
 // the relative state arrives as scalars (r4 unused for ND == 4): an array reference would put the caller's `rel` in
 // local memory
 template <int ND>
@@ -353,26 +507,47 @@ __device__ __noinline__ double pair_value_scattered(const GridDev& vg, double r0
     if (isnan(v)) return INFINITY;
     return v;
 }
+// float32 arithmetic (no packed table, or a NaN position)
+template <int ND>
+__device__ __noinline__ double pair_value_scattered_f32(const GridDev& vg, double r0, double r1, double r2, double r3, double r4) {
+    double rel[ND];
+    rel[0] = r0; rel[1] = r1; rel[2] = r2; rel[3] = r3;
+    if constexpr (ND == 5) rel[4] = r4;
+    Stencil32f<ND> st;
+    stencil32f_setup<ND>(vg, rel, st);
+    if (!st.valid) return INFINITY;
+    const double v = stencil32f_value<ND>(vg, st);
+    if (isnan(v)) return INFINITY;
+    return v;
+}
 
-// raw (unshifted) HJ value of a relative state; +inf = outside the declared range / NaN
-template <int ND, int PER>
+// raw (unshifted) HJ value of a relative state; +inf = outside the declared range / NaN. F32: LSM_FLAG_INTERP_FLOAT32
+template <int ND, int PER, bool F32 = false>
 __device__ __forceinline__ double pair_value_rel(const GridDev& vg, const double (&rel)[ND]) {
-    if (vg.packed != nullptr) {
-        double v;
-        if (packed_value<ND, PER>(vg, rel, v)) return isnan(v) ? INFINITY : v;
+    if constexpr (F32) {
+        if (vg.packed != nullptr) {
+            double v;
+            if (packed_value_f32<ND, PER>(vg, rel, v)) return isnan(v) ? INFINITY : v;
+        }
+        return pair_value_scattered_f32<ND>(vg, rel[0], rel[1], rel[2], rel[3], ND == 5 ? rel[ND - 1] : 0.0);
+    } else {
+        if (vg.packed != nullptr) {
+            double v;
+            if (packed_value<ND, PER>(vg, rel, v)) return isnan(v) ? INFINITY : v;
+        }
+        return pair_value_scattered<ND>(vg, rel[0], rel[1], rel[2], rel[3], ND == 5 ? rel[ND - 1] : 0.0);
     }
-    return pair_value_scattered<ND>(vg, rel[0], rel[1], rel[2], rel[3], ND == 5 ? rel[ND - 1] : 0.0);
 }
 
 // raw (unshifted) HJ value of the pair (ego, other); +inf = outside the declared range / NaN
-template <int DYN>
+template <int DYN, bool F32 = false>
 __device__ __forceinline__ double pair_value_raw(const GridDev& vg, double ex, double ey, double e2, double e3,
                                                  double ox, double oy, double o2, double o3) {
     // safety_filter.py:192-201, 345-354
     constexpr int ND = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5;
     double rel[ND];
     relative_state_rot<DYN>(ex, ey, e2, e3, ox, oy, o2, o3, rel);
-    return pair_value_rel<ND, kPeriodicRuntime>(vg, rel);
+    return pair_value_rel<ND, kPeriodicRuntime, F32>(vg, rel);
 }
 
 // Relative state of (ego i, other j) from an emit record, i.e. from the state the agent kernel left behind: positions
@@ -423,9 +598,11 @@ __device__ __forceinline__ double shift_value(double raw, double sep, const Grid
 //   * pair_rec = 0: the SoA state tensors and the curriculum ratio. In front of the agent kernel (the state may have
 //     been edited after the last record was written), and behind a masked reset, which leaves the records of envs
 //     outside the mask untouched (they may predate a set_state or never have been written).
+//
+// F32 = LSM_FLAG_INTERP_FLOAT32: the float32 lookup from the same corner-packed table (packed_value_f32).
 // ---------------------------------------------------------------------------------------------
 constexpr int kPairThreads = 128;
-template <int DYN, int N, int L, int O, int PER>
+template <int DYN, int N, int L, int O, int PER, bool F32>
 __global__ void __launch_bounds__(kPairThreads) lsm_pair_kernel(const __grid_constant__ KParams kp) {
     using REC = EmitRec<DYN, N, L, O>;
     constexpr int ND = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5;
@@ -462,7 +639,7 @@ __global__ void __launch_bounds__(kPairThreads) lsm_pair_kernel(const __grid_con
                                     af[LSM_AF_S3 * fs + ia], af[LSM_AF_X * fs + ja], af[LSM_AF_Y * fs + ja],
                                     af[LSM_AF_S2 * fs + ja], af[LSM_AF_S3 * fs + ja], rel);
         }
-        kp.pairval[(size_t)env * (N * N) + (i * N + j)] = pair_value_rel<ND, PER>(kp.vg, rel);
+        kp.pairval[(size_t)env * (N * N) + (i * N + j)] = pair_value_rel<ND, PER, F32>(kp.vg, rel);
     }
     tl_end(kp.timeline, TL_PAIR_BODY_END);
     if (kp.pair_late && blockIdx.x == 0 && threadIdx.x == 0) pdl_wait();
@@ -471,7 +648,7 @@ __global__ void __launch_bounds__(kPairThreads) lsm_pair_kernel(const __grid_con
 
 // in-kernel variant for internal steps after the first (states changed inside the launch): pair-parallel over
 // the warp's environments, shifted values into P.fval
-template <int DYN, int N, int L, int O>
+template <int DYN, int N, int L, int O, bool F32>
 __device__ __noinline__ void pair_phase(const GridDev* __restrict__ vg, EmitRec<DYN, N, L, O>* Rw, AgentScratch<DYN, N, L>* Pw,
                                        int nenv, int lane) {
     const GridDev& g = *vg;
@@ -482,7 +659,7 @@ __device__ __noinline__ void pair_phase(const GridDev* __restrict__ vg, EmitRec<
         AgentScratch<DYN, N, L>& P = Pw[el];
         if (!P.cur_filter || i == j || R.done[0][i] || R.done[0][j]) continue;
         const double2 pi = R.pos[i], pj = R.pos[j];
-        P.fval[r] = shift_value(pair_value_raw<DYN>(g, pi.x, pi.y, P.as2[i], P.as3[i], pj.x, pj.y, P.as2[j], P.as3[j]),
+        P.fval[r] = shift_value(pair_value_raw<DYN, F32>(g, pi.x, pi.y, P.as2[i], P.as3[i], pj.x, pj.y, P.as2[j], P.as3[j]),
                                 P.cur_sep, g);
     }
 }
@@ -492,7 +669,7 @@ __device__ __noinline__ void pair_phase(const GridDev* __restrict__ vg, EmitRec<
 // state). The per-agent chain is latency bound (~20 % issue utilisation), so these lookups ride on idle issue slots of
 // warps that are resident anyway - no pair kernel competing with the emit kernel for the SMs, one launch less. Same
 // conditions and arithmetic as lsm_pair_kernel (raw values; entries of done agents / filter-off envs are left alone).
-template <int DYN, int N, int L, int O>
+template <int DYN, int N, int L, int O, bool F32>
 __device__ __noinline__ void pair_tail_phase(const GridDev* __restrict__ vg, const EmitRec<DYN, N, L, O>* Rw, double* __restrict__ pairval,
                                             int env0, int nenv, unsigned on_mask, int lane) {
     const GridDev& g = *vg;
@@ -503,7 +680,7 @@ __device__ __noinline__ void pair_tail_phase(const GridDev* __restrict__ vg, con
         if (!((on_mask >> ((el * N) & 31)) & 1u) || !R.next_filter || i == j || R.done[1][i] || R.done[1][j]) continue;
         double rel[DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5];
         pair_rel_rec<DYN, N, L, O>(R, i, j, rel);
-        pairval[(size_t)(env0 + el) * (N * N) + r] = pair_value_rel<DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5, kPeriodicRuntime>(g, rel);
+        pairval[(size_t)(env0 + el) * (N * N) + r] = pair_value_rel<DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5, kPeriodicRuntime, F32>(g, rel);
     }
 }
 
@@ -721,7 +898,7 @@ __device__ __noinline__ double potential_conflict_penalty(const EmitRec<DYN, N, 
 }
 
 // reward_hj_value (navigation_graph_safe.py:830-837, core.py:459-468)
-template <int DYN, int N, int L, int O>
+template <int DYN, int N, int L, int O, bool F32>
 __device__ __noinline__ double hj_value_reward(const GridDev* __restrict__ vg, const EmitRec<DYN, N, L, O>& R,
                                               const AgentScratch<DYN, N, L>& P, int ai, double x, double y, double sep, double cvalue_rew) {
     const GridDev& g = *vg;
@@ -732,7 +909,7 @@ __device__ __noinline__ double hj_value_reward(const GridDev* __restrict__ vg, c
         if (adone) continue;
         // as2/as3 hold the pre-update states
         const double2 pa = R.pos[a];
-        const double v = shift_value(pair_value_raw<DYN>(g, x, y, P.as2[ai], P.as3[ai], pa.x, pa.y, P.as2[a], P.as3[a]), sep, g);
+        const double v = shift_value(pair_value_raw<DYN, F32>(g, x, y, P.as2[ai], P.as3[ai], pa.x, pa.y, P.as2[a], P.as3[a]), sep, g);
         const double cvp = fabs(pymin(v - 0.4, 0.0));
         r += cvalue_rew * cvp;
     }
@@ -778,7 +955,10 @@ __device__ __noinline__ void episode_summary(const KParams& kp, int le, int env,
     }
 }
 
-template <int DYN, int N, int L, int O, int BLOCK, int MINB>
+// F32 = LSM_FLAG_INTERP_FLOAT32: every grid lookup (filter gradient, airtaxi TTR term, in-kernel pair values, HJ_VALUE
+// reward) in float32 arithmetic. A compile-time choice: this kernel is bound by instruction fetch, and unused flag code
+// compiled into it costs time (DESIGN.md 3).
+template <int DYN, int N, int L, int O, int BLOCK, int MINB, bool F32>
 __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_constant__ KParams kp) {
     using REC = EmitRec<DYN, N, L, O>;
     using SCR = AgentScratch<DYN, N, L>;
@@ -960,7 +1140,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 // for later internal steps
                 const bool precomputed = it == 0 && kp.pairval != nullptr;
                 if (any_filter != 0u && !precomputed) {
-                    pair_phase<DYN, N, L, O>(&kp.vg, Rw, Pw, nenv, lane);
+                    pair_phase<DYN, N, L, O, F32>(&kp.vg, Rw, Pw, nenv, lane);
                     __syncwarp();
                 }
                 if (agent_on && q.world_filter) {
@@ -992,7 +1172,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                             // `min distance > coordination_range` as an exact test on the squared distance
                             const double best_d = (best_d2 >= kp.r2_gt) ? INFINITY : 0.0;
                             const double2 po = R.pos[kv];
-                            filter_resolve<DYN, LeanGrad>(kp, best_d, best_v, !isinf(best_v), x, y, s2, s3, po.x, po.y, P.as2[kv], P.as3[kv],
+                            filter_resolve<DYN, LeanGrad<F32>>(kp, best_d, best_v, !isinf(best_v), x, y, s2, s3, po.x, po.y, P.as2[kv], P.as3[kv],
                                                 raw0, raw1, P.rawx[kv], P.rawy[kv], safe0, safe1, filt, hsc[0], hsc[1]);
                         }
                     }
@@ -1054,9 +1234,16 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                         double rpx, rpy;
                         rotate_into(x - gx, y - gy, P.lcos[goal_pre], P.lsin[goal_pre], rpx, rpy);   // tabulated cos / sin(gh)
                         const double rs[4] = { rpx, rpy, theta - gh, speed };
-                        Stencil32<4> st;
-                        stencil32_setup<4>(kp.tg, rs, st);
-                        double ttr = st.valid ? stencil32_value<4>(kp.tg, st) : NAN;
+                        double ttr;
+                        if constexpr (F32) {
+                            Stencil32f<4> st;
+                            stencil32f_setup<4>(kp.tg, rs, st);
+                            ttr = st.valid ? stencil32f_value<4>(kp.tg, st) : NAN;
+                        } else {
+                            Stencil32<4> st;
+                            stencil32_setup<4>(kp.tg, rs, st);
+                            ttr = st.valid ? stencil32_value<4>(kp.tg, st) : NAN;
+                        }
                         if (isnan(ttr)) ttr = kp.tg.ttr_max;
                         rew -= 0.04 * ttr;
                         rew -= sen * cra;
@@ -1141,7 +1328,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                     if (!done) rew += q.diff_rew * action_diff;
                 }
                 if (c.flags & LSM_FLAG_HJ_VALUE)
-                    rew += hj_value_reward<DYN, N, L, O>(&kp.vg, R, P, ai, x, y, q.sep, q.cvalue_rew);
+                    rew += hj_value_reward<DYN, N, L, O, F32>(&kp.vg, R, P, ai, x, y, q.sep, q.cvalue_rew);
                 rew = clipd(rew, c.min_reward, c.max_reward);
                 if (!done_post) {
                     ep_len += 1;
@@ -1343,7 +1530,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 for (int k = lane; k < Q; k += 32) dst[k] = src[k];
             }
             // placement 4: next step's HJ pair values from the records still in shared memory
-            if (kp.pair_tail) pair_tail_phase<DYN, N, L, O>(&kp.vg, Rw, kp.pairval, env0, nenv, on_mask, lane);
+            if (kp.pair_tail) pair_tail_phase<DYN, N, L, O, F32>(&kp.vg, Rw, kp.pairval, env0, nenv, on_mask, lane);
         }
         __syncwarp();
         LSM_PHASE_STAMP(PH_EMIT_REC);

@@ -73,6 +73,9 @@ static int agent_minb() {
 static int env_int(const char* name, int dflt) { const char* e = std::getenv(name); return e ? std::atoi(e) : dflt; }
 #endif
 
+// The agent and pair kernels exist in two arithmetics of the HJ grid lookups (LSM_FLAG_INTERP_FLOAT32: float32, else
+// float64), chosen at compile time; spec_fns picks the pair of the handle's mode. The emit and edge-count kernels make no
+// grid lookups and serve both modes.
 struct SpecFns {
     const void* pair;         // lsm_pair_kernel for the periodic-dimension mask pair_periodic (kPairPeriodic)
     const void* pair_rt;      // the same kernel reading the mask from the bound grid (any other grid)
@@ -95,9 +98,9 @@ static void cfg2_emit_variant(SpecFns* f) {
 
 #endif
 
-static bool spec_fns_base(int dynamics, int N, int L, int O, SpecFns* f);
-static bool spec_fns(int dynamics, int N, int L, int O, SpecFns* f) {
-    if (!spec_fns_base(dynamics, N, L, O, f)) return false;
+static bool spec_fns_base(int dynamics, int N, int L, int O, bool f32, SpecFns* f);
+static bool spec_fns(int dynamics, int N, int L, int O, bool f32, SpecFns* f) {
+    if (!spec_fns_base(dynamics, N, L, O, f32, f)) return false;
 #ifdef LSM_EXPERIMENTS
     if (dynamics == LSM_DYN_DOUBLE_INTEGRATOR && N == 8 && L == 2 && O == 0) {
         const int w = env_int("LSM_WPE", 0);
@@ -109,21 +112,24 @@ static bool spec_fns(int dynamics, int N, int L, int O, SpecFns* f) {
     return true;
 }
 
+// LSM_AGENT_MINB=3 (lab build) has float64 instantiations only
 #ifdef LSM_EXPERIMENTS
-#define LSM_AGENT_FN(DYN_, N_, L_, O_) (agent_minb() == 3 ? (const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, 3> \
-                                                          : (const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, kAgentMinB>)
+#define LSM_AGENT_FN(DYN_, N_, L_, O_, F32_) (agent_minb() == 3 && !(F32_) ? (const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, 3, false> \
+                                                                          : (const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, kAgentMinB, F32_>)
 #define LSM_EMIT_PIE_FN(DYN_, N_, L_, O_, WPE_, EMINB_) ((const void*)lsm_emit_kernel<DYN_, N_, L_, O_, WPE_, EMINB_, true>)
 #else
-#define LSM_AGENT_FN(DYN_, N_, L_, O_) ((const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, kAgentMinB>)
+#define LSM_AGENT_FN(DYN_, N_, L_, O_, F32_) ((const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, kAgentMinB, F32_>)
 #define LSM_EMIT_PIE_FN(DYN_, N_, L_, O_, WPE_, EMINB_) nullptr   /* "pair values inside the emit kernel": experiments only */
 #endif
-static bool spec_fns_base(int dynamics, int N, int L, int O, SpecFns* f) {
+static bool spec_fns_base(int dynamics, int N, int L, int O, bool f32, SpecFns* f) {
 #define X(DYN_, N_, L_, O_, WPE_, EMINB_)                                                         \
     if (dynamics == DYN_ && N == N_ && L == L_ && O == O_) {                                      \
-        f->pair = (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPairPeriodic<DYN_>>;            \
-        f->pair_rt = (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPeriodicRuntime>;            \
+        f->pair = f32 ? (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPairPeriodic<DYN_>, true>  \
+                      : (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPairPeriodic<DYN_>, false>; \
+        f->pair_rt = f32 ? (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPeriodicRuntime, true>  \
+                         : (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPeriodicRuntime, false>; \
         f->pair_periodic = kPairPeriodic<DYN_>;                                                   \
-        f->agent = LSM_AGENT_FN(DYN_, N_, L_, O_);                                                \
+        f->agent = f32 ? LSM_AGENT_FN(DYN_, N_, L_, O_, true) : LSM_AGENT_FN(DYN_, N_, L_, O_, false); \
         f->emit = (const void*)lsm_emit_kernel<DYN_, N_, L_, O_, WPE_, EMINB_>;                   \
         f->emit_pie = LSM_EMIT_PIE_FN(DYN_, N_, L_, O_, WPE_, EMINB_);                            \
         f->edge_count = (const void*)lsm_edge_count_kernel<DYN_, N_, L_, O_>;                     \
@@ -143,9 +149,12 @@ static const void* generic_ptr(int dynamics) {
                                                  : (const void*)lsm_generic_kernel<LSM_DYN_AIRTAXI>;
 }
 
+static bool kp_interp_f32(const KParams& kp) { return (kp.c.flags & LSM_FLAG_INTERP_FLOAT32) != 0; }
+
+// the geometry is the same in both interpolation modes
 bool spec_available(int dynamics, int N, int L, int O, SpecGeometry* g) {
     SpecFns f;
-    if (!spec_fns(dynamics, N, L, O, &f)) return false;
+    if (!spec_fns(dynamics, N, L, O, false, &f)) return false;
     g->rec_bytes = f.rec_bytes; g->scratch_bytes = f.scratch_bytes; g->agent_block = kAgentBlock;
     g->emit_smem = f.emit_smem; g->emit_threads = f.emit_threads; g->pair_block = kPairBlock;
     return true;
@@ -161,17 +170,17 @@ static cudaError_t prepare_one(const void* fn, int block_threads, int smem_bytes
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, fn, block_threads, smem_bytes);
 }
 
-cudaError_t kernel_prepare(int dynamics, int N, int L, int O, bool spec, int smem_bytes, int block_threads, int* regs,
+cudaError_t kernel_prepare(int dynamics, int N, int L, int O, bool f32, bool spec, int smem_bytes, int block_threads, int* regs,
                            int* blocks_per_sm) {
     SpecFns f;
     const void* fn = generic_ptr(dynamics);
-    if (spec) { if (!spec_fns(dynamics, N, L, O, &f)) return cudaErrorInvalidValue; fn = f.agent; }
+    if (spec) { if (!spec_fns(dynamics, N, L, O, f32, &f)) return cudaErrorInvalidValue; fn = f.agent; }
     return prepare_one(fn, block_threads, smem_bytes, regs, blocks_per_sm);
 }
 
-cudaError_t spec_prepare_aux(int dynamics, int N, int L, int O, int* emit_regs, int* emit_blocks_per_sm, int* pair_regs) {
+cudaError_t spec_prepare_aux(int dynamics, int N, int L, int O, bool f32, int* emit_regs, int* emit_blocks_per_sm, int* pair_regs) {
     SpecFns f;
-    if (!spec_fns(dynamics, N, L, O, &f)) return cudaErrorInvalidValue;
+    if (!spec_fns(dynamics, N, L, O, f32, &f)) return cudaErrorInvalidValue;
     cudaError_t e = prepare_one(f.emit, f.emit_threads, f.emit_smem, emit_regs, emit_blocks_per_sm);
     if (e != cudaSuccess) return e;
     if (f.emit_pie != nullptr) { int r = 0, b = 0; e = prepare_one(f.emit_pie, f.emit_threads, f.emit_smem, &r, &b); if (e != cudaSuccess) return e; }
@@ -224,7 +233,7 @@ cudaError_t kernel_launch(const KParams& kp, bool spec, int grid_blocks, int blo
                           cudaStream_t stream, const void* persist_ptr, size_t persist_bytes) {
     SpecFns f;
     const void* fn = generic_ptr(kp.c.dynamics);
-    if (spec) { if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, &f)) return cudaErrorInvalidValue; fn = f.agent; }
+    if (spec) { if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, kp_interp_f32(kp), &f)) return cudaErrorInvalidValue; fn = f.agent; }
 #ifdef LSM_EXPERIMENTS
     if (spec) {
         // LSM_AGENT_SMEM=<bytes>: pad the agent kernel's dynamic shared memory so that fewer blocks fit an SM and the
@@ -242,7 +251,7 @@ cudaError_t kernel_launch(const KParams& kp, bool spec, int grid_blocks, int blo
 
 cudaError_t spec_launch_pair(const KParams& kp, cudaStream_t stream, const void* persist_ptr, size_t persist_bytes) {
     SpecFns f;
-    if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, &f)) return cudaErrorInvalidValue;
+    if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, kp_interp_f32(kp), &f)) return cudaErrorInvalidValue;
     // one thread per ordered pair i != j, 32-bit task indices in the kernel
     const long long tasks = (long long)(kp.env_end - kp.env_begin) * kp.N * (kp.N - 1);
     if (tasks > INT_MAX) return cudaErrorInvalidValue;
@@ -272,10 +281,11 @@ static cudaError_t emit_blocks_per_sm(const SpecFns& f, bool reserve_pair, bool 
 #ifndef LSM_EXPERIMENTS
     // the answer depends only on (kernel, reserve_pair): asked once per process, not on every launch (two occupancy /
     // attribute queries cost more host time than the launch itself)
-    struct Memo { const void* fn; bool reserve; int bps; };
+    struct Memo { const void* fn; const void* pair; bool reserve; int bps; };
     static thread_local Memo memo[32];
     static thread_local int memo_n = 0;
-    for (int k = 0; k < memo_n; ++k) if (memo[k].fn == fn && memo[k].reserve == reserve_pair) { *out = memo[k].bps; return cudaSuccess; }
+    for (int k = 0; k < memo_n; ++k)
+        if (memo[k].fn == fn && memo[k].pair == f.pair && memo[k].reserve == reserve_pair) { *out = memo[k].bps; return cudaSuccess; }
 #endif
     cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, fn, f.emit_threads, f.emit_smem);
     if (e != cudaSuccess) return e;
@@ -295,15 +305,15 @@ static cudaError_t emit_blocks_per_sm(const SpecFns& f, bool reserve_pair, bool 
 #ifdef LSM_EXPERIMENTS
     { const int v = env_int("LSM_EMIT_BPS", 0); if (v >= 1 && v < bps) bps = v; }
 #else
-    if (memo_n < 32) { memo[memo_n].fn = fn; memo[memo_n].reserve = reserve_pair; memo[memo_n].bps = bps; ++memo_n; }
+    if (memo_n < 32) { memo[memo_n].fn = fn; memo[memo_n].pair = f.pair; memo[memo_n].reserve = reserve_pair; memo[memo_n].bps = bps; ++memo_n; }
 #endif
     *out = bps;
     return cudaSuccess;
 }
 
-cudaError_t spec_emit_blocks_per_sm(int dynamics, int N, int L, int O, bool reserve_pair, bool pie, int* out, int* regs) {
+cudaError_t spec_emit_blocks_per_sm(int dynamics, int N, int L, int O, bool f32, bool reserve_pair, bool pie, int* out, int* regs) {
     SpecFns f;
-    if (!spec_fns(dynamics, N, L, O, &f)) return cudaErrorInvalidValue;
+    if (!spec_fns(dynamics, N, L, O, f32, &f)) return cudaErrorInvalidValue;
     if (regs != nullptr) {
         cudaFuncAttributes fa;
         cudaError_t e = cudaFuncGetAttributes(&fa, (pie && f.emit_pie != nullptr) ? f.emit_pie : f.emit);
@@ -315,7 +325,7 @@ cudaError_t spec_emit_blocks_per_sm(int dynamics, int N, int L, int O, bool rese
 
 cudaError_t spec_launch_emit(const KParams& kp, cudaStream_t stream, const void* persist_ptr, size_t persist_bytes, bool reserve_pair, bool pie) {
     SpecFns f;
-    if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, &f)) return cudaErrorInvalidValue;
+    if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, kp_interp_f32(kp), &f)) return cudaErrorInvalidValue;
     // persistent blocks: as many as are resident at once, each loops over environments
     static int sm_count = 0;
     if (sm_count == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev); }
@@ -342,7 +352,7 @@ int edge_count_envs_per_block(long long envs) {
 
 cudaError_t spec_launch_edge_count(const KParams& kp, cudaStream_t stream) {
     SpecFns f;
-    if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, &f)) return cudaErrorInvalidValue;
+    if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, kp_interp_f32(kp), &f)) return cudaErrorInvalidValue;
     const long long envs = kp.env_end - kp.env_begin;
     long long blocks = (envs + kp.edge_envs_per_block - 1) / kp.edge_envs_per_block;
     if (blocks < 1) blocks = 1;
