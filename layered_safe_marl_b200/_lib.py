@@ -4,6 +4,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+from typing import Optional
 
 from . import _build
 
@@ -70,28 +71,30 @@ EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_dest
                     'lsm_set_compact_adjacency', 'lsm_expand_adjacency_host', 'lsm_set_edge_output', 'lsm_world_graph', 'lsm_fetch_host', 'lsm_step_host',
                     'lsm_episode_stats', 'lsm_debug_pair_values')
 
-_lib = None
+_libs = {}          # one CDLL per path: the product library and the per-shape libraries (_build.build_shape)
 
 
 def lib_path() -> str:
     return _build.LIB_PATH
 
 
-def load():
-    """Load liblsm_b200.so (building it first if the sources are newer). Raises if unavailable."""
-    global _lib
-    if _lib is not None:
-        return _lib
-    path = _build.LIB_PATH
-    alt = os.environ.get('LSM_LIB')     # experiments: an A/B build of the same sources (see _build.build)
-    if alt:
-        path = alt
-    elif _build.needs_build():
-        try:
-            _build.build()
-        except Exception as exc:  # no nvcc on the box and no prebuilt library: fail loudly
-            if not os.path.exists(path):
-                raise RuntimeError(f"liblsm_b200.so is missing and could not be built: {exc}") from exc
+def load(path: Optional[str] = None):
+    """Load liblsm_b200.so (building it first if the sources are newer), or with `path` the library at that path (a
+    per-shape library of _build.build_shape). One CDLL per path and process. Raises if unavailable."""
+    key = path
+    if key in _libs:
+        return _libs[key]
+    if path is None:
+        path = _build.LIB_PATH
+        alt = os.environ.get('LSM_LIB')     # experiments: an A/B build of the same sources (see _build.build)
+        if alt:
+            path = alt
+        elif _build.needs_build():
+            try:
+                _build.build()
+            except Exception as exc:  # no nvcc on the box and no prebuilt library: fail loudly
+                if not os.path.exists(path):
+                    raise RuntimeError(f"liblsm_b200.so is missing and could not be built: {exc}") from exc
     lib = C.CDLL(path)
     lib.lsm_abi_version.restype = C.c_int
     lib.lsm_last_error.restype = C.c_char_p
@@ -124,11 +127,13 @@ def load():
     for name in EXPORTED_SYMBOLS:
         if name not in ('lsm_abi_version', 'lsm_last_error'):
             getattr(lib, name).restype = C.c_int
-    _lib = lib
+    _libs[key] = lib
     return lib
 
 
-def check(rc: int, what: str):
+def check(rc: int, what: str, lib=None):
+    """Raise on a non-zero return code; the message is `lsm_last_error` of `lib`, the library that returned `rc` (default:
+    the product library)."""
     if rc != 0:
-        msg = load().lsm_last_error()
+        msg = (lib if lib is not None else load()).lsm_last_error()
         raise RuntimeError(f"{what} failed (code {rc}): {msg.decode() if msg else ''}")

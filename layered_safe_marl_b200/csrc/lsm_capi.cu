@@ -821,12 +821,17 @@ int lsm_set_compact_adjacency(lsm_handle* h, float* adj_base, uint32_t* adj_keep
     return 0;
 }
 
+// entities of the largest environment lsm_create accepts (agents + landmarks + obstacles), rounded up to the 4-float
+// steps of the vector path: the host expansion's per-row buffers hold this many entries
+constexpr int kMaxEntities = LSM_MAX_AGENTS + LSM_MAX_LANDMARKS + LSM_MAX_OBSTACLES;
+constexpr int kRowCap = (kMaxEntities + 3) / 4 * 4;
+
 // one environment range of the host-side adjacency expansion (pure data movement: every float is copied or zero)
 static void expand_adjacency_range(const float* adj_base, const uint32_t* adj_keep, float* adj, int64_t e0, int64_t e1, int N, int E,
                                    bool cached_stores) {
     const int W = (E + 31) / 32, EE = E * E;
     const bool vec = (EE % 4) == 0;          // every observer matrix starts 16-byte aligned
-    alignas(16) float row[LSM_MAX_AGENTS + LSM_MAX_LANDMARKS + 4];
+    alignas(16) float row[kRowCap];
     for (int64_t e = e0; e < e1; ++e) {
         const float* base = adj_base + e * EE;
         for (int i = 0; i < N; ++i) {
@@ -846,7 +851,7 @@ static void expand_adjacency_range(const float* adj_base, const uint32_t* adj_ke
                     continue;
                 }
                 // rows are 16-byte multiples: build the column mask once per observer, stream the rows
-                alignas(16) uint32_t cm[LSM_MAX_AGENTS + LSM_MAX_LANDMARKS + 4];
+                alignas(16) uint32_t cm[kRowCap];
                 for (int b = 0; b < E; ++b) cm[b] = ((keep[b >> 5] >> (b & 31)) & 1u) ? 0xffffffffu : 0u;
                 for (int a = 0; a < E; ++a) {
                     const bool ka = (keep[a >> 5] >> (a & 31)) & 1u;
@@ -884,7 +889,7 @@ static int resolve_host_threads(int threads, int64_t num_envs) {
 int lsm_expand_adjacency_host(const float* adj_base, const uint32_t* adj_keep, float* adj, int64_t num_envs, int32_t N, int32_t E,
                               int32_t threads, int32_t cached_stores) {
     if (adj_base == nullptr || adj_keep == nullptr || adj == nullptr) return fail(1, "lsm_expand_adjacency_host: null argument");
-    if (num_envs < 0 || N < 1 || N > LSM_MAX_AGENTS || E < N || E > LSM_MAX_AGENTS + LSM_MAX_LANDMARKS)
+    if (num_envs < 0 || N < 1 || N > LSM_MAX_AGENTS || E < N || E > kMaxEntities)
         return fail(2, "lsm_expand_adjacency_host: bad sizes");
     if (((uintptr_t)adj & 3u) || (((E * E) % 4) == 0 && ((uintptr_t)adj & 15u)))
         return fail(2, "lsm_expand_adjacency_host: adj must be 16-byte aligned (4-byte when E*E is not a multiple of 4)");
@@ -909,6 +914,7 @@ int lsm_fetch_host(lsm_handle* h, const lsm_host_io* io, void* stream) {
     if (io->adj == nullptr || io->adj_base_staging == nullptr || io->adj_keep_staging == nullptr)
         return fail(2, "lsm_fetch_host: adj, adj_base_staging and adj_keep_staging are required");
     const int N = h->kp.N, E = h->kp.E, W = (E + 31) / 32, EE = E * E;
+    if (E > kMaxEntities) return fail(2, "lsm_fetch_host: more entities than the host expansion holds");
     if (((uintptr_t)io->adj & 3u) || ((EE % 4) == 0 && ((uintptr_t)io->adj & 15u)))
         return fail(2, "lsm_fetch_host: adj must be 16-byte aligned (4-byte when E*E is not a multiple of 4)");
     const int64_t n = h->kp.b.num_envs;

@@ -128,6 +128,8 @@ __global__ void __launch_bounds__(32 * kEdgeCountWarps) lsm_edge_count_kernel(co
     using REC = EmitRec<DYN, N, L, O>;
     constexpr int E = REC::E, W = REC::W;
     constexpr int T = 32 * kEdgeCountWarps;
+    static_assert(sizeof(unsigned) * kEdgeCountWarps * (E * W + N * W) + sizeof(int) * kEdgeMaxEnvsPerBlock * N <= 40 * 1024,
+                  "static shared memory of the edge-count kernel stays under the 48 KB static limit");
     __shared__ unsigned s_rowmask[kEdgeCountWarps][E * W];
     __shared__ unsigned s_keep[kEdgeCountWarps][N * W];
     __shared__ int s_cnt[kEdgeMaxEnvsPerBlock * N];

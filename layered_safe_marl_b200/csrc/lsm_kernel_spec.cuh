@@ -61,6 +61,11 @@ struct __align__(16) EmitRec {
     static constexpr int E = N + M + O;
     static constexpr int W = (E + 31) / 32;
     static constexpr int CA = M + O;      // first agent-goal entry of cst
+    // the domain lsm_create accepts (lsm_b200.h LSM_MAX_*): 8-bit landmark indices, 16-bit entity indices in pair_tab
+    static_assert(N >= 1 && N <= LSM_MAX_AGENTS, "1 <= N <= 32: one lane per agent");
+    static_assert(L >= 2 && M <= LSM_MAX_LANDMARKS, "L >= 2 and N * L <= 128");
+    static_assert(O >= 0 && O <= LSM_MAX_OBSTACLES, "0 <= O <= 32");
+    static_assert(W <= 6, "at most 192 entities: 6 mask words");
     double2 pos[E + 2 * N];
     double2 vel[2 * N + 1];
     float4 cst[M + O + 2 * N];
@@ -607,6 +612,7 @@ __global__ void __launch_bounds__(kPairThreads) lsm_pair_kernel(const __grid_con
     using REC = EmitRec<DYN, N, L, O>;
     constexpr int ND = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5;
     constexpr unsigned T = N * (N - 1);
+    constexpr unsigned TD = T > 0 ? T : 1, ND1 = N > 1 ? N - 1 : 1;   // N = 1: no tasks; the divisors stay non-zero
     pdl_launch_dependents();
     if (!kp.pair_late) pdl_wait();
     tl_start(kp.timeline, TL_PAIR_START);
@@ -614,8 +620,8 @@ __global__ void __launch_bounds__(kPairThreads) lsm_pair_kernel(const __grid_con
     // grid-stride: the late placement runs a bounded number of blocks per SM (lsm_kernels.cu) so that these fp64-heavy
     // warps take a fixed share of the issue slots next to the emit kernel's producers
     for (unsigned t = blockIdx.x * blockDim.x + threadIdx.x; t < tasks; t += gridDim.x * blockDim.x) {
-        const unsigned el = t / T, r = t - el * T;
-        const int i = (int)(r / (N - 1)), jj = (int)(r - (unsigned)i * (N - 1));
+        const unsigned el = t / TD, r = t - el * TD;
+        const int i = (int)(r / ND1), jj = (int)(r - (unsigned)i * ND1);
         const int j = jj + (jj >= i);
         const int env = kp.env_begin + (int)el;
         double rel[ND];
@@ -1580,7 +1586,8 @@ struct __align__(16) EmitShared {
     unsigned sel[N * GEO::W];                                // KParams::sel_tab, read once per block (not once per environment)
     // fused COO edge output: non-zero bit mask of every row of the thresholded matrix, exclusive row offsets per observer
     unsigned rowmask[GEO::E * GEO::W];
-    unsigned short rowoff[N * GEO::E];      // <= E * (E - 1) = 18 240 for the largest configuration
+    unsigned short rowoff[N * GEO::E];      // <= E * (E - 1): 36 672 at the largest shape lsm_create accepts (E = 192)
+    static_assert(GEO::E * (GEO::E - 1) <= 65535, "rowoff holds an observer's edge count in 16 bits");
     long long gbase[N];
     long long range_base;
 };

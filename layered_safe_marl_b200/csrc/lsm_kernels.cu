@@ -50,6 +50,37 @@ namespace lsm {
     X(LSM_DYN_AIRTAXI, 10, 2, 4, LSM_AIR_WPE, 5)       \
     X(LSM_DYN_DOUBLE_INTEGRATOR, 8, 2, 4, 4, 4)
 
+// Launch shape of the emit kernel for a shape built on demand (-DLSM_SHAPE below; _build.build_shape), derived
+// at compile time instead of measured:
+//   WPE   warps per environment. The emit kernel's per-environment phases give one thread per entity or per observer row,
+//         so warps beyond ~E / 4 idle; the measured list picks 1 warp at E = 9, 2 at E = 12 and 4 at E = 24 and
+//         above, except the 8-agent airtaxi entry (E = 24), measured best at 2.
+//   EMINB resident blocks per SM the register budget targets: as many EmitShared blocks as the SM's shared memory holds
+//         (1 KB per block reserved by the hardware), at most 512 threads per SM as the list caps it (16 / 8 / 4 blocks
+//         of 1 / 2 / 4 warps). E >= ~150 leaves one block per SM.
+template <int DYN, int N, int L, int O>
+struct ShapeLaunch {
+    static constexpr int E = N + N * L + O;
+    static constexpr int WPE = E <= 9 ? 1 : E <= 16 ? 2 : 4;
+    static constexpr int kSmemPerSm = 233472, kSmemOptin = 232448, kBlockReserved = 1024;
+    static constexpr int SMEM = (int)sizeof(EmitShared<DYN, N, L, O, WPE>);
+    static_assert(SMEM <= kSmemOptin, "the emit kernel's shared memory exceeds the per-block opt-in of sm_100");
+    static constexpr int FIT = kSmemPerSm / (SMEM + kBlockReserved);
+    static constexpr int CAP = 16 / WPE;
+    static constexpr int EMINB = FIT < 1 ? 1 : FIT > CAP ? CAP : FIT;
+};
+
+#ifdef LSM_SHAPE
+// a library of exactly one specialised shape (plus the generic kernels). LSM_SHAPE = decimal digits DNNLLOO: dynamics,
+// agents, landmarks per agent, obstacles (one integer: nvcc splits a -D value at commas)
+constexpr int kShapeDyn = (LSM_SHAPE) / 1000000, kShapeN = (LSM_SHAPE) / 10000 % 100, kShapeL = (LSM_SHAPE) / 100 % 100,
+              kShapeO = (LSM_SHAPE) % 100;
+static_assert(kShapeDyn == LSM_DYN_DOUBLE_INTEGRATOR || kShapeDyn == LSM_DYN_AIRTAXI, "LSM_SHAPE: dynamics 0 or 1");
+using ShapeLaunchT = ShapeLaunch<kShapeDyn, kShapeN, kShapeL, kShapeO>;
+#undef LSM_SPEC_LIST
+#define LSM_SPEC_LIST(X) X(kShapeDyn, kShapeN, kShapeL, kShapeO, ShapeLaunchT::WPE, ShapeLaunchT::EMINB)
+#endif
+
 constexpr int kAgentBlock = 128;
 constexpr int kAgentMinB = 2;
 constexpr int kPairBlock = kPairThreads;

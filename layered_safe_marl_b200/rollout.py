@@ -126,7 +126,7 @@ class DeviceGraphRolloutBuffer:
             so_ptr = C.c_void_p(self.share_obs[s + 1].data_ptr()) if self.use_centralized_V else None
             _lib.check(env.lib.lsm_rollout_insert(env._h, C.c_void_p(self.obs[s + 1].data_ptr()), C.c_void_p(self._done_u8.data_ptr()),
                                                   so_ptr, C.c_void_p(self.masks[s + 1].data_ptr()),
-                                                  C.c_void_p(self.active_masks[s + 1].data_ptr()), env._stream()), 'lsm_rollout_insert')
+                                                  C.c_void_p(self.active_masks[s + 1].data_ptr()), env._stream()), 'lsm_rollout_insert', env.lib)
             if not self.use_centralized_V:
                 self.share_obs[s + 1].copy_(self.obs[s + 1])
         else:

@@ -25,7 +25,7 @@ from typing import Optional
 import numpy as np
 import torch
 
-from . import _lib
+from . import _build, _lib
 from . import layout as LY
 from .config import (DYN_DOUBLE_INTEGRATOR, FLAG_SHARED_REWARD, FLAG_USE_SAFETY_FILTER, FLAG_HJ_VALUE,
                      RewardBinaryConfig, RewardWeightConfig, ScenarioParams, scenario_params_from_args)
@@ -160,7 +160,15 @@ class B200GraphVecEnv:
         cfg = make_config_struct(p)
         self._cfg = cfg
         self._h = C.c_void_p()
-        _lib.check(self.lib.lsm_create(C.byref(cfg), C.byref(self._h)), 'lsm_create')
+        self._check(self.lib.lsm_create(C.byref(cfg), C.byref(self._h)), 'lsm_create')
+        if bool(getattr(args, 'specialise_shape', False)) and not os.environ.get('LSM_LIB') and \
+                self.launch_info()['specialised'] == 0:
+            # a shape the product library runs on the generic kernel: the library of exactly this shape (built by nvcc
+            # on first use, _build.build_shape), which runs the specialised pipeline
+            self.lib.lsm_destroy(self._h)
+            self._h = C.c_void_p()
+            self.lib = _lib.load(_build.build_shape(p.dynamics, N, self.L, self.O))
+            self._check(self.lib.lsm_create(C.byref(cfg), C.byref(self._h)), 'lsm_create')
         if tuning:
             # launch-shape overrides (include/lsm_b200.h lsm_tuning): chunks, pair_placement, packed_grid, use_graph
             unknown = set(tuning) - {'chunks', 'pair_placement', 'packed_grid', 'use_graph'}
@@ -168,7 +176,7 @@ class B200GraphVecEnv:
                 raise ValueError(f"unknown tuning keys {sorted(unknown)}")
             t = _lib.LsmTuning(int(tuning.get('chunks', 0)), int(tuning.get('pair_placement', -1)),
                                int(tuning.get('packed_grid', -1)), int(tuning.get('use_graph', -1)))
-            _lib.check(self.lib.lsm_set_tuning(self._h, C.byref(t)), 'lsm_set_tuning')
+            self._check(self.lib.lsm_set_tuning(self._h, C.byref(t)), 'lsm_set_tuning')
 
         # --- grids (HjDataHandle / TTR loading); synthetic when none is given
         needs_vg = bool(p.flags & (FLAG_USE_SAFETY_FILTER | FLAG_HJ_VALUE))
@@ -178,12 +186,12 @@ class B200GraphVecEnv:
             if value_grid is None:
                 value_grid = synthetic_di_grid() if p.dynamics == DYN_DOUBLE_INTEGRATOR else synthetic_airtaxi_grid()
             self.value_grid = _DeviceGrid(value_grid, self.device)
-            _lib.check(self.lib.lsm_set_value_grid(self._h, C.byref(self.value_grid.desc)), 'lsm_set_value_grid')
+            self._check(self.lib.lsm_set_value_grid(self._h, C.byref(self.value_grid.desc)), 'lsm_set_value_grid')
         if p.dynamics != DYN_DOUBLE_INTEGRATOR:
             if ttr_grid is None:
                 ttr_grid = synthetic_ttr_grid()
             self.ttr_grid = _DeviceGrid(ttr_grid, self.device)
-            _lib.check(self.lib.lsm_set_ttr_grid(self._h, C.byref(self.ttr_grid.desc)), 'lsm_set_ttr_grid')
+            self._check(self.lib.lsm_set_ttr_grid(self._h, C.byref(self.ttr_grid.desc)), 'lsm_set_ttr_grid')
 
         # --- state + output buffers in HBM
         n, M = self.n, self.M
@@ -226,7 +234,7 @@ class B200GraphVecEnv:
         b.reward_individual = self.reward_individual.data_ptr() if self.reward_individual is not None else None
         b.obstacles = self.obstacles.data_ptr() if self.O > 0 else None
         self._buffers = b
-        _lib.check(self.lib.lsm_bind_buffers(self._h, C.byref(b)), 'lsm_bind_buffers')
+        self._check(self.lib.lsm_bind_buffers(self._h, C.byref(b)), 'lsm_bind_buffers')
         # pinned staging for host-side callers (the unmodified runner hands numpy one-hot actions)
         self._act_pinned = None
         self._act_dev = None
@@ -262,7 +270,7 @@ class B200GraphVecEnv:
             cpt['node_h'] = torch.zeros((n, N, E, Fr), dtype=f32).pin_memory()
             cpt['reward_h'] = torch.zeros((n, N), dtype=f32).pin_memory()
             cpt['done_h'] = torch.zeros((n, N), dtype=torch.uint8).pin_memory()
-            _lib.check(self.lib.lsm_set_compact_adjacency(self._h, C.c_void_p(cpt['base'].data_ptr()),
+            self._check(self.lib.lsm_set_compact_adjacency(self._h, C.c_void_p(cpt['base'].data_ptr()),
                                                           C.c_void_p(cpt['keep'].data_ptr())), 'lsm_set_compact_adjacency')
             self._compact = cpt
 
@@ -288,10 +296,13 @@ class B200GraphVecEnv:
             res += [cpt['reward_h'].numpy(), cpt['done_h'].numpy().view(np.bool_)]
         return res
 
+    def _check(self, rc: int, what: str):
+        _lib.check(rc, what, self.lib)
+
     # ------------------------------------------------------------------------------------------
     def launch_info(self) -> dict:
         li = _lib.LsmLaunchInfo()
-        _lib.check(self.lib.lsm_get_launch_info(self._h, C.byref(li)), 'lsm_get_launch_info')
+        self._check(self.lib.lsm_get_launch_info(self._h, C.byref(li)), 'lsm_get_launch_info')
         return {k: int(getattr(li, k)) for k, _ in _lib.LsmLaunchInfo._fields_}
 
     def _stream(self):
@@ -362,7 +373,7 @@ class B200GraphVecEnv:
                 # compact adjacency over PCIe, expanded by the library's host threads while the later ranges and node_obs
                 # are still in flight (lsm_fetch_host); returns when every host array is complete
                 io = self._host_io(with_step)
-                _lib.check(self.lib.lsm_fetch_host(self._h, C.byref(io), self._stream()), 'lsm_fetch_host')
+                self._check(self.lib.lsm_fetch_host(self._h, C.byref(io), self._stream()), 'lsm_fetch_host')
                 return self._host_results(with_step)
             # generic-kernel configurations: dense adjacency straight into pinned buffers
             if self._host_out is None:
@@ -391,7 +402,7 @@ class B200GraphVecEnv:
     def reset(self, num_current_episode: int = 0, copy: bool = False):
         """GraphSubprocVecEnv.reset (env_wrappers.py:998-1005): every env draws a new scenario."""
         self._step_id += 1
-        _lib.check(self.lib.lsm_reset(self._h, None, int(num_current_episode), self.seed, 1, self._stream()),
+        self._check(self.lib.lsm_reset(self._h, None, int(num_current_episode), self.seed, 1, self._stream()),
                    'lsm_reset')
         obs, agent_id, node_obs, adj = self._outputs(False, copy)
         infos = LazyInfos(self, self._step_id, reset_only=True)
@@ -400,25 +411,25 @@ class B200GraphVecEnv:
     def reset_from_state(self, num_current_episode: int = 0):
         """reset bookkeeping + observation for the currently injected agents / landmarks (no sampling)."""
         self._step_id += 1
-        _lib.check(self.lib.lsm_reset(self._h, None, int(num_current_episode), self.seed, 0, self._stream()),
+        self._check(self.lib.lsm_reset(self._h, None, int(num_current_episode), self.seed, 0, self._stream()),
                    'lsm_reset')
         return self._outputs(False, False)
 
     def observe(self):
         """Re-emit obs / node_obs / adj from the current state (after set_state)."""
-        _lib.check(self.lib.lsm_observe(self._h, self._stream()), 'lsm_observe')
+        self._check(self.lib.lsm_observe(self._h, self._stream()), 'lsm_observe')
         return self._outputs(False, False)
 
     def emit_only(self):
         """Relaunch the graph-emission kernel alone (measurement hook; rewrites node_obs / adj with the same values)."""
-        _lib.check(self.lib.lsm_emit_only(self._h, self._stream()), 'lsm_emit_only')
+        self._check(self.lib.lsm_emit_only(self._h, self._stream()), 'lsm_emit_only')
 
     def debug_timeline(self, arm: bool = True):
         """Diagnostics: read the per-kernel %globaltimer timeline of the launches since the last arm (dict of ns relative
         to the first kernel's start, or None when nothing was armed), then re-arm / disarm."""
         out = (C.c_uint64 * 7)()
         had = getattr(self, '_tl_armed', False)
-        _lib.check(self.lib.lsm_debug_timeline(self._h, int(bool(arm)), out if had else None), 'lsm_debug_timeline')
+        self._check(self.lib.lsm_debug_timeline(self._h, int(bool(arm)), out if had else None), 'lsm_debug_timeline')
         self._tl_armed = bool(arm)
         if not had:
             return None
@@ -445,14 +456,14 @@ class B200GraphVecEnv:
             self._step_id += 1
             io = self._host_io(True)
             ptr = C.c_void_p(a.ctypes.data)
-            _lib.check(self.lib.lsm_step_host(self._h, None if a.ndim == 3 else ptr, ptr if a.ndim == 3 else None, ep,
+            self._check(self.lib.lsm_step_host(self._h, None if a.ndim == 3 else ptr, ptr if a.ndim == 3 else None, ep,
                                               self.seed, int(self.auto_reset), C.byref(io), self._stream()), 'lsm_step_host')
             obs, agent_id, node_obs, adj, rewards, dones = self._host_results(True)
             infos = LazyInfos(self, self._step_id, reset_only=False)
             return obs, agent_id, node_obs, adj, rewards, dones, infos
         idx_ptr, onehot_ptr = self._stage_actions(actions)
         self._step_id += 1
-        _lib.check(self.lib.lsm_step(self._h, idx_ptr, onehot_ptr, ep, self.seed, int(self.auto_reset),
+        self._check(self.lib.lsm_step(self._h, idx_ptr, onehot_ptr, ep, self.seed, int(self.auto_reset),
                                      self._stream()), 'lsm_step')
         obs, agent_id, node_obs, adj, rewards, dones = self._outputs(True, copy)
         infos = LazyInfos(self, self._step_id, reset_only=False)
@@ -489,7 +500,7 @@ class B200GraphVecEnv:
         obs, node_obs, adj = chk(obs, self.obs, 'obs'), chk(node_obs, self.node_obs, 'node_obs'), chk(adj, self.adj, 'adj')
         reward, done = chk(reward, self.reward, 'reward'), chk(done, self.done, 'done')
         ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
-        _lib.check(self.lib.lsm_set_output_buffers(self._h, ptr(obs), ptr(node_obs), ptr(adj), ptr(reward), ptr(done)),
+        self._check(self.lib.lsm_set_output_buffers(self._h, ptr(obs), ptr(node_obs), ptr(adj), ptr(reward), ptr(done)),
                    'lsm_set_output_buffers')
         for name, t in (('obs', obs), ('node_obs', node_obs), ('adj', adj), ('reward', reward), ('done', done)):
             if t is not None:
@@ -511,7 +522,7 @@ class B200GraphVecEnv:
             self._edge_counts = torch.empty((graphs,), dtype=torch.int32, device=self.device)
             self._edge_offsets = torch.empty((graphs + 1,), dtype=torch.int64, device=self.device)
             self._edge_cap = cap
-        _lib.check(self.lib.lsm_edge_list(self._h, C.c_void_p(a.data_ptr()), C.c_void_p(self._edge_index.data_ptr()),
+        self._check(self.lib.lsm_edge_list(self._h, C.c_void_p(a.data_ptr()), C.c_void_p(self._edge_index.data_ptr()),
                                           C.c_void_p(self._edge_attr.data_ptr()), C.c_void_p(self._edge_counts.data_ptr()),
                                           C.c_void_p(self._edge_offsets.data_ptr()), self._edge_cap, self._stream()),
                    'lsm_edge_list')
@@ -536,12 +547,12 @@ class B200GraphVecEnv:
         self.edge_capacity = cap
         self._edge_dense = bool(dense_adj)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.lsm_set_edge_output(self._h, C.c_void_p(self.edge_index.data_ptr()), C.c_void_p(self.edge_attr.data_ptr()),
+            self._check(self.lib.lsm_set_edge_output(self._h, C.c_void_p(self.edge_index.data_ptr()), C.c_void_p(self.edge_attr.data_ptr()),
                                                     C.c_void_p(self.edge_counts.data_ptr()), C.c_void_p(self.edge_offsets.data_ptr()),
                                                     cap, int(bool(dense_adj))), 'lsm_set_edge_output')
 
     def disable_edge_output(self):
-        _lib.check(self.lib.lsm_set_edge_output(self._h, None, None, None, None, 0, 1), 'lsm_set_edge_output')
+        self._check(self.lib.lsm_set_edge_output(self._h, None, None, None, None, 0, 1), 'lsm_set_edge_output')
         self.edge_index = self.edge_attr = self.edge_counts = self.edge_offsets = None
         self._edge_dense = True
 
@@ -566,14 +577,14 @@ class B200GraphVecEnv:
         ew = torch.empty((cap,), dtype=torch.float64, device=self.device)
         cnt = torch.empty((n,), dtype=torch.int32, device=self.device)
         off = torch.empty((n + 1,), dtype=torch.int64, device=self.device)
-        _lib.check(self.lib.lsm_world_graph(self._h, C.c_void_p(ei.data_ptr()), C.c_void_p(ew.data_ptr()), C.c_void_p(cnt.data_ptr()),
+        self._check(self.lib.lsm_world_graph(self._h, C.c_void_p(ei.data_ptr()), C.c_void_p(ew.data_ptr()), C.c_void_p(cnt.data_ptr()),
                                             C.c_void_p(off.data_ptr()), cap, self._stream()), 'lsm_world_graph')
         nnz = int(off[-1].item())
         return ei[:, :nnz], ew[:nnz], off
 
     def invalidate(self):
         """Call after writing the state tensors (agent_f64, agent_i32, env_f64, landmarks) directly."""
-        _lib.check(self.lib.lsm_invalidate(self._h), 'lsm_invalidate')
+        self._check(self.lib.lsm_invalidate(self._h), 'lsm_invalidate')
 
     def set_state(self, s: dict):
         dev = self.device
@@ -627,7 +638,7 @@ class B200GraphVecEnv:
         if b is not None:
             b = np.ascontiguousarray(b, dtype=np.float64)
             bp = b.ctypes.data_as(C.c_void_p)
-        _lib.check(self.lib.lsm_math_eval(int(op), a.ctypes.data_as(C.c_void_p), bp, out.ctypes.data_as(C.c_void_p), a.size),
+        self._check(self.lib.lsm_math_eval(int(op), a.ctypes.data_as(C.c_void_p), bp, out.ctypes.data_as(C.c_void_p), a.size),
                    'lsm_math_eval')
         return out
 
@@ -671,7 +682,7 @@ class B200GraphVecEnv:
         # column sums + env count in one launch of the library (lsm_episode_stats), then at most one all-reduce of 9 doubles
         sums = torch.empty((LY.EP_COUNT + 1,), dtype=torch.float64, device=self.device)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.lsm_episode_stats(self._h, C.c_void_p(sums.data_ptr()), self._stream()), 'lsm_episode_stats')
+            self._check(self.lib.lsm_episode_stats(self._h, C.c_void_p(sums.data_ptr()), self._stream()), 'lsm_episode_stats')
         if reduce_group is None:
             vals = (sums[:-1] / sums[-1]).cpu().numpy()
             return {k: float(vals[j]) for j, k in enumerate(LY.EP_INFO_KEYS)}
