@@ -26,6 +26,9 @@
  *                HjDataHandle.__init__                     multiagent/safety_filter.py:154-168
  *                TTR grid loading in make_world            navigation_graph_safe.py:128-138
  *   lsm_create   Scenario.make_world (constants only)      navigation_graph_safe.py:58-262
+ *   lsm_safety_filter  both safety handles' apply_safety_filter for caller-owned states
+ *                                                          multiagent/safety_filter.py:203-260, 378-433
+ *   lsm_hj_lookup      get_value_of_relative_state + gradient  multiagent/safety_filter.py:192-201, 345-354
  */
 #ifndef LSM_B200_H
 #define LSM_B200_H
@@ -359,6 +362,53 @@ int lsm_debug_timeline(lsm_handle *h, int arm, uint64_t *out_ns);
  * are defined: envs whose curriculum has the filter on, i != j, both agents not done. Returns 6 when the
  * configuration keeps no pair values (generic kernel). */
 int lsm_debug_pair_values(lsm_handle *h, double *out, void *stream);
+
+/* The HJ safety filter as a standalone batched operator, for states the environment does not own (another simulator,
+ * hardware, logged trajectories). Both entry points need a handle with a value grid (lsm_set_value_grid); buffers need
+ * not be bound. They use the handle's dynamics, grid, interpolation mode (LSM_FLAG_INTERP_FLOAT32) and its config's dt,
+ * cbf_rate and coordination_range, evaluate the relative state in the form of the specialised pipeline (one sincos of
+ * the ego heading per pair), launch on `stream` and never synchronise. All pointers are DEVICE pointers; states are
+ * double integrator [x, y, vx, vy] or airtaxi [x, y, theta, v]; d = 4 (double integrator) | 5 (airtaxi).
+ *
+ * lsm_safety_filter: the safety handle's apply_safety_filter (safety_filter.py:203-260, 378-433) for num_rows
+ * independent egos, each against num_slots candidate others. Per row: distance and HJ value of every active slot, the
+ * FIRST minimum of each in ascending slot order (np.argmin), the value shifted by -(sep - grid separation), then the
+ * range test against coordination_range, gradient, bang-bang below 0.4 or CBF-QP, clipping and
+ * filtered = |u - u_ref| > 1e-4, exactly as lsm_step computes it for one ego. index is the deconflicting slot, also when
+ * the row stays unfiltered because of range; -1 and value +inf when no slot is active. If every active value is +inf
+ * (NaN state) index is the first active slot, value +inf and the row is unfiltered. */
+typedef struct lsm_filter_io {
+    int64_t num_rows;                   /* B >= 0 */
+    int32_t num_slots;                  /* M >= 0 */
+    int32_t _reserved;
+    const double *ego;                  /* [B][4] */
+    const double *others;               /* [B][M][4] (may be NULL when M == 0) */
+    const double *ego_action;           /* [B][2]    decoded control of the ego */
+    const double *other_actions;        /* [B][M][2] decoded reference controls of the others (may be NULL when M == 0) */
+    const uint8_t *active;              /* [B][M] slot mask (0 = absent) or NULL = every slot active */
+    const double *separation_distance;  /* [B] or NULL = the grid's own separation (no shift) */
+    double *safe_action;                /* [B][2] out */
+    uint8_t *filtered;                  /* [B] out, or NULL */
+    int32_t *index;                     /* [B] out, or NULL */
+    double *value;                      /* [B] out, or NULL */
+} lsm_filter_io;
+int lsm_safety_filter(lsm_handle *h, const lsm_filter_io *io, void *stream);
+
+/* lsm_hj_lookup: get_value_of_relative_state (safety_filter.py:192-201, 345-354) and the gradient (:245, :418) for
+ * num_points points, given as relative states (rel non-NULL) or as (ego, other) state pairs. value: +inf for a NaN
+ * relative state, shifted like the filter's; a finite point outside the grid box is interpolated with the grid's index
+ * clamp, as the env does. grad: every component NaN for a NaN relative state. */
+typedef struct lsm_lookup_io {
+    int64_t num_points;                 /* K >= 0 */
+    const double *rel;                  /* [K][d] or NULL: then ego / other */
+    const double *ego;                  /* [K][4] */
+    const double *other;                /* [K][4] */
+    const double *separation_distance;  /* [K] or NULL = the grid's own separation */
+    double *value;                      /* [K] out */
+    double *grad;                       /* [K][d] out, or NULL */
+    double *rel_out;                    /* [K][d] out: the relative state used, or NULL */
+} lsm_lookup_io;
+int lsm_hj_lookup(lsm_handle *h, const lsm_lookup_io *io, void *stream);
 
 #ifdef __cplusplus
 }

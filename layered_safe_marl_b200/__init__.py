@@ -5,8 +5,9 @@ from .config import (AirTaxiConfig, DoubleIntegratorConfig, RewardBinaryConfig, 
                      ScenarioParams, scenario_params_from_args)
 from .vec_env import B200GraphDummyVecEnv, B200GraphVecEnv
 from .rollout import DeviceGraphRolloutBuffer
+from .safety_filter import SafetyFilter
 from . import eval_scenarios
 
 __all__ = ['AirTaxiConfig', 'DoubleIntegratorConfig', 'RewardBinaryConfig', 'RewardWeightConfig',
            'ScenarioParams', 'scenario_params_from_args', 'B200GraphVecEnv', 'B200GraphDummyVecEnv',
-           'DeviceGraphRolloutBuffer', 'eval_scenarios']
+           'DeviceGraphRolloutBuffer', 'SafetyFilter', 'eval_scenarios']

@@ -64,12 +64,24 @@ class LsmHostIo(C.Structure):
                 ('threads', C.c_int32), ('chunks', C.c_int32), ('cached_stores', C.c_int32), ('_reserved', C.c_int32)]
 
 
+class LsmFilterIo(C.Structure):
+    _fields_ = [('num_rows', C.c_int64), ('num_slots', C.c_int32), ('_reserved', C.c_int32),
+                ('ego', C.c_void_p), ('others', C.c_void_p), ('ego_action', C.c_void_p), ('other_actions', C.c_void_p),
+                ('active', C.c_void_p), ('separation_distance', C.c_void_p), ('safe_action', C.c_void_p),
+                ('filtered', C.c_void_p), ('index', C.c_void_p), ('value', C.c_void_p)]
+
+
+class LsmLookupIo(C.Structure):
+    _fields_ = [('num_points', C.c_int64), ('rel', C.c_void_p), ('ego', C.c_void_p), ('other', C.c_void_p),
+                ('separation_distance', C.c_void_p), ('value', C.c_void_p), ('grad', C.c_void_p), ('rel_out', C.c_void_p)]
+
+
 EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_destroy', 'lsm_set_value_grid',
                     'lsm_set_ttr_grid', 'lsm_bind_buffers', 'lsm_get_launch_info', 'lsm_step', 'lsm_reset',
                     'lsm_observe', 'lsm_emit_only', 'lsm_invalidate', 'lsm_set_output_buffers', 'lsm_edge_list',
                     'lsm_debug_timeline', 'lsm_rollout_insert', 'lsm_math_eval', 'lsm_math_eval_device', 'lsm_set_tuning',
                     'lsm_set_compact_adjacency', 'lsm_expand_adjacency_host', 'lsm_set_edge_output', 'lsm_world_graph', 'lsm_fetch_host', 'lsm_step_host',
-                    'lsm_episode_stats', 'lsm_debug_pair_values')
+                    'lsm_episode_stats', 'lsm_debug_pair_values', 'lsm_safety_filter', 'lsm_hj_lookup')
 
 _libs = {}          # one CDLL per path: the product library and the per-shape libraries (_build.build_shape)
 
@@ -122,6 +134,8 @@ def load(path: Optional[str] = None):
     lib.lsm_set_edge_output.argtypes = [C.c_void_p] * 5 + [C.c_int64, C.c_int]
     lib.lsm_world_graph.argtypes = [C.c_void_p] * 5 + [C.c_int64, C.c_void_p]
     lib.lsm_episode_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.lsm_safety_filter.argtypes = [C.c_void_p, C.POINTER(LsmFilterIo), C.c_void_p]
+    lib.lsm_hj_lookup.argtypes = [C.c_void_p, C.POINTER(LsmLookupIo), C.c_void_p]
     lib.lsm_math_eval.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
     lib.lsm_math_eval_device.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
     for name in EXPORTED_SYMBOLS:

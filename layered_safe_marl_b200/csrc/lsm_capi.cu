@@ -1172,6 +1172,51 @@ int lsm_debug_pair_values(lsm_handle* h, double* out, void* stream) {
     return 0;
 }
 
+// the standalone filter operator needs the handle's value grid only (no bound buffers)
+static int filter_op_check_grid(const lsm_handle* h, const char* who) {
+    if (!h->kp.has_vg) return fail(5, std::string(who) + ": the handle has no value grid (call lsm_set_value_grid first)");
+    const int want = h->kp.c.dynamics == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5;
+    if (h->kp.vg.ndim != want) return fail(2, std::string(who) + ": the value grid's dimensionality does not match the dynamics");
+    return 0;
+}
+
+int lsm_safety_filter(lsm_handle* h, const lsm_filter_io* io, void* stream) {
+    if (h == nullptr || io == nullptr) return fail(1, "lsm_safety_filter: null argument");
+    if (int rc = filter_op_check_grid(h, "lsm_safety_filter")) return rc;
+    if (io->num_rows < 0 || io->num_slots < 0) return fail(2, "lsm_safety_filter: num_rows and num_slots must be >= 0");
+    if (io->num_rows == 0) return 0;
+    if (io->ego == nullptr || io->ego_action == nullptr || io->safe_action == nullptr)
+        return fail(2, "lsm_safety_filter: ego, ego_action and safe_action are required");
+    if (io->num_slots > 0 && (io->others == nullptr || io->other_actions == nullptr))
+        return fail(2, "lsm_safety_filter: others and other_actions are required when num_slots > 0");
+    DeviceGuard guard(h->device);
+    lsm::FilterOpArgs a;
+    a.rows = io->num_rows; a.slots = io->num_slots;
+    a.ego = io->ego; a.others = io->others; a.ego_action = io->ego_action; a.other_actions = io->other_actions;
+    a.active = io->active; a.sep = io->separation_distance;
+    a.safe_action = io->safe_action; a.filtered = io->filtered; a.index = io->index; a.value = io->value;
+    const cudaError_t e = lsm::safety_filter_launch(h->kp, a, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "lsm_safety_filter");
+    return 0;
+}
+
+int lsm_hj_lookup(lsm_handle* h, const lsm_lookup_io* io, void* stream) {
+    if (h == nullptr || io == nullptr) return fail(1, "lsm_hj_lookup: null argument");
+    if (int rc = filter_op_check_grid(h, "lsm_hj_lookup")) return rc;
+    if (io->num_points < 0) return fail(2, "lsm_hj_lookup: num_points must be >= 0");
+    if (io->num_points == 0) return 0;
+    if (io->value == nullptr) return fail(2, "lsm_hj_lookup: value is required");
+    if (io->rel == nullptr && (io->ego == nullptr || io->other == nullptr))
+        return fail(2, "lsm_hj_lookup: give either rel or both ego and other");
+    DeviceGuard guard(h->device);
+    lsm::LookupArgs a;
+    a.points = io->num_points; a.rel = io->rel; a.ego = io->ego; a.other = io->other; a.sep = io->separation_distance;
+    a.value = io->value; a.grad = io->grad; a.rel_out = io->rel_out;
+    const cudaError_t e = lsm::hj_lookup_launch(h->kp, a, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_lookup");
+    return 0;
+}
+
 int lsm_debug_timeline(lsm_handle* h, int arm, uint64_t* out_ns) {
     if (h == nullptr) return fail(1, "lsm_debug_timeline: null handle");
     DeviceGuard guard(h->device);

@@ -30,6 +30,35 @@ cudaError_t episode_stats_launch(const double* ep_info, long long n, double* out
 cudaError_t rollout_insert_launch(const float* obs, const uint8_t* done, float* share_obs, float* masks, float* active_masks,
                                   long long n, int N, int D, cudaStream_t stream);
 cudaError_t math_eval_launch(int op, const double* a, const double* b, double* out, long long n, cudaStream_t stream);
+// standalone filter operator (lsm_filter_op.cuh): device pointers of lsm_filter_io / lsm_lookup_io
+struct FilterOpArgs {
+    long long rows;
+    int slots;
+    const double* ego;              // [rows][4]
+    const double* others;           // [rows][slots][4]
+    const double* ego_action;       // [rows][2]
+    const double* other_actions;    // [rows][slots][2]
+    const uint8_t* active;          // [rows][slots] or NULL (all active)
+    const double* sep;              // [rows] or NULL (the grid's own separation: no shift)
+    double* safe_action;            // [rows][2]
+    uint8_t* filtered;              // [rows] or NULL
+    int32_t* index;                 // [rows] or NULL
+    double* value;                  // [rows] or NULL
+};
+
+struct LookupArgs {
+    long long points;
+    const double* rel;              // [points][ND] or NULL: then (ego, other) pairs
+    const double* ego;              // [points][4]
+    const double* other;            // [points][4]
+    const double* sep;              // [points] or NULL
+    double* value;                  // [points]
+    double* grad;                   // [points][ND] or NULL
+    double* rel_out;                // [points][ND] or NULL
+};
+// lsm_filter_op.cuh: the handle's dynamics and interpolation mode; no-op for zero rows / points
+cudaError_t safety_filter_launch(const KParams& kp, const FilterOpArgs& a, cudaStream_t stream);
+cudaError_t hj_lookup_launch(const KParams& kp, const LookupArgs& a, cudaStream_t stream);
 cudaError_t pad_grads_launch(const float* grads, float* grads8, long long cells);
 cudaError_t edge_list_launch(const float* adj, int32_t* counts, long long* offsets, long long* edge_index, float* edge_attr,
                              long long num_graphs, int E, long long capacity, cudaStream_t stream);

@@ -3,6 +3,7 @@
 //   lsm_kernel_spec.cuh     kernels specialised at compile time on (dynamics, N, L) - the fast path
 //   lsm_kernel_generic.cuh  run-time N / L fallback for every other configuration
 //   lsm_step_common.cuh     dynamics, HJ filter resolution, grid interpolation shared by both
+//   lsm_filter_op.cuh       the same filter as a standalone batched operator (lsm_safety_filter / lsm_hj_lookup)
 //
 // Specialised path: three launches per step (per-agent physics -> graph emission -> next step's pair values), see
 // lsm_kernel_spec.cuh. Generic path ("warp per env group", one fused launch): a warp owns EPW consecutive
@@ -15,6 +16,7 @@
 // observer i selects "post" for agents <= i and "pre" for agents > i.
 #include "lsm_kernel_generic.cuh"
 #include "lsm_kernel_spec.cuh"
+#include "lsm_filter_op.cuh"
 #include "lsm_edges.cuh"
 #include "lsm_rollout.cuh"
 #include "lsm_host.h"
@@ -437,6 +439,50 @@ cudaError_t math_eval_launch(int op, const double* a, const double* b, double* o
     if (n <= 0) return cudaSuccess;
     lsm_math_eval_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(op, a, b, out, n);
     return cudaGetLastError();
+}
+
+// the standalone filter operator: instantiation of the handle's dynamics and interpolation mode, on the caller's stream
+static int sm_count_cached() {
+    static int sm_count = 0;
+    if (sm_count == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev); }
+    return sm_count;
+}
+
+cudaError_t safety_filter_launch(const KParams& kp, const FilterOpArgs& a, cudaStream_t stream) {
+    if (a.rows <= 0) return cudaSuccess;
+    const bool f32 = kp_interp_f32(kp), di = kp.c.dynamics == LSM_DYN_DOUBLE_INTEGRATOR;
+    const void* fn = di ? (f32 ? (const void*)lsm_safety_filter_kernel<LSM_DYN_DOUBLE_INTEGRATOR, true>
+                               : (const void*)lsm_safety_filter_kernel<LSM_DYN_DOUBLE_INTEGRATOR, false>)
+                        : (f32 ? (const void*)lsm_safety_filter_kernel<LSM_DYN_AIRTAXI, true>
+                               : (const void*)lsm_safety_filter_kernel<LSM_DYN_AIRTAXI, false>);
+    // one tile of kFopRows rows per block; beyond 32 blocks per SM the blocks stride over the tiles
+    long long blocks = (a.rows + kFopRows - 1) / kFopRows;
+    const long long cap = (long long)sm_count_cached() * 32;
+    if (blocks > cap) blocks = cap;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)blocks, 1, 1);
+    cfg.blockDim = dim3(kFopThreads, 1, 1);
+    cfg.stream = stream;
+    void* args[] = { (void*)&kp, (void*)&a };
+    return cudaLaunchKernelExC(&cfg, fn, args);
+}
+
+cudaError_t hj_lookup_launch(const KParams& kp, const LookupArgs& a, cudaStream_t stream) {
+    if (a.points <= 0) return cudaSuccess;
+    const bool f32 = kp_interp_f32(kp), di = kp.c.dynamics == LSM_DYN_DOUBLE_INTEGRATOR;
+    const void* fn = di ? (f32 ? (const void*)lsm_hj_lookup_kernel<LSM_DYN_DOUBLE_INTEGRATOR, true>
+                               : (const void*)lsm_hj_lookup_kernel<LSM_DYN_DOUBLE_INTEGRATOR, false>)
+                        : (f32 ? (const void*)lsm_hj_lookup_kernel<LSM_DYN_AIRTAXI, true>
+                               : (const void*)lsm_hj_lookup_kernel<LSM_DYN_AIRTAXI, false>);
+    long long blocks = (a.points + kLookupThreads - 1) / kLookupThreads;
+    const long long cap = (long long)sm_count_cached() * 64;
+    if (blocks > cap) blocks = cap;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)blocks, 1, 1);
+    cfg.blockDim = dim3(kLookupThreads, 1, 1);
+    cfg.stream = stream;
+    void* args[] = { (void*)&kp, (void*)&a };
+    return cudaLaunchKernelExC(&cfg, fn, args);
 }
 
 cudaError_t pad_grads_launch(const float* grads, float* grads8, long long cells) {
