@@ -350,6 +350,34 @@ int lsm_invalidate(lsm_handle *h);
  * configuration has no separate emission launch. */
 int lsm_emit_only(lsm_handle *h, void *stream);
 
+/* Rollout storage by emit record (specialised pipeline only). The graph observation of one environment at one step is a
+ * pure function of its emit record (emit_record_bytes of lsm_launch_info, 1-7 % of the dense node_obs + adj bytes) and
+ * of the handle's constants (radius, graph_feat_type), so a rollout can keep the records and rebuild any observer's
+ * graph when a learner asks for it.
+ *
+ * lsm_copy_records: copy the num_envs * emit_record_bytes records that the last lsm_step / lsm_reset / lsm_observe left
+ * behind to `dst` (device or pinned host memory) with one cudaMemcpyAsync on `stream`. After a masked reset the envs
+ * outside the mask keep the record of their previous step, which is also what their node_obs / adj still hold. Returns
+ * 6 on a generic-kernel handle, 5 when no buffers are bound. */
+int lsm_copy_records(lsm_handle *h, void *dst, void *stream);
+
+/* lsm_emit_from_records: for each item k, the node rows and the masked thresholded adjacency matrix that observer
+ * observer[k] received at the step of record record[k], byte for byte what the step's emission wrote to its node_obs /
+ * adj. Uses the handle's shape, graph_feat_type and coordination_range; needs no bound buffers, launches on `stream`
+ * and never synchronises. An item whose record is outside [0, num_records) or whose observer is outside [0, N) gets
+ * zero-filled outputs. Returns 6 on a generic-kernel handle. */
+typedef struct lsm_record_emit_io {
+    int64_t num_items;          /* B >= 0 */
+    int64_t num_records;        /* records in the store */
+    const void *records;        /* DEVICE [num_records][emit_record_bytes], 16-byte aligned, written by lsm_copy_records
+                                   of a handle of the same library and shape */
+    const int64_t *record;      /* DEVICE [B] */
+    const int32_t *observer;    /* DEVICE [B] */
+    float *node_obs;            /* DEVICE [B][E][F] out (F = 7 with graph_feat_type global), 16-byte aligned, or NULL */
+    float *adj;                 /* DEVICE [B][E][E] out, 16-byte aligned, or NULL */
+} lsm_record_emit_io;
+int lsm_emit_from_records(lsm_handle *h, const lsm_record_emit_io *io, void *stream);
+
 /* Diagnostics (never on the product path): per-kernel timeline of the launches that follow. If `out_ns` is non-NULL
  * and a timeline is armed, synchronises the device and copies 7 %globaltimer values (ns) out: pair first-block-in,
  * pair last-body-out, agent in / out, emit in / out, pair grid out. `arm` != 0 (re)arms the recording for the next

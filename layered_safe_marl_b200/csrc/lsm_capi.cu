@@ -1160,6 +1160,39 @@ int lsm_emit_only(lsm_handle* h, void* stream) {
     return 0;
 }
 
+int lsm_copy_records(lsm_handle* h, void* dst, void* stream) {
+    if (h == nullptr) return fail(1, "lsm_copy_records: null handle");
+    if (!h->spec) return fail(6, "lsm_copy_records: this configuration runs the fused generic kernel (no emit records)");
+    if (!h->have_buffers) return fail(5, "lsm_copy_records: lsm_bind_buffers has not been called");
+    if (dst == nullptr) return fail(2, "lsm_copy_records: null destination");
+    DeviceGuard guard(h->device);
+    const size_t bytes = (size_t)h->kp.b.num_envs * (size_t)h->geo.rec_bytes;
+    const cudaError_t e = cudaMemcpyAsync(dst, h->d_emit_rec, bytes, cudaMemcpyDefault, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "lsm_copy_records");
+    return 0;
+}
+
+int lsm_emit_from_records(lsm_handle* h, const lsm_record_emit_io* io, void* stream) {
+    if (h == nullptr || io == nullptr) return fail(1, "lsm_emit_from_records: null argument");
+    if (!h->spec) return fail(6, "lsm_emit_from_records: this configuration runs the fused generic kernel (no emit records)");
+    if (io->num_items < 0 || io->num_records < 0) return fail(2, "lsm_emit_from_records: num_items and num_records must be >= 0");
+    if (io->num_items == 0 || (io->node_obs == nullptr && io->adj == nullptr)) return 0;
+    if (io->record == nullptr || io->observer == nullptr) return fail(2, "lsm_emit_from_records: record and observer are required");
+    if (io->num_records > 0 && io->records == nullptr) return fail(2, "lsm_emit_from_records: null record store");
+    if (((uintptr_t)io->records & 15u) || ((uintptr_t)io->node_obs & 15u) || ((uintptr_t)io->adj & 15u))
+        return fail(2, "lsm_emit_from_records: records, node_obs and adj must be 16-byte aligned");
+    DeviceGuard guard(h->device);
+    lsm::RecordEmitArgs a;
+    a.num_items = io->num_items; a.num_records = io->num_records;
+    a.records = (const unsigned char*)io->records; a.record = (const long long*)io->record; a.observer = io->observer;
+    a.node_obs = io->node_obs; a.adj = io->adj;
+    a.sel_tab = h->kp.sel_tab; a.r2_lt = h->kp.r2_lt; a.r2_nz = h->kp.r2_nz;
+    a.gfeat = (h->kp.c.flags & LSM_FLAG_GRAPH_FEAT_GLOBAL) != 0;
+    const cudaError_t e = lsm::spec_launch_record_emit(h->kp.c.dynamics, h->kp.N, h->kp.L, h->kp.O, a, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "lsm_emit_from_records");
+    return 0;
+}
+
 int lsm_debug_pair_values(lsm_handle* h, double* out, void* stream) {
     if (h == nullptr) return fail(1, "lsm_debug_pair_values: null handle");
     if (!h->have_buffers) return fail(5, "lsm_debug_pair_values: lsm_bind_buffers has not been called");

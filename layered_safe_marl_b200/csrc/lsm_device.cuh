@@ -129,6 +129,19 @@ struct KParams {
 #endif
 };
 
+// lsm_emit_from_records: items (record, observer) of a caller-owned record store, re-emitted with a handle's constants
+struct RecordEmitArgs {
+    long long num_items, num_records;
+    const unsigned char* records;   // [num_records][sizeof(EmitRec)], 16-byte aligned
+    const long long* record;        // [num_items]
+    const int* observer;            // [num_items]
+    float* node_obs;                // [num_items][E][F or 7] or NULL
+    float* adj;                     // [num_items][E][E] or NULL
+    const uint32_t* sel_tab;        // KParams::sel_tab
+    double r2_lt, r2_nz;            // KParams::r2_lt / r2_nz
+    int gfeat;                      // LSM_FLAG_GRAPH_FEAT_GLOBAL
+};
+
 // timeline slots: first block in / last block out of each kernel of the pipeline (ns, %globaltimer)
 enum { TL_PAIR_START = 0, TL_PAIR_BODY_END, TL_AGENT_START, TL_AGENT_END, TL_EMIT_START, TL_EMIT_END, TL_PAIR_END, TL_COUNT };
 __device__ __forceinline__ unsigned long long globaltimer_ns() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }

@@ -1701,6 +1701,80 @@ __device__ __noinline__ void emit_edges(EmitShared<DYN, N, L, O, WPE>& S, const 
     __syncthreads();
 }
 
+// ---------------------------------------------------------------------------------------------
+// graph emission from one record: shared by lsm_emit_kernel (every observer of an env) and lsm_record_emit_kernel (one
+// observer of one stored record), so that both write the same bytes
+// ---------------------------------------------------------------------------------------------
+// float32 adjacency entry of an entity pair at squared distance d2: non-zero strictly inside the radius and above r2_nz
+__device__ __forceinline__ float adj_value(double d2, double r2_lt, double r2_nz) {
+    const float d2f = fmaxf((float)d2, 1.0e-30f);
+    float rs;
+    asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(rs) : "f"(d2f));
+    return (d2 < r2_lt && d2 > r2_nz) ? d2f * rs : 0.0f;
+}
+
+// entities one mask word of an observer keeps: an entity whose owner is <= the observer (sel) is seen after this step's
+// goal update (disconnected after), any other before it
+__device__ __forceinline__ unsigned keep_word(unsigned disc_post, unsigned disc_pre, unsigned sel) {
+    return ~((disc_post & sel) | (disc_pre & ~sel));
+}
+
+// node-feature row r = i * E + e (observer i, entity e) of the record: F floats, or 7 with graph_feat_type 'global'
+template <int DYN, int N, int L, int O>
+__device__ __forceinline__ void node_feature_row(const EmitRec<DYN, N, L, O>& R, int r, bool gfeat, float* o) {
+    using REC = EmitRec<DYN, N, L, O>;
+    constexpr int M = REC::M, E = REC::E;
+    const int i = r / E, e = r - i * E;
+    const double2 pi = R.pos[i], vi = R.vel[N + i];
+    const bool is_agent = e < N;
+    const int sel = (e <= i) ? N : 0;     // agents <= i are seen after their own update
+    const int vidx = is_agent ? sel + e : 2 * N;
+    const int gidx = is_agent ? E + sel + e : e;
+    const int cidx = is_agent ? REC::CA + sel + e : e - N;
+    if (gfeat) {
+        // an agent's goal is its FIRST landmark (optimal_match_index = arange, navigation_graph_safe.py:179), a
+        // landmark's goal is itself; velocities are world-frame (landmarks: zero)
+        const double2 pe = R.pos[e], ve = R.vel[vidx], ge = is_agent ? R.pos[N + e] : pe;
+        o[0] = (float)ve.x; o[1] = (float)ve.y; o[2] = (float)pe.x; o[3] = (float)pe.y;
+        o[4] = (float)ge.x; o[5] = (float)ge.y; o[6] = is_agent ? 0.0f : ((O == 0 || e < N + M) ? 1.0f : 2.0f);
+        (void)gidx; (void)cidx; (void)pi; (void)vi;
+    } else if constexpr (DYN == LSM_DYN_DOUBLE_INTEGRATOR) {
+        // utils.py:201-255: [p_e - p_i, v_e - v_i, goal_e - p_i, sin gh, cos gh, gspeed, type]
+        const double2 pe = R.pos[e], ve = R.vel[vidx], ge = R.pos[gidx];
+        const float4 cc = R.cst[cidx];
+        float2* o2 = reinterpret_cast<float2*>(o);   // rows are 40 B: 8 B aligned
+        o2[0] = make_float2((float)(pe.x - pi.x), (float)(pe.y - pi.y));
+        o2[1] = make_float2((float)(ve.x - vi.x), (float)(ve.y - vi.y));
+        o2[2] = make_float2((float)(ge.x - pi.x), (float)(ge.y - pi.y));
+        o2[3] = make_float2(cc.x, cc.y);
+        o2[4] = make_float2(cc.z, cc.w);
+    } else {
+        const double ci = R.air.cth[i], si = R.air.sth[i];
+        if (e < N) {
+            const int g = R.air.goal[sel ? 1 : 0][e];
+            const double2 pe = R.pos[e], ve = R.vel[vidx], ge = R.pos[gidx];
+            double rx, ry, gx, gy;
+            rotate_into(pe.x - pi.x, pe.y - pi.y, ci, si, rx, ry);
+            rotate_into(ge.x - pi.x, ge.y - pi.y, ci, si, gx, gy);
+            const double ce = R.air.cth[e], se = R.air.sth[e];
+            o[0] = (float)rx; o[1] = (float)ry; o[2] = (float)norm2(ve.x - vi.x, ve.y - vi.y);
+            o[3] = (float)(se * ci - ce * si); o[4] = (float)(ce * ci + se * si);
+            o[5] = (float)gx; o[6] = (float)gy;
+            o[7] = (float)(R.air.lsin[g] * ci - R.air.lcos[g] * si); o[8] = (float)(R.air.lcos[g] * ci + R.air.lsin[g] * si);
+            o[9] = (float)R.air.lsp[g]; o[10] = 0.0f;
+        } else {
+            const int m = e - N;
+            const double2 pe = R.pos[e];
+            double rx, ry;
+            rotate_into(pe.x - pi.x, pe.y - pi.y, ci, si, rx, ry);
+            const float sh = (float)(R.air.lsin[m] * ci - R.air.lcos[m] * si), ch = (float)(R.air.lcos[m] * ci + R.air.lsin[m] * si);
+            o[0] = (float)rx; o[1] = (float)ry; o[2] = (float)R.air.spd_post[i];
+            o[3] = sh; o[4] = ch; o[5] = (float)rx; o[6] = (float)ry; o[7] = sh; o[8] = ch;
+            o[9] = (float)R.air.lsp[m]; o[10] = (O == 0 || e < N + M) ? 1.0f : 2.0f;
+        }
+    }
+}
+
 // PIE ("pair in emit"): also compute the next step's HJ pair values per environment after its copies are issued - the
 // placement that wins for few agents (one launch less; the lookups of an 8-agent environment occupy half a block once).
 // For many agents the per-block chain gets long and lsm_pair_kernel behind this kernel is faster (see lsm_capi.cu).
@@ -1837,10 +1911,7 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
                     const double2 pb = R.pos[b];
                     const double dx = pa.x - pb.x, dy = pa.y - pb.y;
                     const double d2 = dx * dx + dy * dy;
-                    const float d2f = fmaxf((float)d2, 1.0e-30f);
-                    float rs;
-                    asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(rs) : "f"(d2f));
-                    const float v = (d2 < r2_lt && d2 > r2_nz) ? d2f * rs : 0.0f;
+                    const float v = adj_value(d2, r2_lt, r2_nz);
                     dthr[a * E + b] = v; dthr[b * E + a] = v;
                 }
             }
@@ -1866,7 +1937,7 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
             for (int k = tid; k < N * W; k += T) {
                 const int w = k % W;
                 const unsigned sel = S.sel[k];
-                S.keepm[k] = ~((S.disc[1][w] & sel) | (S.disc[0][w] & ~sel));
+                S.keepm[k] = keep_word(S.disc[1][w], S.disc[0][w], sel);
             }
             __syncthreads();
         }
@@ -1927,57 +1998,7 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
         const bool gfeat = (kp.c.flags & LSM_FLAG_GRAPH_FEAT_GLOBAL) != 0;
         const int Fr = gfeat ? 7 : F;
         float* nbase = kp.b.node_obs + (size_t)ee * (ROWS * Fr);
-        auto node_row = [&](int r, float* o) {
-            const int i = r / E, e = r - i * E;
-            const double2 pi = R.pos[i], vi = R.vel[N + i];
-            const bool is_agent = e < N;
-            const int sel = (e <= i) ? N : 0;     // agents <= i are seen after their own update
-            const int vidx = is_agent ? sel + e : 2 * N;
-            const int gidx = is_agent ? E + sel + e : e;
-            const int cidx = is_agent ? REC::CA + sel + e : e - N;
-            if (gfeat) {
-                // an agent's goal is its FIRST landmark (optimal_match_index = arange, navigation_graph_safe.py:179), a
-                // landmark's goal is itself; velocities are world-frame (landmarks: zero)
-                const double2 pe = R.pos[e], ve = R.vel[vidx], ge = is_agent ? R.pos[N + e] : pe;
-                o[0] = (float)ve.x; o[1] = (float)ve.y; o[2] = (float)pe.x; o[3] = (float)pe.y;
-                o[4] = (float)ge.x; o[5] = (float)ge.y; o[6] = is_agent ? 0.0f : ((O == 0 || e < N + M) ? 1.0f : 2.0f);
-                (void)gidx; (void)cidx; (void)pi; (void)vi;
-            } else if constexpr (DYN == LSM_DYN_DOUBLE_INTEGRATOR) {
-                // utils.py:201-255: [p_e - p_i, v_e - v_i, goal_e - p_i, sin gh, cos gh, gspeed, type]
-                const double2 pe = R.pos[e], ve = R.vel[vidx], ge = R.pos[gidx];
-                const float4 cc = R.cst[cidx];
-                float2* o2 = reinterpret_cast<float2*>(o);   // rows are 40 B: 8 B aligned
-                o2[0] = make_float2((float)(pe.x - pi.x), (float)(pe.y - pi.y));
-                o2[1] = make_float2((float)(ve.x - vi.x), (float)(ve.y - vi.y));
-                o2[2] = make_float2((float)(ge.x - pi.x), (float)(ge.y - pi.y));
-                o2[3] = make_float2(cc.x, cc.y);
-                o2[4] = make_float2(cc.z, cc.w);
-            } else {
-                const double ci = R.air.cth[i], si = R.air.sth[i];
-                if (e < N) {
-                    const int g = R.air.goal[sel ? 1 : 0][e];
-                    const double2 pe = R.pos[e], ve = R.vel[vidx], ge = R.pos[gidx];
-                    double rx, ry, gx, gy;
-                    rotate_into(pe.x - pi.x, pe.y - pi.y, ci, si, rx, ry);
-                    rotate_into(ge.x - pi.x, ge.y - pi.y, ci, si, gx, gy);
-                    const double ce = R.air.cth[e], se = R.air.sth[e];
-                    o[0] = (float)rx; o[1] = (float)ry; o[2] = (float)norm2(ve.x - vi.x, ve.y - vi.y);
-                    o[3] = (float)(se * ci - ce * si); o[4] = (float)(ce * ci + se * si);
-                    o[5] = (float)gx; o[6] = (float)gy;
-                    o[7] = (float)(R.air.lsin[g] * ci - R.air.lcos[g] * si); o[8] = (float)(R.air.lcos[g] * ci + R.air.lsin[g] * si);
-                    o[9] = (float)R.air.lsp[g]; o[10] = 0.0f;
-                } else {
-                    const int m = e - N;
-                    const double2 pe = R.pos[e];
-                    double rx, ry;
-                    rotate_into(pe.x - pi.x, pe.y - pi.y, ci, si, rx, ry);
-                    const float sh = (float)(R.air.lsin[m] * ci - R.air.lcos[m] * si), ch = (float)(R.air.lcos[m] * ci + R.air.lsin[m] * si);
-                    o[0] = (float)rx; o[1] = (float)ry; o[2] = (float)R.air.spd_post[i];
-                    o[3] = sh; o[4] = ch; o[5] = (float)rx; o[6] = (float)ry; o[7] = sh; o[8] = ch;
-                    o[9] = (float)R.air.lsp[m]; o[10] = (O == 0 || e < N + M) ? 1.0f : 2.0f;
-                }
-            }
-        };
+        auto node_row = [&](int r, float* o) { node_feature_row<DYN, N, L, O>(R, r, gfeat, o); };
         bool adj_sent = false;
         for (int c = 0; c < NCHUNK; ++c) {
             const int r0 = c * CR;
@@ -2038,6 +2059,114 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
     cp_async_wait_all();
     tl_end(kp.timeline, TL_EMIT_END);
 #undef LSM_DBG
+}
+
+// ---------------------------------------------------------------------------------------------
+// lsm_record_emit_kernel: graph emission from stored records (lsm_emit_from_records). One item = (record, observer i):
+// observer i's node rows (E, F) and masked thresholded matrix (E, E), byte for byte what lsm_emit_kernel wrote for that
+// observer, through the same three helpers. A group of WPI warps owns one item at a time (WPI grows with E so that the
+// E * E stores of an item spread over more lanes); a block holds GPB groups, each synchronising on its own named barrier.
+// ---------------------------------------------------------------------------------------------
+template <int DYN, int N, int L, int O>
+struct RecordEmitGeom {
+    using REC = EmitRec<DYN, N, L, O>;
+    static constexpr int E = REC::E, W = REC::W, EE = E * E;
+    static constexpr int F = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 10 : 11;
+    static constexpr int WPI = E <= 32 ? 1 : E < 64 ? 2 : 4;      // warps per item
+    static constexpr int GPB = 8 / WPI;                             // items in flight per 256-thread block
+    static constexpr int THREADS = 32 * WPI * GPB;
+    struct __align__(16) Slot {
+        REC rec;
+        alignas(16) float nodes[E * F];
+        unsigned keep[W];
+    };
+    static constexpr int SMEM = (int)sizeof(Slot) * GPB;
+};
+
+template <int DYN, int N, int L, int O>
+__global__ void __launch_bounds__(RecordEmitGeom<DYN, N, L, O>::THREADS) lsm_record_emit_kernel(const __grid_constant__ RecordEmitArgs a) {
+    using GEO = RecordEmitGeom<DYN, N, L, O>;
+    using REC = EmitRec<DYN, N, L, O>;
+    constexpr int M = REC::M, E = GEO::E, W = GEO::W, EE = GEO::EE, WPI = GEO::WPI, GPB = GEO::GPB;
+    constexpr int TG = 32 * WPI;                      // threads per item
+    constexpr int Q = (int)(sizeof(REC) / 16);
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int g = threadIdx.x / TG, t = threadIdx.x - g * TG, lane = t & 31;
+    typename GEO::Slot& S = reinterpret_cast<typename GEO::Slot*>(smem_raw)[g];
+    auto group_sync = [&]() {
+        if (WPI == 1) __syncwarp();
+        else asm volatile("bar.sync %0, %1;" :: "r"(1 + g), "r"(TG) : "memory");
+    };
+    const int Fr = a.gfeat ? 7 : GEO::F;
+    const int NF = E * Fr;                            // node floats per item
+    for (long long it = (long long)blockIdx.x * GPB + g; it < a.num_items; it += (long long)gridDim.x * GPB) {
+        const long long rec = a.record[it];
+        const int i = a.observer[it];
+        float* const adj = a.adj != nullptr ? a.adj + it * EE : nullptr;
+        float* const nob = a.node_obs != nullptr ? a.node_obs + it * NF : nullptr;
+        if (rec < 0 || rec >= a.num_records || i < 0 || i >= N) {     // invalid item: zero-filled outputs
+            if (adj != nullptr) for (int k = t; k < EE; k += TG) __stcs(adj + k, 0.0f);
+            if (nob != nullptr) for (int k = t; k < NF; k += TG) __stcs(nob + k, 0.0f);
+            continue;
+        }
+        group_sync();                                 // the previous item's readers of S are done
+        {
+            const int4* src = reinterpret_cast<const int4*>(a.records + rec * (long long)sizeof(REC));
+            int4* dst = reinterpret_cast<int4*>(&S.rec);
+            for (int k = t; k < Q; k += TG) cp_async16(dst + k, src + k);
+            cp_async_commit();
+            cp_async_wait_all();
+        }
+        group_sync();
+        const REC& R = S.rec;
+        // observer i's keep masks, as lsm_emit_kernel derives them (no masking at all when nothing is disconnected after
+        // the step)
+        if (t < 32) {
+            unsigned pre[W], post[W], any_disc = 0u;
+#pragma unroll
+            for (int w = 0; w < W; ++w) {
+                const int e = w * 32 + lane;
+                bool dpre = false, dpost = false;
+                if (e < N) { dpre = R.done[0][e] != 0; dpost = R.done[1][e] != 0; }
+                else if (e < N + M) {       // obstacles (e >= N + M) are never disconnected
+                    const int m = e - N, order = m / N, owner = m - order * N;
+                    dpre = R.reached[0][owner] > order; dpost = R.reached[1][owner] > order;
+                }
+                pre[w] = __ballot_sync(0xffffffffu, dpre); post[w] = __ballot_sync(0xffffffffu, dpost);
+                any_disc |= post[w];
+            }
+            if (lane < W) {
+#pragma unroll
+                for (int w = 0; w < W; ++w)
+                    if (w == lane) S.keep[w] = any_disc != 0u ? keep_word(post[w], pre[w], a.sel_tab[i * W + w]) : 0xffffffffu;
+            }
+        }
+        // node rows of observer i, assembled in shared memory
+        if (nob != nullptr)
+            for (int e = t; e < E; e += TG) node_feature_row<DYN, N, L, O>(R, i * E + e, a.gfeat != 0, S.nodes + e * Fr);
+        group_sync();
+        // masked thresholded matrix: every entry from the two positions (the float64 d2 is symmetric bit for bit)
+        if (adj != nullptr) {
+            const double r2_lt = a.r2_lt, r2_nz = a.r2_nz;
+            for (int k = t; k < EE; k += TG) {
+                const int ra = k / E, cb = k - ra * E;
+                const double2 pa = R.pos[ra], pb = R.pos[cb];
+                const double dx = pa.x - pb.x, dy = pa.y - pb.y;
+                const float v = adj_value(dx * dx + dy * dy, r2_lt, r2_nz);
+                const bool keep = ((S.keep[ra >> 5] >> (ra & 31)) & 1u) && ((S.keep[cb >> 5] >> (cb & 31)) & 1u);
+                __stcs(adj + k, keep ? v : 0.0f);
+            }
+        }
+        if (nob != nullptr) {
+            if (NF % 4 == 0) {
+                for (int k = t; k < NF / 4; k += TG) __stcs(reinterpret_cast<float4*>(nob) + k, reinterpret_cast<const float4*>(S.nodes)[k]);
+            } else if (NF % 2 == 0) {
+                for (int k = t; k < NF / 2; k += TG) __stcs(reinterpret_cast<float2*>(nob) + k, reinterpret_cast<const float2*>(S.nodes)[k]);
+            } else {
+                for (int k = t; k < NF; k += TG) __stcs(nob + k, S.nodes[k]);
+            }
+        }
+    }
 }
 
 }  // namespace lsm

@@ -117,6 +117,8 @@ struct SpecFns {
     const void* emit_pie;     // emit kernel that also computes the next step's pair values (placement "emit")
     const void* edge_count;   // per-graph edge counts + range prefix for the fused COO output
     int rec_bytes, scratch_bytes, emit_smem, emit_threads;
+    const void* record_emit;  // lsm_record_emit_kernel (lsm_emit_from_records)
+    int record_emit_smem, record_emit_threads, record_emit_items;   // items in flight per block
 };
 
 #ifdef LSM_EXPERIMENTS
@@ -170,6 +172,10 @@ static bool spec_fns_base(int dynamics, int N, int L, int O, bool f32, SpecFns* 
         f->scratch_bytes = (int)sizeof(AgentScratch<DYN_, N_, L_>);                               \
         f->emit_smem = (int)sizeof(EmitShared<DYN_, N_, L_, O_, WPE_>);                           \
         f->emit_threads = 32 * WPE_;                                                              \
+        f->record_emit = (const void*)lsm_record_emit_kernel<DYN_, N_, L_, O_>;                   \
+        f->record_emit_smem = RecordEmitGeom<DYN_, N_, L_, O_>::SMEM;                             \
+        f->record_emit_threads = RecordEmitGeom<DYN_, N_, L_, O_>::THREADS;                       \
+        f->record_emit_items = RecordEmitGeom<DYN_, N_, L_, O_>::GPB;                             \
         return true;                                                                              \
     }
     LSM_SPEC_LIST(X)
@@ -373,6 +379,24 @@ cudaError_t spec_launch_emit(const KParams& kp, cudaStream_t stream, const void*
 #endif
     if (pie && f.emit_pie == nullptr) return cudaErrorInvalidValue;
     return launch_one(pie ? f.emit_pie : f.emit, kp, grid, f.emit_threads, f.emit_smem, stream, persist_ptr, persist_bytes, true);
+}
+
+cudaError_t spec_launch_record_emit(int dynamics, int N, int L, int O, const RecordEmitArgs& a, cudaStream_t stream) {
+    SpecFns f;
+    if (!spec_fns(dynamics, N, L, O, false, &f)) return cudaErrorInvalidValue;
+    if (a.num_items <= 0) return cudaSuccess;
+    static int sm_count = 0;
+    if (sm_count == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev); }
+    if (f.record_emit_smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(f.record_emit, cudaFuncAttributeMaxDynamicSharedMemorySize, f.record_emit_smem);
+        if (e != cudaSuccess) return e;
+    }
+    // blocks loop over the items: at most as many as 8 blocks of 256 threads per SM (a full SM) hold
+    long long blocks = (a.num_items + f.record_emit_items - 1) / f.record_emit_items;
+    if (blocks > 8LL * sm_count) blocks = 8LL * sm_count;
+    void* args[] = { (void*)&a };
+    return cudaLaunchKernel(f.record_emit, dim3((unsigned)blocks), dim3((unsigned)f.record_emit_threads), args,
+                            (size_t)f.record_emit_smem, stream);
 }
 
 int edge_count_envs_per_block(long long envs) {

@@ -15,18 +15,25 @@ array twice (np.stack in the vec-env, `.copy()` in the buffer).
 With `zero_copy=True` the simulator's kernels write obs / node_obs / adj / rewards straight into the
 buffer's slot for the next step (lsm_set_output_buffers re-binds the output pointers, no copy at all).
 
+With `graph_storage='records'` (requires `zero_copy=True` and the specialised pipeline) the buffer keeps the graph
+observation of every slot as the per-env emit records the step left behind (`records`, 1-7 % of the dense node_obs +
+adj bytes) instead of node_obs / adj: the env writes its dense outputs into ONE scratch pair the acting forward reads,
+and `graph_rows` / `graph_batch` re-emit any (step, env, agent) row on the GPU, bit for bit what the dense buffer holds
+(lsm_copy_records / lsm_emit_from_records). The other fields, share_obs included, are stored as in the dense mode.
+
 torch is used for storage and for the few elementwise mask operations; the learner (policy, GAE
 consumers, minibatch generators) is out of scope.
 """
 from __future__ import annotations
 
+import numpy as np
 import torch
 
 
 class DeviceGraphRolloutBuffer:
     def __init__(self, env, episode_length: int, use_centralized_V: bool = True, gamma: float = 0.99,
                  gae_lambda: float = 0.95, use_gae: bool = True, use_proper_time_limits: bool = False,
-                 recurrent_N: int = 1, hidden_size: int = 64, zero_copy: bool = False):
+                 recurrent_N: int = 1, hidden_size: int = 64, zero_copy: bool = False, graph_storage: str = 'dense'):
         self.env = env
         self.episode_length = T = int(episode_length)
         self.n_rollout_threads = n = env.num_envs
@@ -36,14 +43,30 @@ class DeviceGraphRolloutBuffer:
         self._use_gae, self._use_proper_time_limits = bool(use_gae), bool(use_proper_time_limits)
         self.recurrent_N, self.hidden_size = int(recurrent_N), int(hidden_size)
         self.zero_copy = bool(zero_copy)
+        if graph_storage not in ('dense', 'records'):
+            raise ValueError(f"graph_storage must be 'dense' or 'records', got {graph_storage!r}")
+        self.graph_storage = graph_storage
         dev, f32 = env.device, torch.float32
         E, D, F = env.E, env.D, env.F
         so = D * N if self.use_centralized_V else D
         sa = N if self.use_centralized_V else 1
         self.share_obs = torch.zeros((T + 1, n, N, so), dtype=f32, device=dev)
         self.obs = torch.zeros((T + 1, n, N, D), dtype=f32, device=dev)
-        self.node_obs = torch.zeros((T + 1, n, N, E, F), dtype=f32, device=dev)
-        self.adj = torch.zeros((T + 1, n, N, E, E), dtype=f32, device=dev)
+        if graph_storage == 'records':
+            if not self.zero_copy:
+                raise ValueError("graph_storage='records' needs zero_copy=True: the records are those of the env's own step")
+            R = env.record_bytes()
+            if R == 0:
+                raise ValueError("graph_storage='records' needs the specialised pipeline, and this shape runs the generic "
+                                 "kernel (set args.specialise_shape to build a library for it)")
+            self.records = torch.zeros((T + 1, n, R), dtype=torch.uint8, device=dev)
+            self.node_obs = self.adj = None
+            # the dense outputs of the current step only (what the acting forward reads)
+            self._graph_scratch = (torch.zeros((n, N, E, F), dtype=f32, device=dev), torch.zeros((n, N, E, E), dtype=f32, device=dev))
+        else:
+            self.records = None
+            self.node_obs = torch.zeros((T + 1, n, N, E, F), dtype=f32, device=dev)
+            self.adj = torch.zeros((T + 1, n, N, E, E), dtype=f32, device=dev)
         self.agent_id = torch.zeros((T + 1, n, N, 1), dtype=torch.int32, device=dev)
         self.share_agent_id = torch.zeros((T + 1, n, N, sa), dtype=torch.int32, device=dev)
         self.rnn_states = torch.zeros((T + 1, n, N, self.recurrent_N, self.hidden_size), dtype=f32, device=dev)
@@ -83,7 +106,8 @@ class DeviceGraphRolloutBuffer:
         if not self.zero_copy:
             return
         s = self.step
-        self.env.set_output_buffers(obs=self.obs[s + 1], node_obs=self.node_obs[s + 1], adj=self.adj[s + 1],
+        node_obs, adj = self._graph_scratch if self.records is not None else (self.node_obs[s + 1], self.adj[s + 1])
+        self.env.set_output_buffers(obs=self.obs[s + 1], node_obs=node_obs, adj=adj,
                                     reward=self.rewards[s].view(self.n_rollout_threads, self.num_agents),
                                     done=self._done_u8)
         self._bound_slot = s
@@ -91,8 +115,11 @@ class DeviceGraphRolloutBuffer:
     def warmup(self, reset_out=None, num_current_episode: int = 0):
         """GMPERunner.warmup (graph_mpe_runner.py:253-300): reset the envs, fill slot 0."""
         if self.zero_copy:
-            self.env.set_output_buffers(obs=self.obs[0], node_obs=self.node_obs[0], adj=self.adj[0])
+            node_obs, adj = self._graph_scratch if self.records is not None else (self.node_obs[0], self.adj[0])
+            self.env.set_output_buffers(obs=self.obs[0], node_obs=node_obs, adj=adj)
             reset_out = self.env.reset(num_current_episode)
+            if self.records is not None:
+                self.env.copy_records(self.records[0])
         elif reset_out is None:
             reset_out = self.env.reset(num_current_episode)
         obs, agent_id, node_obs, adj = reset_out[:4]
@@ -129,6 +156,11 @@ class DeviceGraphRolloutBuffer:
                                                   C.c_void_p(self.active_masks[s + 1].data_ptr()), env._stream()), 'lsm_rollout_insert', env.lib)
             if not self.use_centralized_V:
                 self.share_obs[s + 1].copy_(self.obs[s + 1])
+            if self.records is not None:
+                env.copy_records(self.records[s + 1])
+        elif self.records is not None:
+            raise RuntimeError("graph_storage='records' stores the env's own step: insert the output of the step that "
+                               "followed warmup / the previous insert")
         else:
             dones_env = dones.all(dim=1)                                   # np.all(dones, axis=1)
             masks = (~dones).to(torch.float32).unsqueeze(-1)               # masks[dones] = 0
@@ -151,10 +183,11 @@ class DeviceGraphRolloutBuffer:
 
     def after_update(self):
         """Copy the last time step to index 0 (graph_buffer.py:253-283)."""
-        for name in ('share_obs', 'obs', 'node_obs', 'adj', 'agent_id', 'share_agent_id', 'rnn_states',
+        for name in ('share_obs', 'obs', 'node_obs', 'adj', 'records', 'agent_id', 'share_agent_id', 'rnn_states',
                      'rnn_states_critic', 'masks', 'bad_masks', 'active_masks', 'available_actions'):
             t = getattr(self, name)
-            t[0].copy_(t[-1])
+            if t is not None:
+                t[0].copy_(t[-1])
         self.bind_next_slot()
 
     def compute_returns(self, next_value):
@@ -177,6 +210,61 @@ class DeviceGraphRolloutBuffer:
                 if self._use_proper_time_limits:
                     r = r * self.bad_masks[step + 1] + (1 - self.bad_masks[step + 1]) * self.value_preds[step]
                 self.returns[step] = r
+
+    def graph_rows(self, t, env, agent, node_obs=None, adj=None):
+        """Graph observation rows (node_obs[t, env, agent], adj[t, env, agent]) for B index triples, t in [0, T]:
+        -> ((B, E, F), (B, E, E)). Dense storage gathers them; records storage re-emits them on the GPU. Host (CPU tensor
+        or numpy) indices out of range raise IndexError; out-of-range CUDA indices give zero rows in records storage."""
+        T1, n = self.episode_length + 1, self.n_rollout_threads
+        dev = self.env.device
+        on_dev = all(torch.is_tensor(x) and x.is_cuda for x in (t, env, agent))
+        if not on_dev:
+            t, env, agent = (torch.as_tensor(np.asarray(x)).reshape(-1).to(torch.int64) for x in (t, env, agent))
+            for x, bound, name in ((t, T1, 't'), (env, n, 'env'), (agent, self.num_agents, 'agent')):
+                if x.numel() and (int(x.min()) < 0 or int(x.max()) >= bound):
+                    raise IndexError(f"{name} out of range [0, {bound})")
+            t, env, agent = t.to(dev), env.to(dev), agent.to(dev)
+        t, env, agent = (x.reshape(-1).to(torch.int64) for x in (t, env, agent))
+        if self.records is None:
+            no, ad = self.node_obs[t, env, agent], self.adj[t, env, agent]
+            if node_obs is not None:
+                node_obs.copy_(no); no = node_obs
+            if adj is not None:
+                adj.copy_(ad); ad = adj
+            return no, ad
+        # an env index out of range must not alias another env's record: it becomes an invalid record
+        ok = (t >= 0) & (t < T1) & (env >= 0) & (env < n)
+        record = torch.where(ok, t * n + env, torch.full_like(t, -1))
+        return self.env.emit_from_records(self.records, record, agent, node_obs, adj)
+
+    def graph_batch(self, rows, node_obs=None, adj=None):
+        """Rows of the (T, n, N) flattening a minibatch generator indexes: equal to
+        (node_obs[:-1].reshape(-1, E, F)[rows], adj[:-1].reshape(-1, E, E)[rows]) of the dense storage."""
+        T, n, N = self.episode_length, self.n_rollout_threads, self.num_agents
+        if not (torch.is_tensor(rows) and rows.is_cuda):
+            rows = torch.as_tensor(np.asarray(rows)).reshape(-1).to(torch.int64)
+            if rows.numel() and (int(rows.min()) < 0 or int(rows.max()) >= T * n * N):
+                raise IndexError(f"row out of range [0, {T * n * N})")
+            rows = rows.to(self.env.device)
+        rows = rows.reshape(-1).to(torch.int64)
+        if self.records is None:
+            E = self.env.E
+            no = self.node_obs[:-1].reshape(-1, E, self.node_obs.shape[-1])[rows]
+            ad = self.adj[:-1].reshape(-1, E, E)[rows]
+            if node_obs is not None:
+                node_obs.copy_(no); no = node_obs
+            if adj is not None:
+                adj.copy_(ad); ad = adj
+            return no, ad
+        # row r is record r // N of the first T slots (an out-of-range row: a record index outside them), observer r % N
+        return self.env.emit_from_records(self.records[:-1], torch.div(rows, N, rounding_mode='floor'), rows % N, node_obs, adj)
+
+    def graph_nbytes(self) -> int:
+        """Bytes of graph-observation storage: node_obs + adj (dense), or the records plus the one-step dense scratch
+        pair (records). Every other field (share_obs, the largest of them) is the same in both modes."""
+        if self.records is None:
+            return self.node_obs.nbytes + self.adj.nbytes
+        return self.records.nbytes + sum(x.nbytes for x in self._graph_scratch)
 
     def runner_view(self):
         """Adapter for an UNMODIFIED `GMPERunner.collect` (graph_mpe_runner.py:398-415), which evaluates
@@ -231,6 +319,19 @@ class _FieldView:
         return _ConcatSlot(self._t[step])
 
 
+class _ScratchFieldView:
+    """node_obs / adj of a records-storage buffer: only the current step is held densely."""
+
+    def __init__(self, buf, k):
+        self._buf, self._k = buf, k
+
+    def __getitem__(self, step):
+        if step != self._buf.step:
+            raise IndexError(f"graph_storage='records' holds node_obs / adj densely for the current step ({self._buf.step}) "
+                             f"only, not step {step}: use graph_rows / graph_batch")
+        return _ConcatSlot(self._buf._graph_scratch[self._k])
+
+
 class _RunnerView:
     _FIELDS = ('share_obs', 'obs', 'node_obs', 'adj', 'agent_id', 'share_agent_id', 'rnn_states', 'rnn_states_critic', 'masks',
                'available_actions', 'active_masks')
@@ -239,6 +340,8 @@ class _RunnerView:
         self._buf = buf
 
     def __getattr__(self, name):
+        if name in ('node_obs', 'adj') and self._buf.records is not None:
+            return _ScratchFieldView(self._buf, 0 if name == 'node_obs' else 1)
         if name in _RunnerView._FIELDS:
             return _FieldView(getattr(self._buf, name))
         return getattr(self._buf, name)

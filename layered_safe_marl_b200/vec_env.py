@@ -424,6 +424,57 @@ class B200GraphVecEnv:
         """Relaunch the graph-emission kernel alone (measurement hook; rewrites node_obs / adj with the same values)."""
         self._check(self.lib.lsm_emit_only(self._h, self._stream()), 'lsm_emit_only')
 
+    def record_bytes(self) -> int:
+        """emit_record_bytes of the handle (0 on the generic kernel); asked once, it is fixed per handle."""
+        if getattr(self, '_rec_bytes', None) is None:
+            self._rec_bytes = self.launch_info()['emit_record_bytes']
+        return self._rec_bytes
+
+    def copy_records(self, dst):
+        """Copy the emit records of the last step / reset / observe into `dst`, a contiguous uint8 CUDA tensor of
+        num_envs * emit_record_bytes bytes (lsm_copy_records; specialised pipeline only)."""
+        assert dst.is_cuda and dst.dtype == torch.uint8 and dst.is_contiguous() and dst.numel() == self.n * self.record_bytes(), \
+            "dst: contiguous uint8 CUDA tensor of the records' size"
+        self._check(self.lib.lsm_copy_records(self._h, C.c_void_p(dst.data_ptr()), self._stream()), 'lsm_copy_records')
+
+    def emit_from_records(self, records, record, observer, node_obs=None, adj=None):
+        """Re-emit graph observations from stored records (lsm_emit_from_records) on torch's current stream.
+
+        records: uint8 CUDA tensor whose last dimension is emit_record_bytes (copy_records output, any leading shape);
+        record / observer: B indices into the flattened records and the observing agent. CPU tensors or numpy arrays
+        are range-checked here (IndexError); CUDA tensors go to the kernel unchecked, which zero-fills invalid items.
+        -> (node_obs (B, E, F), adj (B, E, E)), written into the given tensors or into new ones."""
+        R = self.record_bytes()
+        if R == 0:
+            raise RuntimeError("emit_from_records needs the specialised pipeline (this handle runs the generic kernel)")
+        assert records.is_cuda and records.dtype == torch.uint8 and records.is_contiguous() and records.shape[-1] == R, \
+            f"records: contiguous uint8 CUDA tensor with a last dimension of {R} bytes"
+        num_records = records.numel() // R
+        record, observer = self._item_index(record, num_records, torch.int64), self._item_index(observer, self.N, torch.int32)
+        if record.shape != observer.shape:
+            raise ValueError(f"record and observer must have the same shape, got {tuple(record.shape)} and {tuple(observer.shape)}")
+        B, E = record.numel(), self.E
+        if node_obs is None:
+            node_obs = torch.empty((B, E, self.F), dtype=torch.float32, device=self.device)
+        if adj is None:
+            adj = torch.empty((B, E, E), dtype=torch.float32, device=self.device)
+        for t, shape, name in ((node_obs, (B, E, self.F), 'node_obs'), (adj, (B, E, E), 'adj')):
+            assert t.is_cuda and t.dtype == torch.float32 and t.is_contiguous() and tuple(t.shape) == shape, \
+                f"{name}: need a contiguous float32 CUDA tensor of shape {shape}"
+        io = _lib.LsmRecordEmitIo(B, num_records, records.data_ptr(), record.data_ptr(), observer.data_ptr(),
+                                  node_obs.data_ptr(), adj.data_ptr())
+        self._check(self.lib.lsm_emit_from_records(self._h, C.byref(io), self._stream()), 'lsm_emit_from_records')
+        return node_obs, adj
+
+    def _item_index(self, idx, bound: int, dtype):
+        """Index tensor for the kernel: host indices are checked against [0, bound); device indices are not."""
+        if torch.is_tensor(idx) and idx.is_cuda:
+            return idx.reshape(-1).to(dtype).contiguous()
+        idx = torch.as_tensor(np.asarray(idx)).reshape(-1).to(torch.int64)
+        if idx.numel() and (int(idx.min()) < 0 or int(idx.max()) >= bound):
+            raise IndexError(f"index out of range [0, {bound})")
+        return idx.to(device=self.device, dtype=dtype)
+
     def debug_timeline(self, arm: bool = True):
         """Diagnostics: read the per-kernel %globaltimer timeline of the launches since the last arm (dict of ns relative
         to the first kernel's start, or None when nothing was armed), then re-arm / disarm."""
