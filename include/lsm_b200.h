@@ -29,6 +29,8 @@
  *   lsm_safety_filter  both safety handles' apply_safety_filter for caller-owned states
  *                                                          multiagent/safety_filter.py:203-260, 378-433
  *   lsm_hj_lookup      get_value_of_relative_state + gradient  multiagent/safety_filter.py:192-201, 345-354
+ *   lsm_edges_from_records  TransformerConvNet.process_adj on a learner minibatch of stored rollout rows, straight from
+ *                      the stored emit records (no dense adjacency)  onpolicy/algorithms/utils/gnn.py:376-407
  */
 #ifndef LSM_B200_H
 #define LSM_B200_H
@@ -377,6 +379,31 @@ typedef struct lsm_record_emit_io {
     float *adj;                 /* DEVICE [B][E][E] out, 16-byte aligned, or NULL */
 } lsm_record_emit_io;
 int lsm_emit_from_records(lsm_handle *h, const lsm_record_emit_io *io, void *stream);
+
+/* lsm_edges_from_records: the COO edge list of the matrices lsm_emit_from_records would write for the same items, in the
+ * order and layout of the reference's TransformerConvNet.process_adj (gnn.py:376-407) over the (B, E, E) batch: item k's
+ * non-zero entries in row-major order, edge_index row 0 = k * E + row, row 1 = k * E + col, edge_attr = the matrix entry
+ * bit for bit. No dense matrix is written or read. Two passes over the same items:
+ *   edge_index == NULL  counting pass: writes counts and offsets (exclusive prefix, offsets[B] = nnz on the device).
+ *                       Zero items: only offsets[0] = 0.
+ *   otherwise           fill pass: reads the offsets of a counting pass and writes only positions in [0, capacity), so a
+ *                       short capacity or a stale offsets array never writes out of bounds. Zero items: nothing.
+ * Items with an out-of-range record or observer have no edges. Uses the handle's shape and coordination_range, needs no
+ * bound buffers, keeps no per-handle scratch, launches on `stream` and never synchronises (two streams may use one
+ * handle at once). Returns 6 on a generic-kernel handle, 2 on negative sizes, missing arrays or misaligned records. */
+typedef struct lsm_record_edges_io {
+    int64_t num_items;          /* B >= 0 */
+    int64_t num_records;        /* records in the store */
+    const void *records;        /* as lsm_record_emit_io */
+    const int64_t *record;      /* DEVICE [B] */
+    const int32_t *observer;    /* DEVICE [B] */
+    int32_t *counts;            /* DEVICE [B]   edges per item (counting pass) */
+    int64_t *offsets;           /* DEVICE [B+1] offsets[B] = nnz (written by the counting pass, read by the fill pass) */
+    int64_t *edge_index;        /* DEVICE [2][capacity], or NULL (counting pass) */
+    float *edge_attr;           /* DEVICE [capacity] */
+    int64_t capacity;
+} lsm_record_edges_io;
+int lsm_edges_from_records(lsm_handle *h, const lsm_record_edges_io *io, void *stream);
 
 /* Diagnostics (never on the product path): per-kernel timeline of the launches that follow. If `out_ns` is non-NULL
  * and a timeline is armed, synchronises the device and copies 7 %globaltimer values (ns) out: pair first-block-in,

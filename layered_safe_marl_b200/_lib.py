@@ -81,13 +81,19 @@ class LsmRecordEmitIo(C.Structure):
                 ('observer', C.c_void_p), ('node_obs', C.c_void_p), ('adj', C.c_void_p)]
 
 
+class LsmRecordEdgesIo(C.Structure):
+    _fields_ = [('num_items', C.c_int64), ('num_records', C.c_int64), ('records', C.c_void_p), ('record', C.c_void_p),
+                ('observer', C.c_void_p), ('counts', C.c_void_p), ('offsets', C.c_void_p), ('edge_index', C.c_void_p),
+                ('edge_attr', C.c_void_p), ('capacity', C.c_int64)]
+
+
 EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_destroy', 'lsm_set_value_grid',
                     'lsm_set_ttr_grid', 'lsm_bind_buffers', 'lsm_get_launch_info', 'lsm_step', 'lsm_reset',
                     'lsm_observe', 'lsm_emit_only', 'lsm_invalidate', 'lsm_set_output_buffers', 'lsm_edge_list',
                     'lsm_debug_timeline', 'lsm_rollout_insert', 'lsm_math_eval', 'lsm_math_eval_device', 'lsm_set_tuning',
                     'lsm_set_compact_adjacency', 'lsm_expand_adjacency_host', 'lsm_set_edge_output', 'lsm_world_graph', 'lsm_fetch_host', 'lsm_step_host',
                     'lsm_episode_stats', 'lsm_debug_pair_values', 'lsm_safety_filter', 'lsm_hj_lookup',
-                    'lsm_copy_records', 'lsm_emit_from_records')
+                    'lsm_copy_records', 'lsm_emit_from_records', 'lsm_edges_from_records')
 
 _libs = {}          # one CDLL per path: the product library and the per-shape libraries (_build.build_shape)
 
@@ -144,6 +150,7 @@ def load(path: Optional[str] = None):
     lib.lsm_hj_lookup.argtypes = [C.c_void_p, C.POINTER(LsmLookupIo), C.c_void_p]
     lib.lsm_copy_records.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     lib.lsm_emit_from_records.argtypes = [C.c_void_p, C.POINTER(LsmRecordEmitIo), C.c_void_p]
+    lib.lsm_edges_from_records.argtypes = [C.c_void_p, C.POINTER(LsmRecordEdgesIo), C.c_void_p]
     lib.lsm_math_eval.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
     lib.lsm_math_eval_device.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
     for name in EXPORTED_SYMBOLS:

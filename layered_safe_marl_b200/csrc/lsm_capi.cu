@@ -1193,6 +1193,33 @@ int lsm_emit_from_records(lsm_handle* h, const lsm_record_emit_io* io, void* str
     return 0;
 }
 
+int lsm_edges_from_records(lsm_handle* h, const lsm_record_edges_io* io, void* stream) {
+    if (h == nullptr || io == nullptr) return fail(1, "lsm_edges_from_records: null argument");
+    if (!h->spec) return fail(6, "lsm_edges_from_records: this configuration runs the fused generic kernel (no emit records)");
+    if (io->num_items < 0 || io->num_records < 0 || io->capacity < 0)
+        return fail(2, "lsm_edges_from_records: num_items, num_records and capacity must be >= 0");
+    const bool fill = io->edge_index != nullptr;
+    if (io->offsets == nullptr) return fail(2, "lsm_edges_from_records: offsets is required");
+    if (io->num_items > 0) {
+        if (fill ? io->edge_attr == nullptr : io->counts == nullptr)
+            return fail(2, "lsm_edges_from_records: the count pass needs counts, the fill pass edge_attr");
+        if (io->record == nullptr || io->observer == nullptr) return fail(2, "lsm_edges_from_records: record and observer are required");
+        if (io->num_records > 0 && io->records == nullptr) return fail(2, "lsm_edges_from_records: null record store");
+        if ((uintptr_t)io->records & 15u) return fail(2, "lsm_edges_from_records: records must be 16-byte aligned");
+    }
+    DeviceGuard guard(h->device);
+    lsm::RecordEdgesArgs a;
+    a.num_items = io->num_items; a.num_records = io->num_records;
+    a.records = (const unsigned char*)io->records; a.record = (const long long*)io->record; a.observer = io->observer;
+    a.counts = io->counts; a.offsets = (const long long*)io->offsets;
+    a.edge_index = (long long*)io->edge_index; a.edge_attr = io->edge_attr; a.capacity = io->capacity;
+    a.sel_tab = h->kp.sel_tab; a.r2_lt = h->kp.r2_lt; a.r2_nz = h->kp.r2_nz;
+    const cudaError_t e = lsm::spec_launch_record_edges(h->kp.c.dynamics, h->kp.N, h->kp.L, h->kp.O, a, (long long*)io->offsets,
+                                                        fill, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "lsm_edges_from_records");
+    return 0;
+}
+
 int lsm_debug_pair_values(lsm_handle* h, double* out, void* stream) {
     if (h == nullptr) return fail(1, "lsm_debug_pair_values: null handle");
     if (!h->have_buffers) return fail(5, "lsm_debug_pair_values: lsm_bind_buffers has not been called");

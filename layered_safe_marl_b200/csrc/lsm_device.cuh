@@ -142,6 +142,21 @@ struct RecordEmitArgs {
     int gfeat;                      // LSM_FLAG_GRAPH_FEAT_GLOBAL
 };
 
+// lsm_edges_from_records: the COO edge list of the same items' matrices (count pass, then fill pass)
+struct RecordEdgesArgs {
+    long long num_items, num_records;
+    const unsigned char* records;   // [num_records][sizeof(EmitRec)], 16-byte aligned
+    const long long* record;        // [num_items]
+    const int* observer;            // [num_items]
+    int32_t* counts;                // count pass: [num_items] out
+    const long long* offsets;       // fill pass: [num_items + 1], the count pass's prefix
+    long long* edge_index;          // fill pass: [2][capacity]
+    float* edge_attr;               // fill pass: [capacity]
+    long long capacity;
+    const uint32_t* sel_tab;        // KParams::sel_tab
+    double r2_lt, r2_nz;            // KParams::r2_lt / r2_nz
+};
+
 // timeline slots: first block in / last block out of each kernel of the pipeline (ns, %globaltimer)
 enum { TL_PAIR_START = 0, TL_PAIR_BODY_END, TL_AGENT_START, TL_AGENT_END, TL_EMIT_START, TL_EMIT_END, TL_PAIR_END, TL_COUNT };
 __device__ __forceinline__ unsigned long long globaltimer_ns() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }

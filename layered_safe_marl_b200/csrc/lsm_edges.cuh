@@ -7,7 +7,7 @@
 //     edge_attr  = adj[graph, row, col]                  (nnz, 1) float32
 // with B = num_envs * N graphs (the runner concatenates the agent axis into the batch, graph_mpe_runner.py:398-410).
 //
-// Two ways to get it. (1) lsm_set_edge_output: the step pipeline itself writes the list (lsm_edge_count_kernel<DYN,N,L>
+// Three ways to get it. (1) lsm_set_edge_output: the step pipeline itself writes the list (lsm_edge_count_kernel<DYN,N,L>
 // below + the edge section of lsm_emit_kernel), the dense adjacency becomes optional and nothing is read back.
 // (2) lsm_edge_list: a post-pass over ANY dense adjacency tensor (a rollout-buffer slot, a user tensor) -
 // three launches, all HBM / L2 streaming integer work (no tensor cores):
@@ -16,6 +16,9 @@
 //   lsm_edge_fill_kernel    one warp per graph: row-major walk in chunks of 32 entries, ballot + prefix popcount
 //                           compaction, writes starting at offsets[g]
 // The dense matrices are read twice; they were just written by the emit kernel and mostly sit in the 126 MB L2.
+// (3) lsm_edges_from_records: the list of (stored record, observer) items of a rollout store - a learner minibatch -
+// computed from the records like (1), with no dense matrix (lsm_record_emit_kernel_edge_count / _edge_fill in
+// lsm_kernel_spec.cuh, lsm_edge_scan_kernel between them).
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>

@@ -23,6 +23,10 @@ cudaError_t spec_launch_emit(const KParams& kp, cudaStream_t stream, const void*
 cudaError_t spec_emit_blocks_per_sm(int dynamics, int N, int L, int O, bool f32, bool reserve_pair, bool pie, int* out, int* regs);
 // lsm_record_emit_kernel of the shape (a shape without a specialisation: cudaErrorInvalidValue); no-op for zero items
 cudaError_t spec_launch_record_emit(int dynamics, int N, int L, int O, const RecordEmitArgs& a, cudaStream_t stream);
+// lsm_record_emit_kernel_edge_count + lsm_edge_scan_kernel into `offsets` (fill == false), or
+// lsm_record_emit_kernel_edge_fill (fill == true); zero items: the count pass only sets offsets[0] = 0
+cudaError_t spec_launch_record_edges(int dynamics, int N, int L, int O, const RecordEdgesArgs& a, long long* offsets, bool fill,
+                                     cudaStream_t stream);
 int edge_count_envs_per_block(long long envs);
 cudaError_t spec_launch_edge_count(const KParams& kp, cudaStream_t stream);
 cudaError_t world_graph_launch(const KParams& kp, int32_t* counts, long long* offsets, long long* edge_index, double* edge_weight,

@@ -1706,6 +1706,7 @@ __device__ __noinline__ void emit_edges(EmitShared<DYN, N, L, O, WPE>& S, const 
 // observer of one stored record), so that both write the same bytes
 // ---------------------------------------------------------------------------------------------
 // float32 adjacency entry of an entity pair at squared distance d2: non-zero strictly inside the radius and above r2_nz
+// (the non-zero value is at least ~1e-15: d2f >= 1e-30, so "adj_value != 0" is exactly that float64 test)
 __device__ __forceinline__ float adj_value(double d2, double r2_lt, double r2_nz) {
     const float d2f = fmaxf((float)d2, 1.0e-30f);
     float rs;
@@ -2067,6 +2068,45 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
 // observer, through the same three helpers. A group of WPI warps owns one item at a time (WPI grows with E so that the
 // E * E stores of an item spread over more lanes); a block holds GPB groups, each synchronising on its own named barrier.
 // ---------------------------------------------------------------------------------------------
+// observer i's keep masks of a stored record, as lsm_emit_kernel derives them (no masking at all when nothing is
+// disconnected after the step). Called by one whole warp; lanes < W write keep[lane].
+template <int DYN, int N, int L, int O>
+__device__ __forceinline__ void record_keep_words(const EmitRec<DYN, N, L, O>& R, const uint32_t* sel_tab, int i, int lane,
+                                                  unsigned* keep) {
+    using REC = EmitRec<DYN, N, L, O>;
+    constexpr int M = REC::M, W = REC::W;
+    unsigned pre[W], post[W], any_disc = 0u;
+#pragma unroll
+    for (int w = 0; w < W; ++w) {
+        const int e = w * 32 + lane;
+        bool dpre = false, dpost = false;
+        if (e < N) { dpre = R.done[0][e] != 0; dpost = R.done[1][e] != 0; }
+        else if (e < N + M) {       // obstacles (e >= N + M) are never disconnected
+            const int m = e - N, order = m / N, owner = m - order * N;
+            dpre = R.reached[0][owner] > order; dpost = R.reached[1][owner] > order;
+        }
+        pre[w] = __ballot_sync(0xffffffffu, dpre); post[w] = __ballot_sync(0xffffffffu, dpost);
+        any_disc |= post[w];
+    }
+    if (lane < W) {
+#pragma unroll
+        for (int w = 0; w < W; ++w)
+            if (w == lane) keep[w] = any_disc != 0u ? keep_word(post[w], pre[w], sel_tab[i * W + w]) : 0xffffffffu;
+    }
+}
+
+// copy stored record `rec` into shared memory with cp.async: thread t of the TG threads of an item group; returns when
+// this thread's copies have landed (the caller synchronises the group)
+template <typename REC, int TG>
+__device__ __forceinline__ void stage_record(REC& S, const unsigned char* records, long long rec, int t) {
+    constexpr int Q = (int)(sizeof(REC) / 16);
+    const int4* src = reinterpret_cast<const int4*>(records + rec * (long long)sizeof(REC));
+    int4* dst = reinterpret_cast<int4*>(&S);
+    for (int k = t; k < Q; k += TG) cp_async16(dst + k, src + k);
+    cp_async_commit();
+    cp_async_wait_all();
+}
+
 template <int DYN, int N, int L, int O>
 struct RecordEmitGeom {
     using REC = EmitRec<DYN, N, L, O>;
@@ -2087,9 +2127,8 @@ template <int DYN, int N, int L, int O>
 __global__ void __launch_bounds__(RecordEmitGeom<DYN, N, L, O>::THREADS) lsm_record_emit_kernel(const __grid_constant__ RecordEmitArgs a) {
     using GEO = RecordEmitGeom<DYN, N, L, O>;
     using REC = EmitRec<DYN, N, L, O>;
-    constexpr int M = REC::M, E = GEO::E, W = GEO::W, EE = GEO::EE, WPI = GEO::WPI, GPB = GEO::GPB;
+    constexpr int E = GEO::E, EE = GEO::EE, WPI = GEO::WPI, GPB = GEO::GPB;
     constexpr int TG = 32 * WPI;                      // threads per item
-    constexpr int Q = (int)(sizeof(REC) / 16);
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int g = threadIdx.x / TG, t = threadIdx.x - g * TG, lane = t & 31;
     typename GEO::Slot& S = reinterpret_cast<typename GEO::Slot*>(smem_raw)[g];
@@ -2110,37 +2149,10 @@ __global__ void __launch_bounds__(RecordEmitGeom<DYN, N, L, O>::THREADS) lsm_rec
             continue;
         }
         group_sync();                                 // the previous item's readers of S are done
-        {
-            const int4* src = reinterpret_cast<const int4*>(a.records + rec * (long long)sizeof(REC));
-            int4* dst = reinterpret_cast<int4*>(&S.rec);
-            for (int k = t; k < Q; k += TG) cp_async16(dst + k, src + k);
-            cp_async_commit();
-            cp_async_wait_all();
-        }
+        stage_record<REC, TG>(S.rec, a.records, rec, t);
         group_sync();
         const REC& R = S.rec;
-        // observer i's keep masks, as lsm_emit_kernel derives them (no masking at all when nothing is disconnected after
-        // the step)
-        if (t < 32) {
-            unsigned pre[W], post[W], any_disc = 0u;
-#pragma unroll
-            for (int w = 0; w < W; ++w) {
-                const int e = w * 32 + lane;
-                bool dpre = false, dpost = false;
-                if (e < N) { dpre = R.done[0][e] != 0; dpost = R.done[1][e] != 0; }
-                else if (e < N + M) {       // obstacles (e >= N + M) are never disconnected
-                    const int m = e - N, order = m / N, owner = m - order * N;
-                    dpre = R.reached[0][owner] > order; dpost = R.reached[1][owner] > order;
-                }
-                pre[w] = __ballot_sync(0xffffffffu, dpre); post[w] = __ballot_sync(0xffffffffu, dpost);
-                any_disc |= post[w];
-            }
-            if (lane < W) {
-#pragma unroll
-                for (int w = 0; w < W; ++w)
-                    if (w == lane) S.keep[w] = any_disc != 0u ? keep_word(post[w], pre[w], a.sel_tab[i * W + w]) : 0xffffffffu;
-            }
-        }
+        if (t < 32) record_keep_words<DYN, N, L, O>(R, a.sel_tab, i, lane, S.keep);
         // node rows of observer i, assembled in shared memory
         if (nob != nullptr)
             for (int e = t; e < E; e += TG) node_feature_row<DYN, N, L, O>(R, i * E + e, a.gfeat != 0, S.nodes + e * Fr);
@@ -2167,6 +2179,148 @@ __global__ void __launch_bounds__(RecordEmitGeom<DYN, N, L, O>::THREADS) lsm_rec
             }
         }
     }
+}
+
+// ---------------------------------------------------------------------------------------------
+// lsm_record_emit_kernel_edge_count / lsm_record_emit_kernel_edge_fill (lsm_edges_from_records): the COO edge list of
+// the matrices lsm_record_emit_kernel writes for the same items, in the order of the reference's process_adj, without
+// the dense matrices. Item k's edges are the non-zero entries of its masked matrix in row-major order, at node indices
+// k * E + row and k * E + col. The count kernel writes counts[k], lsm_edge_scan_kernel turns the counts into offsets,
+// and the fill kernel ranks each row's entries with a ballot and popcounts and writes them from offsets[k]. Same item
+// groups as lsm_record_emit_kernel, same record staging and keep masks; the pattern is "adj_value != 0" and the value
+// adj_value, so the edges are exactly the dense matrix's non-zeros and an edge_attr entry is bit for bit its entry.
+// ---------------------------------------------------------------------------------------------
+template <int DYN, int N, int L, int O>
+struct RecordEdgesGeom {
+    using REC = EmitRec<DYN, N, L, O>;
+    static constexpr int E = REC::E, W = REC::W;
+    static constexpr int WPI = RecordEmitGeom<DYN, N, L, O>::WPI;     // warps per item
+    static constexpr int GPB = 8 / WPI;                                 // items in flight per 256-thread block
+    static constexpr int THREADS = 32 * WPI * GPB;
+    struct __align__(16) Slot {
+        REC rec;
+        unsigned keep[W];
+        unsigned rowmask[E * W];    // fill: kept non-zero entries of every row
+        int rowoff[E];              // fill: exclusive prefix of the row counts; count: the per-warp totals
+    };
+    static constexpr int SMEM = (int)sizeof(Slot) * GPB;
+};
+
+template <int DYN, int N, int L, int O, bool FILL>
+__device__ __forceinline__ void record_edges_items(const RecordEdgesArgs& a) {
+    using GEO = RecordEdgesGeom<DYN, N, L, O>;
+    using REC = EmitRec<DYN, N, L, O>;
+    constexpr int E = GEO::E, W = GEO::W, WPI = GEO::WPI, GPB = GEO::GPB;
+    constexpr int TG = 32 * WPI;                      // threads per item
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int g = threadIdx.x / TG, t = threadIdx.x - g * TG, lane = t & 31, wg = t >> 5;
+    typename GEO::Slot& S = reinterpret_cast<typename GEO::Slot*>(smem_raw)[g];
+    auto group_sync = [&]() {
+        if (WPI == 1) __syncwarp();
+        else asm volatile("bar.sync %0, %1;" :: "r"(1 + g), "r"(TG) : "memory");
+    };
+    const double r2_lt = a.r2_lt, r2_nz = a.r2_nz;
+    const unsigned lt = (1u << lane) - 1u;
+    for (long long it = (long long)blockIdx.x * GPB + g; it < a.num_items; it += (long long)gridDim.x * GPB) {
+        const long long rec = a.record[it];
+        const int i = a.observer[it];
+        if (rec < 0 || rec >= a.num_records || i < 0 || i >= N) {     // invalid item: no edges
+            if (!FILL && t == 0) a.counts[it] = 0;
+            continue;
+        }
+        group_sync();                                 // the previous item's readers of S are done
+        stage_record<REC, TG>(S.rec, a.records, rec, t);
+        group_sync();
+        const REC& R = S.rec;
+        if (t < 32) record_keep_words<DYN, N, L, O>(R, a.sel_tab, i, lane, S.keep);
+        group_sync();
+        // kept non-zero entries of every row: warp wg of the group takes rows wg, wg + WPI, ...; one ballot per 32 columns
+        int cnt = 0;
+        for (int ra = wg; ra < E; ra += WPI) {
+            const bool ka = (S.keep[ra >> 5] >> (ra & 31)) & 1u;
+            const double2 pa = R.pos[ra];
+            int rc = 0;
+#pragma unroll
+            for (int w = 0; w < W; ++w) {
+                const int cb = w * 32 + lane;
+                bool nz = false;
+                if (ka && cb < E) {
+                    const double2 pb = R.pos[cb];
+                    const double dx = pa.x - pb.x, dy = pa.y - pb.y;
+                    nz = adj_value(dx * dx + dy * dy, r2_lt, r2_nz) != 0.0f;
+                }
+                const unsigned m = __ballot_sync(0xffffffffu, nz) & S.keep[w];
+                if (FILL && lane == 0) S.rowmask[ra * W + w] = m;
+                rc += __popc(m);
+            }
+            if (FILL) { if (lane == 0) S.rowoff[ra] = rc; }
+            else cnt += rc;
+        }
+        if (!FILL) {
+            if (WPI == 1) {
+                if (lane == 0) a.counts[it] = cnt;
+            } else {
+                if (lane == 0) S.rowoff[wg] = cnt;
+                group_sync();
+                if (t == 0) {
+                    int c = 0;
+#pragma unroll
+                    for (int w = 0; w < WPI; ++w) c += S.rowoff[w];
+                    a.counts[it] = c;
+                }
+            }
+            continue;
+        }
+        group_sync();
+        // exclusive prefix of the row counts (the group's first warp)
+        if (t < 32) {
+            int running = 0;
+            for (int c0 = 0; c0 < E; c0 += 32) {
+                const int ra = c0 + lane;
+                const int v = ra < E ? S.rowoff[ra] : 0;
+                int incl = v;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) { const int u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
+                if (ra < E) S.rowoff[ra] = running + incl - v;
+                running += __shfl_sync(0xffffffffu, incl, 31);
+            }
+        }
+        group_sync();
+        // edges of row ra at offsets[it] + rowoff[ra] + rank among the row's kept non-zeros; a position outside
+        // [0, capacity) (a short capacity, or offsets of other items) is never written
+        const long long base = a.offsets[it], node0 = it * E;
+        long long* const src = a.edge_index;
+        long long* const dst = a.edge_index + a.capacity;
+        const unsigned long long cap = (unsigned long long)a.capacity;
+        for (int ra = wg; ra < E; ra += WPI) {
+            long long p0 = base + S.rowoff[ra];
+            const double2 pa = R.pos[ra];
+#pragma unroll
+            for (int w = 0; w < W; ++w) {
+                const unsigned m = S.rowmask[ra * W + w];
+                const long long p = p0 + __popc(m & lt);
+                if (((m >> lane) & 1u) && (unsigned long long)p < cap) {
+                    const int cb = w * 32 + lane;
+                    const double2 pb = R.pos[cb];
+                    const double dx = pa.x - pb.x, dy = pa.y - pb.y;
+                    src[p] = node0 + ra; dst[p] = node0 + cb; a.edge_attr[p] = adj_value(dx * dx + dy * dy, r2_lt, r2_nz);
+                }
+                p0 += __popc(m);
+            }
+        }
+    }
+}
+
+template <int DYN, int N, int L, int O>
+__global__ void __launch_bounds__(RecordEdgesGeom<DYN, N, L, O>::THREADS)
+lsm_record_emit_kernel_edge_count(const __grid_constant__ RecordEdgesArgs a) {
+    record_edges_items<DYN, N, L, O, false>(a);
+}
+
+template <int DYN, int N, int L, int O>
+__global__ void __launch_bounds__(RecordEdgesGeom<DYN, N, L, O>::THREADS)
+lsm_record_emit_kernel_edge_fill(const __grid_constant__ RecordEdgesArgs a) {
+    record_edges_items<DYN, N, L, O, true>(a);
 }
 
 }  // namespace lsm

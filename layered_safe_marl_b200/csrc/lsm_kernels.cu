@@ -119,6 +119,9 @@ struct SpecFns {
     int rec_bytes, scratch_bytes, emit_smem, emit_threads;
     const void* record_emit;  // lsm_record_emit_kernel (lsm_emit_from_records)
     int record_emit_smem, record_emit_threads, record_emit_items;   // items in flight per block
+    const void* record_edge_count;  // lsm_record_emit_kernel_edge_count / _edge_fill (lsm_edges_from_records)
+    const void* record_edge_fill;
+    int record_edges_smem, record_edges_threads, record_edges_items;
 };
 
 #ifdef LSM_EXPERIMENTS
@@ -176,6 +179,11 @@ static bool spec_fns_base(int dynamics, int N, int L, int O, bool f32, SpecFns* 
         f->record_emit_smem = RecordEmitGeom<DYN_, N_, L_, O_>::SMEM;                             \
         f->record_emit_threads = RecordEmitGeom<DYN_, N_, L_, O_>::THREADS;                       \
         f->record_emit_items = RecordEmitGeom<DYN_, N_, L_, O_>::GPB;                             \
+        f->record_edge_count = (const void*)lsm_record_emit_kernel_edge_count<DYN_, N_, L_, O_>;  \
+        f->record_edge_fill = (const void*)lsm_record_emit_kernel_edge_fill<DYN_, N_, L_, O_>;    \
+        f->record_edges_smem = RecordEdgesGeom<DYN_, N_, L_, O_>::SMEM;                           \
+        f->record_edges_threads = RecordEdgesGeom<DYN_, N_, L_, O_>::THREADS;                     \
+        f->record_edges_items = RecordEdgesGeom<DYN_, N_, L_, O_>::GPB;                           \
         return true;                                                                              \
     }
     LSM_SPEC_LIST(X)
@@ -397,6 +405,29 @@ cudaError_t spec_launch_record_emit(int dynamics, int N, int L, int O, const Rec
     void* args[] = { (void*)&a };
     return cudaLaunchKernel(f.record_emit, dim3((unsigned)blocks), dim3((unsigned)f.record_emit_threads), args,
                             (size_t)f.record_emit_smem, stream);
+}
+
+cudaError_t spec_launch_record_edges(int dynamics, int N, int L, int O, const RecordEdgesArgs& a, long long* offsets, bool fill,
+                                     cudaStream_t stream) {
+    SpecFns f;
+    if (!spec_fns(dynamics, N, L, O, false, &f)) return cudaErrorInvalidValue;
+    if (a.num_items <= 0) return fill ? cudaSuccess : cudaMemsetAsync(offsets, 0, sizeof(long long), stream);
+    static int sm_count = 0;
+    if (sm_count == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev); }
+    const void* fn = fill ? f.record_edge_fill : f.record_edge_count;
+    if (f.record_edges_smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, f.record_edges_smem);
+        if (e != cudaSuccess) return e;
+    }
+    // blocks loop over the items, as in spec_launch_record_emit
+    long long blocks = (a.num_items + f.record_edges_items - 1) / f.record_edges_items;
+    if (blocks > 8LL * sm_count) blocks = 8LL * sm_count;
+    void* args[] = { (void*)&a };
+    cudaError_t e = cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3((unsigned)f.record_edges_threads), args,
+                                     (size_t)f.record_edges_smem, stream);
+    if (e != cudaSuccess || fill) return e;
+    lsm_edge_scan_kernel<<<1, 1024, 0, stream>>>(a.counts, offsets, a.num_items);
+    return cudaGetLastError();
 }
 
 int edge_count_envs_per_block(long long envs) {

@@ -211,10 +211,15 @@ class DeviceGraphRolloutBuffer:
                     r = r * self.bad_masks[step + 1] + (1 - self.bad_masks[step + 1]) * self.value_preds[step]
                 self.returns[step] = r
 
-    def graph_rows(self, t, env, agent, node_obs=None, adj=None):
+    def graph_rows(self, t, env, agent, node_obs=None, adj=None, edges: bool = False):
         """Graph observation rows (node_obs[t, env, agent], adj[t, env, agent]) for B index triples, t in [0, T]:
         -> ((B, E, F), (B, E, E)). Dense storage gathers them; records storage re-emits them on the GPU. Host (CPU tensor
-        or numpy) indices out of range raise IndexError; out-of-range CUDA indices give zero rows in records storage."""
+        or numpy) indices out of range raise IndexError; out-of-range CUDA indices give zero rows in records storage.
+        With edges=True the matrices come as the edge list the GNN builds from them instead:
+        -> (node_obs (B, E, F), edge_index (2, nnz) int64, edge_attr (nnz, 1) float32), equal to process_adj(adj) of
+        the rows; records storage computes it from the records without any dense matrix (one host sync to read nnz)."""
+        if edges and adj is not None:
+            raise ValueError("adj is not written with edges=True")
         T1, n = self.episode_length + 1, self.n_rollout_threads
         dev = self.env.device
         on_dev = all(torch.is_tensor(x) and x.is_cuda for x in (t, env, agent))
@@ -229,17 +234,23 @@ class DeviceGraphRolloutBuffer:
             no, ad = self.node_obs[t, env, agent], self.adj[t, env, agent]
             if node_obs is not None:
                 node_obs.copy_(no); no = node_obs
+            if edges:
+                return (no,) + process_adj(ad)
             if adj is not None:
                 adj.copy_(ad); ad = adj
             return no, ad
         # an env index out of range must not alias another env's record: it becomes an invalid record
         ok = (t >= 0) & (t < T1) & (env >= 0) & (env < n)
         record = torch.where(ok, t * n + env, torch.full_like(t, -1))
-        return self.env.emit_from_records(self.records, record, agent, node_obs, adj)
+        return self._emit(self.records, record, agent, node_obs, adj, edges)
 
-    def graph_batch(self, rows, node_obs=None, adj=None):
+    def graph_batch(self, rows, node_obs=None, adj=None, edges: bool = False):
         """Rows of the (T, n, N) flattening a minibatch generator indexes: equal to
-        (node_obs[:-1].reshape(-1, E, F)[rows], adj[:-1].reshape(-1, E, E)[rows]) of the dense storage."""
+        (node_obs[:-1].reshape(-1, E, F)[rows], adj[:-1].reshape(-1, E, E)[rows]) of the dense storage.
+        With edges=True: (node_obs rows, *process_adj(adj rows)) - item b of the edge list is position b of `rows` -
+        which records storage computes from the records without any dense matrix (one host sync to read nnz)."""
+        if edges and adj is not None:
+            raise ValueError("adj is not written with edges=True")
         T, n, N = self.episode_length, self.n_rollout_threads, self.num_agents
         if not (torch.is_tensor(rows) and rows.is_cuda):
             rows = torch.as_tensor(np.asarray(rows)).reshape(-1).to(torch.int64)
@@ -253,11 +264,21 @@ class DeviceGraphRolloutBuffer:
             ad = self.adj[:-1].reshape(-1, E, E)[rows]
             if node_obs is not None:
                 node_obs.copy_(no); no = node_obs
+            if edges:
+                return (no,) + process_adj(ad)
             if adj is not None:
                 adj.copy_(ad); ad = adj
             return no, ad
         # row r is record r // N of the first T slots (an out-of-range row: a record index outside them), observer r % N
-        return self.env.emit_from_records(self.records[:-1], torch.div(rows, N, rounding_mode='floor'), rows % N, node_obs, adj)
+        return self._emit(self.records[:-1], torch.div(rows, N, rounding_mode='floor'), rows % N, node_obs, adj, edges)
+
+    def _emit(self, records, record, observer, node_obs, adj, edges):
+        """Records storage: the rows' node_obs and adj, or node_obs and the edge list (lsm_emit_from_records without
+        the matrices, then lsm_edges_from_records)."""
+        if not edges:
+            return self.env.emit_from_records(records, record, observer, node_obs, adj)
+        no, _ = self.env.emit_from_records(records, record, observer, node_obs, dense_adj=False)
+        return (no,) + self.env.edges_from_records(records, record, observer)
 
     def graph_nbytes(self) -> int:
         """Bytes of graph-observation storage: node_obs + adj (dense), or the records plus the one-step dense scratch
@@ -309,6 +330,14 @@ class _ConcatSlot:
     @property
     def tensor(self):
         return self._t
+
+
+def process_adj(adj):
+    """The reference's TransformerConvNet.process_adj (onpolicy/algorithms/utils/gnn.py:376-407) on a (B, E, E) batch:
+    -> (edge_index (2, nnz) int64 = [b * E + row, b * E + col] of the non-zeros in row-major order, edge_attr (nnz, 1))."""
+    nz = adj.nonzero()
+    base = nz[:, 0] * adj.shape[1]
+    return torch.stack([base + nz[:, 1], base + nz[:, 2]], dim=0), adj[nz[:, 0], nz[:, 1], nz[:, 2]].unsqueeze(1)
 
 
 class _FieldView:

@@ -437,34 +437,64 @@ class B200GraphVecEnv:
             "dst: contiguous uint8 CUDA tensor of the records' size"
         self._check(self.lib.lsm_copy_records(self._h, C.c_void_p(dst.data_ptr()), self._stream()), 'lsm_copy_records')
 
-    def emit_from_records(self, records, record, observer, node_obs=None, adj=None):
+    def emit_from_records(self, records, record, observer, node_obs=None, adj=None, dense_adj: bool = True):
         """Re-emit graph observations from stored records (lsm_emit_from_records) on torch's current stream.
 
         records: uint8 CUDA tensor whose last dimension is emit_record_bytes (copy_records output, any leading shape);
         record / observer: B indices into the flattened records and the observing agent. CPU tensors or numpy arrays
         are range-checked here (IndexError); CUDA tensors go to the kernel unchecked, which zero-fills invalid items.
-        -> (node_obs (B, E, F), adj (B, E, E)), written into the given tensors or into new ones."""
+        -> (node_obs (B, E, F), adj (B, E, E)), written into the given tensors or into new ones. With dense_adj=False
+        the matrices are not written and adj is None (edges_from_records gives their edge list)."""
+        num_records, record, observer = self._record_items(records, record, observer, 'emit_from_records')
+        B, E = record.numel(), self.E
+        if node_obs is None:
+            node_obs = torch.empty((B, E, self.F), dtype=torch.float32, device=self.device)
+        if adj is None and dense_adj:
+            adj = torch.empty((B, E, E), dtype=torch.float32, device=self.device)
+        elif not dense_adj and adj is not None:
+            raise ValueError("adj given with dense_adj=False")
+        for t, shape, name in ((node_obs, (B, E, self.F), 'node_obs'), (adj, (B, E, E), 'adj')):
+            assert t is None or (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous() and tuple(t.shape) == shape), \
+                f"{name}: need a contiguous float32 CUDA tensor of shape {shape}"
+        io = _lib.LsmRecordEmitIo(B, num_records, records.data_ptr(), record.data_ptr(), observer.data_ptr(),
+                                  node_obs.data_ptr(), adj.data_ptr() if adj is not None else None)
+        self._check(self.lib.lsm_emit_from_records(self._h, C.byref(io), self._stream()), 'lsm_emit_from_records')
+        return node_obs, adj
+
+    def edges_from_records(self, records, record, observer):
+        """COO edge list of the matrices emit_from_records would write for the same items (lsm_edges_from_records),
+        computed from the records without any dense matrix: -> (edge_index (2, nnz) int64, edge_attr (nnz, 1) float32),
+        what the reference's TransformerConvNet.process_adj (gnn.py:376-407) returns for that (B, E, E) batch. Indices
+        are handled as by emit_from_records; an invalid CUDA item has no edges. A counting pass, one host sync to read
+        nnz, allocations of exactly nnz edges, then the fill pass."""
+        num_records, record, observer = self._record_items(records, record, observer, 'edges_from_records')
+        B = record.numel()
+        counts = torch.empty((B,), dtype=torch.int32, device=self.device)
+        offsets = torch.empty((B + 1,), dtype=torch.int64, device=self.device)
+        io = _lib.LsmRecordEdgesIo(B, num_records, records.data_ptr(), record.data_ptr(), observer.data_ptr(),
+                                   counts.data_ptr(), offsets.data_ptr(), None, None, 0)
+        self._check(self.lib.lsm_edges_from_records(self._h, C.byref(io), self._stream()), 'lsm_edges_from_records')
+        nnz = int(offsets[B].item())
+        edge_index = torch.empty((2, nnz), dtype=torch.int64, device=self.device)
+        edge_attr = torch.empty((nnz, 1), dtype=torch.float32, device=self.device)
+        if nnz > 0:
+            io.edge_index, io.edge_attr, io.capacity = edge_index.data_ptr(), edge_attr.data_ptr(), nnz
+            self._check(self.lib.lsm_edges_from_records(self._h, C.byref(io), self._stream()), 'lsm_edges_from_records')
+        return edge_index, edge_attr
+
+    def _record_items(self, records, record, observer, what: str):
+        """-> (num_records, record int64, observer int32) of a record store and its items, checked as documented in
+        emit_from_records."""
         R = self.record_bytes()
         if R == 0:
-            raise RuntimeError("emit_from_records needs the specialised pipeline (this handle runs the generic kernel)")
+            raise RuntimeError(f"{what} needs the specialised pipeline (this handle runs the generic kernel)")
         assert records.is_cuda and records.dtype == torch.uint8 and records.is_contiguous() and records.shape[-1] == R, \
             f"records: contiguous uint8 CUDA tensor with a last dimension of {R} bytes"
         num_records = records.numel() // R
         record, observer = self._item_index(record, num_records, torch.int64), self._item_index(observer, self.N, torch.int32)
         if record.shape != observer.shape:
             raise ValueError(f"record and observer must have the same shape, got {tuple(record.shape)} and {tuple(observer.shape)}")
-        B, E = record.numel(), self.E
-        if node_obs is None:
-            node_obs = torch.empty((B, E, self.F), dtype=torch.float32, device=self.device)
-        if adj is None:
-            adj = torch.empty((B, E, E), dtype=torch.float32, device=self.device)
-        for t, shape, name in ((node_obs, (B, E, self.F), 'node_obs'), (adj, (B, E, E), 'adj')):
-            assert t.is_cuda and t.dtype == torch.float32 and t.is_contiguous() and tuple(t.shape) == shape, \
-                f"{name}: need a contiguous float32 CUDA tensor of shape {shape}"
-        io = _lib.LsmRecordEmitIo(B, num_records, records.data_ptr(), record.data_ptr(), observer.data_ptr(),
-                                  node_obs.data_ptr(), adj.data_ptr())
-        self._check(self.lib.lsm_emit_from_records(self._h, C.byref(io), self._stream()), 'lsm_emit_from_records')
-        return node_obs, adj
+        return num_records, record, observer
 
     def _item_index(self, idx, bound: int, dtype):
         """Index tensor for the kernel: host indices are checked against [0, bound); device indices are not."""
