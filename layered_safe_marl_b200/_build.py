@@ -3,6 +3,7 @@
     python -m layered_safe_marl_b200._build                      the product library (liblsm_b200.so)
     python -m layered_safe_marl_b200._build --shape airtaxi,6,2,0
                                                                  the library of one specialised shape (build_shape)
+    python -m layered_safe_marl_b200._build --ppo                the PPO-input library (liblsm_b200_ppo.so, build_ppo)
 """
 from __future__ import annotations
 
@@ -32,11 +33,25 @@ MAX_AGENTS, MAX_LANDMARKS, MAX_OBSTACLES = 32, 128, 32
 DYNAMICS_TAG = {0: 'di', 1: 'at'}
 
 
-def needs_build(path: str = LIB_PATH) -> bool:
+def needs_build(path: str = LIB_PATH, deps=DEPS) -> bool:
     if not os.path.exists(path):
         return True
     t = os.path.getmtime(path)
-    return any(os.path.getmtime(p) > t for p in DEPS)
+    return any(os.path.getmtime(p) > t for p in deps)
+
+
+# the PPO-input kernels (returns, advantages, advantage moments): no env handle, so a library of their own
+PPO_LIB_PATH = os.path.join(HERE, 'liblsm_b200_ppo.so')
+PPO_SOURCES = [os.path.join(CSRC, 'lsm_ppo.cu')]
+PPO_DEPS = PPO_SOURCES + [os.path.join(os.path.dirname(HERE), 'include', 'lsm_b200_ppo.h')]
+
+
+def build_ppo(force: bool = False, verbose: bool = False) -> str:
+    """liblsm_b200_ppo.so from csrc/lsm_ppo.cu with the product library's flags; rebuilt when a source is newer."""
+    if not force and not needs_build(PPO_LIB_PATH, PPO_DEPS):
+        return PPO_LIB_PATH
+    _nvcc([], PPO_LIB_PATH, verbose, sources=PPO_SOURCES)
+    return PPO_LIB_PATH
 
 
 EXP_LIB_PATH = os.path.join(HERE, 'liblsm_b200_exp.so')
@@ -50,9 +65,9 @@ def build_experiments(extra_flags=(), verbose: bool = False) -> str:
     return EXP_LIB_PATH
 
 
-def _nvcc(extra_flags, out_path: str, verbose: bool = False) -> None:
+def _nvcc(extra_flags, out_path: str, verbose: bool = False, sources=SOURCES) -> None:
     nvcc = os.environ.get('NVCC', 'nvcc')
-    cmd = [nvcc] + NVCC_FLAGS + list(extra_flags) + (['-Xptxas', '-v'] if verbose else []) + ['-o', out_path] + SOURCES
+    cmd = [nvcc] + NVCC_FLAGS + list(extra_flags) + (['-Xptxas', '-v'] if verbose else []) + ['-o', out_path] + list(sources)
     try:
         proc = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     except OSError as exc:
@@ -134,9 +149,14 @@ def main(argv=None) -> None:
     ap = argparse.ArgumentParser(prog='python -m layered_safe_marl_b200._build', description=__doc__.splitlines()[0])
     ap.add_argument('--shape', action='append', default=[], metavar='DYNAMICS,N,L,O',
                     help='build the library of one specialised shape (repeatable), e.g. airtaxi,6,2,0')
+    ap.add_argument('--ppo', action='store_true', help='build the PPO-input library (liblsm_b200_ppo.so)')
     ap.add_argument('--force', action='store_true', help='rebuild even when the library is up to date')
     ap.add_argument('--verbose', action='store_true', help='print ptxas resource usage')
     a = ap.parse_args(argv)
+    if a.ppo:
+        print(build_ppo(force=a.force, verbose=a.verbose))
+        if not a.shape:
+            return
     if not a.shape:
         print(build(force=a.force, verbose=a.verbose))
         return

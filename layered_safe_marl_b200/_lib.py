@@ -87,6 +87,16 @@ class LsmRecordEdgesIo(C.Structure):
                 ('edge_attr', C.c_void_p), ('capacity', C.c_int64)]
 
 
+class LsmReturnsIo(C.Structure):
+    """include/lsm_b200_ppo.h lsm_returns_io."""
+    _fields_ = [('T', C.c_int64), ('columns', C.c_int64), ('rewards', C.c_void_p), ('value_preds', C.c_void_p),
+                ('next_value', C.c_void_p), ('masks', C.c_void_p), ('bad_masks', C.c_void_p), ('returns', C.c_void_p),
+                ('advantages', C.c_void_p), ('active_masks', C.c_void_p), ('value_scale', C.c_void_p),
+                ('value_shift', C.c_void_p), ('scratch', C.c_void_p), ('stats64', C.c_void_p), ('stats', C.c_void_p),
+                ('gamma', C.c_float), ('gamma_lambda', C.c_float), ('use_gae', C.c_int32),
+                ('use_proper_time_limits', C.c_int32)]
+
+
 EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_destroy', 'lsm_set_value_grid',
                     'lsm_set_ttr_grid', 'lsm_bind_buffers', 'lsm_get_launch_info', 'lsm_step', 'lsm_reset',
                     'lsm_observe', 'lsm_emit_only', 'lsm_invalidate', 'lsm_set_output_buffers', 'lsm_edge_list',
@@ -94,6 +104,8 @@ EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_dest
                     'lsm_set_compact_adjacency', 'lsm_expand_adjacency_host', 'lsm_set_edge_output', 'lsm_world_graph', 'lsm_fetch_host', 'lsm_step_host',
                     'lsm_episode_stats', 'lsm_debug_pair_values', 'lsm_safety_filter', 'lsm_hj_lookup',
                     'lsm_copy_records', 'lsm_emit_from_records', 'lsm_edges_from_records')
+
+PPO_EXPORTED_SYMBOLS = ('lsm_ppo_abi_version', 'lsm_ppo_last_error', 'lsm_compute_returns', 'lsm_returns_scratch_bytes')
 
 _libs = {}          # one CDLL per path: the product library and the per-shape libraries (_build.build_shape)
 
@@ -156,6 +168,29 @@ def load(path: Optional[str] = None):
     for name in EXPORTED_SYMBOLS:
         if name not in ('lsm_abi_version', 'lsm_last_error'):
             getattr(lib, name).restype = C.c_int
+    _libs[key] = lib
+    return lib
+
+
+def load_ppo():
+    """Load liblsm_b200_ppo.so (include/lsm_b200_ppo.h), building it first if the sources are newer. Once per process."""
+    key = _build.PPO_LIB_PATH
+    if key in _libs:
+        return _libs[key]
+    if _build.needs_build(key, _build.PPO_DEPS):
+        try:
+            _build.build_ppo()
+        except Exception as exc:
+            if not os.path.exists(key):
+                raise RuntimeError(f"liblsm_b200_ppo.so is missing and could not be built: {exc}") from exc
+    lib = C.CDLL(key)
+    lib.lsm_ppo_abi_version.restype = C.c_int
+    lib.lsm_ppo_last_error.restype = C.c_char_p
+    lib.lsm_compute_returns.argtypes = [C.POINTER(LsmReturnsIo), C.c_void_p]
+    lib.lsm_compute_returns.restype = C.c_int
+    lib.lsm_returns_scratch_bytes.argtypes = [C.c_int64]
+    lib.lsm_returns_scratch_bytes.restype = C.c_int64
+    lib.lsm_last_error = lib.lsm_ppo_last_error      # check(rc, what, lib) reads this library's own error string
     _libs[key] = lib
     return lib
 

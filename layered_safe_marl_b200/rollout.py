@@ -6,7 +6,8 @@ Mirrors the environment-facing half of the reference's host-side loop
     GraphReplayBuffer.__init__      onpolicy/utils/graph_buffer.py:45-166   (field names, shapes, dtypes)
     GraphReplayBuffer.insert        onpolicy/utils/graph_buffer.py:168-251
     GraphReplayBuffer.after_update  onpolicy/utils/graph_buffer.py:253-283
-    GraphReplayBuffer.compute_returns (GAE / discounted sum, no value normaliser)   graph_buffer.py:285-373
+    GraphReplayBuffer.compute_returns (GAE / discounted sum, optional value denormalisation)   graph_buffer.py:285-373
+    GraphReplayBuffer.feed_forward_generator / recurrent_generator   graph_buffer.py (after compute_returns)
 
 but keeps every array in HBM, so one rollout step never crosses PCIe: the reference builds `masks`,
 `active_masks`, `share_obs` and the one-hot actions with numpy on the host and copies every observation
@@ -21,10 +22,15 @@ adj bytes) instead of node_obs / adj: the env writes its dense outputs into ONE 
 and `graph_rows` / `graph_batch` re-emit any (step, env, agent) row on the GPU, bit for bit what the dense buffer holds
 (lsm_copy_records / lsm_emit_from_records). The other fields, share_obs included, are stored as in the dense mode.
 
-torch is used for storage and for the few elementwise mask operations; the learner (policy, GAE
-consumers, minibatch generators) is out of scope.
+torch is used for storage and for the few elementwise mask operations. The PPO inputs come from the device too:
+compute_returns / compute_advantages run one kernel of liblsm_b200_ppo.so on CUDA buffers (returns, raw advantages and
+their active-entry moments in one pass), and feed_forward_batches / recurrent_batches serve the reference generators'
+minibatches, the graph fields through graph_rows in either storage. The policy, the GNN and the value normaliser belong
+to the learner.
 """
 from __future__ import annotations
+
+import warnings
 
 import numpy as np
 import torch
@@ -190,26 +196,128 @@ class DeviceGraphRolloutBuffer:
                 t[0].copy_(t[-1])
         self.bind_next_slot()
 
-    def compute_returns(self, next_value):
-        """graph_buffer.py:285-373 without a value normaliser (popart / valuenorm belong to the learner)."""
-        T = self.rewards.shape[0]
-        if self._use_gae:
-            self.value_preds[-1].copy_(next_value.reshape(self.value_preds[-1].shape))
-            gae = torch.zeros_like(self.value_preds[0])
-            for step in reversed(range(T)):
-                delta = self.rewards[step] + self.gamma * self.value_preds[step + 1] * self.masks[step + 1] \
-                    - self.value_preds[step]
-                gae = delta + self.gamma * self.gae_lambda * self.masks[step + 1] * gae
-                if self._use_proper_time_limits:
-                    gae = gae * self.bad_masks[step + 1]
-                self.returns[step] = gae + self.value_preds[step]
+    def compute_returns(self, next_value, value_scale=None, value_shift=None):
+        """graph_buffer.py:285-373. With value_scale / value_shift (1-element float32 tensors, given together) every value
+        prediction the recursion reads is denormalised as v * value_scale + value_shift, the ValueNorm / PopArt
+        `denormalize` with value_scale = sqrt(var) and value_shift = mean. CUDA buffers run one kernel
+        (lsm_compute_returns), bit for bit the torch loop below, which CPU buffers run. No host sync on CUDA."""
+        if self.rewards.is_cuda:
+            self._returns_kernel(next_value, value_scale, value_shift)
+            return
+        returns_loop(self.rewards, self.value_preds, self.returns, self.masks, self.bad_masks, next_value, self.gamma,
+                     self.gae_lambda, self._use_gae, self._use_proper_time_limits, value_scale, value_shift)
+
+    def compute_advantages(self, normalize: bool = True, value_scale=None, value_shift=None):
+        """The advantages GR_MAPPO.train feeds its generators, after compute_returns (with the same value_scale /
+        value_shift): adv = returns[:-1] - d(value_preds[:-1]), then with `normalize`
+        (adv - mean) / (std + 1e-5), mean and std over the entries with active_masks[:-1] != 0 (np.nanmean / np.nanstd,
+        taken in float64 and rounded to float32; NaN when no entry is active).
+        -> (advantages (T, n, N, 1) float32, mean, std) with mean / std 0-dim float32 tensors on the buffer's device.
+        CUDA buffers take the raw advantages and their moments from one pass of lsm_compute_returns, which recomputes the
+        returns from the next value compute_returns stored (value_preds[T] with GAE, returns[T] otherwise) and writes
+        the same bits again; no host sync."""
+        if self.rewards.is_cuda:
+            adv, stats = self._returns_kernel(None, value_scale, value_shift, advantages=True)
+            mean, std = stats[0], stats[1]
         else:
-            self.returns[-1].copy_(next_value.reshape(self.returns[-1].shape))
-            for step in reversed(range(T)):
-                r = self.returns[step + 1] * self.gamma * self.masks[step + 1] + self.rewards[step]
-                if self._use_proper_time_limits:
-                    r = r * self.bad_masks[step + 1] + (1 - self.bad_masks[step + 1]) * self.value_preds[step]
-                self.returns[step] = r
+            d = _denormalizer(value_scale, value_shift)
+            adv = self.returns[:-1] - d(self.value_preds[:-1])
+            a = adv.numpy().astype(np.float64)
+            a[self.active_masks[:-1].numpy() == 0] = np.nan
+            with warnings.catch_warnings():          # "Mean of empty slice" when no entry is active
+                warnings.simplefilter('ignore', RuntimeWarning)
+                mean, std = np.float32(np.nanmean(a)), np.float32(np.nanstd(a))
+            mean, std = torch.tensor(mean), torch.tensor(std)
+        if normalize:
+            adv = (adv - mean) / (std + 1e-5)
+        return adv, mean, std
+
+    def _returns_kernel(self, next_value, value_scale, value_shift, advantages: bool = False):
+        """returns_kernel on the buffer's arrays. next_value None: the one the last compute_returns stored.
+        With `advantages`: -> (raw advantages (T, n, N, 1), stats (2,) float32 = mean, std)."""
+        if next_value is None:
+            next_value = self.value_preds[-1] if self._use_gae else self.returns[-1]
+        adv = stats = None
+        if advantages:
+            adv = torch.empty_like(self.rewards)
+            stats = torch.empty((2,), dtype=torch.float32, device=self.rewards.device)
+        returns_kernel(self.rewards, self.value_preds, self.returns, self.masks, self.bad_masks, next_value, self.gamma,
+                       self.gae_lambda, self._use_gae, self._use_proper_time_limits, value_scale, value_shift,
+                       advantages=adv, active_masks=self.active_masks if advantages else None, stats=stats)
+        return adv, stats
+
+    # ------------------------------------------------------------------------------------------
+    # minibatches (graph_buffer.py feed_forward_generator / recurrent_generator) from the device buffer
+    _BATCH_FIELDS = (('share_obs', 'share_obs'), ('obs', 'obs'), ('agent_id', 'agent_id'),
+                     ('share_agent_id', 'share_agent_id'), ('rnn_states', 'rnn_states'),
+                     ('rnn_states_critic', 'rnn_states_critic'), ('actions', 'actions'), ('value_preds', 'value_preds'),
+                     ('returns', 'returns'), ('masks', 'masks'), ('active_masks', 'active_masks'),
+                     ('old_action_log_probs', 'action_log_probs'), ('available_actions', 'available_actions'))
+
+    def _perm(self, count, perm, generator):
+        dev = self.rewards.device
+        if perm is None:
+            return torch.randperm(count, device=dev, generator=generator)
+        return torch.as_tensor(perm).reshape(-1).to(device=dev, dtype=torch.int64)
+
+    def _batch(self, t, e, a, advantages, edges, rnn_rows=None):
+        """One minibatch at (t, env, agent) index triples: every field a gather, the graph fields from graph_rows."""
+        out = {}
+        for key, name in self._BATCH_FIELDS:
+            x = getattr(self, name)
+            if name in ('rnn_states', 'rnn_states_critic') and rnn_rows is not None:
+                out[key] = x[rnn_rows]
+            else:
+                out[key] = x[t, e, a]
+        out['adv_targ'] = advantages[t, e, a]
+        g = self.graph_rows(t, e, a, edges=edges)
+        out['node_obs'] = g[0]
+        if edges:
+            out['edge_index'], out['edge_attr'] = g[1], g[2]
+        else:
+            out['adj'] = g[1]
+        return out
+
+    def feed_forward_batches(self, advantages, num_mini_batch: int, mini_batch_size=None, edges: bool = False, perm=None,
+                             generator=None):
+        """graph_buffer.py feed_forward_generator over the (T, n, N) flattening of the rows: mini_batch_size =
+        T * n * N // num_mini_batch unless given, batch i = rows perm[i * mbs:(i + 1) * mbs] (the remainder is dropped).
+        `advantages`: (T, n, N, 1), e.g. compute_advantages()[0]. Yields dicts keyed by the reference's batch names
+        (share_obs, obs, node_obs, adj, agent_id, share_agent_id, rnn_states, rnn_states_critic, actions, value_preds,
+        returns, masks, active_masks, old_action_log_probs, adv_targ, available_actions), each (mbs, ...); with
+        edges=True edge_index / edge_attr (process_adj of the rows) replace adj. perm: a permutation of the rows on any
+        device, default torch.randperm on the buffer's device (with `generator`). No host sync per batch except the nnz
+        read of edges=True."""
+        T, n, N = self.episode_length, self.n_rollout_threads, self.num_agents
+        batch_size = T * n * N
+        mbs = batch_size // num_mini_batch if mini_batch_size is None else int(mini_batch_size)
+        perm = self._perm(batch_size, perm, generator)
+        for i in range(num_mini_batch):
+            rows = perm[i * mbs:(i + 1) * mbs]
+            t = torch.div(rows, n * N, rounding_mode='floor')
+            e = torch.div(rows, N, rounding_mode='floor') % n
+            yield self._batch(t, e, rows % N, advantages, edges)
+
+    def recurrent_batches(self, advantages, num_mini_batch: int, data_chunk_length: int, edges: bool = False, perm=None,
+                          generator=None):
+        """graph_buffer.py recurrent_generator: rows follow the (n, N, T) flattening, chunk c is rows [c * L, (c + 1) * L)
+        (a chunk may cross from one (env, agent) column into the next when T % L != 0, as in the reference), there are
+        T * n * N // L chunks and mbs = chunks // num_mini_batch per batch. Batch row l * mbs + j is row perm[j] * L + l
+        (the reference's np.stack(axis=1) then _flatten); rnn_states / rnn_states_critic are taken at each chunk's first
+        row, (mbs, recurrent_N, hidden). Fields, perm and syncs as feed_forward_batches."""
+        T, n, N = self.episode_length, self.n_rollout_threads, self.num_agents
+        L = int(data_chunk_length)
+        chunks = T * n * N // L
+        mbs = chunks // num_mini_batch
+        perm = self._perm(chunks, perm, generator)
+        ar = torch.arange(L, device=perm.device, dtype=torch.int64)
+        for i in range(num_mini_batch):
+            first = perm[i * mbs:(i + 1) * mbs] * L
+            rows = (first.view(1, -1) + ar.view(-1, 1)).reshape(-1)          # l-major: row l * mbs + j
+            t, col = rows % T, torch.div(rows, T, rounding_mode='floor')
+            rt, rcol = first % T, torch.div(first, T, rounding_mode='floor')
+            yield self._batch(t, torch.div(col, N, rounding_mode='floor'), col % N, advantages, edges,
+                              rnn_rows=(rt, torch.div(rcol, N, rounding_mode='floor'), rcol % N))
 
     def graph_rows(self, t, env, agent, node_obs=None, adj=None, edges: bool = False):
         """Graph observation rows (node_obs[t, env, agent], adj[t, env, agent]) for B index triples, t in [0, T]:
@@ -299,6 +407,89 @@ class DeviceGraphRolloutBuffer:
         """np.eye(n)[actions] of GMPERunner.collect (graph_mpe_runner.py:431-433), on device. The simulator also
         accepts the integer indices directly, which skips this tensor altogether."""
         return torch.nn.functional.one_hot(actions.reshape(actions.shape[0], actions.shape[1]).long(), n_actions).to(torch.float32)
+
+
+def _denormalizer(value_scale, value_shift):
+    """v -> v * value_scale + value_shift (two rounded float32 ops), or the identity without them."""
+    if (value_scale is None) != (value_shift is None):
+        raise ValueError("value_scale and value_shift are given together or not at all")
+    if value_scale is None:
+        return lambda v: v
+    return lambda v: v * value_scale + value_shift
+
+
+def returns_kernel(rewards, value_preds, returns, masks, bad_masks, next_value, gamma: float, gae_lambda: float,
+                   use_gae: bool, use_proper_time_limits: bool, value_scale=None, value_shift=None, advantages=None,
+                   active_masks=None, stats=None, stats64=None):
+    """returns_loop as one CUDA kernel (lsm_compute_returns of liblsm_b200_ppo.so), bit for bit, on torch's current
+    stream and without a host sync. Arrays are contiguous float32 CUDA tensors whose leading dimension is the step:
+    rewards (T, ...), value_preds / returns / masks / bad_masks / active_masks (T + 1, ...), next_value one step's worth.
+    Optional outputs of the same pass: advantages (T, ...) = returns[t] - d(value_preds[t]); with active_masks, stats (2,)
+    float32 = mean, std and stats64 (3,) float64 = count, mean, std of those advantages over the entries with
+    active_masks[t] != 0, t < T (population std, float64 accumulation, NaN when no entry is active)."""
+    import ctypes as C
+    from . import _lib
+    lib = _lib.load_ppo()
+    T, dev = rewards.shape[0], rewards.device
+    cols = value_preds[0].numel()
+    if (value_scale is None) != (value_shift is None):
+        raise ValueError("value_scale and value_shift are given together or not at all")
+    if value_scale is not None:
+        value_scale, value_shift = (torch.as_tensor(x).to(device=dev, dtype=torch.float32).reshape(1).contiguous()
+                                    for x in (value_scale, value_shift))
+    next_value = next_value.to(device=dev, dtype=torch.float32).contiguous()
+    moments = stats is not None or stats64 is not None
+    if moments and active_masks is None:
+        raise ValueError("the advantage moments need active_masks")
+    for x, rows, name in ((rewards, T, 'rewards'), (value_preds, T + 1, 'value_preds'), (returns, T + 1, 'returns'),
+                          (masks, T + 1, 'masks'), (bad_masks, T + 1, 'bad_masks'), (advantages, T, 'advantages'),
+                          (active_masks, T + 1, 'active_masks')):
+        if x is not None and not (x.is_cuda and x.device == dev and x.dtype == torch.float32 and x.is_contiguous()
+                                  and x.numel() == rows * cols):
+            raise ValueError(f"{name}: need a contiguous float32 tensor of {rows} x {cols} on {dev}")
+    if next_value.numel() != cols:
+        raise ValueError(f"next_value: need {cols} values, got {next_value.numel()}")
+    for x, k, dt, name in ((stats, 2, torch.float32, 'stats'), (stats64, 3, torch.float64, 'stats64')):
+        if x is not None and not (x.device == dev and x.dtype == dt and x.is_contiguous() and x.numel() == k):
+            raise ValueError(f"{name}: need {k} contiguous {dt} values on {dev}")
+    scratch = None
+    if moments:
+        scratch = torch.empty((int(lib.lsm_returns_scratch_bytes(cols)) + 7) // 8, dtype=torch.float64, device=dev)
+    ptr = lambda x: C.c_void_p(x.data_ptr()) if x is not None else None
+    io = _lib.LsmReturnsIo(T, cols, ptr(rewards), ptr(value_preds), ptr(next_value), ptr(masks), ptr(bad_masks),
+                           ptr(returns), ptr(advantages), ptr(active_masks), ptr(value_scale), ptr(value_shift),
+                           ptr(scratch), ptr(stats64), ptr(stats),
+                           # the multipliers the torch loop applies: float32(gamma), float32(gamma * gae_lambda in double)
+                           float(np.float32(gamma)), float(np.float32(gamma * gae_lambda)),
+                           int(bool(use_gae)), int(bool(use_proper_time_limits)))
+    with torch.cuda.device(dev):
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(lib.lsm_compute_returns(C.byref(io), stream), 'lsm_compute_returns', lib)
+
+
+def returns_loop(rewards, value_preds, returns, masks, bad_masks, next_value, gamma: float, gae_lambda: float,
+                 use_gae: bool, use_proper_time_limits: bool, value_scale=None, value_shift=None):
+    """GraphReplayBuffer.compute_returns (graph_buffer.py:285-373) as eager torch ops, in place on (T[+1], ...) tensors
+    of any device: what DeviceGraphRolloutBuffer.compute_returns runs on CPU buffers, and the reference the kernel is
+    tested against bit for bit. value_scale / value_shift: the value normaliser's denormalize (see compute_returns)."""
+    d = _denormalizer(value_scale, value_shift)
+    T = rewards.shape[0]
+    if use_gae:
+        value_preds[-1].copy_(next_value.reshape(value_preds[-1].shape))
+        gae = torch.zeros_like(value_preds[0])
+        for step in reversed(range(T)):
+            delta = rewards[step] + gamma * d(value_preds[step + 1]) * masks[step + 1] - d(value_preds[step])
+            gae = delta + gamma * gae_lambda * masks[step + 1] * gae
+            if use_proper_time_limits:
+                gae = gae * bad_masks[step + 1]
+            returns[step] = gae + d(value_preds[step])
+    else:
+        returns[-1].copy_(next_value.reshape(returns[-1].shape))
+        for step in reversed(range(T)):
+            r = returns[step + 1] * gamma * masks[step + 1] + rewards[step]
+            if use_proper_time_limits:
+                r = r * bad_masks[step + 1] + (1 - bad_masks[step + 1]) * d(value_preds[step])
+            returns[step] = r
 
 
 class _ConcatSlot:
