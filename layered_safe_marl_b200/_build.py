@@ -4,6 +4,7 @@
     python -m layered_safe_marl_b200._build --shape airtaxi,6,2,0
                                                                  the library of one specialised shape (build_shape)
     python -m layered_safe_marl_b200._build --ppo                the PPO-input library (liblsm_b200_ppo.so, build_ppo)
+    python -m layered_safe_marl_b200._build --hj                 the HJ reachability solver (liblsm_b200_hj.so, build_hj)
 """
 from __future__ import annotations
 
@@ -52,6 +53,20 @@ def build_ppo(force: bool = False, verbose: bool = False) -> str:
         return PPO_LIB_PATH
     _nvcc([], PPO_LIB_PATH, verbose, sources=PPO_SOURCES)
     return PPO_LIB_PATH
+
+
+# the HJ reachability solver (value functions for the safety filter): no env handle, so a library of its own
+HJ_LIB_PATH = os.path.join(HERE, 'liblsm_b200_hj.so')
+HJ_SOURCES = [os.path.join(CSRC, 'lsm_hj.cu')]
+HJ_DEPS = HJ_SOURCES + [os.path.join(os.path.dirname(HERE), 'include', f) for f in ('lsm_b200_hj.h', 'lsm_math.h')]
+
+
+def build_hj(force: bool = False, verbose: bool = False) -> str:
+    """liblsm_b200_hj.so from csrc/lsm_hj.cu with the product library's flags; rebuilt when a source is newer."""
+    if not force and not needs_build(HJ_LIB_PATH, HJ_DEPS):
+        return HJ_LIB_PATH
+    _nvcc([], HJ_LIB_PATH, verbose, sources=HJ_SOURCES)
+    return HJ_LIB_PATH
 
 
 EXP_LIB_PATH = os.path.join(HERE, 'liblsm_b200_exp.so')
@@ -150,11 +165,15 @@ def main(argv=None) -> None:
     ap.add_argument('--shape', action='append', default=[], metavar='DYNAMICS,N,L,O',
                     help='build the library of one specialised shape (repeatable), e.g. airtaxi,6,2,0')
     ap.add_argument('--ppo', action='store_true', help='build the PPO-input library (liblsm_b200_ppo.so)')
+    ap.add_argument('--hj', action='store_true', help='build the HJ reachability solver (liblsm_b200_hj.so)')
     ap.add_argument('--force', action='store_true', help='rebuild even when the library is up to date')
     ap.add_argument('--verbose', action='store_true', help='print ptxas resource usage')
     a = ap.parse_args(argv)
-    if a.ppo:
-        print(build_ppo(force=a.force, verbose=a.verbose))
+    if a.ppo or a.hj:
+        if a.ppo:
+            print(build_ppo(force=a.force, verbose=a.verbose))
+        if a.hj:
+            print(build_hj(force=a.force, verbose=a.verbose))
         if not a.shape:
             return
     if not a.shape:

@@ -97,6 +97,12 @@ class LsmReturnsIo(C.Structure):
                 ('use_proper_time_limits', C.c_int32)]
 
 
+class LsmHjProblem(C.Structure):
+    """include/lsm_b200_hj.h lsm_hj_problem."""
+    _fields_ = [('dynamics', C.c_int32), ('shape', C.c_int32 * 5), ('lo', C.c_double * 5), ('hi', C.c_double * 5),
+                ('cfl', C.c_double)]
+
+
 EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_destroy', 'lsm_set_value_grid',
                     'lsm_set_ttr_grid', 'lsm_bind_buffers', 'lsm_get_launch_info', 'lsm_step', 'lsm_reset',
                     'lsm_observe', 'lsm_emit_only', 'lsm_invalidate', 'lsm_set_output_buffers', 'lsm_edge_list',
@@ -106,6 +112,9 @@ EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_dest
                     'lsm_copy_records', 'lsm_emit_from_records', 'lsm_edges_from_records')
 
 PPO_EXPORTED_SYMBOLS = ('lsm_ppo_abi_version', 'lsm_ppo_last_error', 'lsm_compute_returns', 'lsm_returns_scratch_bytes')
+
+HJ_EXPORTED_SYMBOLS = ('lsm_hj_abi_version', 'lsm_hj_last_error', 'lsm_hj_work_bytes', 'lsm_hj_dissipation',
+                       'lsm_hj_solve')
 
 _libs = {}          # one CDLL per path: the product library and the per-shape libraries (_build.build_shape)
 
@@ -191,6 +200,32 @@ def load_ppo():
     lib.lsm_returns_scratch_bytes.argtypes = [C.c_int64]
     lib.lsm_returns_scratch_bytes.restype = C.c_int64
     lib.lsm_last_error = lib.lsm_ppo_last_error      # check(rc, what, lib) reads this library's own error string
+    _libs[key] = lib
+    return lib
+
+
+def load_hj():
+    """Load liblsm_b200_hj.so (include/lsm_b200_hj.h), building it first if the sources are newer. Once per process."""
+    key = _build.HJ_LIB_PATH
+    if key in _libs:
+        return _libs[key]
+    if _build.needs_build(key, _build.HJ_DEPS):
+        try:
+            _build.build_hj()
+        except Exception as exc:
+            if not os.path.exists(key):
+                raise RuntimeError(f"liblsm_b200_hj.so is missing and could not be built: {exc}") from exc
+    lib = C.CDLL(key)
+    lib.lsm_hj_abi_version.restype = C.c_int
+    lib.lsm_hj_last_error.restype = C.c_char_p
+    lib.lsm_hj_work_bytes.argtypes = [C.POINTER(LsmHjProblem)]
+    lib.lsm_hj_work_bytes.restype = C.c_int64
+    lib.lsm_hj_dissipation.argtypes = [C.POINTER(LsmHjProblem), C.POINTER(C.c_double), C.POINTER(C.c_double)]
+    lib.lsm_hj_dissipation.restype = C.c_int
+    lib.lsm_hj_solve.argtypes = [C.POINTER(LsmHjProblem), C.c_void_p, C.POINTER(C.c_double), C.c_int32, C.c_void_p,
+                                 C.c_void_p, C.c_void_p]
+    lib.lsm_hj_solve.restype = C.c_int
+    lib.lsm_last_error = lib.lsm_hj_last_error       # check(rc, what, lib) reads this library's own error string
     _libs[key] = lib
     return lib
 
