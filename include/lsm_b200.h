@@ -161,7 +161,7 @@ typedef struct lsm_buffers {
 } lsm_buffers;
 
 /* Launch-shape choices a caller may override (lsm_set_tuning, right after lsm_create; 0 / -1 = automatic). These are
- * the product's only knobs; ablation switches live in the LSM_EXPERIMENTS build (liblsm_b200_exp.so), not here. */
+ * the library's only knobs: it reads no environment variable. */
 typedef struct lsm_tuning {
     int32_t chunks;               /* env ranges one step is split into on library-owned streams (1..16); 0 = automatic
                                      (4 from 0.4 GB of observations per step, else 1) */

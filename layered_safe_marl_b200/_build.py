@@ -69,17 +69,6 @@ def build_hj(force: bool = False, verbose: bool = False) -> str:
     return HJ_LIB_PATH
 
 
-EXP_LIB_PATH = os.path.join(HERE, 'liblsm_b200_exp.so')
-
-
-def build_experiments(extra_flags=(), verbose: bool = False) -> str:
-    """The lab build of the same sources: -DLSM_EXPERIMENTS compiles the ablation switches (LSM_DEBUG, LSM_WPE, LSM_PAIR,
-    LSM_AGENT_MINB, ... read from the environment) and the alternative kernel instantiations that the product library
-    does not contain. Tools select it with LSM_LIB=<path>."""
-    build(force=True, verbose=verbose, extra_flags=['-DLSM_EXPERIMENTS'] + list(extra_flags), out_path=EXP_LIB_PATH)
-    return EXP_LIB_PATH
-
-
 def _nvcc(extra_flags, out_path: str, verbose: bool = False, sources=SOURCES) -> None:
     nvcc = os.environ.get('NVCC', 'nvcc')
     cmd = [nvcc] + NVCC_FLAGS + list(extra_flags) + (['-Xptxas', '-v'] if verbose else []) + ['-o', out_path] + list(sources)
@@ -95,7 +84,7 @@ def _nvcc(extra_flags, out_path: str, verbose: bool = False, sources=SOURCES) ->
 
 def build(force: bool = False, verbose: bool = False, extra_flags=(), out_path: str = LIB_PATH) -> str:
     """`extra_flags` / `out_path` build an A/B variant (extra -D switches) next to the product library; a variant
-    is selected at run time with LSM_LIB=<path> (experiments only)."""
+    is selected at run time with LSM_LIB=<path>."""
     if not force and not needs_build() and out_path == LIB_PATH:
         return LIB_PATH
     _nvcc(extra_flags, out_path, verbose)

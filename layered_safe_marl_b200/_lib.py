@@ -131,7 +131,7 @@ def load(path: Optional[str] = None):
         return _libs[key]
     if path is None:
         path = _build.LIB_PATH
-        alt = os.environ.get('LSM_LIB')     # experiments: an A/B build of the same sources (see _build.build)
+        alt = os.environ.get('LSM_LIB')     # A/B builds: another build of the sources (see _build.build)
         if alt:
             path = alt
         elif _build.needs_build():

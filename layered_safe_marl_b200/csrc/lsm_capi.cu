@@ -105,24 +105,15 @@ struct lsm_handle {
     uint16_t* d_pair_tab = nullptr;
     uint32_t* d_sel_tab = nullptr;
     uint32_t* d_pair32 = nullptr;
-    size_t persist_bytes = 0;
-    size_t max_window = 0;
     bool spec = false;          // compile-time specialised pipeline available for (dynamics, N, L)
     int bytes_per_env = 0;      // shared memory of one environment (agent kernel: emit record + scratch)
     int epw_max = 1;            // 32 / G
     int smem_optin = 0;
-    int forced_epw = 0;         // LSM_EPW environment override (experiments)
-    lsm::SpecGeometry geo = {};
-    int emit_regs = 0, emit_blocks_per_sm = 0, pair_regs = 0;
-    bool l2_persist = false;            // LSM_L2_PERSIST=1: persisting access-policy window on the value grid
+    lsm::SpecTable tab = {};    // kernels and launch geometry of the specialised pipeline (spec)
     bool pairval_valid = false;         // d_pairval holds the HJ pair values of the CURRENT state (written by the last emit launch)
     double* d_pairval = nullptr;        // library-owned scratch of the specialised pipeline
     unsigned char* d_emit_rec = nullptr;
     unsigned long long* d_timeline = nullptr;   // diagnostics only (lsm_debug_timeline)
-#ifdef LSM_EXPERIMENTS
-    unsigned long long* d_phase = nullptr;      // lab build: agent-kernel phase stamps (lsm_debug_phase_stamps)
-    size_t phase_bytes = 0;
-#endif
     float* d_vpacked = nullptr;          // corner-packed copy of the value grid (GridDev::packed)
     // chunked launches: big batches are split into `chunks` env ranges on library-owned streams so that the latency-bound
     // agent kernel of one range runs beside the HBM-bound emit kernel of another (fork / join with events, no host sync)
@@ -153,7 +144,7 @@ struct lsm_handle {
     bool g_key_valid = false, g_seen_valid = false;
     long long g_replays = 0, g_captures = 0;
     lsm_tuning tuning = { 0, -1, -1, -1 };   // lsm_set_tuning (0 / -1 = automatic)
-    int pair_placement = 0;             // 0 late (lsm_pair_kernel behind the emit kernel), 1 inside the emit kernel, 2 in front of the agent kernel, 3 between agent and emit kernel
+    int pair_placement = 0;             // 0 late (lsm_pair_kernel behind the emit kernel), 2 in front of the agent kernel, 3 between agent and emit kernel, 4 tail of the agent kernel
 };
 
 extern "C" {
@@ -188,19 +179,6 @@ int lsm_create(const lsm_config* cfg, lsm_handle** out) {
     e = cudaGetDeviceProperties(&prop, h->device);
     if (e != cudaSuccess) { delete h; return cuda_fail(e, "cudaGetDeviceProperties"); }
     h->sm_count = prop.multiProcessorCount;
-    h->max_window = (size_t)prop.accessPolicyMaxWindowSize;
-    // An L2 persisting set-aside for the HJ grid is OFF by default: carving 32 MB out of the 126 MB L2 slowed the
-    // step's 107 MB store stream by 25-35 % on B200 (plain 16-byte stores of the adjacency bytes: 22.6 -> 16.8 us;
-    // whole cfg2 step 52.5 -> 47.9 us), while the 3-24 MB grids stay L2-resident on their own. LSM_L2_PERSIST=1 opts in.
-#ifdef LSM_EXPERIMENTS
-    h->l2_persist = std::getenv("LSM_L2_PERSIST") != nullptr;
-#endif
-    if (prop.persistingL2CacheMaxSize > 0 && h->l2_persist) {
-        size_t want = (size_t)prop.persistingL2CacheMaxSize;
-        if (want > ((size_t)32 << 20)) want = (size_t)32 << 20;
-        cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want);   // best effort
-        cudaGetLastError();
-    }
 
     lsm::KParams& kp = h->kp;
     kp.c = *cfg;
@@ -285,32 +263,17 @@ int lsm_create(const lsm_config* cfg, lsm_handle** out) {
     // grid lookups, so that the float64 kernels carry none of its code
     // (the obstacle extension is specialised for the shapes LSM_SPEC_LIST names with O > 0; other obstacle counts: generic)
     const bool f32 = (cfg->flags & LSM_FLAG_INTERP_FLOAT32) != 0;
-    h->spec = lsm::spec_available(cfg->dynamics, N, L, O, &h->geo);
-#ifdef LSM_EXPERIMENTS
-    { const char* force_generic = std::getenv("LSM_FORCE_GENERIC"); if (force_generic != nullptr && force_generic[0] == '1') h->spec = false; }
-#endif
+    h->spec = lsm::spec_table(cfg->dynamics, N, L, O, f32, &h->tab);
     // where the next step's HJ pair values are computed (measured, DESIGN.md 3): in lsm_pair_kernel behind the emit kernel
     // ("late") for the 4-D double-integrator grid; between the agent and the emit kernel ("middle") for the 5-D airtaxi
     // grid, whose lookups are half an emit kernel's worth of work and hurt it more when they share the SMs.
     // lsm_set_tuning overrides.
     h->pair_placement = cfg->dynamics == LSM_DYN_AIRTAXI ? 3 : 0;
-#ifdef LSM_EXPERIMENTS
-    if (const char* pp = std::getenv("LSM_PAIR")) {
-        if (!std::strcmp(pp, "late")) h->pair_placement = 0;
-        else if (!std::strcmp(pp, "emit")) h->pair_placement = 1;
-        else if (!std::strcmp(pp, "front")) h->pair_placement = 2;
-        else if (!std::strcmp(pp, "middle")) h->pair_placement = 3;
-    }
-    // the in-emit pair values (placement 1) exist in float64 only: a float32 handle keeps its default placement
-    if (f32 && h->pair_placement == 1) h->pair_placement = cfg->dynamics == LSM_DYN_AIRTAXI ? 3 : 0;
-    { const char* fe = std::getenv("LSM_EPW"); h->forced_epw = fe ? std::atoi(fe) : 0; }
-#endif
     if (h->spec) {
-        h->bytes_per_env = h->geo.rec_bytes + h->geo.scratch_bytes;
-        // agent kernel: one lane per agent, 32/N envs per warp (LSM_EPW overrides for experiments)
+        h->bytes_per_env = h->tab.rec_bytes + h->tab.scratch_bytes;
+        // agent kernel: one lane per agent, 32/N envs per warp
         h->epw_max = 32 / N; kp.EPW = h->epw_max;
-        if (h->forced_epw >= 1 && h->forced_epw <= h->epw_max) kp.EPW = h->forced_epw;
-        int wpb = h->geo.agent_block / 32;
+        int wpb = h->tab.agent_block / 32;
         while (wpb > 1 && h->bytes_per_env * kp.EPW * wpb > h->smem_optin) --wpb;
         h->warps_per_block = wpb;
         h->block_threads = 32 * wpb;
@@ -330,15 +293,16 @@ int lsm_create(const lsm_config* cfg, lsm_handle** out) {
         delete h;
         return fail(4, "lsm_create: one environment group does not fit in shared memory");
     }
-    e = lsm::kernel_prepare(cfg->dynamics, N, L, O, f32, h->spec, h->smem_per_block, h->block_threads, &h->regs, &h->blocks_per_sm);
+    e = lsm::kernel_prepare(h->spec ? h->tab.agent : lsm::generic_ptr(cfg->dynamics), h->block_threads, h->smem_per_block, &h->regs,
+                            &h->blocks_per_sm);
     if (e != cudaSuccess) { delete h; return cuda_fail(e, "kernel_prepare"); }
     if (h->blocks_per_sm < 1) { delete h; return fail(4, "lsm_create: kernel does not fit on an SM"); }
     h->grid_cap = h->sm_count * h->blocks_per_sm;
     if (h->spec) {
-        if (h->geo.emit_smem > h->smem_optin) { delete h; return fail(4, "lsm_create: emit record does not fit in shared memory"); }
-        e = lsm::spec_prepare_aux(cfg->dynamics, N, L, O, f32, &h->emit_regs, &h->emit_blocks_per_sm, &h->pair_regs);
-        if (e != cudaSuccess) { delete h; return cuda_fail(e, "spec_prepare_aux"); }
-        if (h->emit_blocks_per_sm < 1) { delete h; return fail(4, "lsm_create: emit kernel does not fit on an SM"); }
+        if (h->tab.emit_smem > h->smem_optin) { delete h; return fail(4, "lsm_create: emit record does not fit in shared memory"); }
+        e = lsm::spec_prepare(&h->tab);
+        if (e != cudaSuccess) { delete h; return cuda_fail(e, "spec_prepare"); }
+        if (h->tab.emit_blocks_per_sm < 1) { delete h; return fail(4, "lsm_create: emit kernel does not fit on an SM"); }
     }
 
     // lookup tables
@@ -387,9 +351,6 @@ int lsm_destroy(lsm_handle* h) {
     if (h->d_pairval) cudaFree(h->d_pairval);
     if (h->d_emit_rec) cudaFree(h->d_emit_rec);
     if (h->d_timeline) cudaFree(h->d_timeline);
-#ifdef LSM_EXPERIMENTS
-    if (h->d_phase) cudaFree(h->d_phase);
-#endif
     if (h->d_vpacked) cudaFree(h->d_vpacked);
     if (h->d_grads8) cudaFree(h->d_grads8);
     if (h->d_edge_local) cudaFree(h->d_edge_local);
@@ -437,8 +398,6 @@ int lsm_set_value_grid(lsm_handle* h, const lsm_grid_desc* g) {
     h->kp.has_vg = 1;
     size_t cells = 1;
     for (int k = 0; k < g->ndim; ++k) cells *= (size_t)g->shape[k];
-    h->persist_bytes = cells * sizeof(float);
-    if (h->persist_bytes > h->max_window) h->persist_bytes = h->max_window;
     // corner-packed copy for the pair kernel (one aligned chunk per lookup; the same table serves the float64 and the
     // float32 lookups); lsm_tuning.packed_grid = 0 keeps the scattered gathers; tables larger than 2 GiB are not built.
     DeviceGuard guard(h->device);
@@ -482,19 +441,13 @@ int lsm_set_ttr_grid(lsm_handle* h, const lsm_grid_desc* g) {
 int lsm_set_tuning(lsm_handle* h, const lsm_tuning* t) {
     if (h == nullptr || t == nullptr) return fail(1, "lsm_set_tuning: null argument");
     if (t->chunks < 0 || t->chunks > 16) return fail(2, "lsm_set_tuning: chunks must be 0 (automatic) or 1..16");
-    if (t->pair_placement != -1 && t->pair_placement != 0 && t->pair_placement != 2 && t->pair_placement != 3 && t->pair_placement != 4) {
-#ifdef LSM_EXPERIMENTS
-        if (t->pair_placement != 1)
-#endif
+    if (t->pair_placement != -1 && t->pair_placement != 0 && t->pair_placement != 2 && t->pair_placement != 3 && t->pair_placement != 4)
         return fail(2, "lsm_set_tuning: pair_placement must be -1 (automatic), 0 (behind the emit kernel), 2 (in front of the agent kernel), 3 (between them) or 4 (tail of the agent kernel)");
-    }
     if (t->packed_grid < -1 || t->packed_grid > 1) return fail(2, "lsm_set_tuning: packed_grid must be -1, 0 or 1");
     if (t->use_graph < -1 || t->use_graph > 1) return fail(2, "lsm_set_tuning: use_graph must be -1, 0 or 1");
     if (h->have_buffers || h->kp.has_vg) return fail(5, "lsm_set_tuning: call it right after lsm_create (before lsm_set_value_grid / lsm_bind_buffers)");
     h->tuning = *t;
-    // placement 1 (lab build) has no float32 form: a float32 handle keeps its placement (see lsm_create)
-    const bool f32 = (h->kp.c.flags & LSM_FLAG_INTERP_FLOAT32) != 0;
-    if (t->pair_placement >= 0 && !(f32 && t->pair_placement == 1)) h->pair_placement = t->pair_placement;
+    if (t->pair_placement >= 0) h->pair_placement = t->pair_placement;
     return 0;
 }
 
@@ -545,7 +498,7 @@ int lsm_bind_buffers(lsm_handle* h, const lsm_buffers* b) {
         if (h->d_emit_rec) { cudaFree(h->d_emit_rec); h->d_emit_rec = nullptr; }
         const size_t N = (size_t)h->kp.N;
         cudaError_t e = cudaMalloc(&h->d_pairval, (size_t)b->num_envs * N * N * sizeof(double));
-        if (e == cudaSuccess) e = cudaMalloc(&h->d_emit_rec, (size_t)b->num_envs * (size_t)h->geo.rec_bytes);
+        if (e == cudaSuccess) e = cudaMalloc(&h->d_emit_rec, (size_t)b->num_envs * (size_t)h->tab.rec_bytes);
         if (e != cudaSuccess) return cuda_fail(e, "lsm_bind_buffers: scratch allocation");
         h->kp.emit_rec = h->d_emit_rec;
         h->pairval_valid = false;
@@ -555,7 +508,6 @@ int lsm_bind_buffers(lsm_handle* h, const lsm_buffers* b) {
 
 int lsm_get_launch_info(lsm_handle* h, lsm_launch_info* out) {
     if (h == nullptr || out == nullptr) return fail(1, "lsm_get_launch_info: null argument");
-    DeviceGuard guard(h->device);
     const long long ngroups = h->have_buffers ? (h->kp.b.num_envs + h->kp.EPW - 1) / h->kp.EPW : 0;
     long long blocks = (ngroups + h->warps_per_block - 1) / h->warps_per_block;
     if (!h->spec && blocks > h->grid_cap) blocks = h->grid_cap;
@@ -563,21 +515,13 @@ int lsm_get_launch_info(lsm_handle* h, lsm_launch_info* out) {
     out->envs_per_warp = h->kp.EPW; out->smem_bytes_per_block = h->smem_per_block; out->regs_per_thread = h->regs;
     out->blocks_per_sm = h->blocks_per_sm; out->sm_count = h->sm_count;
     out->specialised = h->spec ? 1 : 0;
-    out->emit_block_threads = h->spec ? h->geo.emit_threads : 0;
-    out->emit_smem_bytes_per_block = h->spec ? h->geo.emit_smem : 0;
-    out->emit_regs_per_thread = h->emit_regs; out->emit_blocks_per_sm = h->emit_blocks_per_sm;
+    out->emit_block_threads = h->tab.emit_threads;
+    out->emit_smem_bytes_per_block = h->tab.emit_smem;
+    out->emit_regs_per_thread = h->tab.emit_regs; out->emit_blocks_per_sm = h->tab.emit_blocks_per_sm;
     const bool pair_path_li = h->spec && (h->kp.c.flags & LSM_FLAG_USE_SAFETY_FILTER) && h->kp.has_vg;
-    if (h->spec) {   // the emit kernel / grid lsm_step launches (room left for the pair kernel with placement "late")
-        int bps = 0, regs = 0;
-        if (lsm::spec_emit_blocks_per_sm(h->kp.c.dynamics, h->kp.N, h->kp.L, h->kp.O, (h->kp.c.flags & LSM_FLAG_INTERP_FLOAT32) != 0,
-                                         pair_path_li && h->pair_placement == 0,
-                                         pair_path_li && h->pair_placement == 1, &bps, &regs) == cudaSuccess) {
-            out->emit_blocks_per_sm = bps; out->emit_regs_per_thread = regs;
-        }
-    }
-    out->pair_regs_per_thread = h->pair_regs;
-    out->launches_per_step = h->spec ? ((pair_path_li && h->pair_placement != 1 && h->pair_placement != 4) ? 3 : 2) : 1;   // agent, emit [, pair]
-    out->emit_record_bytes = h->spec ? h->geo.rec_bytes : 0;
+    out->pair_regs_per_thread = h->tab.pair_regs;
+    out->launches_per_step = h->spec ? ((pair_path_li && h->pair_placement != 4) ? 3 : 2) : 1;   // agent, emit [, pair]
+    out->emit_record_bytes = h->tab.rec_bytes;
     {
         const int K = (h->spec && h->chunks > 1 && ngroups >= 4LL * h->chunks * h->warps_per_block) ? h->chunks : 1;
         out->chunks = K;
@@ -602,14 +546,8 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
     kp.env_mask = env_mask; kp.episode = (long long)episode; kp.seed = (unsigned long long)seed;
     const long long ngroups = (kp.b.num_envs + kp.EPW - 1) / kp.EPW;
     DeviceGuard guard(h->device);
-#ifdef LSM_EXPERIMENTS
-    { const char* dbg = std::getenv("LSM_DEBUG"); kp.debug = dbg ? std::atoi(dbg) : 0; }
-#else
-    kp.debug = 0;
-#endif
-    const void* persist = (h->l2_persist && mode == lsm::MODE_STEP && h->kp.has_vg && needs_vg) ? (const void*)h->kp.vg.values : nullptr;
-    const bool pair_path = h->spec && (c.flags & LSM_FLAG_USE_SAFETY_FILTER) && h->kp.has_vg && !(kp.debug & 2);
-    const int placement = (kp.debug & 32) ? 2 : h->pair_placement;   // LSM_DEBUG 32: K_a in front of the agent kernel on every step
+    const bool pair_path = h->spec && (c.flags & LSM_FLAG_USE_SAFETY_FILTER) && h->kp.has_vg;
+    const int placement = h->pair_placement;
     const bool was_valid = h->pairval_valid;
 
     const bool edges = h->spec && kp.edge_index != nullptr;
@@ -647,12 +585,13 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
             // previous launch (emit kernel / late pair kernel); recomputed here when the state was edited in between
             k.pairval = h->d_pairval;
             if (!was_valid || placement == 2) {
-                e = lsm::spec_launch_pair(k, s, persist, h->persist_bytes);
+                e = lsm::spec_launch_pair(k, h->tab, h->sm_count, s);
                 if (e != cudaSuccess) return e;
             }
         }
         // K_b (specialised: per-agent physics) or the fused generic kernel
-        e = lsm::kernel_launch(k, h->spec, (int)blocks, h->block_threads, h->smem_per_block, s, persist, h->persist_bytes);
+        e = lsm::kernel_launch(h->spec ? h->tab.agent : lsm::generic_ptr(c.dynamics), k, (unsigned)blocks, h->block_threads,
+                               h->smem_per_block, s, h->spec);
         if (e != cudaSuccess) return e;
         if (h->spec) {
             if (pair_path && placement == 3) {
@@ -660,7 +599,7 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
                 k.pairval = h->d_pairval;
                 k.pair_late = 0;
                 k.pair_rec = rec_fresh ? 1 : 0;
-                e = lsm::spec_launch_pair(k, s, persist, h->persist_bytes);
+                e = lsm::spec_launch_pair(k, h->tab, h->sm_count, s);
                 k.pair_rec = 0;
                 if (e != cudaSuccess) return e;
             }
@@ -668,7 +607,7 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
                 // fused COO output: where every graph's edges start (counts + prefix inside this range); the emit kernel of
                 // a later range also needs the totals of the earlier ones -> ordered by events, never by spinning
                 k.pairval = nullptr;
-                e = lsm::spec_launch_edge_count(k, s);
+                e = lsm::spec_launch_edge_count(k, h->tab, s);
                 if (e != cudaSuccess) return e;
                 if (nq > 1) {
                     if ((e = cudaEventRecord(h->ev_count[q], s)) != cudaSuccess) return e;
@@ -676,19 +615,16 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
                         if ((e = cudaStreamWaitEvent(s, h->ev_count[r], 0)) != cudaSuccess) return e;
                 }
             }
-            if (!(k.debug & 1)) {
-                // K_c: graph observation (persistent blocks) [+ the next step's pair values, placement 1]
-                const bool pie = pair_path && placement == 1;
-                k.pairval = pie ? h->d_pairval : nullptr;
-                e = lsm::spec_launch_emit(k, s, persist, h->persist_bytes, pair_path && placement == 0, pie);
-                if (e != cudaSuccess) return e;
-            }
+            // K_c: graph observation (persistent blocks)
+            k.pairval = nullptr;
+            e = lsm::spec_launch_emit(k, h->tab, h->sm_count, s);
+            if (e != cudaSuccess) return e;
             if (pair_path && placement == 0) {
                 // K_a for the NEXT step, beside the emit kernel's drain (see lsm_pair_kernel)
                 k.pairval = h->d_pairval;
-                k.pair_late = (k.debug & 1) ? 0 : 1;
+                k.pair_late = 1;
                 k.pair_rec = rec_fresh ? 1 : 0;
-                e = lsm::spec_launch_pair(k, s, persist, h->persist_bytes);
+                e = lsm::spec_launch_pair(k, h->tab, h->sm_count, s);
                 if (e != cudaSuccess) return e;
             }
         }
@@ -699,8 +635,7 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
     const int K = (h->spec && h->chunks > 1 && ngroups >= 4LL * h->chunks * h->warps_per_block) ? h->chunks : 1;
     // graph replay: single-range steps of the specialised pipeline (the launch-latency-bound sizes); opt-in - measured on
     // B200 it cuts the host time of a step from ~25 to ~9 us but adds ~1 us of device time (DESIGN.md 3)
-    bool use_graph = h->spec && K == 1 && mode == lsm::MODE_STEP && h->tuning.use_graph == 1 && kp.timeline == nullptr &&
-                     kp.debug == 0 && persist == nullptr;
+    bool use_graph = h->spec && K == 1 && mode == lsm::MODE_STEP && h->tuning.use_graph == 1 && kp.timeline == nullptr;
     if (use_graph) {
         cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
         if (cudaStreamIsCapturing((cudaStream_t)stream, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone) {
@@ -775,8 +710,8 @@ static int launch(lsm_handle* h, int mode, int flag, const int32_t* action_idx, 
     if (h->spec) {
         h->pairval_valid = false;
         if (pair_path && (placement == 0 || placement == 3)) h->pairval_valid = true;
-        // placements 1 and 4: a masked reset refreshes only the masked environments, the others keep what they had
-        if (pair_path && ((placement == 1 && !(kp.debug & 1)) || placement == 4))
+        // placement 4: a masked reset refreshes only the masked environments, the others keep what they had
+        if (pair_path && placement == 4)
             h->pairval_valid = env_mask == nullptr ? true : (was_valid && mode != lsm::MODE_STEP);
     }
     return 0;
@@ -1141,21 +1076,13 @@ int lsm_emit_only(lsm_handle* h, void* stream) {
     lsm::KParams kp = h->kp;
     kp.mode = lsm::MODE_OBSERVE; kp.env_mask = nullptr;
     DeviceGuard guard(h->device);
-#ifdef LSM_EXPERIMENTS
-    { const char* dbg = std::getenv("LSM_DEBUG"); kp.debug = dbg ? std::atoi(dbg) : 0; }
-#else
-    kp.debug = 0;
-#endif
     kp.pair_late = 0;
     kp.grp_begin = 0; kp.env_begin = 0; kp.env_end = (int)kp.b.num_envs;
     if (kp.edge_index != nullptr && h->chunks > 1) kp.edge_index = nullptr;   // the per-range prefixes of a chunked step do not describe one launch
     kp.edge_range = 0; kp.edge_num_ranges = 1;
     kp.edge_envs_per_block = lsm::edge_count_envs_per_block(kp.b.num_envs); kp.edge_block_ofs = 0;
-    const bool pair_path = (kp.c.flags & LSM_FLAG_USE_SAFETY_FILTER) && kp.has_vg && !(kp.debug & 2);
-    const int placement = (kp.debug & 32) ? 2 : h->pair_placement;
-    const bool pie = pair_path && placement == 1;     // the same kernel, grid and work as inside lsm_step
-    kp.pairval = pie ? h->d_pairval : nullptr;
-    cudaError_t e = lsm::spec_launch_emit(kp, (cudaStream_t)stream, nullptr, 0, pair_path && placement == 0, pie);
+    kp.pairval = nullptr;     // the same kernel, grid and work as inside lsm_step
+    cudaError_t e = lsm::spec_launch_emit(kp, h->tab, h->sm_count, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "lsm_emit_only");
     return 0;
 }
@@ -1166,7 +1093,7 @@ int lsm_copy_records(lsm_handle* h, void* dst, void* stream) {
     if (!h->have_buffers) return fail(5, "lsm_copy_records: lsm_bind_buffers has not been called");
     if (dst == nullptr) return fail(2, "lsm_copy_records: null destination");
     DeviceGuard guard(h->device);
-    const size_t bytes = (size_t)h->kp.b.num_envs * (size_t)h->geo.rec_bytes;
+    const size_t bytes = (size_t)h->kp.b.num_envs * (size_t)h->tab.rec_bytes;
     const cudaError_t e = cudaMemcpyAsync(dst, h->d_emit_rec, bytes, cudaMemcpyDefault, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "lsm_copy_records");
     return 0;
@@ -1188,7 +1115,7 @@ int lsm_emit_from_records(lsm_handle* h, const lsm_record_emit_io* io, void* str
     a.node_obs = io->node_obs; a.adj = io->adj;
     a.sel_tab = h->kp.sel_tab; a.r2_lt = h->kp.r2_lt; a.r2_nz = h->kp.r2_nz;
     a.gfeat = (h->kp.c.flags & LSM_FLAG_GRAPH_FEAT_GLOBAL) != 0;
-    const cudaError_t e = lsm::spec_launch_record_emit(h->kp.c.dynamics, h->kp.N, h->kp.L, h->kp.O, a, (cudaStream_t)stream);
+    const cudaError_t e = lsm::spec_launch_record_emit(h->tab, h->sm_count, a, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "lsm_emit_from_records");
     return 0;
 }
@@ -1214,8 +1141,7 @@ int lsm_edges_from_records(lsm_handle* h, const lsm_record_edges_io* io, void* s
     a.counts = io->counts; a.offsets = (const long long*)io->offsets;
     a.edge_index = (long long*)io->edge_index; a.edge_attr = io->edge_attr; a.capacity = io->capacity;
     a.sel_tab = h->kp.sel_tab; a.r2_lt = h->kp.r2_lt; a.r2_nz = h->kp.r2_nz;
-    const cudaError_t e = lsm::spec_launch_record_edges(h->kp.c.dynamics, h->kp.N, h->kp.L, h->kp.O, a, (long long*)io->offsets,
-                                                        fill, (cudaStream_t)stream);
+    const cudaError_t e = lsm::spec_launch_record_edges(h->tab, h->sm_count, a, (long long*)io->offsets, fill, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "lsm_edges_from_records");
     return 0;
 }
@@ -1255,7 +1181,7 @@ int lsm_safety_filter(lsm_handle* h, const lsm_filter_io* io, void* stream) {
     a.ego = io->ego; a.others = io->others; a.ego_action = io->ego_action; a.other_actions = io->other_actions;
     a.active = io->active; a.sep = io->separation_distance;
     a.safe_action = io->safe_action; a.filtered = io->filtered; a.index = io->index; a.value = io->value;
-    const cudaError_t e = lsm::safety_filter_launch(h->kp, a, (cudaStream_t)stream);
+    const cudaError_t e = lsm::safety_filter_launch(h->kp, h->sm_count, a, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "lsm_safety_filter");
     return 0;
 }
@@ -1272,7 +1198,7 @@ int lsm_hj_lookup(lsm_handle* h, const lsm_lookup_io* io, void* stream) {
     lsm::LookupArgs a;
     a.points = io->num_points; a.rel = io->rel; a.ego = io->ego; a.other = io->other; a.sep = io->separation_distance;
     a.value = io->value; a.grad = io->grad; a.rel_out = io->rel_out;
-    const cudaError_t e = lsm::hj_lookup_launch(h->kp, a, (cudaStream_t)stream);
+    const cudaError_t e = lsm::hj_lookup_launch(h->kp, h->sm_count, a, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_lookup");
     return 0;
 }
@@ -1299,39 +1225,5 @@ int lsm_debug_timeline(lsm_handle* h, int arm, uint64_t* out_ns) {
     }
     return 0;
 }
-
-#ifdef LSM_EXPERIMENTS
-// Lab build only: per env group (%globaltimer ns, clock64) at each phase boundary of the specialised agent kernel,
-// [ngroups][lsm::kPhaseSlots][2] uint64 (tools/agent_phases.py). `out` (capacity `cap` uint64) receives the stamps of the
-// steps since the last arm; returns the number of uint64 written through *n_out. arm = 1 clears and keeps stamping.
-int lsm_debug_phase_stamps(lsm_handle* h, int arm, uint64_t* out, long long cap, long long* n_out) {
-    if (h == nullptr) return fail(1, "lsm_debug_phase_stamps: null handle");
-    if (!h->have_buffers) return fail(5, "lsm_debug_phase_stamps: lsm_bind_buffers has not been called");
-    DeviceGuard guard(h->device);
-    cudaError_t e;
-    const size_t words = (size_t)((h->kp.b.num_envs + h->kp.EPW - 1) / h->kp.EPW) * lsm::kPhaseSlots * 2;
-    if (n_out != nullptr) *n_out = 0;
-    if (out != nullptr && h->d_phase != nullptr) {
-        if ((long long)words > cap) return fail(2, "lsm_debug_phase_stamps: output too small");
-        if ((e = cudaDeviceSynchronize()) != cudaSuccess) return cuda_fail(e, "lsm_debug_phase_stamps");
-        if ((e = cudaMemcpy(out, h->d_phase, words * sizeof(uint64_t), cudaMemcpyDeviceToHost)) != cudaSuccess)
-            return cuda_fail(e, "lsm_debug_phase_stamps");
-        if (n_out != nullptr) *n_out = (long long)words;
-    }
-    if (arm) {
-        if (h->phase_bytes < words * sizeof(uint64_t)) {
-            if (h->d_phase) cudaFree(h->d_phase);
-            h->d_phase = nullptr; h->phase_bytes = 0;
-            if ((e = cudaMalloc(&h->d_phase, words * sizeof(uint64_t))) != cudaSuccess) return cuda_fail(e, "lsm_debug_phase_stamps");
-            h->phase_bytes = words * sizeof(uint64_t);
-        }
-        if ((e = cudaMemset(h->d_phase, 0, words * sizeof(uint64_t))) != cudaSuccess) return cuda_fail(e, "lsm_debug_phase_stamps");
-        h->kp.phase_stamps = h->d_phase;
-    } else {
-        h->kp.phase_stamps = nullptr;
-    }
-    return 0;
-}
-#endif
 
 }  // extern "C"

@@ -88,7 +88,6 @@ struct KParams {
     int ngroups;               // ceil(num_envs / EPW); with chunked launches: END of this launch's env-group range
     int grp_begin;             // first env group of this launch (chunked multi-stream launches; 0 otherwise)
     int env_begin, env_end;    // the same range in environments (emit / pair kernels)
-    int debug;                 // LSM_DEBUG experiment switches (0 in production): 1 skip graph emission, 2 skip HJ pair lookups, 4 skip node rows, 8 skip adjacency stores
     const uint32_t* sel_tab;   // [N][W] entities whose owner agent is <= i
     // exact squared thresholds (host): lt(T) = min{t : sqrt_rn(t) >= T} so that d < T <=> d2 < lt(T);
     //                                  gt(T) = min{t : sqrt_rn(t) >  T} so that d > T <=> d2 >= gt(T)
@@ -122,11 +121,6 @@ struct KParams {
     int edge_range, edge_num_ranges;
     int edge_dense;                 // 1: the dense adjacency is written as well
     unsigned long long* timeline;   // diagnostics (lsm_debug_timeline), NULL in production: globaltimer min-start / max-end per kernel
-#ifdef LSM_EXPERIMENTS
-    // lab build only (lsm_debug_phase_stamps): [ngroups][kPhaseSlots][2] (%globaltimer, clock64) of every env group of the
-    // specialised agent kernel at its phase boundaries; NULL = off
-    unsigned long long* phase_stamps;
-#endif
 };
 
 // lsm_emit_from_records: items (record, observer) of a caller-owned record store, re-emitted with a handle's constants
@@ -162,32 +156,6 @@ enum { TL_PAIR_START = 0, TL_PAIR_BODY_END, TL_AGENT_START, TL_AGENT_END, TL_EMI
 __device__ __forceinline__ unsigned long long globaltimer_ns() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
 __device__ __forceinline__ void tl_start(unsigned long long* tl, int slot) { if (tl != nullptr && threadIdx.x == 0) atomicMin(tl + slot, globaltimer_ns()); }
 __device__ __forceinline__ void tl_end(unsigned long long* tl, int slot) { if (tl != nullptr && threadIdx.x == 0) atomicMax(tl + slot, globaltimer_ns()); }
-
-// Phase boundaries of lsm_agent_kernel (lab build, tools/agent_phases.py): slot k is stamped when a warp has finished
-// phase k-1 of one env group. The product library compiles none of this.
-enum {
-    PH_GROUP_START = 0,   // after the grid-dependency wait / top of the group loop
-    PH_LOADS,             // P0: prefetches, env and agent state loads
-    PH_LANDMARKS,         // landmark tables into shared memory, curriculum
-    PH_FILTER,            // P1: action decode, safety filter, integration
-    PH_GOAL,              // P2: goal / reward / done
-    PH_OTHERS,            // other-agent pass, bookkeeping, reward / done stores
-    PH_RESET,             // episode summary and auto-reset
-    PH_WRITEBACK,         // state write-back
-    PH_EMIT_REC,          // emit records to global memory
-    kPhaseSlots
-};
-#ifdef LSM_EXPERIMENTS
-__device__ __forceinline__ void phase_stamp(unsigned long long* ps, int grp, int slot, int lane) {
-    if (ps != nullptr && lane == 0) {
-        unsigned long long* p = ps + ((size_t)grp * kPhaseSlots + slot) * 2;
-        p[0] = globaltimer_ns(); p[1] = (unsigned long long)clock64();
-    }
-}
-#define LSM_PHASE_STAMP(SLOT) phase_stamp(kp.phase_stamps, grp, (SLOT), lane)
-#else
-#define LSM_PHASE_STAMP(SLOT) ((void)0)
-#endif
 
 __device__ __forceinline__ double clipd(double v, double lo, double hi) { return v < lo ? lo : (v > hi ? hi : v); }
 __device__ __forceinline__ double pymax(double a, double b) { return (b > a) ? b : a; }

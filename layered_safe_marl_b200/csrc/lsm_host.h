@@ -3,32 +3,48 @@
 #include "lsm_device.cuh"
 
 namespace lsm {
-struct SpecGeometry {
-    int rec_bytes;        // sizeof(EmitRec): per-env record between the agent and the emit kernel
-    int scratch_bytes;    // sizeof(AgentScratch): per-env physics scratch of the agent kernel
-    int agent_block, pair_block;
+// The kernels and launch geometry of one specialised shape in one interpolation mode: lsm_create fills it once per handle
+// (spec_table, then spec_prepare) and every launcher of the specialised pipeline reads it.
+struct SpecTable {
+    const void* agent;        // lsm_agent_kernel
+    const void* pair;         // lsm_pair_kernel for the periodic-dimension mask pair_periodic (kPairPeriodic)
+    const void* pair_rt;      // the same kernel reading the mask from the bound grid (any other grid)
+    int pair_periodic;
+    const void* emit;
+    const void* edge_count;   // per-graph edge counts + range prefix for the fused COO output
+    int rec_bytes;            // sizeof(EmitRec): per-env record between the agent and the emit kernel
+    int scratch_bytes;        // sizeof(AgentScratch): per-env physics scratch of the agent kernel
+    int agent_block;
     int emit_smem, emit_threads;
+    int emit_regs, emit_blocks_per_sm, pair_regs;   // spec_prepare
+    const void* record_emit;  // lsm_record_emit_kernel (lsm_emit_from_records)
+    int record_emit_smem, record_emit_threads, record_emit_items;   // items in flight per block
+    const void* record_edge_count;  // lsm_record_emit_kernel_edge_count / _edge_fill (lsm_edges_from_records)
+    const void* record_edge_fill;
+    int record_edges_smem, record_edges_threads, record_edges_items;
 };
-bool spec_available(int dynamics, int N, int L, int O, SpecGeometry* g);
-// agent kernel (specialised) or the fused generic kernel
-// f32: the LSM_FLAG_INTERP_FLOAT32 instantiations of the agent / pair kernels (specialised path)
-cudaError_t kernel_prepare(int dynamics, int N, int L, int O, bool f32, bool spec, int smem_bytes, int block_threads, int* regs,
-                           int* blocks_per_sm);
-cudaError_t spec_prepare_aux(int dynamics, int N, int L, int O, bool f32, int* emit_regs, int* emit_blocks_per_sm, int* pair_regs);
+// the table of (dynamics, N, L, O) with the agent / pair kernels of the interpolation mode (f32: LSM_FLAG_INTERP_FLOAT32);
+// false (table zeroed): no specialisation, the shape runs the fused generic kernel
+bool spec_table(int dynamics, int N, int L, int O, bool f32, SpecTable* t);
+// dynamic shared memory opt-in of the emit kernel, its registers and resident blocks per SM, the pair kernel's registers
+cudaError_t spec_prepare(SpecTable* t);
+const void* generic_ptr(int dynamics);
+// dynamic shared memory opt-in of `fn`, its registers and resident blocks per SM
+cudaError_t kernel_prepare(const void* fn, int block_threads, int smem_bytes, int* regs, int* blocks_per_sm);
 cudaError_t upload_magnetic_tables(const double* cos_tab, const double* sin_tab);
-cudaError_t kernel_launch(const KParams& kp, bool spec, int grid_blocks, int block_threads, int smem_bytes,
-                          cudaStream_t stream, const void* persist_ptr, size_t persist_bytes);
-cudaError_t spec_launch_pair(const KParams& kp, cudaStream_t stream, const void* persist_ptr, size_t persist_bytes);
-cudaError_t spec_launch_emit(const KParams& kp, cudaStream_t stream, const void* persist_ptr, size_t persist_bytes, bool reserve_pair, bool pie);
-cudaError_t spec_emit_blocks_per_sm(int dynamics, int N, int L, int O, bool f32, bool reserve_pair, bool pie, int* out, int* regs);
-// lsm_record_emit_kernel of the shape (a shape without a specialisation: cudaErrorInvalidValue); no-op for zero items
-cudaError_t spec_launch_record_emit(int dynamics, int N, int L, int O, const RecordEmitArgs& a, cudaStream_t stream);
+// one kernel taking the KParams block; pdl: programmatic stream serialisation with the launch before it
+cudaError_t kernel_launch(const void* fn, const KParams& kp, unsigned grid_blocks, int block_threads, int smem_bytes,
+                          cudaStream_t stream, bool pdl);
+cudaError_t spec_launch_pair(const KParams& kp, const SpecTable& t, int sm_count, cudaStream_t stream);
+cudaError_t spec_launch_emit(const KParams& kp, const SpecTable& t, int sm_count, cudaStream_t stream);
+// lsm_record_emit_kernel of the shape; no-op for zero items
+cudaError_t spec_launch_record_emit(const SpecTable& t, int sm_count, const RecordEmitArgs& a, cudaStream_t stream);
 // lsm_record_emit_kernel_edge_count + lsm_edge_scan_kernel into `offsets` (fill == false), or
 // lsm_record_emit_kernel_edge_fill (fill == true); zero items: the count pass only sets offsets[0] = 0
-cudaError_t spec_launch_record_edges(int dynamics, int N, int L, int O, const RecordEdgesArgs& a, long long* offsets, bool fill,
+cudaError_t spec_launch_record_edges(const SpecTable& t, int sm_count, const RecordEdgesArgs& a, long long* offsets, bool fill,
                                      cudaStream_t stream);
 int edge_count_envs_per_block(long long envs);
-cudaError_t spec_launch_edge_count(const KParams& kp, cudaStream_t stream);
+cudaError_t spec_launch_edge_count(const KParams& kp, const SpecTable& t, cudaStream_t stream);
 cudaError_t world_graph_launch(const KParams& kp, int32_t* counts, long long* offsets, long long* edge_index, double* edge_weight,
                                long long capacity, cudaStream_t stream);
 cudaError_t pack_grid_launch(const GridDev& g, float* packed, long long cells);
@@ -63,8 +79,8 @@ struct LookupArgs {
     double* rel_out;                // [points][ND] or NULL
 };
 // lsm_filter_op.cuh: the handle's dynamics and interpolation mode; no-op for zero rows / points
-cudaError_t safety_filter_launch(const KParams& kp, const FilterOpArgs& a, cudaStream_t stream);
-cudaError_t hj_lookup_launch(const KParams& kp, const LookupArgs& a, cudaStream_t stream);
+cudaError_t safety_filter_launch(const KParams& kp, int sm_count, const FilterOpArgs& a, cudaStream_t stream);
+cudaError_t hj_lookup_launch(const KParams& kp, int sm_count, const LookupArgs& a, cudaStream_t stream);
 cudaError_t pad_grads_launch(const float* grads, float* grads8, long long cells);
 cudaError_t edge_list_launch(const float* adj, int32_t* counts, long long* offsets, long long* edge_index, float* edge_attr,
                              long long num_graphs, int E, long long capacity, cudaStream_t stream);

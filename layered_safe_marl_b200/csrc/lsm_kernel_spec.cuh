@@ -1002,7 +1002,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
         if (kp.mode == MODE_RESET && kp.env_mask != nullptr && env_on) env_on = kp.env_mask[env] != 0;
         const bool agent_on = env_on && ai < N;
         if (__ballot_sync(0xffffffffu, env_on) == 0u) continue;
-        LSM_PHASE_STAMP(PH_GROUP_START);
         const int nenv = (n - env0) < EPW ? (n - env0) : EPW;   // envs of this group
 
         // ---------------- P0: load ----------------
@@ -1079,7 +1078,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
             if constexpr (O > 0) nobst = aip[LSM_AI_NUM_OBST_COLLISIONS * fstride]; \
         }
         if (kp.mode != MODE_STEP) { LSM_LOAD_MOTION() LSM_LOAD_BOOKKEEPING(false) }
-        LSM_PHASE_STAMP(PH_LOADS);
         // landmark tables of the group's environments: contiguous runs per field
         {
             const int total = nenv * M;
@@ -1112,7 +1110,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
             if (ai == 0) { P.cur_sep = q.sep; P.cur_filter = q.world_filter ? 1 : 0; R.vel[2 * N] = make_double2(0.0, 0.0); }
         }
         __syncwarp();
-        LSM_PHASE_STAMP(PH_LANDMARKS);
 
         bool all_done_env = false;
         const unsigned any_filter = __ballot_sync(0xffffffffu, env_on && q.world_filter);
@@ -1194,7 +1191,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 }
                 __syncwarp();
             }
-            LSM_PHASE_STAMP(PH_FILTER);
             // ---------------- P2: goal / reward / done ----------------
             int goal_pre = 0, goal_post = 0, reached_post = reached, done_post = done;
             double rew = 0.0;
@@ -1279,7 +1275,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 s2 = s2q; s3 = s3q;
             }
             __syncwarp();
-            LSM_PHASE_STAMP(PH_GOAL);
             LSM_LOAD_BOOKKEEPING(true)
             if (agent_on) {
                 // one pass over the other agents: min distance, collisions, episode statistics, proximity rewards.
@@ -1293,10 +1288,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 unsigned pc_mask = 0u;
                 // airtaxi: the loop stays rolled (-5 % code in a kernel bound by instruction fetch: cfg3 0.3385 -> 0.3348 ms, same-box
                 // A/B); the double-integrator kernels measure the same either way and keep the unrolled loop
-#ifndef LSM_OTHERS_UNROLL
-#define LSM_OTHERS_UNROLL 0
-#endif
-                constexpr int kOthersUnroll = LSM_OTHERS_UNROLL > 0 ? LSM_OTHERS_UNROLL : (DYN == LSM_DYN_DOUBLE_INTEGRATOR ? N : 1);
+                constexpr int kOthersUnroll = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? N : 1;
 #pragma unroll kOthersUnroll
                 for (int a = 0; a < N; ++a) {
                     if (a == ai) continue;
@@ -1384,7 +1376,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
             }
             reached = reached_post; done = done_post;
             parity ^= 1;
-            LSM_PHASE_STAMP(PH_OTHERS);
         } else {
             if (agent_on) {
                 double vx, vy;
@@ -1478,7 +1469,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
         } else if (kp.mode == MODE_OBSERVE && agent_on) {
             emit_obs_row<DYN, N, L, O>(R, P, ai, goal_obs, x, y, s2, s3, kp.b.obs + ((size_t)env * N + ai) * Dobs);
         }
-        LSM_PHASE_STAMP(PH_RESET);
 
         // ---------------- state write-back ----------------
         if (kp.mode != MODE_OBSERVE) {
@@ -1509,7 +1499,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                 if constexpr (O > 0) aip[LSM_AI_NUM_OBST_COLLISIONS * fstride] = nobst;
             }
         }
-        LSM_PHASE_STAMP(PH_WRITEBACK);
         // ---------------- emit records -> global memory (consumed by lsm_emit_kernel; L2 resident) ----------------
         if (env_on && ai == 0) R.next_filter = q.world_filter ? 1 : 0;     // q follows a reset's new curriculum ratio
         if constexpr (DYN != LSM_DYN_DOUBLE_INTEGRATOR) {
@@ -1539,7 +1528,6 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
             if (kp.pair_tail) pair_tail_phase<DYN, N, L, O, F32>(&kp.vg, Rw, kp.pairval, env0, nenv, on_mask, lane);
         }
         __syncwarp();
-        LSM_PHASE_STAMP(PH_EMIT_REC);
     }
     tl_end(kp.timeline, TL_AGENT_END);
 }
@@ -1776,10 +1764,7 @@ __device__ __forceinline__ void node_feature_row(const EmitRec<DYN, N, L, O>& R,
     }
 }
 
-// PIE ("pair in emit"): also compute the next step's HJ pair values per environment after its copies are issued - the
-// placement that wins for few agents (one launch less; the lookups of an 8-agent environment occupy half a block once).
-// For many agents the per-block chain gets long and lsm_pair_kernel behind this kernel is faster (see lsm_capi.cu).
-template <int DYN, int N, int L, int O, int WPE, int MINB, bool PIE = false>
+template <int DYN, int N, int L, int O, int WPE, int MINB>
 __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_constant__ KParams kp) {
     using ES = EmitShared<DYN, N, L, O, WPE>;
     using REC = EmitRec<DYN, N, L, O>;
@@ -1792,52 +1777,11 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
     ES& S = *reinterpret_cast<ES*>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31;
     const double r2_lt = kp.r2_lt, r2_nz = kp.r2_nz;
-    // ablation switches exist only in the LSM_EXPERIMENTS build (liblsm_b200_exp.so); the product kernel has none
-#ifdef LSM_EXPERIMENTS
-    const int debug = kp.debug;
-    const int n = (int)kp.b.num_envs;
-#define LSM_DBG(bit) ((debug & (bit)) != 0)
-#else
-#define LSM_DBG(bit) false
-#endif
     // the dependents (normally lsm_pair_kernel, which does not wait at its top) are released only once the agent kernel
     // this launch depends on is complete and flushed
     pdl_wait();
     pdl_launch_dependents();
     tl_start(kp.timeline, TL_EMIT_START);
-#ifdef LSM_EXPERIMENTS
-    if (debug & 64) return;          // experiments: launch + block dispatch floor
-    if (debug & 512) {               // experiments: every bulk copy of this block back to back, nothing else
-        if (tid == 0) {
-            for (int ee = blockIdx.x; ee < n; ee += gridDim.x) {
-                if (GEO::ADJ_BULK) for (int i = 0; i < N; ++i) bulk_store(kp.b.adj + ((size_t)ee * N + i) * EE, S.dthr[0], (unsigned)EE * 4u);
-                if (GEO::NODE_BULK && NCHUNK == 1) bulk_store(kp.b.node_obs + (size_t)ee * (ROWS * F), S.nodes[0], (unsigned)(ROWS * F) * 4u);
-                bulk_store_commit();
-            }
-            bulk_store_wait_read<0>();
-        }
-        return;
-    }
-    if (debug & 2048) {              // experiments: the same bytes, classic grid-strided 16-byte stores (compact moving window)
-        const float4 v = make_float4(1.f, 2.f, 3.f, 4.f);
-        float4* a4 = reinterpret_cast<float4*>(kp.b.adj);
-        const size_t na = (size_t)n * N * EE / 4, nn = (size_t)n * ROWS * F / 4;
-        if (!(debug & 8)) for (size_t k = (size_t)blockIdx.x * T + tid; k < na; k += (size_t)gridDim.x * T) a4[k] = v;
-        float4* n4 = reinterpret_cast<float4*>(kp.b.node_obs);
-        if (!(debug & 4)) for (size_t k = (size_t)blockIdx.x * T + tid; k < nn; k += (size_t)gridDim.x * T) n4[k] = v;
-        return;
-    }
-    if (debug & 1024) {              // experiments: the same bytes with coalesced 16-byte stores from registers
-        const float4 v = make_float4(1.f, 2.f, 3.f, 4.f);
-        for (int ee = blockIdx.x; ee < n; ee += gridDim.x) {
-            float4* a4 = reinterpret_cast<float4*>(kp.b.adj + (size_t)ee * N * EE);
-            if (!(debug & 8)) for (int k = tid; k < N * EE / 4; k += T) a4[k] = v;
-            float4* n4 = reinterpret_cast<float4*>(kp.b.node_obs + (size_t)ee * (ROWS * F));
-            if (!(debug & 4)) for (int k = tid; k < ROWS * F / 4; k += T) n4[k] = v;
-        }
-        return;
-    }
-#endif
     const bool masked_reset = kp.mode == MODE_RESET && kp.env_mask != nullptr;
     // compact adjacency (host-facing callers, lsm_set_compact_adjacency): ONE thresholded E x E matrix per environment +
     // the per-observer keep masks instead of the N masked copies - 1/N of the adjacency bytes cross PCIe and the host
@@ -1877,20 +1821,9 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
         cp_async_commit();
         // (with the fused edge list every env is re-emitted: a masked reset shifts the offsets of all later graphs)
         if (masked_reset && kp.env_mask[ee] == 0 && !edges) continue;
-        if (LSM_DBG(128)) continue;   // experiments: + record load
         ++tiles;
         const REC& R = S.rec[rb];
         float* const dthr = S.dthr[tb];
-#ifdef LSM_EXPERIMENTS
-        if (debug & 256) {           // experiments: the bulk copies alone (whatever the tiles hold), no compute
-            if (tid == 0) {
-                if (GEO::ADJ_BULK) for (int i = 0; i < N; ++i) bulk_store(kp.b.adj + ((size_t)ee * N + i) * EE, dthr, (unsigned)EE * 4u);
-                if (GEO::NODE_BULK && NCHUNK == 1) bulk_store(kp.b.node_obs + (size_t)ee * (ROWS * F), S.nodes[tb], (unsigned)(ROWS * F) * 4u);
-                bulk_store_commit();
-            }
-            continue;
-        }
-#endif
         // (a) thresholded distance matrix: d2 in float64 against the exact squared radius; the stored float32 value is
         //     d2f * rsqrt(d2f). Thread a (one per entity) walks the circular distances d = 1 .. E/2 to entity a + d
         //     (for even E the last distance only needs a < E/2), so every unordered pair is visited once.
@@ -1953,8 +1886,8 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
         }
         // (d) adjacency
         float* abase = kp.b.adj + (size_t)ee * (N * EE);
-        const bool adj_bulk = GEO::ADJ_BULK && any_change == 0u && !LSM_DBG(16) && dense;
-        if (!LSM_DBG(8) && dense) {
+        const bool adj_bulk = GEO::ADJ_BULK && any_change == 0u && dense;
+        if (dense) {
             if (adj_bulk) {
                 // every observer sees the same matrix: mask it once in place; thread 0 sends it N times below
                 if (any_disc != 0u) {
@@ -2011,25 +1944,24 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
                 __syncthreads();
             }
             float* buf = S.nodes[nb];
-            if (!LSM_DBG(4))
-                for (int r = tid; r < nrows; r += T) node_row(r0 + r, buf + r * Fr);
+            for (int r = tid; r < nrows; r += T) node_row(r0 + r, buf + r * Fr);
             if (GEO::NODE_BULK || adj_bulk || compact) bulk_store_fence();
             __syncthreads();
             if (lane == 0) {
                 // the copies of one environment are issued by lane 0 of EVERY warp (observer i by warp i mod WPE, the node
                 // chunk by the last warp) instead of by one thread while the other 127 wait at the next barrier
                 const unsigned long long stream_pol = l2_evict_first();
-                if (adj_bulk && !adj_sent && !LSM_DBG(8)) {
+                if (adj_bulk && !adj_sent) {
 #pragma unroll 1
                     for (int i = warp; i < N; i += WPE) bulk_store(abase + i * EE, dthr, (unsigned)EE * 4u, stream_pol);
                 }
                 if (compact && GEO::ADJ_BULK && !adj_sent && warp == 0)
                     bulk_store(kp.adj_base + (size_t)ee * EE, dthr, (unsigned)EE * 4u, stream_pol);
-                if (GEO::NODE_BULK && !LSM_DBG(4) && warp == WPE - 1) bulk_store(nbase + r0 * Fr, buf, (unsigned)(nrows * Fr) * 4u, stream_pol);
+                if (GEO::NODE_BULK && warp == WPE - 1) bulk_store(nbase + r0 * Fr, buf, (unsigned)(nrows * Fr) * 4u, stream_pol);
                 bulk_store_commit();
             }
             adj_sent = true;
-            if (!GEO::NODE_BULK && !LSM_DBG(4)) {
+            if (!GEO::NODE_BULK) {
                 const int nfl = nrows * Fr;
                 if (Fr % 2 == 0 && (ROWS * Fr) % 2 == 0) {
                     for (int q = tid; q < nfl / 2; q += T)
@@ -2040,26 +1972,11 @@ __global__ void __launch_bounds__(32 * WPE, MINB) lsm_emit_kernel(const __grid_c
                 __syncthreads();
             }
         }
-        // (e) PIE: HJ values of every ordered agent pair for the NEXT step (safety_filter.py:192-201, 345-354): they depend
-        //     only on the state this step leaves behind; the lookups overlap this environment's copies draining to HBM.
-        if constexpr (PIE) {
-            if (kp.pairval != nullptr && R.next_filter) {
-                double* pv = kp.pairval + (size_t)ee * (N * N);
-                for (int t = tid; t < N * N; t += T) {
-                    const int i = t / N, j = t - i * N;
-                    if (i == j || R.done[1][i] || R.done[1][j]) continue;
-                    double rel[DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5];
-                    pair_rel_rec<DYN, N, L, O>(R, i, j, rel);
-                    pv[t] = pair_value_rel<DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5, kPeriodicRuntime>(kp.vg, rel);
-                }
-            }
-        }
     }
     // every bulk copy issued by this block has finished READING shared memory before the block retires
     if (lane == 0) bulk_store_wait_read<0>();
     cp_async_wait_all();
     tl_end(kp.timeline, TL_EMIT_END);
-#undef LSM_DBG
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -22,7 +22,6 @@
 #include "lsm_host.h"
 
 #include <climits>
-#include <cstdlib>
 
 namespace lsm {
 
@@ -30,9 +29,6 @@ namespace lsm {
 // host-side launch helpers (used by lsm_capi.cu)
 // ---------------------------------------------------------------------------------------------
 // (dynamics, N, L, O, warps per env of the emit kernel, resident emit blocks per SM the register budget targets)
-#ifndef LSM_AIR_WPE
-#define LSM_AIR_WPE 4
-#endif
 // BASELINE.json's benchmark shapes (8 / 3 / 32 double-integrator agents, 10 airtaxi agents) and the shapes the
 // reference's own scripts ship with (train.sh: 4 agents, 2 landmarks, either dynamics; eval_airtaxi.sh: 8 and 16 agents;
 // eval_double_integrator.sh: 4 agents; the 16-agent dense golden rollout)
@@ -45,11 +41,11 @@ namespace lsm {
     X(LSM_DYN_DOUBLE_INTEGRATOR, 32, 2, 0, 4, 3)       \
     X(LSM_DYN_DOUBLE_INTEGRATOR, 4, 2, 0, 2, 8)        \
     X(LSM_DYN_DOUBLE_INTEGRATOR, 16, 2, 0, 4, 4)       \
-    X(LSM_DYN_AIRTAXI, 10, 2, 0, LSM_AIR_WPE, 5)       \
+    X(LSM_DYN_AIRTAXI, 10, 2, 0, 4, 5)                 \
     X(LSM_DYN_AIRTAXI, 4, 2, 0, 2, 8)                  \
     X(LSM_DYN_AIRTAXI, 8, 2, 0, 2, 5)                  \
     X(LSM_DYN_AIRTAXI, 16, 2, 0, 4, 4)                 \
-    X(LSM_DYN_AIRTAXI, 10, 2, 4, LSM_AIR_WPE, 5)       \
+    X(LSM_DYN_AIRTAXI, 10, 2, 4, 4, 5)                 \
     X(LSM_DYN_DOUBLE_INTEGRATOR, 8, 2, 4, 4, 4)
 
 // Launch shape of the emit kernel for a shape built on demand (-DLSM_SHAPE below; _build.build_shape), derived
@@ -86,104 +82,42 @@ using ShapeLaunchT = ShapeLaunch<kShapeDyn, kShapeN, kShapeL, kShapeO>;
 constexpr int kAgentBlock = 128;
 constexpr int kAgentMinB = 2;
 constexpr int kPairBlock = kPairThreads;
-// SM room the emit grid leaves for pair blocks (placement "late") and the late pair kernel's grid bound. Swept on B200
-// with the record-reading pair kernel (profiles/experiments/r03_pair_kernel_sweep.txt, r03_pair_kernel_ab.txt): with no
-// room reserved the cfg2 emit kernel gets 6 instead of 5 blocks per SM and ends ~2.5 us earlier; the pair blocks then
-// start as emit blocks retire and finish the lookups in the emit kernel's tail (cfg2 -1.1 us against one reserved
-// block, cfg4 and cfg5 slightly faster too). A grid bound of 16 blocks per SM lets them fill the SMs the emit kernel frees.
-constexpr int kPairResident = 0;
+// Grid bound of the late pair kernel (placement 0). Swept on B200 with the record-reading pair kernel
+// (profiles/experiments/r03_pair_kernel_sweep.txt, r03_pair_kernel_ab.txt): the emit grid reserves no room for pair
+// blocks; they start as emit blocks retire and finish the lookups in the emit kernel's tail, and 16 blocks per SM lets
+// them fill the SMs the emit kernel frees.
 constexpr int kPairLateBlocksPerSm = 16;
 
-// The product library (liblsm_b200.so) has ONE instantiation per kernel and configuration and reads no environment
-// variable. Alternative kernel shapes and ablation switches are compiled only with -DLSM_EXPERIMENTS
-// (liblsm_b200_exp.so, `_build.build_experiments()`; selected by the tools with LSM_LIB=<path>).
-#ifdef LSM_EXPERIMENTS
-// LSM_AGENT_MINB=3 trades ~100-400 B of spills for 12 instead of 8 resident physics warps per SM
-static int agent_minb() {
-    static const int v = [] { const char* e = std::getenv("LSM_AGENT_MINB"); return e ? std::atoi(e) : 0; }();
-    return v;
-}
-static int env_int(const char* name, int dflt) { const char* e = std::getenv(name); return e ? std::atoi(e) : dflt; }
-#endif
-
 // The agent and pair kernels exist in two arithmetics of the HJ grid lookups (LSM_FLAG_INTERP_FLOAT32: float32, else
-// float64), chosen at compile time; spec_fns picks the pair of the handle's mode. The emit and edge-count kernels make no
-// grid lookups and serve both modes.
-struct SpecFns {
-    const void* pair;         // lsm_pair_kernel for the periodic-dimension mask pair_periodic (kPairPeriodic)
-    const void* pair_rt;      // the same kernel reading the mask from the bound grid (any other grid)
-    int pair_periodic;
-    const void* agent; const void* emit;
-    const void* emit_pie;     // emit kernel that also computes the next step's pair values (placement "emit")
-    const void* edge_count;   // per-graph edge counts + range prefix for the fused COO output
-    int rec_bytes, scratch_bytes, emit_smem, emit_threads;
-    const void* record_emit;  // lsm_record_emit_kernel (lsm_emit_from_records)
-    int record_emit_smem, record_emit_threads, record_emit_items;   // items in flight per block
-    const void* record_edge_count;  // lsm_record_emit_kernel_edge_count / _edge_fill (lsm_edges_from_records)
-    const void* record_edge_fill;
-    int record_edges_smem, record_edges_threads, record_edges_items;
-};
-
-#ifdef LSM_EXPERIMENTS
-// LSM_WPE=2|4 selects an alternative emit-kernel shape for the cfg2 specialisation
-template <int WPE_, int EMINB_>
-static void cfg2_emit_variant(SpecFns* f) {
-    f->emit = (const void*)lsm_emit_kernel<LSM_DYN_DOUBLE_INTEGRATOR, 8, 2, 0, WPE_, EMINB_>;
-    f->emit_pie = (const void*)lsm_emit_kernel<LSM_DYN_DOUBLE_INTEGRATOR, 8, 2, 0, WPE_, EMINB_, true>;
-    f->emit_smem = (int)sizeof(EmitShared<LSM_DYN_DOUBLE_INTEGRATOR, 8, 2, 0, WPE_>);
-    f->emit_threads = 32 * WPE_;
-}
-
-#endif
-
-static bool spec_fns_base(int dynamics, int N, int L, int O, bool f32, SpecFns* f);
-static bool spec_fns(int dynamics, int N, int L, int O, bool f32, SpecFns* f) {
-    if (!spec_fns_base(dynamics, N, L, O, f32, f)) return false;
-#ifdef LSM_EXPERIMENTS
-    if (dynamics == LSM_DYN_DOUBLE_INTEGRATOR && N == 8 && L == 2 && O == 0) {
-        const int w = env_int("LSM_WPE", 0);
-        if (w == 1) cfg2_emit_variant<1, 8>(f);
-        if (w == 2) cfg2_emit_variant<2, 8>(f);
-        if (w == 24) cfg2_emit_variant<2, 4>(f);    // two warps per block at half the occupancy target
-    }
-#endif
-    return true;
-}
-
-// LSM_AGENT_MINB=3 (lab build) has float64 instantiations only
-#ifdef LSM_EXPERIMENTS
-#define LSM_AGENT_FN(DYN_, N_, L_, O_, F32_) (agent_minb() == 3 && !(F32_) ? (const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, 3, false> \
-                                                                          : (const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, kAgentMinB, F32_>)
-#define LSM_EMIT_PIE_FN(DYN_, N_, L_, O_, WPE_, EMINB_) ((const void*)lsm_emit_kernel<DYN_, N_, L_, O_, WPE_, EMINB_, true>)
-#else
-#define LSM_AGENT_FN(DYN_, N_, L_, O_, F32_) ((const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, kAgentMinB, F32_>)
-#define LSM_EMIT_PIE_FN(DYN_, N_, L_, O_, WPE_, EMINB_) nullptr   /* "pair values inside the emit kernel": experiments only */
-#endif
-static bool spec_fns_base(int dynamics, int N, int L, int O, bool f32, SpecFns* f) {
+// float64), chosen at compile time; the table holds the pair of the handle's mode. The emit, edge-count and record
+// kernels make no grid lookups and serve both modes.
+bool spec_table(int dynamics, int N, int L, int O, bool f32, SpecTable* t) {
+    *t = SpecTable{};
 #define X(DYN_, N_, L_, O_, WPE_, EMINB_)                                                         \
     if (dynamics == DYN_ && N == N_ && L == L_ && O == O_) {                                      \
-        f->pair = f32 ? (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPairPeriodic<DYN_>, true>  \
+        t->agent = f32 ? (const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, kAgentMinB, true>  \
+                       : (const void*)lsm_agent_kernel<DYN_, N_, L_, O_, kAgentBlock, kAgentMinB, false>; \
+        t->pair = f32 ? (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPairPeriodic<DYN_>, true>  \
                       : (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPairPeriodic<DYN_>, false>; \
-        f->pair_rt = f32 ? (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPeriodicRuntime, true>  \
+        t->pair_rt = f32 ? (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPeriodicRuntime, true>  \
                          : (const void*)lsm_pair_kernel<DYN_, N_, L_, O_, kPeriodicRuntime, false>; \
-        f->pair_periodic = kPairPeriodic<DYN_>;                                                   \
-        f->agent = f32 ? LSM_AGENT_FN(DYN_, N_, L_, O_, true) : LSM_AGENT_FN(DYN_, N_, L_, O_, false); \
-        f->emit = (const void*)lsm_emit_kernel<DYN_, N_, L_, O_, WPE_, EMINB_>;                   \
-        f->emit_pie = LSM_EMIT_PIE_FN(DYN_, N_, L_, O_, WPE_, EMINB_);                            \
-        f->edge_count = (const void*)lsm_edge_count_kernel<DYN_, N_, L_, O_>;                     \
-        f->rec_bytes = (int)sizeof(EmitRec<DYN_, N_, L_, O_>);                                    \
-        f->scratch_bytes = (int)sizeof(AgentScratch<DYN_, N_, L_>);                               \
-        f->emit_smem = (int)sizeof(EmitShared<DYN_, N_, L_, O_, WPE_>);                           \
-        f->emit_threads = 32 * WPE_;                                                              \
-        f->record_emit = (const void*)lsm_record_emit_kernel<DYN_, N_, L_, O_>;                   \
-        f->record_emit_smem = RecordEmitGeom<DYN_, N_, L_, O_>::SMEM;                             \
-        f->record_emit_threads = RecordEmitGeom<DYN_, N_, L_, O_>::THREADS;                       \
-        f->record_emit_items = RecordEmitGeom<DYN_, N_, L_, O_>::GPB;                             \
-        f->record_edge_count = (const void*)lsm_record_emit_kernel_edge_count<DYN_, N_, L_, O_>;  \
-        f->record_edge_fill = (const void*)lsm_record_emit_kernel_edge_fill<DYN_, N_, L_, O_>;    \
-        f->record_edges_smem = RecordEdgesGeom<DYN_, N_, L_, O_>::SMEM;                           \
-        f->record_edges_threads = RecordEdgesGeom<DYN_, N_, L_, O_>::THREADS;                     \
-        f->record_edges_items = RecordEdgesGeom<DYN_, N_, L_, O_>::GPB;                           \
+        t->pair_periodic = kPairPeriodic<DYN_>;                                                   \
+        t->emit = (const void*)lsm_emit_kernel<DYN_, N_, L_, O_, WPE_, EMINB_>;                   \
+        t->edge_count = (const void*)lsm_edge_count_kernel<DYN_, N_, L_, O_>;                     \
+        t->rec_bytes = (int)sizeof(EmitRec<DYN_, N_, L_, O_>);                                    \
+        t->scratch_bytes = (int)sizeof(AgentScratch<DYN_, N_, L_>);                               \
+        t->agent_block = kAgentBlock;                                                             \
+        t->emit_smem = (int)sizeof(EmitShared<DYN_, N_, L_, O_, WPE_>);                           \
+        t->emit_threads = 32 * WPE_;                                                              \
+        t->record_emit = (const void*)lsm_record_emit_kernel<DYN_, N_, L_, O_>;                   \
+        t->record_emit_smem = RecordEmitGeom<DYN_, N_, L_, O_>::SMEM;                             \
+        t->record_emit_threads = RecordEmitGeom<DYN_, N_, L_, O_>::THREADS;                       \
+        t->record_emit_items = RecordEmitGeom<DYN_, N_, L_, O_>::GPB;                             \
+        t->record_edge_count = (const void*)lsm_record_emit_kernel_edge_count<DYN_, N_, L_, O_>;  \
+        t->record_edge_fill = (const void*)lsm_record_emit_kernel_edge_fill<DYN_, N_, L_, O_>;    \
+        t->record_edges_smem = RecordEdgesGeom<DYN_, N_, L_, O_>::SMEM;                           \
+        t->record_edges_threads = RecordEdgesGeom<DYN_, N_, L_, O_>::THREADS;                     \
+        t->record_edges_items = RecordEdgesGeom<DYN_, N_, L_, O_>::GPB;                           \
         return true;                                                                              \
     }
     LSM_SPEC_LIST(X)
@@ -191,23 +125,14 @@ static bool spec_fns_base(int dynamics, int N, int L, int O, bool f32, SpecFns* 
     return false;
 }
 
-static const void* generic_ptr(int dynamics) {
+const void* generic_ptr(int dynamics) {
     return dynamics == LSM_DYN_DOUBLE_INTEGRATOR ? (const void*)lsm_generic_kernel<LSM_DYN_DOUBLE_INTEGRATOR>
                                                  : (const void*)lsm_generic_kernel<LSM_DYN_AIRTAXI>;
 }
 
 static bool kp_interp_f32(const KParams& kp) { return (kp.c.flags & LSM_FLAG_INTERP_FLOAT32) != 0; }
 
-// the geometry is the same in both interpolation modes
-bool spec_available(int dynamics, int N, int L, int O, SpecGeometry* g) {
-    SpecFns f;
-    if (!spec_fns(dynamics, N, L, O, false, &f)) return false;
-    g->rec_bytes = f.rec_bytes; g->scratch_bytes = f.scratch_bytes; g->agent_block = kAgentBlock;
-    g->emit_smem = f.emit_smem; g->emit_threads = f.emit_threads; g->pair_block = kPairBlock;
-    return true;
-}
-
-static cudaError_t prepare_one(const void* fn, int block_threads, int smem_bytes, int* regs, int* blocks_per_sm) {
+cudaError_t kernel_prepare(const void* fn, int block_threads, int smem_bytes, int* regs, int* blocks_per_sm) {
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
     if (e != cudaSuccess) return e;
     cudaFuncAttributes fa;
@@ -217,22 +142,11 @@ static cudaError_t prepare_one(const void* fn, int block_threads, int smem_bytes
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, fn, block_threads, smem_bytes);
 }
 
-cudaError_t kernel_prepare(int dynamics, int N, int L, int O, bool f32, bool spec, int smem_bytes, int block_threads, int* regs,
-                           int* blocks_per_sm) {
-    SpecFns f;
-    const void* fn = generic_ptr(dynamics);
-    if (spec) { if (!spec_fns(dynamics, N, L, O, f32, &f)) return cudaErrorInvalidValue; fn = f.agent; }
-    return prepare_one(fn, block_threads, smem_bytes, regs, blocks_per_sm);
-}
-
-cudaError_t spec_prepare_aux(int dynamics, int N, int L, int O, bool f32, int* emit_regs, int* emit_blocks_per_sm, int* pair_regs) {
-    SpecFns f;
-    if (!spec_fns(dynamics, N, L, O, f32, &f)) return cudaErrorInvalidValue;
-    cudaError_t e = prepare_one(f.emit, f.emit_threads, f.emit_smem, emit_regs, emit_blocks_per_sm);
+cudaError_t spec_prepare(SpecTable* t) {
+    cudaError_t e = kernel_prepare(t->emit, t->emit_threads, t->emit_smem, &t->emit_regs, &t->emit_blocks_per_sm);
     if (e != cudaSuccess) return e;
-    if (f.emit_pie != nullptr) { int r = 0, b = 0; e = prepare_one(f.emit_pie, f.emit_threads, f.emit_smem, &r, &b); if (e != cudaSuccess) return e; }
     int bps = 0;
-    return prepare_one(f.pair, kPairBlock, 0, pair_regs, &bps);
+    return kernel_prepare(t->pair, kPairBlock, 0, &t->pair_regs, &bps);
 }
 
 cudaError_t upload_magnetic_tables(const double* cos_tab, const double* sin_tab) {
@@ -241,33 +155,18 @@ cudaError_t upload_magnetic_tables(const double* cos_tab, const double* sin_tab)
     return cudaMemcpyToSymbol(c_mag_sin, sin_tab, sizeof(double) * kMagSegments);
 }
 
-static cudaError_t launch_one(const void* fn, const KParams& kp, unsigned grid_blocks, int block_threads, int smem_bytes,
-                              cudaStream_t stream, const void* persist_ptr, size_t persist_bytes, bool pdl) {
+cudaError_t kernel_launch(const void* fn, const KParams& kp, unsigned grid_blocks, int block_threads, int smem_bytes,
+                          cudaStream_t stream, bool pdl) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid_blocks, 1, 1);
     cfg.blockDim = dim3((unsigned)block_threads, 1, 1);
     cfg.dynamicSmemBytes = (size_t)smem_bytes;
     cfg.stream = stream;
-    cudaLaunchAttribute attr[2];
+    cudaLaunchAttribute attr[1];
     int nattr = 0;
-#ifdef LSM_EXPERIMENTS
-    static const bool no_pdl = std::getenv("LSM_NO_PDL") != nullptr;
-#else
-    constexpr bool no_pdl = false;
-#endif
-    if (pdl && !no_pdl) {
+    if (pdl) {
         attr[nattr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr[nattr].val.programmaticStreamSerializationAllowed = 1;
-        ++nattr;
-    }
-    if (persist_ptr != nullptr && persist_bytes > 0) {
-        // keep the HJ value grid resident in L2 while the observation stream flows through it
-        attr[nattr].id = cudaLaunchAttributeAccessPolicyWindow;
-        attr[nattr].val.accessPolicyWindow.base_ptr = const_cast<void*>(persist_ptr);
-        attr[nattr].val.accessPolicyWindow.num_bytes = persist_bytes;
-        attr[nattr].val.accessPolicyWindow.hitRatio = 1.0f;
-        attr[nattr].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        attr[nattr].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
         ++nattr;
     }
     cfg.attrs = attr;
@@ -276,155 +175,56 @@ static cudaError_t launch_one(const void* fn, const KParams& kp, unsigned grid_b
     return cudaLaunchKernelExC(&cfg, fn, args);
 }
 
-cudaError_t kernel_launch(const KParams& kp, bool spec, int grid_blocks, int block_threads, int smem_bytes,
-                          cudaStream_t stream, const void* persist_ptr, size_t persist_bytes) {
-    SpecFns f;
-    const void* fn = generic_ptr(kp.c.dynamics);
-    if (spec) { if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, kp_interp_f32(kp), &f)) return cudaErrorInvalidValue; fn = f.agent; }
-#ifdef LSM_EXPERIMENTS
-    if (spec) {
-        // LSM_AGENT_SMEM=<bytes>: pad the agent kernel's dynamic shared memory so that fewer blocks fit an SM and the
-        // rest of the SM stays free for emit / pair blocks of another env range (overlap experiment)
-        static const int pad = env_int("LSM_AGENT_SMEM", 0);
-        if (pad > smem_bytes) {
-            static thread_local const void* done = nullptr;
-            if (done != fn) { cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, pad); done = fn; }
-            smem_bytes = pad;
-        }
-    }
-#endif
-    return launch_one(fn, kp, (unsigned)grid_blocks, block_threads, smem_bytes, stream, persist_ptr, persist_bytes, spec);
-}
-
-cudaError_t spec_launch_pair(const KParams& kp, cudaStream_t stream, const void* persist_ptr, size_t persist_bytes) {
-    SpecFns f;
-    if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, kp_interp_f32(kp), &f)) return cudaErrorInvalidValue;
+cudaError_t spec_launch_pair(const KParams& kp, const SpecTable& t, int sm_count, cudaStream_t stream) {
     // one thread per ordered pair i != j, 32-bit task indices in the kernel
     const long long tasks = (long long)(kp.env_end - kp.env_begin) * kp.N * (kp.N - 1);
     if (tasks > INT_MAX) return cudaErrorInvalidValue;
     int periodic = 0;
     for (int d = 0; d < kp.vg.ndim; ++d) periodic |= kp.vg.periodic[d] ? 1 << d : 0;
-    const void* fn = periodic == f.pair_periodic ? f.pair : f.pair_rt;
+    const void* fn = periodic == t.pair_periodic ? t.pair : t.pair_rt;
     long long blocks = (tasks + kPairBlock - 1) / kPairBlock;
     if (blocks < 1) blocks = 1;
-    if (kp.pair_late) {
-        // beside the emit kernel: a bounded number of resident blocks per SM, each striding over the pairs
-        static int sm_count = 0;
-        if (sm_count == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev); }
-        int bps = kPairLateBlocksPerSm;
-#ifdef LSM_EXPERIMENTS
-        { const int v = env_int("LSM_PAIR_BPS", 0); if (v >= 1) bps = v; }
-#endif
-        if (blocks > (long long)sm_count * bps) blocks = (long long)sm_count * bps;
-    }
-    return launch_one(fn, kp, (unsigned)blocks, kPairBlock, 0, stream, persist_ptr, persist_bytes, true);
+    // beside the emit kernel: a bounded number of resident blocks per SM, each striding over the pairs
+    if (kp.pair_late && blocks > (long long)sm_count * kPairLateBlocksPerSm) blocks = (long long)sm_count * kPairLateBlocksPerSm;
+    return kernel_launch(fn, kp, (unsigned)blocks, kPairBlock, 0, stream, true);
 }
 
-// resident emit blocks per SM: what fits, minus (when the pair kernel runs beside the emit kernel) enough registers /
-// threads for kPairResident pair blocks per SM
-static cudaError_t emit_blocks_per_sm(const SpecFns& f, bool reserve_pair, bool pie, int* out) {
-    int bps = 0;
-    const void* fn = (pie && f.emit_pie != nullptr) ? f.emit_pie : f.emit;
-#ifndef LSM_EXPERIMENTS
-    // the answer depends only on (kernel, reserve_pair): asked once per process, not on every launch (two occupancy /
-    // attribute queries cost more host time than the launch itself)
-    struct Memo { const void* fn; const void* pair; bool reserve; int bps; };
-    static thread_local Memo memo[32];
-    static thread_local int memo_n = 0;
-    for (int k = 0; k < memo_n; ++k)
-        if (memo[k].fn == fn && memo[k].pair == f.pair && memo[k].reserve == reserve_pair) { *out = memo[k].bps; return cudaSuccess; }
-#endif
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, fn, f.emit_threads, f.emit_smem);
-    if (e != cudaSuccess) return e;
-    if (bps < 1) return cudaErrorLaunchOutOfResources;
-    if (reserve_pair) {
-        cudaFuncAttributes fe, fp;
-        if ((e = cudaFuncGetAttributes(&fe, fn)) != cudaSuccess) return e;
-        if ((e = cudaFuncGetAttributes(&fp, f.pair)) != cudaSuccess) return e;
-        auto block_regs = [](int regs, int threads) { return ((regs * 32 + 255) / 256 * 256) * ((threads + 31) / 32); };
-        int resident = kPairResident;
-#ifdef LSM_EXPERIMENTS
-        { const int v = env_int("LSM_PAIR_RESIDENT", -1); if (v >= 0) resident = v; }
-#endif
-        const int need_regs = resident * block_regs(fp.numRegs, kPairBlock), need_thr = resident * kPairBlock;
-        while (bps > 1 && (65536 - bps * block_regs(fe.numRegs, f.emit_threads) < need_regs || 2048 - bps * f.emit_threads < need_thr)) --bps;
-    }
-#ifdef LSM_EXPERIMENTS
-    { const int v = env_int("LSM_EMIT_BPS", 0); if (v >= 1 && v < bps) bps = v; }
-#else
-    if (memo_n < 32) { memo[memo_n].fn = fn; memo[memo_n].pair = f.pair; memo[memo_n].reserve = reserve_pair; memo[memo_n].bps = bps; ++memo_n; }
-#endif
-    *out = bps;
-    return cudaSuccess;
-}
-
-cudaError_t spec_emit_blocks_per_sm(int dynamics, int N, int L, int O, bool f32, bool reserve_pair, bool pie, int* out, int* regs) {
-    SpecFns f;
-    if (!spec_fns(dynamics, N, L, O, f32, &f)) return cudaErrorInvalidValue;
-    if (regs != nullptr) {
-        cudaFuncAttributes fa;
-        cudaError_t e = cudaFuncGetAttributes(&fa, (pie && f.emit_pie != nullptr) ? f.emit_pie : f.emit);
-        if (e != cudaSuccess) return e;
-        *regs = fa.numRegs;
-    }
-    return emit_blocks_per_sm(f, reserve_pair, pie, out);
-}
-
-cudaError_t spec_launch_emit(const KParams& kp, cudaStream_t stream, const void* persist_ptr, size_t persist_bytes, bool reserve_pair, bool pie) {
-    SpecFns f;
-    if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, kp_interp_f32(kp), &f)) return cudaErrorInvalidValue;
+cudaError_t spec_launch_emit(const KParams& kp, const SpecTable& t, int sm_count, cudaStream_t stream) {
     // persistent blocks: as many as are resident at once, each loops over environments
-    static int sm_count = 0;
-    if (sm_count == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev); }
-    int bps = 0;
-    cudaError_t e = emit_blocks_per_sm(f, reserve_pair, pie, &bps);
-    if (e != cudaSuccess) return e;
-    unsigned grid = (unsigned)sm_count * (unsigned)bps;
+    unsigned grid = (unsigned)sm_count * (unsigned)t.emit_blocks_per_sm;
     if (grid > (unsigned)(kp.env_end - kp.env_begin)) grid = (unsigned)(kp.env_end - kp.env_begin);
     if (grid < 1) grid = 1;
-#ifdef LSM_EXPERIMENTS
-    { const unsigned v = (unsigned)env_int("LSM_EMIT_GRID", 0); if (v >= 1 && v < grid) grid = v; }
-#endif
-    if (pie && f.emit_pie == nullptr) return cudaErrorInvalidValue;
-    return launch_one(pie ? f.emit_pie : f.emit, kp, grid, f.emit_threads, f.emit_smem, stream, persist_ptr, persist_bytes, true);
+    return kernel_launch(t.emit, kp, grid, t.emit_threads, t.emit_smem, stream, true);
 }
 
-cudaError_t spec_launch_record_emit(int dynamics, int N, int L, int O, const RecordEmitArgs& a, cudaStream_t stream) {
-    SpecFns f;
-    if (!spec_fns(dynamics, N, L, O, false, &f)) return cudaErrorInvalidValue;
+cudaError_t spec_launch_record_emit(const SpecTable& t, int sm_count, const RecordEmitArgs& a, cudaStream_t stream) {
     if (a.num_items <= 0) return cudaSuccess;
-    static int sm_count = 0;
-    if (sm_count == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev); }
-    if (f.record_emit_smem > 48 * 1024) {
-        const cudaError_t e = cudaFuncSetAttribute(f.record_emit, cudaFuncAttributeMaxDynamicSharedMemorySize, f.record_emit_smem);
+    if (t.record_emit_smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(t.record_emit, cudaFuncAttributeMaxDynamicSharedMemorySize, t.record_emit_smem);
         if (e != cudaSuccess) return e;
     }
     // blocks loop over the items: at most as many as 8 blocks of 256 threads per SM (a full SM) hold
-    long long blocks = (a.num_items + f.record_emit_items - 1) / f.record_emit_items;
+    long long blocks = (a.num_items + t.record_emit_items - 1) / t.record_emit_items;
     if (blocks > 8LL * sm_count) blocks = 8LL * sm_count;
     void* args[] = { (void*)&a };
-    return cudaLaunchKernel(f.record_emit, dim3((unsigned)blocks), dim3((unsigned)f.record_emit_threads), args,
-                            (size_t)f.record_emit_smem, stream);
+    return cudaLaunchKernel(t.record_emit, dim3((unsigned)blocks), dim3((unsigned)t.record_emit_threads), args,
+                            (size_t)t.record_emit_smem, stream);
 }
 
-cudaError_t spec_launch_record_edges(int dynamics, int N, int L, int O, const RecordEdgesArgs& a, long long* offsets, bool fill,
+cudaError_t spec_launch_record_edges(const SpecTable& t, int sm_count, const RecordEdgesArgs& a, long long* offsets, bool fill,
                                      cudaStream_t stream) {
-    SpecFns f;
-    if (!spec_fns(dynamics, N, L, O, false, &f)) return cudaErrorInvalidValue;
     if (a.num_items <= 0) return fill ? cudaSuccess : cudaMemsetAsync(offsets, 0, sizeof(long long), stream);
-    static int sm_count = 0;
-    if (sm_count == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev); }
-    const void* fn = fill ? f.record_edge_fill : f.record_edge_count;
-    if (f.record_edges_smem > 48 * 1024) {
-        const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, f.record_edges_smem);
+    const void* fn = fill ? t.record_edge_fill : t.record_edge_count;
+    if (t.record_edges_smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, t.record_edges_smem);
         if (e != cudaSuccess) return e;
     }
     // blocks loop over the items, as in spec_launch_record_emit
-    long long blocks = (a.num_items + f.record_edges_items - 1) / f.record_edges_items;
+    long long blocks = (a.num_items + t.record_edges_items - 1) / t.record_edges_items;
     if (blocks > 8LL * sm_count) blocks = 8LL * sm_count;
     void* args[] = { (void*)&a };
-    cudaError_t e = cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3((unsigned)f.record_edges_threads), args,
-                                     (size_t)f.record_edges_smem, stream);
+    cudaError_t e = cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3((unsigned)t.record_edges_threads), args,
+                                     (size_t)t.record_edges_smem, stream);
     if (e != cudaSuccess || fill) return e;
     lsm_edge_scan_kernel<<<1, 1024, 0, stream>>>(a.counts, offsets, a.num_items);
     return cudaGetLastError();
@@ -438,13 +238,11 @@ int edge_count_envs_per_block(long long envs) {
     return (int)c;
 }
 
-cudaError_t spec_launch_edge_count(const KParams& kp, cudaStream_t stream) {
-    SpecFns f;
-    if (!spec_fns(kp.c.dynamics, kp.N, kp.L, kp.O, kp_interp_f32(kp), &f)) return cudaErrorInvalidValue;
+cudaError_t spec_launch_edge_count(const KParams& kp, const SpecTable& t, cudaStream_t stream) {
     const long long envs = kp.env_end - kp.env_begin;
     long long blocks = (envs + kp.edge_envs_per_block - 1) / kp.edge_envs_per_block;
     if (blocks < 1) blocks = 1;
-    return launch_one(f.edge_count, kp, (unsigned)blocks, 32 * kEdgeCountWarps, 0, stream, nullptr, 0, true);
+    return kernel_launch(t.edge_count, kp, (unsigned)blocks, 32 * kEdgeCountWarps, 0, stream, true);
 }
 
 cudaError_t world_graph_launch(const KParams& kp, int32_t* counts, long long* offsets, long long* edge_index, double* edge_weight,
@@ -497,13 +295,7 @@ cudaError_t math_eval_launch(int op, const double* a, const double* b, double* o
 }
 
 // the standalone filter operator: instantiation of the handle's dynamics and interpolation mode, on the caller's stream
-static int sm_count_cached() {
-    static int sm_count = 0;
-    if (sm_count == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev); }
-    return sm_count;
-}
-
-cudaError_t safety_filter_launch(const KParams& kp, const FilterOpArgs& a, cudaStream_t stream) {
+cudaError_t safety_filter_launch(const KParams& kp, int sm_count, const FilterOpArgs& a, cudaStream_t stream) {
     if (a.rows <= 0) return cudaSuccess;
     const bool f32 = kp_interp_f32(kp), di = kp.c.dynamics == LSM_DYN_DOUBLE_INTEGRATOR;
     const void* fn = di ? (f32 ? (const void*)lsm_safety_filter_kernel<LSM_DYN_DOUBLE_INTEGRATOR, true>
@@ -512,7 +304,7 @@ cudaError_t safety_filter_launch(const KParams& kp, const FilterOpArgs& a, cudaS
                                : (const void*)lsm_safety_filter_kernel<LSM_DYN_AIRTAXI, false>);
     // one tile of kFopRows rows per block; beyond 32 blocks per SM the blocks stride over the tiles
     long long blocks = (a.rows + kFopRows - 1) / kFopRows;
-    const long long cap = (long long)sm_count_cached() * 32;
+    const long long cap = (long long)sm_count * 32;
     if (blocks > cap) blocks = cap;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)blocks, 1, 1);
@@ -522,7 +314,7 @@ cudaError_t safety_filter_launch(const KParams& kp, const FilterOpArgs& a, cudaS
     return cudaLaunchKernelExC(&cfg, fn, args);
 }
 
-cudaError_t hj_lookup_launch(const KParams& kp, const LookupArgs& a, cudaStream_t stream) {
+cudaError_t hj_lookup_launch(const KParams& kp, int sm_count, const LookupArgs& a, cudaStream_t stream) {
     if (a.points <= 0) return cudaSuccess;
     const bool f32 = kp_interp_f32(kp), di = kp.c.dynamics == LSM_DYN_DOUBLE_INTEGRATOR;
     const void* fn = di ? (f32 ? (const void*)lsm_hj_lookup_kernel<LSM_DYN_DOUBLE_INTEGRATOR, true>
@@ -530,7 +322,7 @@ cudaError_t hj_lookup_launch(const KParams& kp, const LookupArgs& a, cudaStream_
                         : (f32 ? (const void*)lsm_hj_lookup_kernel<LSM_DYN_AIRTAXI, true>
                                : (const void*)lsm_hj_lookup_kernel<LSM_DYN_AIRTAXI, false>);
     long long blocks = (a.points + kLookupThreads - 1) / kLookupThreads;
-    const long long cap = (long long)sm_count_cached() * 64;
+    const long long cap = (long long)sm_count * 64;
     if (blocks > cap) blocks = cap;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)blocks, 1, 1);

@@ -1,12 +1,11 @@
-"""Step time of the float32 interpolation mode (args.interp_float32) on the specialised pipeline against the generic
-fused kernel, beside the float64 product, at the BASELINE shapes. bench.py's flushed method: a 256 MiB L2 flush before
+"""Step time of the float32 interpolation mode (args.interp_float32) on the specialised pipeline beside the float64
+product, at the BASELINE shapes. bench.py's flushed method: a 256 MiB L2 flush before
 every timed step, one CUDA event pair per step, an untimed lead-in of flushes so that the first timed launches are queued.
 
     python tools/interp32_bench.py --runs 3 [--workloads cfg2,cfg3,cfg3_obst4,cfg4] [--steps 60] [--out FILE]
 
-Arms, alternated run by run, each in a process of its own (the library is chosen when it is loaded):
+Arms, alternated run by run, each in a process of its own:
     f32_spec     product library, interp_float32=True   (specialised pipeline, float32 agent / pair kernels)
-    f32_generic  lab library (_build.build_experiments) with LSM_FORCE_GENERIC=1, interp_float32=True
     f64_spec     product library, float64 (the default)
 Every result line carries the card name, power limit and SM clocks read in the same process."""
 from __future__ import annotations
@@ -20,7 +19,7 @@ import sys
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 WORKLOADS = ('cfg2', 'cfg3', 'cfg3_obst4', 'cfg4')
-ARMS = ('f32_spec', 'f32_generic', 'f64_spec')
+ARMS = ('f32_spec', 'f64_spec')
 
 
 def gpu_facts():
@@ -88,18 +87,10 @@ def main():
     a = p.parse_args()
     if a.arm:
         return child(a)
-    sys.path.insert(0, REPO)
-    from layered_safe_marl_b200 import _build
-    exp = _build.EXP_LIB_PATH
-    if not os.path.exists(exp):
-        raise SystemExit(f"{exp} is missing: build the lab library first (_build.build_experiments())")
-    env_of = {'f32_spec': {}, 'f64_spec': {}, 'f32_generic': {'LSM_LIB': exp, 'LSM_FORCE_GENERIC': '1'}}
     lines = []
     for run in range(a.runs):
         for arm in ARMS:
             env = dict(os.environ, PYTHONDONTWRITEBYTECODE='1')
-            env.pop('LSM_LIB', None); env.pop('LSM_FORCE_GENERIC', None)
-            env.update(env_of[arm])
             out = subprocess.run([sys.executable, os.path.abspath(__file__), '--arm', arm, '--workloads', a.workloads,
                                   '--steps', str(a.steps), '--warmup', str(a.warmup)], env=env, capture_output=True, text=True)
             if out.returncode != 0:

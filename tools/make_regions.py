@@ -20,7 +20,7 @@ AGENT = [('prologue', 'lsm_agent_kernel(const __grid_constant__'), ('P0 prefetch
 EMIT = [('prologue + first record prefetch', 'lsm_emit_kernel(const __grid_constant__'), ('loop top: waits / prefetch issue', 'for (int ee = kp.env_begin + blockIdx.x'),
         ('distances', '(a) thresholded distance matrix'), ('masks', '(b) disconnected-entity bit masks'), ('adjacency (mask in place / direct stores)', '(d) adjacency'),
         ('node row builder', '(c) node features: one thread per'), ('node chunks + bulk copy issue', 'bool adj_sent = false;'),
-        ('PIE pair values (not instantiated)', '(e) PIE: HJ values'), ('drain', 'every bulk copy issued by this block has finished READING'),
+        ('drain', 'every bulk copy issued by this block has finished READING'),
         ('end', 'tl_end(kp.timeline, TL_EMIT_END)')]
 tab = AGENT if sys.argv[1] == 'agent' else EMIT
 pos = []

@@ -27,7 +27,7 @@ for t in range(K):
     env.step(acts[10 + t], episode)     # --b2b: warm L2 (no flush), but still one recorded step at a time
     rows.append(env.debug_timeline(True))
 keys = list(rows[0].keys())
-print(a.workload, 'b2b' if a.b2b else 'flushed', os.environ.get('LSM_DEBUG', ''))
+print(a.workload, 'b2b' if a.b2b else 'flushed')
 for k in keys:
     vals = [r[k] for r in rows if r[k] is not None]
     if vals:
