@@ -124,6 +124,8 @@ typedef struct lsm_config {
     double act_tab0[5], act_tab1[5];   /* np.linspace tables of environment.py:387-410 */
 } lsm_config;
 
+/* lsm_set_value_grid / lsm_set_ttr_grid refuse (code 2) a descriptor with a dimension of fewer than 2 nodes or with
+ * 2^31 cells or more, before reading any array; a refused call leaves the grid bound before it in place. */
 typedef struct lsm_grid_desc {
     int32_t ndim;
     int32_t shape[5];

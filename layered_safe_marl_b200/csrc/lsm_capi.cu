@@ -2,6 +2,7 @@
 // Host-only logic: validation, shared-memory layout, lookup tables, launch geometry.
 #include <algorithm>
 #include <atomic>
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -371,22 +372,31 @@ int lsm_destroy(lsm_handle* h) {
     return 0;
 }
 
+// Validates the descriptor completely before it touches the handle: a refused grid leaves the bound one (and its packed
+// table and padded gradient rows) in place. Every lookup (stencil32_setup, stencil32f_setup, packed_value*, interp_f32)
+// forms linear cell indices in int, so grids of 2^31 cells or more are refused.
 static int fill_grid(const lsm_grid_desc* g, lsm::GridDev* d, int want_ndim, bool need_grads, const char* who, bool f32) {
     if (g == nullptr || g->values == nullptr) return fail(1, std::string(who) + ": null grid");
     if (g->ndim != want_ndim) return fail(2, std::string(who) + ": wrong grid dimensionality");
     if (need_grads && g->grads == nullptr) return fail(2, std::string(who) + ": gradient array required");
-    std::memset(d, 0, sizeof(*d));
-    d->ndim = g->ndim;
+    lsm::GridDev v;
+    std::memset(&v, 0, sizeof(v));
+    v.ndim = g->ndim;
+    unsigned long long cells = 1;
     for (int k = 0; k < g->ndim; ++k) {
         if (g->shape[k] < 2) return fail(2, std::string(who) + ": every grid dimension needs >= 2 nodes");
-        d->shape[k] = g->shape[k]; d->periodic[k] = g->periodic[k] ? 1 : 0; d->lo[k] = g->lo[k];
+        cells *= (unsigned long long)g->shape[k];      // < 2^31 before, shape < 2^31: no wrap-around
+        if (cells > (unsigned long long)INT_MAX)
+            return fail(2, std::string(who) + ": the grid has 2^31 cells or more (32-bit cell indices)");
+        v.shape[k] = g->shape[k]; v.periodic[k] = g->periodic[k] ? 1 : 0; v.lo[k] = g->lo[k];
         const double n = (double)g->shape[k];
-        d->spacing[k] = g->periodic[k] ? (g->hi[k] - g->lo[k]) / n : (g->hi[k] - g->lo[k]) / (n - 1.0);
-        d->inv_spacing[k] = 1.0 / d->spacing[k];
+        v.spacing[k] = g->periodic[k] ? (g->hi[k] - g->lo[k]) / n : (g->hi[k] - g->lo[k]) / (n - 1.0);
+        v.inv_spacing[k] = 1.0 / v.spacing[k];
     }
-    d->separation_distance = g->separation_distance; d->ttr_max = g->ttr_max;
-    d->values = g->values; d->grads = g->grads;
-    d->f32 = f32 ? 1 : 0;
+    v.separation_distance = g->separation_distance; v.ttr_max = g->ttr_max;
+    v.values = g->values; v.grads = g->grads;
+    v.f32 = f32 ? 1 : 0;
+    *d = v;
     return 0;
 }
 

@@ -155,10 +155,10 @@ def synthetic_airtaxi_grid(target_separation_distance=AirTaxiConfig.SEPARATION_D
                           data_separation_distance, target_separation_distance)
 
 
-def synthetic_ttr_grid(shape=TTR_GRID_SHAPE) -> HjGrid:
+def synthetic_ttr_grid(shape=TTR_GRID_SHAPE, lo=TTR_GRID_LO, hi=TTR_GRID_HI) -> HjGrid:
     """4-D time-to-reach in the goal frame: distance at nominal speed + a heading-error turn time."""
-    lo = np.asarray(TTR_GRID_LO, dtype=np.float64)
-    hi = np.asarray(TTR_GRID_HI, dtype=np.float64)
+    lo = np.asarray(lo, dtype=np.float64)
+    hi = np.asarray(hi, dtype=np.float64)
     x, y, th, v = _lattice(lo, hi, shape, (False, False, True, False))
     d = np.sqrt(x * x + y * y)
     ttr = d / AirTaxiConfig.V_NOMINAL + 0.5 * np.abs(th) / AirTaxiConfig.ANGULAR_RATE_MAX \

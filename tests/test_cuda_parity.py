@@ -23,11 +23,12 @@ CASES = G.golden_names()
 class CudaAdapter:
     """Gives the CUDA env the attribute surface the shared check_step helper expects."""
 
-    def __init__(self, args, flags, n=1, seed=0, auto_reset=False):
+    def __init__(self, args, flags, n=1, seed=0, auto_reset=False, value_grid=None, ttr_grid=None):
         import torch
         from layered_safe_marl_b200 import B200GraphVecEnv
         self.torch = torch
-        self.env = B200GraphVecEnv(args, num_envs=n, seed=seed, binary_cfg=flags, auto_reset=auto_reset)
+        self.env = B200GraphVecEnv(args, num_envs=n, seed=seed, binary_cfg=flags, auto_reset=auto_reset,
+                                   value_grid=value_grid, ttr_grid=ttr_grid)
 
     def set_state(self, s):
         self.env.set_state(s)
@@ -124,17 +125,20 @@ def _report_divergence(tag, so, sc, ora, cu, prev_state_equal, n):
     return bad
 
 
-def _compare_with_oracle(args, flags, n, T, episode, seed, auto_reset):
+def _compare_with_oracle(args, flags, n, T, episode, seed, auto_reset, grids=None, prepare=None):
     """Same Philox-seeded resets and the same actions through the CUDA env and the C oracle. ZERO tolerance for
     discrete outputs and for the float64 state; float32 observations within tests/_golden.RTOL (the emission uses
-    rsqrt / angle-difference identities, <= 4e-7 relative)."""
+    rsqrt / angle-difference identities, <= 4e-7 relative). `grids`: the (value, TTR) grids both sides bind (default:
+    the synthetic grids); `prepare(env)` runs on the CUDA env before the first reset."""
     import torch
     import oracle_env as O
     from layered_safe_marl_b200 import config as cfg
     params = cfg.scenario_params_from_args(args, binary_cfg=flags)
-    vg, tg = G.value_grid_for(params)
+    vg, tg = G.value_grid_for(params) if grids is None else grids
     ora = O.OracleEnv(params.asdict(), n, value_grid=vg, ttr_grid=tg, seed=seed, nthreads=8)
-    cu = CudaAdapter(args, flags, n=n, seed=seed, auto_reset=auto_reset)
+    cu = CudaAdapter(args, flags, n=n, seed=seed, auto_reset=auto_reset, value_grid=vg, ttr_grid=tg)
+    if prepare is not None:
+        prepare(cu.env)
     # the specialised pipeline evaluates the airtaxi relative position in its rotation form (lsm_step_common.cuh
     # relative_state_rot); the oracle restates both forms (oracle/lsm_oracle.c at_relative_state)
     spec = cu.env.launch_info()['specialised'] == 1

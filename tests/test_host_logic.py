@@ -143,10 +143,14 @@ def test_div_exact_equals_division_on_the_synthetic_grids(which):
     1/b in a sense RN(1/b) does not always meet, so check every dimension of the three synthetic grids: dividends
     a = x - lo for the grid nodes +-8 ulps, the box faces and random positions within two box widths outside."""
     g = dict(di=hj_grid.synthetic_di_grid, airtaxi=hj_grid.synthetic_airtaxi_grid, ttr=hj_grid.synthetic_ttr_grid)[which]()
-    rng = np.random.default_rng(11)
-    for d in range(g.ndim):
-        lo, hi, n = float(g.lo[d]), float(g.hi[d]), g.shape[d]
-        b = (hi - lo) / n if g.periodic[d] else (hi - lo) / (n - 1.0)      # lsm_capi.cu fill_grid
+    check_div_exact(g.lo, g.hi, g.shape, g.periodic, which, np.random.default_rng(11))
+
+
+def check_div_exact(lo_, hi_, shape, periodic, what, rng):
+    """div_exact(x - lo, spacing) == (x - lo) / spacing on every dimension of a grid geometry (see the test above)."""
+    for d in range(len(shape)):
+        lo, hi, n = float(lo_[d]), float(hi_[d]), int(shape[d])
+        b = (hi - lo) / n if periodic[d] else (hi - lo) / (n - 1.0)      # lsm_capi.cu fill_grid
         y = 1.0 / b
         xs = [lo, hi]
         for k in range(n):
@@ -163,7 +167,7 @@ def test_div_exact_equals_division_on_the_synthetic_grids(which):
             q0 = a * y
             r = _fma(-b, q0, a)
             q = _fma(r, y, q0)
-            assert q == a / b, f"{which} dim {d}: x={x!r} a={a!r} b={b!r}: div_exact {q!r} vs {a / b!r}"
+            assert q == a / b, f"{what} dim {d}: x={x!r} a={a!r} b={b!r}: div_exact {q!r} vs {a / b!r}"
 
 
 def test_oracle_interpolation_matches_stub():
