@@ -23,6 +23,20 @@
  *                from the lattice (lsm_hj_dissipation).
  *   time         tau from 0; steps of dt = cfl / sum_i(alpha_i / spacing_i), the last one before each horizon clipped
  *                to land on it; Shu-Osher TVD-RK3.
+ *
+ * The airtaxi time-to-reach grid (DESIGN.md "Time-to-reach grid"; tests/hj_ttr_oracle.py restates it op for op) is the
+ * same scheme on a reach problem, also declared:
+ *   state        [x, y, theta (periodic), v]: one airtaxi relative to its goal, position rotated into the goal's frame,
+ *                heading minus the goal's heading, speed (the point the airtaxi reward looks up).
+ *   Hamiltonian  x' = v cos theta, y' = v sin theta, theta' = w, v' = a; the controls MINIMISE:
+ *                H = p0 v cos theta + p1 v sin theta + sum_k a_k (a_k < 0 ? hi_k : lo_k), a = (p2, p3), with the value
+ *                function solve's float32-rounded boxes w in +-0.1, a in [-0.001, 0.002] and its speed saturation
+ *                (v <= V_MIN: a >= 0; v >= V_MAX: a <= 0; each test restarting from the unsaturated box).
+ *                dV/dtau = min(0, H + sum_i alpha_i (p+_i - p-_i)/2) as above.
+ *   dissipation  alpha = [max |v cos theta|, max |v sin theta|, 0.1, 0.002] over the nodes.
+ *   arrival      ttr = 0 where target <= 0. Elsewhere the first RK3 step whose end value V1 is <= 0 writes
+ *                tau0 + h * (V0 / (V0 - V1)), with tau0, V0 the step's start and h its length; a cell is written once.
+ *                Cells not reached by the horizon stay +inf.
  */
 #ifndef LSM_B200_HJ_H
 #define LSM_B200_HJ_H
@@ -58,6 +72,27 @@ int lsm_hj_dissipation(const lsm_hj_problem *problem, double alpha[5], double *d
  * again. `work`: lsm_hj_work_bytes bytes, 8-byte aligned; `initial` and `out` must not overlap it. */
 int lsm_hj_solve(const lsm_hj_problem *problem, const double *initial, const double *horizons, int32_t K, double *out,
                  void *work, void *stream);
+
+typedef struct lsm_hj_ttr_problem {
+    int32_t shape[4];               /* nodes per dim [x, y, theta, v], each >= 2; theta is periodic */
+    double lo[4];                   /* finite, lo < hi */
+    double hi[4];
+    double cfl;                     /* 0 < cfl <= 1 */
+} lsm_hj_ttr_problem;
+
+/* Bytes of the `work` buffer of the time-to-reach solve: three stage arrays of cells doubles, the coordinate vectors
+ * and the cos / sin table of the theta nodes. 0 when the problem is invalid. */
+int64_t lsm_hj_ttr_work_bytes(const lsm_hj_ttr_problem *problem);
+
+/* Host only: the time-to-reach solve's Lax-Friedrichs coefficients alpha[4] and its CFL time step. */
+int lsm_hj_ttr_dissipation(const lsm_hj_ttr_problem *problem, double alpha[4], double *dt);
+
+/* Solve the reach problem of `target` (cells doubles, <= 0 on the target) to `horizon` (host, finite, >= 0) and write
+ * the first-arrival times to `ttr` (cells doubles; +inf where not reached) and, unless NULL, V(horizon) to
+ * `final_values`. `work`: the work-bytes size above, 8-byte aligned, overlapping none of the other arrays; `ttr` may
+ * alias `target`. */
+int lsm_hj_ttr_solve(const lsm_hj_ttr_problem *problem, const double *target, double horizon, double *ttr,
+                     double *final_values, void *work, void *stream);
 
 #ifdef __cplusplus
 }

@@ -103,6 +103,11 @@ class LsmHjProblem(C.Structure):
                 ('cfl', C.c_double)]
 
 
+class LsmHjTtrProblem(C.Structure):
+    """include/lsm_b200_hj.h lsm_hj_ttr_problem."""
+    _fields_ = [('shape', C.c_int32 * 4), ('lo', C.c_double * 4), ('hi', C.c_double * 4), ('cfl', C.c_double)]
+
+
 EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_destroy', 'lsm_set_value_grid',
                     'lsm_set_ttr_grid', 'lsm_bind_buffers', 'lsm_get_launch_info', 'lsm_step', 'lsm_reset',
                     'lsm_observe', 'lsm_emit_only', 'lsm_invalidate', 'lsm_set_output_buffers', 'lsm_edge_list',
@@ -114,7 +119,7 @@ EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_dest
 PPO_EXPORTED_SYMBOLS = ('lsm_ppo_abi_version', 'lsm_ppo_last_error', 'lsm_compute_returns', 'lsm_returns_scratch_bytes')
 
 HJ_EXPORTED_SYMBOLS = ('lsm_hj_abi_version', 'lsm_hj_last_error', 'lsm_hj_work_bytes', 'lsm_hj_dissipation',
-                       'lsm_hj_solve')
+                       'lsm_hj_solve', 'lsm_hj_ttr_work_bytes', 'lsm_hj_ttr_dissipation', 'lsm_hj_ttr_solve')
 
 _libs = {}          # one CDLL per path: the product library and the per-shape libraries (_build.build_shape)
 
@@ -225,6 +230,13 @@ def load_hj():
     lib.lsm_hj_solve.argtypes = [C.POINTER(LsmHjProblem), C.c_void_p, C.POINTER(C.c_double), C.c_int32, C.c_void_p,
                                  C.c_void_p, C.c_void_p]
     lib.lsm_hj_solve.restype = C.c_int
+    lib.lsm_hj_ttr_work_bytes.argtypes = [C.POINTER(LsmHjTtrProblem)]
+    lib.lsm_hj_ttr_work_bytes.restype = C.c_int64
+    lib.lsm_hj_ttr_dissipation.argtypes = [C.POINTER(LsmHjTtrProblem), C.POINTER(C.c_double), C.POINTER(C.c_double)]
+    lib.lsm_hj_ttr_dissipation.restype = C.c_int
+    lib.lsm_hj_ttr_solve.argtypes = [C.POINTER(LsmHjTtrProblem), C.c_void_p, C.c_double, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.c_void_p]
+    lib.lsm_hj_ttr_solve.restype = C.c_int
     lib.lsm_last_error = lib.lsm_hj_last_error       # check(rc, what, lib) reads this library's own error string
     _libs[key] = lib
     return lib

@@ -7,8 +7,15 @@
 // suffice. The window loads of a warp are 32 consecutive cells at one offset, so every load is coalesced; the reuse
 // between neighbouring cells is served by L1 / L2 (the default grids are 6-26 MB).
 //
-// Every float64 operation is written out in the order of tests/hj_solve_oracle.py, and the library is built with
-// -fmad=false, so the solve is bit for bit the numpy restatement.
+// lsm_hj_ttr_stage_kernel<STAGE>: the same stencil for the airtaxi time-to-reach solve, 4-D [x, y, theta (periodic),
+// v] in the goal's frame, with the controls minimising (a reach problem). Its stage 3 holds V0 = u0[cell] and V1, the
+// step's end value, in registers and writes the first-arrival time of a cell whose V has just crossed to <= 0:
+// tau0 + h * (V0 / (V0 - V1)), once (the slot stays +inf until then). lsm_hj_ttr_init_kernel sets the slot to 0 on
+// the target (l <= 0) and +inf elsewhere. The TTR kernels have their own template and parameters so that the value
+// function kernels above compile exactly as before.
+//
+// Every float64 operation is written out in the order of tests/hj_solve_oracle.py (tests/hj_ttr_oracle.py for the TTR
+// solve), and the library is built with -fmad=false, so the solve is bit for bit the numpy restatement.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -169,6 +176,75 @@ __global__ void __launch_bounds__(BLOCK) lsm_hj_stage_kernel(const StageParams p
     p.out[cell] = v;
 }
 
+// the time-to-reach solve (include/lsm_b200_hj.h lsm_hj_ttr_problem): 4-D, dim 2 periodic
+struct TtrParams {
+    const double* u;                // stencil input (u0, u1 or u2)
+    const double* u0;               // the step's start, read at the cell itself (stages 2 and 3)
+    double* out;
+    double* ttr;                    // first-arrival times, +inf until the cell is reached
+    const double* coords;           // concatenated coordinate vectors
+    const double* cth;              // cos / sin of the theta nodes
+    const double* sth;
+    int64_t cells;
+    int64_t n[4], stride[4], coord_off[4];
+    double inv_dx[4], alpha[4];
+    double h, tau0;                 // the step's length and start
+};
+
+constexpr double UNREACHED = (double)INFINITY;
+
+__global__ void __launch_bounds__(BLOCK) lsm_hj_ttr_init_kernel(const double* __restrict__ l, double* __restrict__ ttr,
+                                                                int64_t cells) {
+    const int64_t cell = (int64_t)blockIdx.x * BLOCK + threadIdx.x;
+    if (cell < cells) ttr[cell] = l[cell] <= 0.0 ? 0.0 : UNREACHED;
+}
+
+// STAGE as lsm_hj_stage_kernel; x' = v cos th, y' = v sin th, th' = w, v' = a with both controls minimising
+template <int STAGE>
+__global__ void __launch_bounds__(BLOCK) lsm_hj_ttr_stage_kernel(const TtrParams p) {
+    const int64_t cell = (int64_t)blockIdx.x * BLOCK + threadIdx.x;
+    if (cell >= p.cells) return;
+    int64_t idx[4];
+    int64_t r = cell;
+#pragma unroll
+    for (int d = 3; d >= 0; --d) { idx[d] = r % p.n[d]; r /= p.n[d]; }
+    double pl[4], pr[4];
+#pragma unroll
+    for (int d = 0; d < 4; ++d) {
+        if (d == 2) derivs<true>(p.u, cell, idx[d], p.n[d], p.stride[d], p.inv_dx[d], pl[d], pr[d]);
+        else derivs<false>(p.u, cell, idx[d], p.n[d], p.stride[d], p.inv_dx[d], pl[d], pr[d]);
+    }
+    double q[4];
+#pragma unroll
+    for (int d = 0; d < 4; ++d) q[d] = (pl[d] + pr[d]) * 0.5;
+    const double c = p.cth[idx[2]], s = p.sth[idx[2]];
+    const double v = p.coords[p.coord_off[3] + idx[3]];
+    const double f0 = v * c, f1 = v * s;
+    double H = q[0] * f0 + q[1] * f1;
+    // the filter solver's speed saturation: each test starts from the unsaturated box
+    double lo3 = AT_AMIN, hi3 = AT_AMAX;
+    if (v <= AT_VMIN) { lo3 = AT_AMIN; hi3 = AT_AMAX; lo3 = 0.0; }
+    if (v >= AT_VMAX) { lo3 = AT_AMIN; hi3 = AT_AMAX; hi3 = 0.0; }
+    const double a[2] = {q[2], q[3]}, lo[2] = {-AT_W, lo3}, hi[2] = {AT_W, hi3};
+#pragma unroll
+    for (int k = 0; k < 2; ++k) H = H + a[k] * (a[k] < 0.0 ? hi[k] : lo[k]);
+    double diss = p.alpha[0] * ((pr[0] - pl[0]) * 0.5);
+#pragma unroll
+    for (int d = 1; d < 4; ++d) diss = diss + p.alpha[d] * ((pr[d] - pl[d]) * 0.5);
+    const double hh = H + diss;
+    const double L = hh < 0.0 ? hh : 0.0;
+    const double next = __ldg(p.u + cell) + p.h * L;
+    if (STAGE == 0) p.out[cell] = next;
+    else if (STAGE == 1) p.out[cell] = 0.75 * p.u0[cell] + 0.25 * next;
+    else {
+        const double v0 = p.u0[cell];
+        const double v1 = C13 * v0 + C23 * next;
+        p.out[cell] = v1;
+        // a cell with a time has V <= 0 at a step end; every other one has V0 > 0, so V0 - V1 > 0
+        if (v1 <= 0.0 && p.ttr[cell] == UNREACHED) p.ttr[cell] = p.tau0 + p.h * (v0 / (v0 - v1));
+    }
+}
+
 template <int DYN>
 cudaError_t launch_step(StageParams p, double* u0, double* u1, double* u2, double h, cudaStream_t st) {
     const unsigned grid = (unsigned)((p.cells + BLOCK - 1) / BLOCK);
@@ -182,6 +258,19 @@ cudaError_t launch_step(StageParams p, double* u0, double* u1, double* u2, doubl
     return cudaGetLastError();
 }
 
+cudaError_t launch_ttr_step(TtrParams p, double* u0, double* u1, double* u2, double tau0, double h, cudaStream_t st) {
+    const unsigned grid = (unsigned)((p.cells + BLOCK - 1) / BLOCK);
+    p.h = h;
+    p.tau0 = tau0;
+    p.u = u0; p.u0 = u0; p.out = u1;
+    lsm_hj_ttr_stage_kernel<0><<<grid, BLOCK, 0, st>>>(p);
+    p.u = u1; p.out = u2;
+    lsm_hj_ttr_stage_kernel<1><<<grid, BLOCK, 0, st>>>(p);
+    p.u = u2; p.out = u0;
+    lsm_hj_ttr_stage_kernel<2><<<grid, BLOCK, 0, st>>>(p);
+    return cudaGetLastError();
+}
+
 constexpr int64_t MAX_CELLS = (int64_t)1 << 38;      // keeps the launch grid within 2^31 - 1 blocks
 
 struct Lattice {
@@ -190,44 +279,59 @@ struct Lattice {
     double sp[5] = {0, 0, 0, 0, 0};
     std::vector<double> coords;     // concatenated per dim
     int64_t off[5] = {0, 0, 0, 0, 0};
-    std::vector<double> cth, sth;   // airtaxi theta nodes
+    std::vector<double> cth, sth;   // cos / sin of the periodic dim's (theta's) nodes
 };
 
-// -> 0 and the lattice, or 2 with the message in g_err
-int check_problem(const lsm_hj_problem* pr, const char* fn, Lattice& L) {
-    if (!pr) return fail(2, std::string(fn) + ": problem is NULL");
-    if (pr->dynamics != 0 && pr->dynamics != 1)
-        return fail(2, std::string(fn) + ": dynamics must be 0 (double integrator) or 1 (airtaxi)");
-    if (!(pr->cfl > 0.0 && pr->cfl <= 1.0)) return fail(2, std::string(fn) + ": cfl must be in (0, 1]");
-    L.nd = pr->dynamics == 0 ? 4 : 5;
-    const int periodic = pr->dynamics == 0 ? -1 : 2;
+// -> 0 and the lattice of nd dims (`periodic`: the periodic dim, -1 for none), or 2 with the message in g_err
+int build_lattice(int nd, int periodic, const int32_t* shape, const double* lo_, const double* hi_, double cfl,
+                  const std::string& fn, Lattice& L) {
+    if (!(cfl > 0.0 && cfl <= 1.0)) return fail(2, fn + ": cfl must be in (0, 1]");
+    L.nd = nd;
     L.cells = 1;
     for (int d = 0; d < L.nd; ++d) {
-        const double lo = pr->lo[d], hi = pr->hi[d];
-        if (pr->shape[d] < 2) return fail(2, std::string(fn) + ": every dim needs at least 2 nodes");
-        if (!(std::isfinite(lo) && std::isfinite(hi) && lo < hi))
-            return fail(2, std::string(fn) + ": every dim needs finite lo < hi");
-        L.cells *= pr->shape[d];
-        if (L.cells > MAX_CELLS) return fail(2, std::string(fn) + ": grid too large");
-        L.sp[d] = d == periodic ? (hi - lo) / (double)pr->shape[d] : (hi - lo) / (double)(pr->shape[d] - 1);
+        const double lo = lo_[d], hi = hi_[d];
+        if (shape[d] < 2) return fail(2, fn + ": every dim needs at least 2 nodes");
+        if (!(std::isfinite(lo) && std::isfinite(hi) && lo < hi)) return fail(2, fn + ": every dim needs finite lo < hi");
+        L.cells *= shape[d];
+        if (L.cells > MAX_CELLS) return fail(2, fn + ": grid too large");
+        L.sp[d] = d == periodic ? (hi - lo) / (double)shape[d] : (hi - lo) / (double)(shape[d] - 1);
     }
     for (int d = 0; d < L.nd; ++d) {
         L.off[d] = (int64_t)L.coords.size();
-        for (int k = 0; k < pr->shape[d]; ++k) L.coords.push_back(pr->lo[d] + L.sp[d] * (double)k);
+        for (int k = 0; k < shape[d]; ++k) L.coords.push_back(lo_[d] + L.sp[d] * (double)k);
     }
-    if (pr->dynamics == 1)
-        for (int k = 0; k < pr->shape[2]; ++k) {
-            const double th = L.coords[L.off[2] + k];
+    if (periodic >= 0)
+        for (int k = 0; k < shape[periodic]; ++k) {
+            const double th = L.coords[L.off[periodic] + k];
             L.cth.push_back(lsm_cos(th));
             L.sth.push_back(lsm_sin(th));
         }
     return 0;
 }
 
+int check_problem(const lsm_hj_problem* pr, const char* fn, Lattice& L) {
+    if (!pr) return fail(2, std::string(fn) + ": problem is NULL");
+    if (pr->dynamics != 0 && pr->dynamics != 1)
+        return fail(2, std::string(fn) + ": dynamics must be 0 (double integrator) or 1 (airtaxi)");
+    return build_lattice(pr->dynamics == 0 ? 4 : 5, pr->dynamics == 0 ? -1 : 2, pr->shape, pr->lo, pr->hi, pr->cfl, fn,
+                         L);
+}
+
+int check_ttr_problem(const lsm_hj_ttr_problem* pr, const char* fn, Lattice& L) {
+    if (!pr) return fail(2, std::string(fn) + ": problem is NULL");
+    return build_lattice(4, 2, pr->shape, pr->lo, pr->hi, pr->cfl, fn, L);
+}
+
 double max_abs(const double* v, int n) {
     double m = 0.0;
     for (int k = 0; k < n; ++k) m = fmax(m, fabs(v[k]));
     return m;
+}
+
+double cfl_step(const Lattice& L, const double* alpha, double cfl) {
+    double s = alpha[0] / L.sp[0];
+    for (int d = 1; d < L.nd; ++d) s = s + alpha[d] / L.sp[d];
+    return cfl / s;
 }
 
 void dissipation(const lsm_hj_problem* pr, const Lattice& L, double alpha[5], double* dt) {
@@ -253,13 +357,39 @@ void dissipation(const lsm_hj_problem* pr, const Lattice& L, double alpha[5], do
         alpha[3] = fmax(fabs(AT_AMIN), fabs(AT_AMAX));
         alpha[4] = alpha[3];
     }
-    double s = alpha[0] / L.sp[0];
-    for (int d = 1; d < L.nd; ++d) s = s + alpha[d] / L.sp[d];
-    *dt = pr->cfl / s;
+    *dt = cfl_step(L, alpha, pr->cfl);
 }
 
-int64_t aux_doubles(const lsm_hj_problem* pr, const Lattice& L) {
-    return (int64_t)L.coords.size() + (pr->dynamics == 1 ? 2 * (int64_t)pr->shape[2] : 0);
+// TTR: alpha = [max |v cos th|, max |v sin th|, W, max(|a_min|, |a_max|)] over the nodes
+void ttr_dissipation(const lsm_hj_ttr_problem* pr, const Lattice& L, double alpha[4], double* dt) {
+    const double* c = L.coords.data();
+    double f0 = 0.0, f1 = 0.0;
+    for (int t = 0; t < pr->shape[2]; ++t)
+        for (int k = 0; k < pr->shape[3]; ++k) {
+            const double v = c[L.off[3] + k];
+            f0 = fmax(f0, fabs(v * L.cth[t]));
+            f1 = fmax(f1, fabs(v * L.sth[t]));
+        }
+    alpha[0] = f0;
+    alpha[1] = f1;
+    alpha[2] = AT_W;
+    alpha[3] = fmax(fabs(AT_AMIN), fabs(AT_AMAX));
+    *dt = cfl_step(L, alpha, pr->cfl);
+}
+
+int64_t aux_doubles(const Lattice& L) { return (int64_t)(L.coords.size() + L.cth.size() + L.sth.size()); }
+
+// the coordinate vectors, then cos and sin of the theta nodes, to aux (aux_doubles doubles). Pageable sources:
+// cudaMemcpyAsync stages them before it returns, so the lattice may go out of scope.
+cudaError_t upload_lattice(const Lattice& L, double* aux, cudaStream_t st) {
+    cudaError_t e = cudaMemcpyAsync(aux, L.coords.data(), L.coords.size() * sizeof(double), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && !L.cth.empty()) {
+        e = cudaMemcpyAsync(aux + L.coords.size(), L.cth.data(), L.cth.size() * sizeof(double), cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess)
+            e = cudaMemcpyAsync(aux + L.coords.size() + L.cth.size(), L.sth.data(), L.sth.size() * sizeof(double),
+                                cudaMemcpyHostToDevice, st);
+    }
+    return e;
 }
 
 }  // namespace
@@ -272,7 +402,7 @@ const char* lsm_hj_last_error(void) { return g_err.c_str(); }
 int64_t lsm_hj_work_bytes(const lsm_hj_problem* problem) {
     Lattice L;
     if (check_problem(problem, "lsm_hj_work_bytes", L) != 0) return 0;
-    return (3 * L.cells + aux_doubles(problem, L)) * (int64_t)sizeof(double);
+    return (3 * L.cells + aux_doubles(L)) * (int64_t)sizeof(double);
 }
 
 int lsm_hj_dissipation(const lsm_hj_problem* problem, double alpha[5], double* dt) {
@@ -307,14 +437,7 @@ int lsm_hj_solve(const lsm_hj_problem* problem, const double* initial, const dou
     double* u1 = u0 + cells;
     double* u2 = u1 + cells;
     double* aux = u2 + cells;
-    // pageable sources: cudaMemcpyAsync stages them before it returns, so the host vectors may go out of scope
-    cudaError_t e = cudaMemcpyAsync(aux, L.coords.data(), L.coords.size() * sizeof(double), cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess && problem->dynamics == 1) {
-        e = cudaMemcpyAsync(aux + L.coords.size(), L.cth.data(), L.cth.size() * sizeof(double), cudaMemcpyHostToDevice, st);
-        if (e == cudaSuccess)
-            e = cudaMemcpyAsync(aux + L.coords.size() + L.cth.size(), L.sth.data(), L.sth.size() * sizeof(double),
-                                cudaMemcpyHostToDevice, st);
-    }
+    cudaError_t e = upload_lattice(L, aux, st);
     if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_solve: upload of the lattice");
     e = cudaMemcpyAsync(u0, initial, bytes, cudaMemcpyDeviceToDevice, st);
     if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_solve: copy of the initial values");
@@ -345,6 +468,77 @@ int lsm_hj_solve(const lsm_hj_problem* problem, const double* initial, const dou
         }
         e = cudaMemcpyAsync(out + (int64_t)k * cells, u0, bytes, cudaMemcpyDeviceToDevice, st);
         if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_solve: snapshot");
+    }
+    return 0;
+}
+
+int64_t lsm_hj_ttr_work_bytes(const lsm_hj_ttr_problem* problem) {
+    Lattice L;
+    if (check_ttr_problem(problem, "lsm_hj_ttr_work_bytes", L) != 0) return 0;
+    return (3 * L.cells + aux_doubles(L)) * (int64_t)sizeof(double);
+}
+
+int lsm_hj_ttr_dissipation(const lsm_hj_ttr_problem* problem, double alpha[4], double* dt) {
+    Lattice L;
+    if (const int rc = check_ttr_problem(problem, "lsm_hj_ttr_dissipation", L)) return rc;
+    if (!alpha || !dt) return fail(2, "lsm_hj_ttr_dissipation: alpha and dt must be non-NULL");
+    ttr_dissipation(problem, L, alpha, dt);
+    return 0;
+}
+
+int lsm_hj_ttr_solve(const lsm_hj_ttr_problem* problem, const double* target, double horizon, double* ttr,
+                     double* final_values, void* work, void* stream) {
+    Lattice L;
+    if (const int rc = check_ttr_problem(problem, "lsm_hj_ttr_solve", L)) return rc;
+    if (!target || !ttr || !work) return fail(2, "lsm_hj_ttr_solve: target, ttr and work must be non-NULL");
+    if ((reinterpret_cast<uintptr_t>(work) % alignof(double)) != 0)
+        return fail(2, "lsm_hj_ttr_solve: work must be 8-byte aligned");
+    if (!(std::isfinite(horizon) && horizon >= 0.0)) return fail(2, "lsm_hj_ttr_solve: horizon must be finite and >= 0");
+    double alpha[4], dt;
+    ttr_dissipation(problem, L, alpha, &dt);
+    if (!(dt > 0.0 && std::isfinite(dt)))
+        return fail(2, "lsm_hj_ttr_solve: the CFL time step is not positive and finite");
+
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int64_t cells = L.cells, bytes = cells * (int64_t)sizeof(double);
+    double* u0 = static_cast<double*>(work);
+    double* u1 = u0 + cells;
+    double* u2 = u1 + cells;
+    double* aux = u2 + cells;
+    cudaError_t e = upload_lattice(L, aux, st);
+    if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_ttr_solve: upload of the lattice");
+    e = cudaMemcpyAsync(u0, target, bytes, cudaMemcpyDeviceToDevice, st);
+    if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_ttr_solve: copy of the target");
+    const unsigned grid = (unsigned)((cells + BLOCK - 1) / BLOCK);
+    lsm_hj_ttr_init_kernel<<<grid, BLOCK, 0, st>>>(u0, ttr, cells);     // from the copy: ttr may alias target
+    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "lsm_hj_ttr_init_kernel");
+
+    TtrParams p{};
+    p.ttr = ttr;
+    p.coords = aux;
+    p.cth = aux + L.coords.size();
+    p.sth = p.cth + problem->shape[2];
+    p.cells = cells;
+    int64_t stride = 1;
+    for (int d = 3; d >= 0; --d) {
+        p.n[d] = problem->shape[d];
+        p.stride[d] = stride;
+        stride *= problem->shape[d];
+        p.coord_off[d] = L.off[d];
+        p.inv_dx[d] = 1.0 / L.sp[d];
+        p.alpha[d] = alpha[d];
+    }
+    double tau = 0.0;
+    while (tau < horizon) {
+        const double tau0 = tau;
+        double h;
+        if (horizon - tau <= dt) { h = horizon - tau; tau = horizon; }
+        else { h = dt; tau = tau + dt; }
+        if ((e = launch_ttr_step(p, u0, u1, u2, tau0, h, st)) != cudaSuccess) return cuda_fail(e, "lsm_hj_ttr_stage_kernel");
+    }
+    if (final_values) {
+        e = cudaMemcpyAsync(final_values, u0, bytes, cudaMemcpyDeviceToDevice, st);
+        if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_ttr_solve: copy of the final values");
     }
     return 0;
 }

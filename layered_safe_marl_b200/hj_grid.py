@@ -8,7 +8,9 @@ not available offline, so this module also provides **deterministic synthetic gr
 reference's dimensionality (4-D double integrator `[x, y, dvx, dvy]`, 5-D airtaxi
 `[x_r, y_r, theta_rel (periodic), v_a, v_b]`, 4-D TTR `[x, y, theta (periodic), v]`).
 Their SHAPE is assumed (the Drive files' shape is not recoverable offline) and every report
-says "synthetic grid".
+says "synthetic grid". They are only the defaults: `reachability.value_grid` and
+`reachability.ttr_grid` compute real value and time-to-reach grids on the GPU for the same
+consumers.
 
 Gradients follow the declared semantics of the oracle (`oracle/ref_stubs/hj_reachability`):
 central differences inside, first-order one-sided at non-periodic ends, wrap on periodic dims.

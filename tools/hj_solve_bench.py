@@ -1,6 +1,8 @@
 """Time the HJ reachability solver (liblsm_b200_hj.so) on one GPU and print one JSON line per measurement.
 
     python tools/hj_solve_bench.py [--out FILE.jsonl] [--steps 20] [--eager-max-cells 30000000]
+    python tools/hj_solve_bench.py --ttr [--out FILE.jsonl] [--steps 20]
+
 
 Per lattice (the two default lattices and refined ones of 10^7-10^8 cells):
 - stage_us: per-stage kernel time from CUDA events, (solve to 2S steps - solve to S steps) / (3 S), so the initial
@@ -12,6 +14,9 @@ Per lattice (the two default lattices and refined ones of 10^7-10^8 cells):
   counts as one op), the achieved FP64 op rate and the share of the measured HBM copy bandwidth (a 4 GiB
   device-to-device copy in the same run);
 - convergence: max|V(H) - V(H/2)| of each default lattice at its default horizon.
+With --ttr, the airtaxi time-to-reach solve (reachability.solve_ttr) on the default TTR lattice and a refined one,
+with the same stage_us / solve_ms / rate / bound fields (no eager baseline) and, per lattice, the fraction of cells
+still unreached at the default horizon and at twice it.
 The card's name, power limit and max SM clock are read in the same run.
 """
 from __future__ import annotations
@@ -40,6 +45,10 @@ PER_DIM = 12 + 2 * WENO_OPS + 2 + 4
 OPS = {0: 4 * PER_DIM + 11 + 6, 1: 5 * PER_DIM + 19 + 6}
 # compulsory traffic per cell and stage: the stencil input read once, u0 read (stages 2 and 3), the output written
 BYTES = (8 + 8 * 2 / 3 + 8)
+# TTR: 4 dims; Hamiltonian 9 (v cos, v sin, two products and a sum, two control terms); 6 as above. Stage 3's arrival
+# test reads the ttr slot only where V <= 0 and writes it once per cell, so it is left out of the per-stage bound.
+TTR_OPS = 4 * PER_DIM + 9 + 6
+TTR_CASES = [('ttr_default', hj_grid.TTR_GRID_SHAPE), ('ttr_refined', (81, 81, 48, 17))]
 
 CASES = [('di_default', 0, hj_grid.DI_GRID_SHAPE, hj_grid.DI_GRID_LO, hj_grid.DI_GRID_HI),
          ('at_default', 1, hj_grid.AIRTAXI_GRID_SHAPE, hj_grid.AIRTAXI_GRID_LO, hj_grid.AIRTAXI_GRID_HI),
@@ -146,17 +155,50 @@ class Eager:
         return HO.C13 * u + HO.C23 * (u2 + h * self.rate(u2))
 
 
+def run_ttr(steps, peak):
+    lo, hi = hj_grid.TTR_GRID_LO, hj_grid.TTR_GRID_HI
+    H = R.DEFAULT_TTR_HORIZON
+    out = []
+    for name, shape in TTR_CASES:
+        cells = int(np.prod(shape))
+        alpha, dt = R.ttr_dissipation(shape, lo, hi)
+        l = torch.as_tensor(R.ttr_target(shape, lo, hi), device='cuda')
+        S = steps
+        t1 = timed(lambda: R.solve_ttr(l, lo, hi, S * dt), reps=3)
+        t2 = timed(lambda: R.solve_ttr(l, lo, hi, 2 * S * dt), reps=3)
+        stage_us = (t2 - t1) * 1e3 / (3 * S)
+        rec = dict(what='ttr_solve', case=name, shape=list(shape), cells=cells, dt=dt, alpha=list(alpha),
+                   stage_us=round(stage_us, 2), cell_updates_per_s=cells / (3 * stage_us * 1e-6),
+                   fp64_ops_per_cell_stage=TTR_OPS, min_bytes_per_cell_stage=round(BYTES, 2),
+                   fp64_ops_per_s=TTR_OPS * cells / (stage_us * 1e-6),
+                   hbm_share_of_copy_peak=round(BYTES * cells / (stage_us * 1e-6) / (peak * 1e9), 4),
+                   horizon=H, steps=math.ceil(H / dt))
+        rec['solve_ms'] = round(timed(lambda: R.solve_ttr(l, lo, hi, H), reps=3), 3)
+        for k, h in (('unreached_at_H', H), ('unreached_at_2H', 2 * H)):
+            ttr = R.solve_ttr(l, lo, hi, h)[0]
+            rec[k] = float(torch.isinf(ttr).double().mean())
+            if k == 'unreached_at_H':
+                rec['ttr_max_finite'] = float(ttr[torch.isfinite(ttr)].max())
+        out.append(rec)
+        del l
+        torch.cuda.empty_cache()
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument('--out', default=None, help='append the JSON lines to this file as well')
     ap.add_argument('--steps', type=int, default=20, help='RK3 steps S of the per-stage difference')
     ap.add_argument('--eager-max-cells', type=int, default=30_000_000, help='skip the eager baseline above this size')
+    ap.add_argument('--ttr', action='store_true', help='time the airtaxi time-to-reach solve instead')
     a = ap.parse_args()
     assert torch.cuda.is_available(), "needs a CUDA device"
     info = gpu_info()
     peak = copy_peak_gbs()
     lines = [dict(what='setup', gpu=info, hbm_copy_peak_gbs=round(peak, 1))]
-    for name, dyn, shape, lo, hi in CASES:
+    if a.ttr:
+        lines += run_ttr(a.steps, peak)
+    for name, dyn, shape, lo, hi in ([] if a.ttr else CASES):
         cells = int(np.prod(shape))
         alpha, dt = R.dissipation(dyn, shape, lo, hi)
         l = torch.as_tensor(R.target(dyn, shape, lo, hi, SEP[dyn]), device='cuda')
