@@ -23,12 +23,12 @@ CASES = G.golden_names()
 class CudaAdapter:
     """Gives the CUDA env the attribute surface the shared check_step helper expects."""
 
-    def __init__(self, args, flags, n=1, seed=0, auto_reset=False, value_grid=None, ttr_grid=None):
+    def __init__(self, args, flags, n=1, seed=0, auto_reset=False, value_grid=None, ttr_grid=None, tuning=None):
         import torch
         from layered_safe_marl_b200 import B200GraphVecEnv
         self.torch = torch
         self.env = B200GraphVecEnv(args, num_envs=n, seed=seed, binary_cfg=flags, auto_reset=auto_reset,
-                                   value_grid=value_grid, ttr_grid=ttr_grid)
+                                   value_grid=value_grid, ttr_grid=ttr_grid, tuning=tuning)
 
     def set_state(self, s):
         self.env.set_state(s)
@@ -125,18 +125,21 @@ def _report_divergence(tag, so, sc, ora, cu, prev_state_equal, n):
     return bad
 
 
-def _compare_with_oracle(args, flags, n, T, episode, seed, auto_reset, grids=None, prepare=None):
+def _compare_with_oracle(args, flags, n, T, episode, seed, auto_reset, grids=None, prepare=None, tuning=None,
+                         after_reset=None, actions=None, on_step=None):
     """Same Philox-seeded resets and the same actions through the CUDA env and the C oracle. ZERO tolerance for
     discrete outputs and for the float64 state; float32 observations within tests/_golden.RTOL (the emission uses
     rsqrt / angle-difference identities, <= 4e-7 relative). `grids`: the (value, TTR) grids both sides bind (default:
-    the synthetic grids); `prepare(env)` runs on the CUDA env before the first reset."""
+    the synthetic grids); `prepare(env)` runs on the CUDA env before the first reset; `tuning`: the CUDA env's launch
+    overrides; `after_reset(ora, cu)` may edit both states after the reset; `actions(rng, t)` draws step t's action
+    indices (default: uniform); `on_step(t, actions, pre, post)` sees the oracle's state before and after each step."""
     import torch
     import oracle_env as O
     from layered_safe_marl_b200 import config as cfg
     params = cfg.scenario_params_from_args(args, binary_cfg=flags)
     vg, tg = G.value_grid_for(params) if grids is None else grids
     ora = O.OracleEnv(params.asdict(), n, value_grid=vg, ttr_grid=tg, seed=seed, nthreads=8)
-    cu = CudaAdapter(args, flags, n=n, seed=seed, auto_reset=auto_reset, value_grid=vg, ttr_grid=tg)
+    cu = CudaAdapter(args, flags, n=n, seed=seed, auto_reset=auto_reset, value_grid=vg, ttr_grid=tg, tuning=tuning)
     if prepare is not None:
         prepare(cu.env)
     # the specialised pipeline evaluates the airtaxi relative position in its rotation form (lsm_step_common.cuh
@@ -147,6 +150,8 @@ def _compare_with_oracle(args, flags, n, T, episode, seed, auto_reset, grids=Non
         ora.reset(episode=episode, sample=True)
         cu.env.reset(episode)
         torch.cuda.synchronize()
+        if after_reset is not None:
+            after_reset(ora, cu)
         rng = np.random.default_rng(seed + 7)
         state_equal = np.ones(n, dtype=bool)
 
@@ -175,9 +180,12 @@ def _compare_with_oracle(args, flags, n, T, episode, seed, auto_reset, grids=Non
 
         compare('reset')
         for t in range(T):
-            a = rng.integers(0, 25, (n, params.num_agents)).astype(np.int32)
+            a = (rng.integers(0, 25, (n, params.num_agents)) if actions is None else actions(rng, t)).astype(np.int32)
+            pre = ora.get_state() if on_step is not None else None
             ora.step(a, episode=episode, auto_reset=auto_reset)
             cu.step(a, episode=episode)
+            if on_step is not None:
+                on_step(t, a, pre, ora.get_state())
             compare(f't={t}')
             G.assert_close(cu.ep_info, ora.ep_info, f't={t} ep_info')
     finally:
