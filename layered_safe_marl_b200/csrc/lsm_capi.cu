@@ -373,8 +373,8 @@ int lsm_destroy(lsm_handle* h) {
 }
 
 // Validates the descriptor completely before it touches the handle: a refused grid leaves the bound one (and its packed
-// table and padded gradient rows) in place. Every lookup (stencil32_setup, stencil32f_setup, packed_value*, interp_f32)
-// forms linear cell indices in int, so grids of 2^31 cells or more are refused.
+// table and padded gradient rows) in place. The lookups (lsm_grid.cuh) form linear cell indices in int, so grids of 2^31
+// cells or more are refused.
 static int fill_grid(const lsm_grid_desc* g, lsm::GridDev* d, int want_ndim, bool need_grads, const char* who, bool f32) {
     if (g == nullptr || g->values == nullptr) return fail(1, std::string(who) + ": null grid");
     if (g->ndim != want_ndim) return fail(2, std::string(who) + ": wrong grid dimensionality");
@@ -429,7 +429,7 @@ int lsm_set_value_grid(lsm_handle* h, const lsm_grid_desc* g) {
     }
     if (h->d_grads8) { cudaFree(h->d_grads8); h->d_grads8 = nullptr; }
     h->kp.vg.grads8 = nullptr;
-    if (h->spec && g->ndim == 5) {     // always: stencil32_grad<5> has no scattered alternative (104 MB for 41x41x24x9x9)
+    if (g->ndim == 5) {     // every handle: the 5-D gradient lookup reads only these rows (104 MB for 41x41x24x9x9)
         cudaError_t e = cudaMalloc(&h->d_grads8, cells * 8 * sizeof(float));
         if (e == cudaSuccess) e = lsm::pad_grads_launch(g->grads, h->d_grads8, (long long)cells);
         if (e == cudaSuccess) e = cudaDeviceSynchronize();

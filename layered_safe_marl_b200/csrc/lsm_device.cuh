@@ -163,6 +163,24 @@ __device__ __forceinline__ double pymin(double a, double b) { return (b < a) ? b
 __device__ __forceinline__ double norm2(double a, double b) { return sqrt(a * a + b * b); }
 __device__ __forceinline__ double f32r(double v) { return (double)(float)v; }
 
+// L2 eviction-priority hints (createpolicy): the 100 MB - 10 GB observation stream of one step is written evict-first
+// and the HJ grids are gathered evict-last, so the stream does not push the few-MB grids out of the 126 MB L2 - without
+// them the pair kernel's gathers miss to HBM and its reads interleave with the emit kernel's write stream.
+__device__ __forceinline__ unsigned long long l2_evict_first() {
+    unsigned long long p; asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p)); return p;
+}
+__device__ __forceinline__ unsigned long long l2_evict_last() {
+    unsigned long long p; asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p)); return p;
+}
+__device__ __forceinline__ float ldg_hint(const float* p, unsigned long long pol) {
+    float v; asm("ld.global.nc.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(v) : "l"(p), "l"(pol)); return v;
+}
+__device__ __forceinline__ float4 ldg_hint(const float4* p, unsigned long long pol) {
+    float4 v;
+    asm("ld.global.nc.L2::cache_hint.v4.f32 {%0, %1, %2, %3}, [%4], %5;" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol));
+    return v;
+}
+
 // ---------------------------------------------------------------------------------------------
 // Philox4x32-10 (Salmon et al. 2011): counter based, keyed by (seed, env, reset_count), so a device
 // reset can be replayed exactly by an independent CPU implementation of the same generator
@@ -196,165 +214,6 @@ struct Rng {
     }
     __device__ double uniform(double lo, double hi) { return lo + (hi - lo) * uniform01(); }
 };
-
-// ---------------------------------------------------------------------------------------------
-// Regular-grid multilinear interpolation (declared semantics: DESIGN.md "grid interpolation").
-// NC == 0: scalar value; NC == ND: all gradient components in one pass (shared stencil).
-// Corner order: binary counting, dim 0 slowest; weight = ((w0*w1)*w2)..; sequential accumulation.
-// ---------------------------------------------------------------------------------------------
-template <int ND>
-struct Stencil {
-    long long stride_lo[ND];   // linear offset contribution of the low / high index per dim
-    long long stride_hi[ND];
-    double wlo[ND], whi[ND];
-    bool valid;
-};
-
-template <int ND>
-__device__ __forceinline__ void stencil_setup(const GridDev& g, const double (&x)[ND], Stencil<ND>& s) {
-    s.valid = true;
-    long long mul = 1;
-#pragma unroll
-    for (int d = ND - 1; d >= 0; --d) {
-        double pos = (x[d] - g.lo[d]) / g.spacing[d];
-        if (isnan(pos)) s.valid = false;
-        pos = clipd(pos, -1.0e9, 1.0e9);
-        double fl = floor(pos);
-        double whi = pos - fl;
-        s.wlo[d] = 1.0 - whi; s.whi[d] = whi;
-        long long il = (long long)fl, ih = il + 1, n = g.shape[d];
-        if (g.periodic[d]) {
-            il %= n; if (il < 0) il += n;
-            ih %= n; if (ih < 0) ih += n;
-        } else {
-            il = il < 0 ? 0 : (il > n - 1 ? n - 1 : il);
-            ih = ih < 0 ? 0 : (ih > n - 1 ? n - 1 : ih);
-        }
-        s.stride_lo[d] = il * mul; s.stride_hi[d] = ih * mul;
-        mul *= n;
-    }
-}
-
-template <int ND>
-__device__ __forceinline__ double stencil_value(const GridDev& g, const Stencil<ND>& s) {
-    double acc = 0.0;
-#pragma unroll
-    for (int corner = 0; corner < (1 << ND); ++corner) {
-        double weight = 0.0; long long lin = 0;
-#pragma unroll
-        for (int d = 0; d < ND; ++d) {
-            const int bit = (corner >> (ND - 1 - d)) & 1;
-            const double wd = bit ? s.whi[d] : s.wlo[d];
-            weight = (d == 0) ? wd : weight * wd;
-            lin += bit ? s.stride_hi[d] : s.stride_lo[d];
-        }
-        acc = acc + weight * (double)__ldg(g.values + lin);
-    }
-    return acc;
-}
-
-template <int ND>
-__device__ __forceinline__ void stencil_grad(const GridDev& g, const Stencil<ND>& s, double (&out)[ND]) {
-#pragma unroll
-    for (int d = 0; d < ND; ++d) out[d] = 0.0;
-#pragma unroll
-    for (int corner = 0; corner < (1 << ND); ++corner) {
-        double weight = 0.0; long long lin = 0;
-#pragma unroll
-        for (int d = 0; d < ND; ++d) {
-            const int bit = (corner >> (ND - 1 - d)) & 1;
-            const double wd = bit ? s.whi[d] : s.wlo[d];
-            weight = (d == 0) ? wd : weight * wd;
-            lin += bit ? s.stride_hi[d] : s.stride_lo[d];
-        }
-        if (ND == 4) {
-            const float4 v = __ldg(reinterpret_cast<const float4*>(g.grads) + lin);
-            out[0] = out[0] + weight * (double)v.x; out[1] = out[1] + weight * (double)v.y;
-            out[2] = out[2] + weight * (double)v.z; out[3] = out[3] + weight * (double)v.w;
-        } else {
-#pragma unroll
-            for (int d = 0; d < ND; ++d) out[d] = out[d] + weight * (double)__ldg(g.grads + lin * ND + d);
-        }
-    }
-}
-
-// Declared FLOAT32 interpolation (LSM_FLAG_INTERP_FLOAT32; the reference never enables jax_enable_x64, so the real
-// hj_reachability.Grid.interpolate runs in float32): state, domain_lo and spacing rounded to float32, position / floor /
-// weights / weight products / corner sum all float32, same corner order and index handling as the float64 mode, no FMA.
-// One out-of-line function for values (ncomp == 0 -> out[0]) and gradient rows (ncomp == ND); scattered gathers - this
-// mode exists for parity with the real library's arithmetic, not for speed. Returns false for a NaN position.
-template <int ND>
-__device__ __noinline__ bool interp_f32(const GridDev& g, const double* x, int ncomp, double* out) {
-    float wlo[ND], whi[ND];
-    int lo[ND], hi[ND];
-    int mul = 1;
-    bool ok = true;
-#pragma unroll
-    for (int d = ND - 1; d >= 0; --d) {
-        float pos = ((float)x[d] - (float)g.lo[d]) / (float)g.spacing[d];
-        if (isnan(pos)) ok = false;
-        pos = fminf(fmaxf(pos, -1.0e9f), 1.0e9f);
-        const float fl = floorf(pos);
-        const float w = pos - fl;
-        wlo[d] = 1.0f - w; whi[d] = w;
-        const int n = g.shape[d];
-        int il = (int)fl, ih = il + 1;
-        if (g.periodic[d]) {
-            il %= n; if (il < 0) il += n;
-            ih %= n; if (ih < 0) ih += n;
-        } else {
-            il = min(max(il, 0), n - 1);
-            ih = min(max(ih, 0), n - 1);
-        }
-        lo[d] = il * mul; hi[d] = ih * mul;
-        mul *= n;
-    }
-    if (!ok) return false;
-    float acc[ND];
-#pragma unroll
-    for (int c = 0; c < ND; ++c) acc[c] = 0.0f;
-#pragma unroll
-    for (int corner = 0; corner < (1 << ND); ++corner) {
-        float weight = 0.0f; int lin = 0;
-#pragma unroll
-        for (int d = 0; d < ND; ++d) {
-            const int bit = (corner >> (ND - 1 - d)) & 1;
-            const float wd = bit ? whi[d] : wlo[d];
-            weight = (d == 0) ? wd : weight * wd;
-            lin += bit ? hi[d] : lo[d];
-        }
-        if (ncomp == 0) acc[0] = acc[0] + weight * __ldg(g.values + lin);
-        else {
-#pragma unroll
-            for (int c = 0; c < ND; ++c) acc[c] = acc[c] + weight * __ldg(g.grads + (size_t)lin * ND + c);
-        }
-    }
-    if (ncomp == 0) out[0] = (double)acc[0];
-    else {
-#pragma unroll
-        for (int c = 0; c < ND; ++c) out[c] = (double)acc[c];
-    }
-    return true;
-}
-
-// Call-site wrappers: private copies go through the out-of-line function, so the CALLER's `x` / `out` arrays never have
-// their address taken (that would move them from registers to local memory on the float64 path as well).
-template <int ND>
-__device__ __forceinline__ double interp_f32_value(const GridDev& g, const double (&x)[ND]) {
-    double xin[ND], v;
-#pragma unroll
-    for (int d = 0; d < ND; ++d) xin[d] = x[d];
-    return interp_f32<ND>(g, xin, 0, &v) ? v : NAN;
-}
-template <int ND>
-__device__ __forceinline__ void interp_f32_grad(const GridDev& g, const double (&x)[ND], double (&out)[ND]) {
-    double xin[ND], o[ND];
-#pragma unroll
-    for (int d = 0; d < ND; ++d) xin[d] = x[d];
-    const bool ok = interp_f32<ND>(g, xin, ND, o);
-#pragma unroll
-    for (int d = 0; d < ND; ++d) out[d] = ok ? o[d] : NAN;
-}
 
 // ---------------------------------------------------------------------------------------------
 // Curriculum scalars: navigation_graph_safe.py:324-366, :1101-1122, :319-322

@@ -4,7 +4,7 @@
 //   relative state   relative_state_rot (one sincos per ego; identical to the literal form for the double integrator)
 //   HJ value         pair_value_rel: corner-packed table when the handle built one, else the scattered stencil
 //   filter           filter_resolve (gradient, least-restrictive bang-bang below 0.4 or CBF-QP, clipping, filtered flag)
-//   gradient         padded 5-D rows / float4 4-D rows (LeanGrad) when present, else the scattered rows (ClassicGrad)
+//   gradient         grid_grad: float4 rows (4-D) / padded rows (5-D, built for every handle by lsm_set_value_grid)
 // F32 = LSM_FLAG_INTERP_FLOAT32 of the handle, chosen at compile time like the agent and pair kernels.
 //
 // lsm_safety_filter_kernel: a block owns kFopRows rows at a time. Phase 1: kFopLanes threads per row evaluate distance and
@@ -21,22 +21,6 @@ constexpr int kFopRows = 32;                    // rows per block tile = owner t
 constexpr int kFopLanes = 8;                    // slot lanes per row in phase 1
 constexpr int kFopThreads = kFopRows * kFopLanes;
 constexpr int kLookupThreads = 128;
-
-// gradient lookup of the operator: the specialised pipeline's rows when the handle carries them (every 4-D grid; 5-D grids of
-// specialised handles), the scattered rows otherwise (5-D grid of a handle on the generic kernel). Both give the declared
-// Grid.interpolate gradient bit for bit. Relative state in the rotation form, like pair_value_raw.
-template <bool F32>
-struct OpGrad {
-    static constexpr bool kRotRel = true;
-    template <int ND>
-    __device__ __forceinline__ static void eval(const GridDev& g, const double (&rel)[ND], double (&out)[ND]) {
-        if constexpr (ND == 4) LeanGrad<F32>::template eval<ND>(g, rel, out);
-        else {
-            if (g.grads8 != nullptr) LeanGrad<F32>::template eval<ND>(g, rel, out);
-            else ClassicGrad::template eval<ND>(g, rel, out);
-        }
-    }
-};
 
 template <int DYN, bool F32>
 __global__ void __launch_bounds__(kFopThreads) lsm_safety_filter_kernel(const __grid_constant__ KParams kp,
@@ -111,8 +95,8 @@ __global__ void __launch_bounds__(kFopThreads) lsm_safety_filter_kernel(const __
                 const double* ou = a.other_actions + ((size_t)row * M + kv) * 2;
                 double rse = 0.0, rce = 1.0;
                 if constexpr (DYN != LSM_DYN_DOUBLE_INTEGRATOR) lsm_sincos(r2, &rse, &rce);
-                filter_resolve<DYN, OpGrad<F32>>(kp, sqrt(best_d2), best_v, !isinf(best_v), rx, ry, r2, r3, o[0], o[1], o[2], o[3],
-                                                 raw0, raw1, ou[0], ou[1], safe0, safe1, filt, rse, rce);
+                filter_resolve<DYN, true, F32>(kp, sqrt(best_d2), best_v, !isinf(best_v), rx, ry, r2, r3, o[0], o[1], o[2], o[3],
+                                               raw0, raw1, ou[0], ou[1], safe0, safe1, filt, rse, rce);
             }
             a.safe_action[(size_t)row * 2] = safe0;
             a.safe_action[(size_t)row * 2 + 1] = safe1;
@@ -152,7 +136,7 @@ __global__ void __launch_bounds__(kLookupThreads) lsm_hj_lookup_kernel(const __g
             if (nan_pos) {
 #pragma unroll
                 for (int d = 0; d < ND; ++d) g[d] = NAN;
-            } else OpGrad<F32>::template eval<ND>(kp.vg, rel, g);
+            } else grid_grad<ND, F32>(kp.vg, rel, g);
 #pragma unroll
             for (int d = 0; d < ND; ++d) a.grad[(size_t)k * ND + d] = g[d];
         }

@@ -61,8 +61,8 @@ __device__ void safety_filter_agent(const KParams& kp, const Curriculum& q, cons
     }
     if (kv < 0) return;                         // no other active agent
     deconf = kv;
-    filter_resolve<DYN>(kp, best_d, best_v, kv_in_range, ex, ey, e2, e3, S.ax[kv], S.ay[kv], S.as2[kv], S.as3[kv],
-                        raw0, raw1, S.rawx[kv], S.rawy[kv], safe0, safe1, filtered);
+    filter_resolve<DYN, false>(kp, best_d, best_v, kv_in_range, ex, ey, e2, e3, S.ax[kv], S.ay[kv], S.as2[kv], S.as3[kv],
+                               raw0, raw1, S.rawx[kv], S.rawy[kv], safe0, safe1, filtered);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -283,10 +283,7 @@ __global__ void __launch_bounds__(256) lsm_generic_kernel(const __grid_constant_
                         double rpx, rpy;
                         rotate_into(x - gx, y - gy, lsm_cos(gh), lsm_sin(gh), rpx, rpy);
                         const double rs[4] = { rpx, rpy, theta - gh, speed };
-                        Stencil<4> st;
-                        stencil_setup<4>(kp.tg, rs, st);
-                        double ttr = st.valid ? stencil_value<4>(kp.tg, st) : NAN;
-                        if (kp.tg.f32) ttr = interp_f32_value<4>(kp.tg, rs);
+                        double ttr = grid_value_rt(kp.tg, rs);
                         if (isnan(ttr)) ttr = kp.tg.ttr_max;
                         rew -= 0.04 * ttr;
                         rew -= sen * cra;

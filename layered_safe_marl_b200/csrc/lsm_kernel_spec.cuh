@@ -19,9 +19,8 @@
 // one range overlaps the HBM-bound emit kernel of another.
 //
 // Same decisions as the generic kernel for every thresholded quantity:
-//   * the HJ stencil uses 32-bit indices and an exactly rounded division by the grid spacing through its
-//     precomputed reciprocal (Markstein: q0 = a*y, r = fma(-b,q0,a), q = fma(r,y,q0) equals RN(a/b);
-//     checked on the CPU in tests/test_host_logic.py).
+//   * the HJ grid lookups are the shared ones of lsm_grid.cuh (the value from the corner-packed table, which
+//     reproduces the stencil bit for bit).
 //   * distances are kept SQUARED in float64; every `d < T` / `d > T` test of the reference becomes
 //     `d2 < T2` against a host-computed exact squared threshold (sqrt_rn is monotone, so
 //     {t : sqrt_rn(t) >= T} is an interval whose lower end the host finds with nextafter). Square roots
@@ -99,450 +98,7 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 // actions, landmark tables, the parity-selected info slots) would otherwise be one more dependent DRAM round trip
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" :: "l"(p)); }
 
-// L2 eviction-priority hints (createpolicy): the 100 MB - 10 GB observation stream of one step is written evict-first
-// and the HJ grids are gathered evict-last, so the stream does not push the few-MB grids out of the 126 MB L2 - without
-// them the pair kernel's gathers miss to HBM and its reads interleave with the emit kernel's write stream.
-__device__ __forceinline__ unsigned long long l2_evict_first() {
-    unsigned long long p; asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p)); return p;
-}
-__device__ __forceinline__ unsigned long long l2_evict_last() {
-    unsigned long long p; asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p)); return p;
-}
-__device__ __forceinline__ float ldg_hint(const float* p, unsigned long long pol) {
-    float v; asm("ld.global.nc.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(v) : "l"(p), "l"(pol)); return v;
-}
-__device__ __forceinline__ float4 ldg_hint(const float4* p, unsigned long long pol) {
-    float4 v;
-    asm("ld.global.nc.L2::cache_hint.v4.f32 {%0, %1, %2, %3}, [%4], %5;" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol));
-    return v;
-}
-
 template <int N> struct Pow2 { static constexpr int value = N <= 1 ? 1 : N <= 2 ? 2 : N <= 4 ? 4 : N <= 8 ? 8 : N <= 16 ? 16 : 32; };
-
-// ---------------------------------------------------------------------------------------------
-// lean stencil: 32-bit indices, exact division through the reciprocal, weight prefixes shared
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ double div_exact(double a, double b, double y /* RN(1/b) */) {
-    const double q0 = a * y;
-    const double r = fma(-b, q0, a);
-    return fma(r, y, q0);
-}
-
-// periodic grid index: i mod n in [0, n). In-grid states land in [0, n) (an angle difference wrapped to one period), so the
-// integer division (~30 instructions) sits behind an "already in range" test. Measured on B200 (same-box A/B,
-// profiles/experiments/r02_wrap_index_ab.txt): for the 5-D airtaxi grid one shared out-of-line copy is faster (cfg3 352.7
-// -> 348.7 us; the unrolled 32-corner stencils are bound by instruction fetch), for the 4-D grids the call costs the
-// pair kernel six registers and a stack frame (cfg2 back-to-back 40.4 -> 43.2 us), so those keep it inline.
-__device__ __noinline__ int wrap_index_slow(int i, int n) { i %= n; if (i < 0) i += n; return i; }
-template <bool OUT_OF_LINE>
-__device__ __forceinline__ int wrap_index(int i, int n) {
-    if constexpr (OUT_OF_LINE) return ((unsigned)i < (unsigned)n) ? i : wrap_index_slow(i, n);
-    else { if ((unsigned)i >= (unsigned)n) { i %= n; if (i < 0) i += n; } return i; }
-}
-
-template <int ND>
-struct Stencil32 {
-    int lo[ND], hi[ND];        // linear offset contributions
-    double wlo[ND], whi[ND];
-    bool valid;
-};
-
-template <int ND>
-__device__ __forceinline__ void stencil32_setup(const GridDev& g, const double (&x)[ND], Stencil32<ND>& s) {
-    s.valid = true;
-    int mul = 1;
-#pragma unroll
-    for (int d = ND - 1; d >= 0; --d) {
-        double pos = div_exact(x[d] - g.lo[d], g.spacing[d], g.inv_spacing[d]);
-        if (isnan(pos)) s.valid = false;
-        if (!(fabs(pos) <= 1.0e9)) pos = pos < 0.0 ? -1.0e9 : 1.0e9;     // declared clamp; never taken in-grid
-        const double fl = floor(pos);
-        const double whi = pos - fl;
-        s.wlo[d] = 1.0 - whi; s.whi[d] = whi;
-        const int n = g.shape[d];
-        int il = (int)fl, ih = il + 1;          // |fl| <= 1e9 fits in int32
-        if (g.periodic[d]) {
-            il = wrap_index<(ND == 5)>(il, n);
-            ih = il + 1 == n ? 0 : il + 1;          // (il + 1) mod n
-        } else {
-            il = min(max(il, 0), n - 1);
-            ih = min(max(ih, 0), n - 1);
-        }
-        s.lo[d] = il * mul; s.hi[d] = ih * mul;
-        mul *= n;
-    }
-}
-
-// value: sum over corners (binary counting, dim 0 slowest) of ((w0*w1)*w2..)*v, sequential adds.
-// All 2^ND loads are issued first (one memory round trip per lookup instead of 2^ND dependent ones).
-template <int ND>
-__device__ __forceinline__ double stencil32_value(const GridDev& g, const Stencil32<ND>& s) {
-    constexpr int NC = 1 << ND;
-    float v[NC];
-    const unsigned long long keep = l2_evict_last();
-#pragma unroll
-    for (int corner = 0; corner < NC; ++corner) {
-        int lin = 0;
-#pragma unroll
-        for (int d = 0; d < ND; ++d) lin += ((corner >> (ND - 1 - d)) & 1) ? s.hi[d] : s.lo[d];
-        v[corner] = ldg_hint(g.values + lin, keep);
-    }
-    double acc = 0.0;
-#pragma unroll
-    for (int corner = 0; corner < NC; ++corner) {
-        double weight = 0.0;
-#pragma unroll
-        for (int d = 0; d < ND; ++d) {
-            const double wd = ((corner >> (ND - 1 - d)) & 1) ? s.whi[d] : s.wlo[d];
-            weight = (d == 0) ? wd : weight * wd;
-        }
-        acc = acc + weight * (double)v[corner];
-    }
-    return acc;
-}
-
-// all gradient components in one pass over the corners (same corner / weight order as the value)
-template <int ND>
-__device__ __forceinline__ void stencil32_grad(const GridDev& g, const Stencil32<ND>& s, double (&out)[ND]) {
-#pragma unroll
-    for (int d = 0; d < ND; ++d) out[d] = 0.0;
-    const unsigned long long keep = l2_evict_last();
-#pragma unroll
-    for (int corner = 0; corner < (1 << ND); ++corner) {
-        double weight = 0.0; int lin = 0;
-#pragma unroll
-        for (int d = 0; d < ND; ++d) {
-            const int bit = (corner >> (ND - 1 - d)) & 1;
-            const double wd = bit ? s.whi[d] : s.wlo[d];
-            weight = (d == 0) ? wd : weight * wd;
-            lin += bit ? s.hi[d] : s.lo[d];
-        }
-        if (ND == 4) {
-            const float4 v = ldg_hint(reinterpret_cast<const float4*>(g.grads) + lin, keep);
-            out[0] = out[0] + weight * (double)v.x; out[1] = out[1] + weight * (double)v.y;
-            out[2] = out[2] + weight * (double)v.z; out[3] = out[3] + weight * (double)v.w;
-        } else if (ND == 5) {
-            // the specialised pipeline always carries the padded rows (lsm_set_value_grid): no run-time alternative inside
-            // the 32 unrolled corners - the per-agent kernel is bound by instruction fetch
-            const float4 a = ldg_hint(reinterpret_cast<const float4*>(g.grads8) + 2 * (size_t)lin, keep);
-            const float4 b = ldg_hint(reinterpret_cast<const float4*>(g.grads8) + 2 * (size_t)lin + 1, keep);
-            out[0] = out[0] + weight * (double)a.x; out[1] = out[1] + weight * (double)a.y;
-            out[2] = out[2] + weight * (double)a.z; out[3] = out[3] + weight * (double)a.w;
-            out[ND - 1] = out[ND - 1] + weight * (double)b.x;
-        } else {
-#pragma unroll
-            for (int d = 0; d < ND; ++d) out[d] = out[d] + weight * (double)ldg_hint(g.grads + lin * ND + d, keep);
-        }
-    }
-}
-
-__global__ void __launch_bounds__(256) lsm_pad_grads_kernel(const float* __restrict__ grads, float* __restrict__ grads8, long long cells) {
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= cells * 8) return;
-    const long long cell = t >> 3; const int d = (int)(t & 7);
-    grads8[t] = d < 5 ? grads[cell * 5 + d] : 0.0f;
-}
-
-// ---------------------------------------------------------------------------------------------
-// float32 stencil (LSM_FLAG_INTERP_FLOAT32, compiled into the F32 instantiations only): the arithmetic of interp_f32
-// (lsm_device.cuh) and of the oracle's interpolate_f32, inline and without pointer arguments. State, lo and spacing
-// rounded to float32, IEEE float32 division (not the float64 reciprocal of div_exact), the declared clamp, float32
-// weights, weight products (dim 0 first) and sequential corner sums in binary counting order; no FMA (-fmad=false).
-// Same 32-bit index handling as stencil32_setup: (il + 1) mod n of the wrapped il equals interp_f32's ih mod n.
-// ---------------------------------------------------------------------------------------------
-template <int ND>
-struct Stencil32f {
-    int lo[ND], hi[ND];
-    float wlo[ND], whi[ND];
-    bool valid;
-};
-
-// float32 grid position of x[d] on dimension d; NaN = invalid
-__device__ __forceinline__ float grid_pos_f32(const GridDev& g, double x, int d) {
-    return __fdiv_rn((float)x - (float)g.lo[d], (float)g.spacing[d]);
-}
-
-template <int ND>
-__device__ __forceinline__ void stencil32f_setup(const GridDev& g, const double (&x)[ND], Stencil32f<ND>& s) {
-    s.valid = true;
-    int mul = 1;
-#pragma unroll
-    for (int d = ND - 1; d >= 0; --d) {
-        float pos = grid_pos_f32(g, x[d], d);
-        if (isnan(pos)) s.valid = false;
-        pos = fminf(fmaxf(pos, -1.0e9f), 1.0e9f);      // declared clamp
-        const float fl = floorf(pos);
-        const float whi = pos - fl;
-        s.wlo[d] = 1.0f - whi; s.whi[d] = whi;
-        const int n = g.shape[d];
-        int il = (int)fl, ih = il + 1;                 // |fl| <= 1e9 fits in int32
-        if (g.periodic[d]) {
-            il = wrap_index<(ND == 5)>(il, n);
-            ih = il + 1 == n ? 0 : il + 1;
-        } else {
-            il = min(max(il, 0), n - 1);
-            ih = min(max(ih, 0), n - 1);
-        }
-        s.lo[d] = il * mul; s.hi[d] = ih * mul;
-        mul *= n;
-    }
-}
-
-template <int ND>
-__device__ __forceinline__ float corner_weight_f32(const float (&wlo)[ND], const float (&whi)[ND], int corner) {
-    float weight = 0.0f;
-#pragma unroll
-    for (int d = 0; d < ND; ++d) {
-        const float wd = ((corner >> (ND - 1 - d)) & 1) ? whi[d] : wlo[d];
-        weight = (d == 0) ? wd : weight * wd;
-    }
-    return weight;
-}
-
-template <int ND>
-__device__ __forceinline__ double stencil32f_value(const GridDev& g, const Stencil32f<ND>& s) {
-    constexpr int NC = 1 << ND;
-    float v[NC];
-    const unsigned long long keep = l2_evict_last();
-#pragma unroll
-    for (int corner = 0; corner < NC; ++corner) {
-        int lin = 0;
-#pragma unroll
-        for (int d = 0; d < ND; ++d) lin += ((corner >> (ND - 1 - d)) & 1) ? s.hi[d] : s.lo[d];
-        v[corner] = ldg_hint(g.values + lin, keep);
-    }
-    float acc = 0.0f;
-#pragma unroll
-    for (int corner = 0; corner < NC; ++corner) acc = acc + corner_weight_f32<ND>(s.wlo, s.whi, corner) * v[corner];
-    return (double)acc;
-}
-
-// gradient rows as in stencil32_grad (float4 rows for 4-D, padded grads8 rows for 5-D), each component summed in
-// float32; a NaN position gives NaN components, as interp_f32_grad does
-template <int ND>
-__device__ __forceinline__ void stencil32f_grad(const GridDev& g, const Stencil32f<ND>& s, double (&out)[ND]) {
-    static_assert(ND == 4 || ND == 5, "the specialised grids are 4-D or 5-D");
-    float acc[ND];
-#pragma unroll
-    for (int d = 0; d < ND; ++d) acc[d] = 0.0f;
-    const unsigned long long keep = l2_evict_last();
-#pragma unroll
-    for (int corner = 0; corner < (1 << ND); ++corner) {
-        const float weight = corner_weight_f32<ND>(s.wlo, s.whi, corner);
-        int lin = 0;
-#pragma unroll
-        for (int d = 0; d < ND; ++d) lin += ((corner >> (ND - 1 - d)) & 1) ? s.hi[d] : s.lo[d];
-        if constexpr (ND == 4) {
-            const float4 v = ldg_hint(reinterpret_cast<const float4*>(g.grads) + lin, keep);
-            acc[0] = acc[0] + weight * v.x; acc[1] = acc[1] + weight * v.y;
-            acc[2] = acc[2] + weight * v.z; acc[3] = acc[3] + weight * v.w;
-        } else {
-            const float4 a = ldg_hint(reinterpret_cast<const float4*>(g.grads8) + 2 * (size_t)lin, keep);
-            const float4 b = ldg_hint(reinterpret_cast<const float4*>(g.grads8) + 2 * (size_t)lin + 1, keep);
-            acc[0] = acc[0] + weight * a.x; acc[1] = acc[1] + weight * a.y;
-            acc[2] = acc[2] + weight * a.z; acc[3] = acc[3] + weight * a.w;
-            acc[ND - 1] = acc[ND - 1] + weight * b.x;
-        }
-    }
-#pragma unroll
-    for (int d = 0; d < ND; ++d) out[d] = s.valid ? (double)acc[d] : NAN;
-}
-
-// gradient lookup of the specialised filter (filter_resolve); F32 = LSM_FLAG_INTERP_FLOAT32
-template <bool F32>
-struct LeanGrad {
-    static constexpr bool kRotRel = true;     // relative_state_rot, like pair_value_raw below
-    template <int ND>
-    __device__ __forceinline__ static void eval(const GridDev& g, const double (&rel)[ND], double (&out)[ND]) {
-        if constexpr (F32) {
-            Stencil32f<ND> st;
-            stencil32f_setup<ND>(g, rel, st);
-            stencil32f_grad<ND>(g, st, out);
-        } else {
-            Stencil32<ND> st;
-            stencil32_setup<ND>(g, rel, st);
-            stencil32_grad<ND>(g, st, out);
-        }
-    }
-};
-
-// ---------------------------------------------------------------------------------------------
-// corner-packed table (GridDev::packed): builder + lookup. The lookup reproduces stencil32_setup + stencil32_value
-// bit for bit (same positions, weights, corner order, sequential adds), including the declared index clamp outside
-// the box; only NaN positions take the scattered path.
-// ---------------------------------------------------------------------------------------------
-// Table extent per dim: n on periodic dims; n + 1 on the others, slot c standing for the index pair
-// (max(c - 1, 0), min(c, n - 1)) - slot 0 is the "both clamped to node 0" pair the declared out-of-box behaviour needs,
-// slot n the "both clamped to node n - 1" pair - so every finite position is served by one chunk.
-template <int ND>
-__global__ void __launch_bounds__(256) lsm_pack_grid_kernel(const float* __restrict__ values, float* __restrict__ packed,
-                                                          GridDev g, long long cells) {
-    constexpr int NC = 1 << ND;
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= cells * NC) return;
-    const long long cell = t / NC; const int corner = (int)(t - cell * NC);
-    long long rem = cell, lin = 0, mul = 1;
-#pragma unroll
-    for (int d = ND - 1; d >= 0; --d) {
-        const int n = g.shape[d];
-        const int ext = g.periodic[d] ? n : n + 1;
-        const int c = (int)(rem % ext); rem /= ext;
-        int il, ih;
-        if (g.periodic[d]) { il = c; ih = c + 1 >= n ? c + 1 - n : c + 1; }
-        else { il = c - 1 < 0 ? 0 : c - 1; ih = c > n - 1 ? n - 1 : c; }
-        lin += (long long)(((corner >> (ND - 1 - d)) & 1) ? ih : il) * mul;
-        mul *= n;
-    }
-    packed[t] = values[lin];
-}
-
-// Which dimensions of a lookup wrap. kPeriodicRuntime reads GridDev::periodic (any grid); any other value is a
-// compile-time mask (bit d = dimension d is periodic), so the per-dimension branch and the inline integer modulo of the
-// dimensions that cannot wrap are not in the code at all. The pair kernel is instantiated for the mask of the grids the
-// specialised shapes are built for (kPairPeriodic) and falls back to the run-time form for any other grid.
-constexpr int kPeriodicRuntime = -1;
-template <int PER>
-__device__ __forceinline__ bool dim_periodic(const GridDev& g, int d) {
-    if constexpr (PER == kPeriodicRuntime) return g.periodic[d] != 0;
-    else return ((PER >> d) & 1) != 0;
-}
-// double integrator: no periodic dimension; airtaxi: the relative heading, dimension 2 (hj_grid.py)
-template <int DYN>
-constexpr int kPairPeriodic = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 0 : 1 << 2;
-
-// reproduces stencil32_setup + stencil32_value bit for bit; false only for NaN positions
-template <int ND, int PER = kPeriodicRuntime>
-__device__ __forceinline__ bool packed_value(const GridDev& g, const double (&x)[ND], double& out) {
-    constexpr int NC = 1 << ND;
-    double wlo[ND], whi[ND];
-    bool ok = true;
-    int cell = 0, mul = 1;
-#pragma unroll
-    for (int d = ND - 1; d >= 0; --d) {
-        double pos = div_exact(x[d] - g.lo[d], g.spacing[d], g.inv_spacing[d]);
-        if (isnan(pos)) ok = false;
-        if (!(fabs(pos) <= 1.0e9)) pos = pos < 0.0 ? -1.0e9 : 1.0e9;     // declared clamp, as in stencil32_setup
-        const double fl = floor(pos);
-        const double w = pos - fl;
-        wlo[d] = 1.0 - w; whi[d] = w;
-        const int n = g.shape[d];
-        if (dim_periodic<PER>(g, d)) {
-            const int il = wrap_index<(ND == 5)>((int)fl, n);
-            cell += il * mul; mul *= n;
-        } else {
-            const int c = min(max((int)fl, -1), n - 1) + 1;
-            cell += c * mul; mul *= n + 1;
-        }
-    }
-    if (!ok) return false;
-    const float4* src = reinterpret_cast<const float4*>(g.packed) + (size_t)cell * (NC / 4);
-    float v[NC];
-#pragma unroll
-    for (int k = 0; k < NC / 4; ++k) {
-        const float4 q = __ldg(src + k);
-        v[4 * k] = q.x; v[4 * k + 1] = q.y; v[4 * k + 2] = q.z; v[4 * k + 3] = q.w;
-    }
-    double acc = 0.0;
-#pragma unroll
-    for (int corner = 0; corner < NC; ++corner) {
-        double weight = 0.0;
-#pragma unroll
-        for (int d = 0; d < ND; ++d) {
-            const double wd = ((corner >> (ND - 1 - d)) & 1) ? whi[d] : wlo[d];
-            weight = (d == 0) ? wd : weight * wd;
-        }
-        acc = acc + weight * (double)v[corner];
-    }
-    out = acc;
-    return true;
-}
-
-// float32 twin of packed_value: reproduces stencil32f_setup + stencil32f_value bit for bit from the same table. The
-// slot c = clamp((int)fl, -1, n - 1) + 1 stands for the index pair interp_f32's clamp gives (non-periodic dims), the
-// wrapped il for the pair (il, (il + 1) mod n) (periodic dims). False only for NaN positions.
-template <int ND, int PER = kPeriodicRuntime>
-__device__ __forceinline__ bool packed_value_f32(const GridDev& g, const double (&x)[ND], double& out) {
-    constexpr int NC = 1 << ND;
-    float wlo[ND], whi[ND];
-    bool ok = true;
-    int cell = 0, mul = 1;
-#pragma unroll
-    for (int d = ND - 1; d >= 0; --d) {
-        float pos = grid_pos_f32(g, x[d], d);
-        if (isnan(pos)) ok = false;
-        pos = fminf(fmaxf(pos, -1.0e9f), 1.0e9f);      // declared clamp, as in stencil32f_setup
-        const float fl = floorf(pos);
-        const float w = pos - fl;
-        wlo[d] = 1.0f - w; whi[d] = w;
-        const int n = g.shape[d];
-        if (dim_periodic<PER>(g, d)) {
-            const int il = wrap_index<(ND == 5)>((int)fl, n);
-            cell += il * mul; mul *= n;
-        } else {
-            const int c = min(max((int)fl, -1), n - 1) + 1;
-            cell += c * mul; mul *= n + 1;
-        }
-    }
-    if (!ok) return false;
-    const float4* src = reinterpret_cast<const float4*>(g.packed) + (size_t)cell * (NC / 4);
-    float v[NC];
-#pragma unroll
-    for (int k = 0; k < NC / 4; ++k) {
-        const float4 q = __ldg(src + k);
-        v[4 * k] = q.x; v[4 * k + 1] = q.y; v[4 * k + 2] = q.z; v[4 * k + 3] = q.w;
-    }
-    float acc = 0.0f;
-#pragma unroll
-    for (int corner = 0; corner < NC; ++corner) acc = acc + corner_weight_f32<ND>(wlo, whi, corner) * v[corner];
-    out = (double)acc;
-    return true;
-}
-
-// the relative state arrives as scalars (r4 unused for ND == 4): an array reference would put the caller's `rel` in
-// local memory
-template <int ND>
-__device__ __noinline__ double pair_value_scattered(const GridDev& vg, double r0, double r1, double r2, double r3, double r4) {
-    double rel[ND];
-    rel[0] = r0; rel[1] = r1; rel[2] = r2; rel[3] = r3;
-    if constexpr (ND == 5) rel[4] = r4;
-    Stencil32<ND> st;
-    stencil32_setup<ND>(vg, rel, st);
-    if (!st.valid) return INFINITY;
-    const double v = stencil32_value<ND>(vg, st);
-    if (isnan(v)) return INFINITY;
-    return v;
-}
-// float32 arithmetic (no packed table, or a NaN position)
-template <int ND>
-__device__ __noinline__ double pair_value_scattered_f32(const GridDev& vg, double r0, double r1, double r2, double r3, double r4) {
-    double rel[ND];
-    rel[0] = r0; rel[1] = r1; rel[2] = r2; rel[3] = r3;
-    if constexpr (ND == 5) rel[4] = r4;
-    Stencil32f<ND> st;
-    stencil32f_setup<ND>(vg, rel, st);
-    if (!st.valid) return INFINITY;
-    const double v = stencil32f_value<ND>(vg, st);
-    if (isnan(v)) return INFINITY;
-    return v;
-}
-
-// raw (unshifted) HJ value of a relative state; +inf = outside the declared range / NaN. F32: LSM_FLAG_INTERP_FLOAT32
-template <int ND, int PER, bool F32 = false>
-__device__ __forceinline__ double pair_value_rel(const GridDev& vg, const double (&rel)[ND]) {
-    if constexpr (F32) {
-        if (vg.packed != nullptr) {
-            double v;
-            if (packed_value_f32<ND, PER>(vg, rel, v)) return isnan(v) ? INFINITY : v;
-        }
-        return pair_value_scattered_f32<ND>(vg, rel[0], rel[1], rel[2], rel[3], ND == 5 ? rel[ND - 1] : 0.0);
-    } else {
-        if (vg.packed != nullptr) {
-            double v;
-            if (packed_value<ND, PER>(vg, rel, v)) return isnan(v) ? INFINITY : v;
-        }
-        return pair_value_scattered<ND>(vg, rel[0], rel[1], rel[2], rel[3], ND == 5 ? rel[ND - 1] : 0.0);
-    }
-}
 
 // raw (unshifted) HJ value of the pair (ego, other); +inf = outside the declared range / NaN
 template <int DYN, bool F32 = false>
@@ -604,7 +160,7 @@ __device__ __forceinline__ double shift_value(double raw, double sep, const Grid
 //     been edited after the last record was written), and behind a masked reset, which leaves the records of envs
 //     outside the mask untouched (they may predate a set_state or never have been written).
 //
-// F32 = LSM_FLAG_INTERP_FLOAT32: the float32 lookup from the same corner-packed table (packed_value_f32).
+// F32 = LSM_FLAG_INTERP_FLOAT32: the float32 lookup from the same corner-packed table (packed_value<.., true>).
 // ---------------------------------------------------------------------------------------------
 constexpr int kPairThreads = 128;
 template <int DYN, int N, int L, int O, int PER, bool F32>
@@ -1175,8 +731,8 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                             // `min distance > coordination_range` as an exact test on the squared distance
                             const double best_d = (best_d2 >= kp.r2_gt) ? INFINITY : 0.0;
                             const double2 po = R.pos[kv];
-                            filter_resolve<DYN, LeanGrad<F32>>(kp, best_d, best_v, !isinf(best_v), x, y, s2, s3, po.x, po.y, P.as2[kv], P.as3[kv],
-                                                raw0, raw1, P.rawx[kv], P.rawy[kv], safe0, safe1, filt, hsc[0], hsc[1]);
+                            filter_resolve<DYN, true, F32>(kp, best_d, best_v, !isinf(best_v), x, y, s2, s3, po.x, po.y, P.as2[kv], P.as3[kv],
+                                                           raw0, raw1, P.rawx[kv], P.rawy[kv], safe0, safe1, filt, hsc[0], hsc[1]);
                         }
                     }
                     deconflict = dec; safety_filtered = filt;
@@ -1236,16 +792,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) lsm_agent_kernel(const __grid_con
                         double rpx, rpy;
                         rotate_into(x - gx, y - gy, P.lcos[goal_pre], P.lsin[goal_pre], rpx, rpy);   // tabulated cos / sin(gh)
                         const double rs[4] = { rpx, rpy, theta - gh, speed };
-                        double ttr;
-                        if constexpr (F32) {
-                            Stencil32f<4> st;
-                            stencil32f_setup<4>(kp.tg, rs, st);
-                            ttr = st.valid ? stencil32f_value<4>(kp.tg, st) : NAN;
-                        } else {
-                            Stencil32<4> st;
-                            stencil32_setup<4>(kp.tg, rs, st);
-                            ttr = st.valid ? stencil32_value<4>(kp.tg, st) : NAN;
-                        }
+                        double ttr = grid_value<4, F32>(kp.tg, rs);
                         if (isnan(ttr)) ttr = kp.tg.ttr_max;
                         rew -= 0.04 * ttr;
                         rew -= sen * cra;

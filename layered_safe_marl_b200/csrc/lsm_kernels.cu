@@ -2,7 +2,8 @@
 //
 //   lsm_kernel_spec.cuh     kernels specialised at compile time on (dynamics, N, L) - the fast path
 //   lsm_kernel_generic.cuh  run-time N / L fallback for every other configuration
-//   lsm_step_common.cuh     dynamics, HJ filter resolution, grid interpolation shared by both
+//   lsm_step_common.cuh     dynamics and HJ filter resolution shared by both
+//   lsm_grid.cuh            the HJ grid lookups of every kernel, in both arithmetics, and the grid-copy builders
 //   lsm_filter_op.cuh       the same filter as a standalone batched operator (lsm_safety_filter / lsm_hj_lookup)
 //
 // Specialised path: three launches per step (per-agent physics -> graph emission -> next step's pair values), see
@@ -130,7 +131,7 @@ const void* generic_ptr(int dynamics) {
                                                  : (const void*)lsm_generic_kernel<LSM_DYN_AIRTAXI>;
 }
 
-static bool kp_interp_f32(const KParams& kp) { return (kp.c.flags & LSM_FLAG_INTERP_FLOAT32) != 0; }
+static bool kp_float32_lookups(const KParams& kp) { return (kp.c.flags & LSM_FLAG_INTERP_FLOAT32) != 0; }
 
 cudaError_t kernel_prepare(const void* fn, int block_threads, int smem_bytes, int* regs, int* blocks_per_sm) {
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
@@ -297,7 +298,7 @@ cudaError_t math_eval_launch(int op, const double* a, const double* b, double* o
 // the standalone filter operator: instantiation of the handle's dynamics and interpolation mode, on the caller's stream
 cudaError_t safety_filter_launch(const KParams& kp, int sm_count, const FilterOpArgs& a, cudaStream_t stream) {
     if (a.rows <= 0) return cudaSuccess;
-    const bool f32 = kp_interp_f32(kp), di = kp.c.dynamics == LSM_DYN_DOUBLE_INTEGRATOR;
+    const bool f32 = kp_float32_lookups(kp), di = kp.c.dynamics == LSM_DYN_DOUBLE_INTEGRATOR;
     const void* fn = di ? (f32 ? (const void*)lsm_safety_filter_kernel<LSM_DYN_DOUBLE_INTEGRATOR, true>
                                : (const void*)lsm_safety_filter_kernel<LSM_DYN_DOUBLE_INTEGRATOR, false>)
                         : (f32 ? (const void*)lsm_safety_filter_kernel<LSM_DYN_AIRTAXI, true>
@@ -316,7 +317,7 @@ cudaError_t safety_filter_launch(const KParams& kp, int sm_count, const FilterOp
 
 cudaError_t hj_lookup_launch(const KParams& kp, int sm_count, const LookupArgs& a, cudaStream_t stream) {
     if (a.points <= 0) return cudaSuccess;
-    const bool f32 = kp_interp_f32(kp), di = kp.c.dynamics == LSM_DYN_DOUBLE_INTEGRATOR;
+    const bool f32 = kp_float32_lookups(kp), di = kp.c.dynamics == LSM_DYN_DOUBLE_INTEGRATOR;
     const void* fn = di ? (f32 ? (const void*)lsm_hj_lookup_kernel<LSM_DYN_DOUBLE_INTEGRATOR, true>
                                : (const void*)lsm_hj_lookup_kernel<LSM_DYN_DOUBLE_INTEGRATOR, false>)
                         : (f32 ? (const void*)lsm_hj_lookup_kernel<LSM_DYN_AIRTAXI, true>

@@ -1,6 +1,6 @@
 // lsm_step_common.cuh - device functions shared by the generic and the specialised step kernels.
 #pragma once
-#include "lsm_device.cuh"
+#include "lsm_grid.cuh"
 
 namespace lsm {
 
@@ -79,56 +79,44 @@ __device__ __forceinline__ void relative_state_rot(double ex, double ey, double 
     relative_state_rot_sc<DYN>(ex, ey, e2, e3, ox, oy, o2, o3, se, ce, r);
 }
 
+// HJ value of the generic kernel (safety_filter.py:192-201, 345-354); out of range (in_range = false, +inf) for a NaN
+// position or a NaN value
 template <int DYN>
 __device__ __forceinline__ double hj_value(const KParams& kp, const Curriculum& q,
                                            const double (&rel)[DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5], bool& in_range) {
-    constexpr int ND = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5;
-    if (kp.vg.f32) {
-        const double v32 = interp_f32_value<ND>(kp.vg, rel);
-        if (isnan(v32)) { in_range = false; return INFINITY; }
-        in_range = true;
-        return v32 - (q.sep - kp.vg.separation_distance);
-    }
-    Stencil<ND> st;
-    stencil_setup<ND>(kp.vg, rel, st);
-    if (!st.valid) { in_range = false; return INFINITY; }
-    const double v = stencil_value<ND>(kp.vg, st);
-    if (isnan(v)) { in_range = false; return INFINITY; }
-    in_range = true;
+    const double v = grid_value_rt(kp.vg, rel);
+    in_range = !isnan(v);
+    if (!in_range) return INFINITY;
     return v - (q.sep - kp.vg.separation_distance);
 }
 
 // Second half of the safety handles (safety_filter.py:225-260, 400-433) once the deconflicting agent
 // `kv` (first minimum of the HJ value) and the smallest distance are known: gradient lookup,
 // least-restrictive bang-bang or CBF-QP, control clipping, filtered flag.
-struct ClassicGrad {
-    static constexpr bool kRotRel = false;
-    template <int ND>
-    __device__ __forceinline__ static void eval(const GridDev& g, const double (&rel)[ND], double (&out)[ND]) {
-        if (g.f32) { interp_f32_grad<ND>(g, rel, out); return; }
-        Stencil<ND> st;
-        stencil_setup<ND>(g, rel, st);
-        stencil_grad<ND>(g, st, out);
-    }
-};
-
-template <int DYN, class GRAD = ClassicGrad>
+// SPEC: the specialised pipeline and the operator - relative state in the rotation form (relative_state_rot_sc, with
+// (se, ce) = lsm_sincos(e2) of the caller), gradient inline in the arithmetic F32. Otherwise the generic kernel - the
+// literal relative_state, gradient in the handle's arithmetic chosen at run time (grid_grad_rt).
+template <int DYN, bool SPEC, bool F32 = false>
 __device__ __forceinline__ void filter_resolve(const KParams& kp, double best_d, double best_v, bool kv_in_range,
                                                double ex, double ey, double e2, double e3,
                                                double ox, double oy, double o2, double o3,
                                                double raw0, double raw1, double oraw0, double oraw1,
                                                double& safe0, double& safe1, int& filtered,
-                                               double se = 0.0, double ce = 1.0 /* kRotRel: lsm_sincos(e2) of the caller */) {
+                                               double se = 0.0, double ce = 1.0) {
     constexpr int ND = DYN == LSM_DYN_DOUBLE_INTEGRATOR ? 4 : 5;
     const lsm_config& c = kp.c;
     if (best_d > c.coordination_range) return;
     if (!kv_in_range) return;
     double rel[ND];
-    if constexpr (GRAD::kRotRel) relative_state_rot_sc<DYN>(ex, ey, e2, e3, ox, oy, o2, o3, se, ce, rel);
-    else relative_state<DYN>(ex, ey, e2, e3, ox, oy, o2, o3, rel);
-    const double uref[4] = { raw0, raw1, oraw0, oraw1 };
     double g[ND];
-    GRAD::template eval<ND>(kp.vg, rel, g);
+    if constexpr (SPEC) {
+        relative_state_rot_sc<DYN>(ex, ey, e2, e3, ox, oy, o2, o3, se, ce, rel);
+        grid_grad<ND, F32>(kp.vg, rel, g);
+    } else {
+        relative_state<DYN>(ex, ey, e2, e3, ox, oy, o2, o3, rel);
+        grid_grad_rt(kp.vg, rel, g);
+    }
+    const double uref[4] = { raw0, raw1, oraw0, oraw1 };
     const double eps_hj = 0.4;
     double u[4]; bool aliased = false;
     const double dt = c.dt;

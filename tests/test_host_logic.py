@@ -138,7 +138,7 @@ def _fma(a, b, c):
 
 @pytest.mark.parametrize('which', ['di', 'airtaxi', 'ttr'])
 def test_div_exact_equals_division_on_the_synthetic_grids(which):
-    """lsm_kernel_spec.cuh div_exact: the HJ stencil divides by the grid spacing b through y = RN(1/b) as
+    """lsm_grid.cuh div_exact: the HJ stencil divides by the grid spacing b through y = RN(1/b) as
     q0 = a*y; r = fma(-b, q0, a); q = fma(r, y, q0). Markstein's proof that q = RN(a/b) assumes y is within one ulp of
     1/b in a sense RN(1/b) does not always meet, so check every dimension of the three synthetic grids: dividends
     a = x - lo for the grid nodes +-8 ulps, the box faces and random positions within two box widths outside."""
@@ -178,6 +178,8 @@ def test_oracle_interpolation_matches_stub():
     grid = hj.Grid(a.lo, a.hi, a.shape, (2,))
     s, keep = O.make_grid(a)
     rng = np.random.default_rng(0)
+    # the float64 arithmetic: an earlier oracle step / reset / observe in the float32 mode leaves the oracle's switch set
+    O.lib().lsmo_set_interp_float32(0)
     for _ in range(200):
         x = rng.uniform(a.lo - 1.0, a.hi + 1.0)
         x[2] = rng.uniform(-10, 10)

@@ -2,8 +2,9 @@
 lsm_emit_from_records): every re-emitted graph row is bit for bit the row the dense buffer stores.
 
 CPU: the ctypes mirror of lsm_record_emit_io; every kernel the library had before the record emission kernel keeps its
-SASS instruction for instruction (tests/golden/sass_kernels_before_record_emit.json: sha256 of each kernel's
-cuobjdump -sass listing), and the only kernels added are its instantiations.
+SASS instruction for instruction (tests/golden/sass_kernels_pinned.json: sha256 of each kernel's cuobjdump -sass
+listing, as the kernels stand since the shared HJ grid lookup of lsm_grid.cuh), and the only kernels added are the
+record emission kernel's instantiations.
 GPU: equality with the dense buffer across shapes, feature modes, chunked steps and auto-resets; disconnected entities
 with flags fixed and changing inside the step; the item edge cases."""
 import ctypes
@@ -55,12 +56,12 @@ def _cuobjdump():
     return exe
 
 
-def test_existing_kernels_keep_their_sass():
+def test_pinned_kernels_keep_their_sass():
     exe = _cuobjdump()
     assert exe is not None, "cuobjdump (CUDA toolkit) not found next to nvcc"
     import sass_diff
     now = sass_diff.kernels(_build.build(), exe)
-    before = json.load(open(os.path.join(REPO, 'tests', 'golden', 'sass_kernels_before_record_emit.json')))
+    before = json.load(open(os.path.join(REPO, 'tests', 'golden', 'sass_kernels_pinned.json')))
     digest = {k: hashlib.sha256('\n'.join(v).encode()).hexdigest() for k, v in now.items()}
     changed = sorted(k for k in before if digest.get(k) != before[k])
     assert not changed, f"kernels whose SASS changed or vanished: {changed}"
