@@ -16,11 +16,21 @@
  *                airtaxi [x_r, y_r, theta_rel (periodic), v_a, v_b].
  *   derivatives  WENO5 (Jiang-Peng) left / right derivatives from v[k-3 .. k+3] per dim; ghosts wrap on periodic dims
  *                and extrapolate away from zero on the others.
- *   Hamiltonian  H(x, p) = p . f(x) + sum_k a_k u*_k, a = p^T G, u*_k = a_k < 0 ? lo_k : hi_k (both agents' controls
- *                maximise, no disturbance), with the filter's drift, control Jacobian, float32-rounded boxes and airtaxi
- *                speed saturation.
+ *   Hamiltonian  H(x, p) = p . f(x) + sum_k a_k u*_k, a = p^T G, with the filter's drift, control Jacobian,
+ *                float32-rounded boxes and airtaxi speed saturation. The controls split into the ego's and the other
+ *                agent's: double integrator [ax_e, ay_e | ax_o, ay_o] (k = 0, 1 | 2, 3), airtaxi [w_a, w_b, a_a, a_b]
+ *                with k = 0, 2 the ego's and k = 1, 3 the other's. The ego's controls maximise, u*_k = a_k < 0 ? lo_k :
+ *                hi_k. The other agent's depend on the game:
+ *                  0 cooperative  maximise as well (lsm_hj_solve; no disturbance);
+ *                  1 adversarial  minimise, u*_k = a_k < 0 ? hi_k : lo_k (a disturbance, disturbance_mode 'min');
+ *                  2 constant     held at 0: their terms are dropped from H (the other keeps its velocity, or its
+ *                                 turn rate and speed).
  *   dissipation  global Lax-Friedrichs: dV/dtau = min(0, H(x, (p- + p+)/2) + sum_i alpha_i (p+_i - p-_i)/2), alpha
- *                from the lattice (lsm_hj_dissipation).
+ *                from the lattice (lsm_hj_dissipation, lsm_hj_game_dissipation): alpha_i = max |f_i| + sum_k max |G_ik|
+ *                max(|lo_k|, |hi_k|) over the controls in play. Cooperative and adversarial: [max|vx|, max|vy|, 1, 1]
+ *                and [f0 + W max|y|, f1 + W max|x|, 2 W, A, A]; constant: [max|vx|, max|vy|, 0.5, 0.5] and
+ *                [f0 + W max|y|, f1 + W max|x|, W, A, 0], with f0 = max |-v_a + v_b cos theta|, f1 = max |v_b sin theta|
+ *                over the nodes, W = 0.1 and A = max(|a_min|, |a_max|) = 0.002 (float32-rounded).
  *   time         tau from 0; steps of dt = cfl / sum_i(alpha_i / spacing_i), the last one before each horizon clipped
  *                to land on it; Shu-Osher TVD-RK3.
  *
@@ -72,6 +82,13 @@ int lsm_hj_dissipation(const lsm_hj_problem *problem, double alpha[5], double *d
  * again. `work`: lsm_hj_work_bytes bytes, 8-byte aligned; `initial` and `out` must not overlap it. */
 int lsm_hj_solve(const lsm_hj_problem *problem, const double *initial, const double *horizons, int32_t K, double *out,
                  void *work, void *stream);
+
+/* lsm_hj_dissipation and lsm_hj_solve for a game: 0 cooperative, 1 adversarial, 2 constant (the Hamiltonian above);
+ * any other value is refused with code 2. Game 0 is lsm_hj_dissipation / lsm_hj_solve bit for bit. The same work
+ * buffer (lsm_hj_work_bytes), arguments and stream rules as those. */
+int lsm_hj_game_dissipation(const lsm_hj_problem *problem, int32_t game, double alpha[5], double *dt);
+int lsm_hj_game_solve(const lsm_hj_problem *problem, int32_t game, const double *initial, const double *horizons,
+                      int32_t K, double *out, void *work, void *stream);
 
 typedef struct lsm_hj_ttr_problem {
     int32_t shape[4];               /* nodes per dim [x, y, theta, v], each >= 2; theta is periodic */

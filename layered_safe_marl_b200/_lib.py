@@ -119,7 +119,8 @@ EXPORTED_SYMBOLS = ('lsm_abi_version', 'lsm_last_error', 'lsm_create', 'lsm_dest
 PPO_EXPORTED_SYMBOLS = ('lsm_ppo_abi_version', 'lsm_ppo_last_error', 'lsm_compute_returns', 'lsm_returns_scratch_bytes')
 
 HJ_EXPORTED_SYMBOLS = ('lsm_hj_abi_version', 'lsm_hj_last_error', 'lsm_hj_work_bytes', 'lsm_hj_dissipation',
-                       'lsm_hj_solve', 'lsm_hj_ttr_work_bytes', 'lsm_hj_ttr_dissipation', 'lsm_hj_ttr_solve')
+                       'lsm_hj_solve', 'lsm_hj_game_dissipation', 'lsm_hj_game_solve', 'lsm_hj_ttr_work_bytes',
+                       'lsm_hj_ttr_dissipation', 'lsm_hj_ttr_solve')
 
 _libs = {}          # one CDLL per path: the product library and the per-shape libraries (_build.build_shape)
 
@@ -230,6 +231,12 @@ def load_hj():
     lib.lsm_hj_solve.argtypes = [C.POINTER(LsmHjProblem), C.c_void_p, C.POINTER(C.c_double), C.c_int32, C.c_void_p,
                                  C.c_void_p, C.c_void_p]
     lib.lsm_hj_solve.restype = C.c_int
+    lib.lsm_hj_game_dissipation.argtypes = [C.POINTER(LsmHjProblem), C.c_int32, C.POINTER(C.c_double),
+                                            C.POINTER(C.c_double)]
+    lib.lsm_hj_game_dissipation.restype = C.c_int
+    lib.lsm_hj_game_solve.argtypes = [C.POINTER(LsmHjProblem), C.c_int32, C.c_void_p, C.POINTER(C.c_double), C.c_int32,
+                                      C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.lsm_hj_game_solve.restype = C.c_int
     lib.lsm_hj_ttr_work_bytes.argtypes = [C.POINTER(LsmHjTtrProblem)]
     lib.lsm_hj_ttr_work_bytes.restype = C.c_int64
     lib.lsm_hj_ttr_dissipation.argtypes = [C.POINTER(LsmHjTtrProblem), C.POINTER(C.c_double), C.POINTER(C.c_double)]

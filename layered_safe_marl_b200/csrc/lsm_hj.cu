@@ -1,8 +1,9 @@
 // lsm_hj.cu - the HJ reachability solver declared in include/lsm_b200_hj.h (liblsm_b200_hj.so).
 //
-// lsm_hj_stage_kernel<DYN, STAGE>: one thread per lattice cell and one launch per TVD-RK3 stage. A thread reads the
-// 7-point window of the stage input along every dim (ghost nodes built in registers), forms the WENO5 left / right
-// derivatives, the global Lax-Friedrichs Hamiltonian and min(0, .), and writes the stage's RK combination
+// lsm_hj_stage_kernel<DYN, STAGE, GAME>: one thread per lattice cell and one launch per TVD-RK3 stage. A thread reads
+// the 7-point window of the stage input along every dim (ghost nodes built in registers), forms the WENO5 left / right
+// derivatives, the global Lax-Friedrichs Hamiltonian of the game (the other agent's controls maximise, minimise or are
+// held at 0; the ego's maximise) and min(0, .), and writes the stage's RK combination
 // c0 * u0 + c1 * (u + h * L(u)). Stage 3 writes in place over u0: a cell reads u0 only at itself, so three stage arrays
 // suffice. The window loads of a warp are 32 consecutive cells at one offset, so every load is coalesced; the reuse
 // between neighbouring cells is served by L1 / L2 (the default grids are 6-26 MB).
@@ -31,8 +32,8 @@ namespace {
 thread_local std::string g_err;
 
 int fail(int code, const std::string& msg) { g_err = msg; return code; }
-int cuda_fail(cudaError_t e, const char* what) {
-    g_err = std::string(what) + ": " + cudaGetErrorString(e);
+int cuda_fail(cudaError_t e, const std::string& what) {
+    g_err = what + ": " + cudaGetErrorString(e);
     return 100 + (int)e;
 }
 
@@ -120,8 +121,23 @@ __device__ __forceinline__ void derivs(const double* __restrict__ u, int64_t cel
     right = weno5(D[5], D[4], D[3], D[2], D[1]);
 }
 
-// STAGE 0: u + h L(u);  1: 3/4 u0 + 1/4 (u + h L(u));  2: 1/3 u0 + 2/3 (u + h L(u))
-template <int DYN, int STAGE>
+// The games (include/lsm_b200_hj.h lsm_hj_game_solve): what the other agent's controls do in H
+enum Game { COOPERATIVE = 0, ADVERSARIAL = 1, CONSTANT = 2 };
+
+// H's term of control k with switching function a and box [lo, hi]: the ego's controls (double integrator k = 0, 1;
+// airtaxi k = 0, 2) maximise; the other agent's maximise (cooperative), minimise (adversarial) or are held at 0
+// (constant: no term)
+template <int DYN, int GAME>
+__device__ __forceinline__ double control_term(double H, int k, double a, double lo, double hi) {
+    const bool other = DYN == 0 ? k >= 2 : (k & 1) != 0;
+    if (GAME == COOPERATIVE || !other) return H + a * (a < 0.0 ? lo : hi);
+    if (GAME == ADVERSARIAL) return H + a * (a < 0.0 ? hi : lo);
+    return H;
+}
+
+// STAGE 0: u + h L(u);  1: 3/4 u0 + 1/4 (u + h L(u));  2: 1/3 u0 + 2/3 (u + h L(u)). GAME is the last template
+// parameter, so the cooperative instantiations are the kernel lsm_hj_solve always ran, with GAME = 0 added to the name.
+template <int DYN, int STAGE, int GAME>
 __global__ void __launch_bounds__(BLOCK) lsm_hj_stage_kernel(const StageParams p) {
     constexpr int ND = Dims<DYN>::ND;
     const int64_t cell = (int64_t)blockIdx.x * BLOCK + threadIdx.x;
@@ -145,7 +161,7 @@ __global__ void __launch_bounds__(BLOCK) lsm_hj_stage_kernel(const StageParams p
         H = q[0] * vx + q[1] * vy;
         const double a[4] = {q[2], q[3], -q[2], -q[3]};
 #pragma unroll
-        for (int k = 0; k < 4; ++k) H = H + a[k] * (a[k] < 0.0 ? -DI_U : DI_U);
+        for (int k = 0; k < 4; ++k) H = control_term<DYN, GAME>(H, k, a[k], -DI_U, DI_U);
     } else {
         const double x = p.coords[p.coord_off[0] + idx[0]], y = p.coords[p.coord_off[1] + idx[1]];
         const double c = p.cth[idx[2]], s = p.sth[idx[2]];
@@ -161,7 +177,7 @@ __global__ void __launch_bounds__(BLOCK) lsm_hj_stage_kernel(const StageParams p
         if (vb >= AT_VMAX) { lo2 = AT_AMIN; hi2 = AT_AMAX; lo3 = AT_AMIN; hi3 = AT_AMAX; hi3 = 0.0; }
         const double lo[4] = {-AT_W, -AT_W, lo2, lo3}, hi[4] = {AT_W, AT_W, hi2, hi3};
 #pragma unroll
-        for (int k = 0; k < 4; ++k) H = H + a[k] * (a[k] < 0.0 ? lo[k] : hi[k]);
+        for (int k = 0; k < 4; ++k) H = control_term<DYN, GAME>(H, k, a[k], lo[k], hi[k]);
     }
     double diss = p.alpha[0] * ((pr[0] - pl[0]) * 0.5);
 #pragma unroll
@@ -245,17 +261,23 @@ __global__ void __launch_bounds__(BLOCK) lsm_hj_ttr_stage_kernel(const TtrParams
     }
 }
 
-template <int DYN>
+template <int DYN, int GAME>
 cudaError_t launch_step(StageParams p, double* u0, double* u1, double* u2, double h, cudaStream_t st) {
     const unsigned grid = (unsigned)((p.cells + BLOCK - 1) / BLOCK);
     p.h = h;
     p.u = u0; p.u0 = u0; p.out = u1;
-    lsm_hj_stage_kernel<DYN, 0><<<grid, BLOCK, 0, st>>>(p);
+    lsm_hj_stage_kernel<DYN, 0, GAME><<<grid, BLOCK, 0, st>>>(p);
     p.u = u1; p.out = u2;
-    lsm_hj_stage_kernel<DYN, 1><<<grid, BLOCK, 0, st>>>(p);
+    lsm_hj_stage_kernel<DYN, 1, GAME><<<grid, BLOCK, 0, st>>>(p);
     p.u = u2; p.out = u0;
-    lsm_hj_stage_kernel<DYN, 2><<<grid, BLOCK, 0, st>>>(p);
+    lsm_hj_stage_kernel<DYN, 2, GAME><<<grid, BLOCK, 0, st>>>(p);
     return cudaGetLastError();
+}
+
+template <int GAME>
+cudaError_t launch_game_step(int dyn, const StageParams& p, double* u0, double* u1, double* u2, double h,
+                             cudaStream_t st) {
+    return dyn == 0 ? launch_step<0, GAME>(p, u0, u1, u2, h, st) : launch_step<1, GAME>(p, u0, u1, u2, h, st);
 }
 
 cudaError_t launch_ttr_step(TtrParams p, double* u0, double* u1, double* u2, double tau0, double h, cudaStream_t st) {
@@ -334,14 +356,16 @@ double cfl_step(const Lattice& L, const double* alpha, double cfl) {
     return cfl / s;
 }
 
-void dissipation(const lsm_hj_problem* pr, const Lattice& L, double alpha[5], double* dt) {
+// alpha_i = max |f_i| + sum_k max |G_ik| max(|lo_k|, |hi_k|) over the controls in play: all four (cooperative,
+// adversarial) or the ego's two (constant)
+void dissipation(const lsm_hj_problem* pr, int game, const Lattice& L, double alpha[5], double* dt) {
     for (int d = 0; d < 5; ++d) alpha[d] = 0.0;
     const double* c = L.coords.data();
     if (pr->dynamics == 0) {
         alpha[0] = max_abs(c + L.off[2], pr->shape[2]);
         alpha[1] = max_abs(c + L.off[3], pr->shape[3]);
-        alpha[2] = DI_U + DI_U;
-        alpha[3] = DI_U + DI_U;
+        alpha[2] = game == CONSTANT ? DI_U : DI_U + DI_U;
+        alpha[3] = game == CONSTANT ? DI_U : DI_U + DI_U;
     } else {
         double f0 = 0.0, f1 = 0.0;
         for (int t = 0; t < pr->shape[2]; ++t)
@@ -353,9 +377,9 @@ void dissipation(const lsm_hj_problem* pr, const Lattice& L, double alpha[5], do
                 }
         alpha[0] = f0 + AT_W * max_abs(c + L.off[1], pr->shape[1]);
         alpha[1] = f1 + AT_W * max_abs(c + L.off[0], pr->shape[0]);
-        alpha[2] = AT_W + AT_W;
+        alpha[2] = game == CONSTANT ? AT_W : AT_W + AT_W;
         alpha[3] = fmax(fabs(AT_AMIN), fabs(AT_AMAX));
-        alpha[4] = alpha[3];
+        alpha[4] = game == CONSTANT ? 0.0 : alpha[3];
     }
     *dt = cfl_step(L, alpha, pr->cfl);
 }
@@ -392,44 +416,40 @@ cudaError_t upload_lattice(const Lattice& L, double* aux, cudaStream_t st) {
     return e;
 }
 
-}  // namespace
-
-extern "C" {
-
-int lsm_hj_abi_version(void) { return LSM_HJ_ABI_VERSION; }
-const char* lsm_hj_last_error(void) { return g_err.c_str(); }
-
-int64_t lsm_hj_work_bytes(const lsm_hj_problem* problem) {
-    Lattice L;
-    if (check_problem(problem, "lsm_hj_work_bytes", L) != 0) return 0;
-    return (3 * L.cells + aux_doubles(L)) * (int64_t)sizeof(double);
-}
-
-int lsm_hj_dissipation(const lsm_hj_problem* problem, double alpha[5], double* dt) {
-    Lattice L;
-    if (const int rc = check_problem(problem, "lsm_hj_dissipation", L)) return rc;
-    if (!alpha || !dt) return fail(2, "lsm_hj_dissipation: alpha and dt must be non-NULL");
-    dissipation(problem, L, alpha, dt);
+int check_game(int32_t game, const std::string& fn) {
+    if (game != COOPERATIVE && game != ADVERSARIAL && game != CONSTANT)
+        return fail(2, fn + ": game must be 0 (cooperative), 1 (adversarial) or 2 (constant)");
     return 0;
 }
 
-int lsm_hj_solve(const lsm_hj_problem* problem, const double* initial, const double* horizons, int32_t K, double* out,
-                 void* work, void* stream) {
+int game_dissipation(const char* fn, const lsm_hj_problem* problem, int32_t game, double alpha[5], double* dt) {
     Lattice L;
-    if (const int rc = check_problem(problem, "lsm_hj_solve", L)) return rc;
+    if (const int rc = check_problem(problem, fn, L)) return rc;
+    if (const int rc = check_game(game, fn)) return rc;
+    if (!alpha || !dt) return fail(2, std::string(fn) + ": alpha and dt must be non-NULL");
+    dissipation(problem, game, L, alpha, dt);
+    return 0;
+}
+
+int solve(const char* fn_, const lsm_hj_problem* problem, int32_t game, const double* initial, const double* horizons,
+          int32_t K, double* out, void* work, void* stream) {
+    const std::string fn(fn_);
+    Lattice L;
+    if (const int rc = check_problem(problem, fn_, L)) return rc;
+    if (const int rc = check_game(game, fn)) return rc;
     if (!initial || !horizons || !out || !work)
-        return fail(2, "lsm_hj_solve: initial, horizons, out and work must be non-NULL");
-    if (K < 1) return fail(2, "lsm_hj_solve: K must be >= 1");
+        return fail(2, fn + ": initial, horizons, out and work must be non-NULL");
+    if (K < 1) return fail(2, fn + ": K must be >= 1");
     if ((reinterpret_cast<uintptr_t>(work) % alignof(double)) != 0)
-        return fail(2, "lsm_hj_solve: work must be 8-byte aligned");
+        return fail(2, fn + ": work must be 8-byte aligned");
     for (int32_t k = 0; k < K; ++k) {
         if (!(std::isfinite(horizons[k]) && horizons[k] >= 0.0))
-            return fail(2, "lsm_hj_solve: horizons must be finite and >= 0");
-        if (k > 0 && horizons[k] < horizons[k - 1]) return fail(2, "lsm_hj_solve: horizons must be non-decreasing");
+            return fail(2, fn + ": horizons must be finite and >= 0");
+        if (k > 0 && horizons[k] < horizons[k - 1]) return fail(2, fn + ": horizons must be non-decreasing");
     }
     double alpha[5], dt;
-    dissipation(problem, L, alpha, &dt);
-    if (!(dt > 0.0 && std::isfinite(dt))) return fail(2, "lsm_hj_solve: the CFL time step is not positive and finite");
+    dissipation(problem, game, L, alpha, &dt);
+    if (!(dt > 0.0 && std::isfinite(dt))) return fail(2, fn + ": the CFL time step is not positive and finite");
 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int64_t cells = L.cells, bytes = cells * (int64_t)sizeof(double);
@@ -438,9 +458,9 @@ int lsm_hj_solve(const lsm_hj_problem* problem, const double* initial, const dou
     double* u2 = u1 + cells;
     double* aux = u2 + cells;
     cudaError_t e = upload_lattice(L, aux, st);
-    if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_solve: upload of the lattice");
+    if (e != cudaSuccess) return cuda_fail(e, fn + ": upload of the lattice");
     e = cudaMemcpyAsync(u0, initial, bytes, cudaMemcpyDeviceToDevice, st);
-    if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_solve: copy of the initial values");
+    if (e != cudaSuccess) return cuda_fail(e, fn + ": copy of the initial values");
 
     StageParams p{};
     p.coords = aux;
@@ -463,13 +483,47 @@ int lsm_hj_solve(const lsm_hj_problem* problem, const double* initial, const dou
             double h;
             if (target - tau <= dt) { h = target - tau; tau = target; }
             else { h = dt; tau = tau + dt; }
-            e = problem->dynamics == 0 ? launch_step<0>(p, u0, u1, u2, h, st) : launch_step<1>(p, u0, u1, u2, h, st);
+            const int dyn = problem->dynamics;
+            e = game == COOPERATIVE ? launch_game_step<COOPERATIVE>(dyn, p, u0, u1, u2, h, st)
+              : game == ADVERSARIAL ? launch_game_step<ADVERSARIAL>(dyn, p, u0, u1, u2, h, st)
+                                    : launch_game_step<CONSTANT>(dyn, p, u0, u1, u2, h, st);
             if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_stage_kernel");
         }
         e = cudaMemcpyAsync(out + (int64_t)k * cells, u0, bytes, cudaMemcpyDeviceToDevice, st);
-        if (e != cudaSuccess) return cuda_fail(e, "lsm_hj_solve: snapshot");
+        if (e != cudaSuccess) return cuda_fail(e, fn + ": snapshot");
     }
     return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int lsm_hj_abi_version(void) { return LSM_HJ_ABI_VERSION; }
+const char* lsm_hj_last_error(void) { return g_err.c_str(); }
+
+int64_t lsm_hj_work_bytes(const lsm_hj_problem* problem) {
+    Lattice L;
+    if (check_problem(problem, "lsm_hj_work_bytes", L) != 0) return 0;
+    return (3 * L.cells + aux_doubles(L)) * (int64_t)sizeof(double);
+}
+
+int lsm_hj_dissipation(const lsm_hj_problem* problem, double alpha[5], double* dt) {
+    return game_dissipation("lsm_hj_dissipation", problem, COOPERATIVE, alpha, dt);
+}
+
+int lsm_hj_game_dissipation(const lsm_hj_problem* problem, int32_t game, double alpha[5], double* dt) {
+    return game_dissipation("lsm_hj_game_dissipation", problem, game, alpha, dt);
+}
+
+int lsm_hj_solve(const lsm_hj_problem* problem, const double* initial, const double* horizons, int32_t K, double* out,
+                 void* work, void* stream) {
+    return solve("lsm_hj_solve", problem, COOPERATIVE, initial, horizons, K, out, work, stream);
+}
+
+int lsm_hj_game_solve(const lsm_hj_problem* problem, int32_t game, const double* initial, const double* horizons,
+                      int32_t K, double* out, void* work, void* stream) {
+    return solve("lsm_hj_game_solve", problem, game, initial, horizons, K, out, work, stream);
 }
 
 int64_t lsm_hj_ttr_work_bytes(const lsm_hj_ttr_problem* problem) {

@@ -8,6 +8,12 @@ float64, the declared scheme of DESIGN.md "HJ value functions" - with the projec
     grid = reachability.value_grid('double_integrator')          # default lattice, 4 s horizon
     env = B200GraphVecEnv(args, value_grid=grid)
 
+`game` chooses what the other agent of the pair does (DESIGN.md "HJ value functions"): 'cooperative' (the default,
+the reference's game: it plays its part of the avoidance manoeuvre), 'adversarial' (it does its worst: the value the
+ego alone can guarantee) or 'constant' (it holds its controls at 0: traffic that runs no filter).
+
+    grid = reachability.value_grid('airtaxi', game='adversarial')
+
 It also computes the airtaxi time-to-reach grid the reward looks up (DESIGN.md "Time-to-reach grid"): the same scheme
 on a reach problem to the goal, with first-arrival times taken during the solve.
 
@@ -32,6 +38,8 @@ NDIM = {0: 4, 1: 5}
 PERIODIC = {0: (False,) * 4, 1: (False, False, True, False, False)}
 # horizons after which the default lattices have converged (DESIGN.md "HJ value functions": max|V(H) - V(H/2)|)
 DEFAULT_HORIZON = {0: 4.0, 1: 60.0}
+# the games of lsm_hj_game_solve (include/lsm_b200_hj.h)
+GAMES = {'cooperative': 0, 'adversarial': 1, 'constant': 2}
 TTR_PERIODIC = (False, False, True, False)
 # horizon of the default TTR lattice: every cell more than 2 km inside the x/y boundary is reached by then
 # (DESIGN.md "Time-to-reach grid")
@@ -51,22 +59,39 @@ def _problem(dyn: int, shape: Sequence[int], lo, hi, cfl: float) -> _lib.LsmHjPr
     return pr
 
 
-def dissipation(dynamics, shape, lo, hi, cfl: float = 0.75):
-    """The global Lax-Friedrichs coefficients (ndim float64) and the CFL time step of a lattice."""
+def parse_game(game) -> int:
+    """'cooperative' / 'adversarial' / 'constant' or its code 0 / 1 / 2 -> the code."""
+    if isinstance(game, str):
+        if game not in GAMES:
+            raise ValueError(f"unknown game {game!r}: one of {sorted(GAMES)}")
+        return GAMES[game]
+    if isinstance(game, (int, np.integer)) and not isinstance(game, bool) and int(game) in GAMES.values():
+        return int(game)
+    raise ValueError(f"unknown game {game!r}: one of {sorted(GAMES)} or its code 0, 1, 2")
+
+
+def dissipation(dynamics, shape, lo, hi, cfl: float = 0.75, game='cooperative'):
+    """The global Lax-Friedrichs coefficients (ndim float64) and the CFL time step of a lattice for a game."""
     dyn = parse_dynamics(dynamics)
+    g = parse_game(game)
     pr = _problem(dyn, shape, lo, hi, cfl)
     lib = _lib.load_hj()
     alpha = (C.c_double * 5)()
     dt = C.c_double()
-    _lib.check(lib.lsm_hj_dissipation(C.byref(pr), alpha, C.byref(dt)), 'lsm_hj_dissipation', lib)
+    if g == 0:
+        _lib.check(lib.lsm_hj_dissipation(C.byref(pr), alpha, C.byref(dt)), 'lsm_hj_dissipation', lib)
+    else:
+        _lib.check(lib.lsm_hj_game_dissipation(C.byref(pr), g, alpha, C.byref(dt)), 'lsm_hj_game_dissipation', lib)
     return np.array(alpha[:NDIM[dyn]], dtype=np.float64), float(dt.value)
 
 
-def solve(dynamics, initial_values: torch.Tensor, lo, hi, horizons, cfl: float = 0.75) -> torch.Tensor:
+def solve(dynamics, initial_values: torch.Tensor, lo, hi, horizons, cfl: float = 0.75,
+          game='cooperative') -> torch.Tensor:
     """V(tau) for each tau in `horizons` (non-decreasing, >= 0) of the backward reachable tube from V(0) =
-    `initial_values` (a CUDA float64 tensor of the lattice's shape): float64 `(K, *shape)` on the same device. Runs on
-    torch's current stream and does not synchronise."""
+    `initial_values` (a CUDA float64 tensor of the lattice's shape) in `game` (GAMES): float64 `(K, *shape)` on the
+    same device. Runs on torch's current stream and does not synchronise."""
     dyn = parse_dynamics(dynamics)
+    g = parse_game(game)
     if not (isinstance(initial_values, torch.Tensor) and initial_values.is_cuda and initial_values.dtype == torch.float64):
         raise TypeError("initial_values must be a CUDA float64 tensor")
     pr = _problem(dyn, initial_values.shape, lo, hi, cfl)
@@ -83,9 +108,12 @@ def solve(dynamics, initial_values: torch.Tensor, lo, hi, horizons, cfl: float =
         work = torch.empty(nbytes, dtype=torch.uint8, device=dev)
         out = torch.empty((h.size,) + tuple(init.shape), dtype=torch.float64, device=dev)
         stream = torch.cuda.current_stream(dev).cuda_stream
-        rc = lib.lsm_hj_solve(C.byref(pr), C.c_void_p(init.data_ptr()), h.ctypes.data_as(C.POINTER(C.c_double)),
-                              int(h.size), C.c_void_p(out.data_ptr()), C.c_void_p(work.data_ptr()), C.c_void_p(stream))
-        _lib.check(rc, 'lsm_hj_solve', lib)
+        args = (C.c_void_p(init.data_ptr()), h.ctypes.data_as(C.POINTER(C.c_double)), int(h.size),
+                C.c_void_p(out.data_ptr()), C.c_void_p(work.data_ptr()), C.c_void_p(stream))
+        if g == 0:
+            _lib.check(lib.lsm_hj_solve(C.byref(pr), *args), 'lsm_hj_solve', lib)
+        else:
+            _lib.check(lib.lsm_hj_game_solve(C.byref(pr), g, *args), 'lsm_hj_game_solve', lib)
     return out
 
 
@@ -101,13 +129,16 @@ def target(dynamics, shape, lo, hi, separation_distance: float) -> np.ndarray:
 
 
 def value_grid(dynamics, separation_distance: Optional[float] = None, shape=None, lo=None, hi=None,
-               horizon: Optional[float] = None, target_separation_distance: Optional[float] = None) -> HjGrid:
+               horizon: Optional[float] = None, target_separation_distance: Optional[float] = None,
+               game='cooperative') -> HjGrid:
     """A computed value function as the `HjGrid` the environment and `SafetyFilter` consume. Solves the tube of
-    l(x) = |x[:2]| - separation_distance to `horizon` on the lattice (defaults: the dynamics' separation distance, the
-    DI_GRID_* / AIRTAXI_GRID_* lattice, 4 s / 60 s) and stores it the way the reference's value-function files do
-    (stored = -V, hj_grid.make_hj_handle), so the filter sees it at `target_separation_distance` (default: the
-    separation distance it was solved for). Solves on the current CUDA device."""
+    l(x) = |x[:2]| - separation_distance in `game` (GAMES) to `horizon` on the lattice (defaults: the dynamics'
+    separation distance, the DI_GRID_* / AIRTAXI_GRID_* lattice, 4 s / 60 s for every game) and stores it the way the
+    reference's value-function files do (stored = -V, hj_grid.make_hj_handle), so the filter sees it at
+    `target_separation_distance` (default: the separation distance it was solved for). Solves on the current CUDA
+    device."""
     dyn = parse_dynamics(dynamics)
+    g = parse_game(game)
     if separation_distance is None:
         separation_distance = (DoubleIntegratorConfig if dyn == 0 else AirTaxiConfig).SEPARATION_DISTANCE
     shape = tuple(shape if shape is not None else (DI_GRID_SHAPE if dyn == 0 else AIRTAXI_GRID_SHAPE))
@@ -118,7 +149,7 @@ def value_grid(dynamics, separation_distance: Optional[float] = None, shape=None
         target_separation_distance = separation_distance
     dev = torch.device('cuda', torch.cuda.current_device())
     l = torch.as_tensor(target(dyn, shape, lo, hi, separation_distance), device=dev)
-    v = solve(dyn, l, lo, hi, [horizon])[0].cpu().numpy()
+    v = solve(dyn, l, lo, hi, [horizon], game=g)[0].cpu().numpy()
     return make_hj_handle(-v, lo, hi, PERIODIC[dyn], separation_distance, target_separation_distance)
 
 

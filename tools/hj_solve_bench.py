@@ -2,6 +2,7 @@
 
     python tools/hj_solve_bench.py [--out FILE.jsonl] [--steps 20] [--eager-max-cells 30000000]
     python tools/hj_solve_bench.py --ttr [--out FILE.jsonl] [--steps 20]
+    python tools/hj_solve_bench.py --game adversarial [--out FILE.jsonl] [--steps 20]
 
 
 Per lattice (the two default lattices and refined ones of 10^7-10^8 cells):
@@ -14,6 +15,8 @@ Per lattice (the two default lattices and refined ones of 10^7-10^8 cells):
   counts as one op), the achieved FP64 op rate and the share of the measured HBM copy bandwidth (a 4 GiB
   device-to-device copy in the same run);
 - convergence: max|V(H) - V(H/2)| of each default lattice at its default horizon.
+With --game, the same value-function measurements for that game of lsm_hj_game_solve ('cooperative', the default,
+'adversarial' or 'constant'); the eager baseline is the cooperative game's only, so other games skip it.
 With --ttr, the airtaxi time-to-reach solve (reachability.solve_ttr) on the default TTR lattice and a refined one,
 with the same stage_us / solve_ms / rate / bound fields (no eager baseline) and, per lattice, the fraction of cells
 still unreached at the default horizon and at twice it.
@@ -191,7 +194,9 @@ def main():
     ap.add_argument('--steps', type=int, default=20, help='RK3 steps S of the per-stage difference')
     ap.add_argument('--eager-max-cells', type=int, default=30_000_000, help='skip the eager baseline above this size')
     ap.add_argument('--ttr', action='store_true', help='time the airtaxi time-to-reach solve instead')
+    ap.add_argument('--game', default='cooperative', choices=sorted(R.GAMES), help='the value-function game')
     a = ap.parse_args()
+    game = a.game
     assert torch.cuda.is_available(), "needs a CUDA device"
     info = gpu_info()
     peak = copy_peak_gbs()
@@ -200,13 +205,14 @@ def main():
         lines += run_ttr(a.steps, peak)
     for name, dyn, shape, lo, hi in ([] if a.ttr else CASES):
         cells = int(np.prod(shape))
-        alpha, dt = R.dissipation(dyn, shape, lo, hi)
+        alpha, dt = R.dissipation(dyn, shape, lo, hi, game=game)
         l = torch.as_tensor(R.target(dyn, shape, lo, hi, SEP[dyn]), device='cuda')
         S = a.steps
-        t1 = timed(lambda: R.solve(dyn, l, lo, hi, [S * dt]), reps=3)
-        t2 = timed(lambda: R.solve(dyn, l, lo, hi, [2 * S * dt]), reps=3)
+        t1 = timed(lambda: R.solve(dyn, l, lo, hi, [S * dt], game=game), reps=3)
+        t2 = timed(lambda: R.solve(dyn, l, lo, hi, [2 * S * dt], game=game), reps=3)
         stage_us = (t2 - t1) * 1e3 / (3 * S)
-        rec = dict(what='solve', case=name, dynamics=dyn, shape=list(shape), cells=cells, dt=dt, alpha=list(alpha),
+        rec = dict(what='solve', game=game, case=name, dynamics=dyn, shape=list(shape), cells=cells, dt=dt,
+                   alpha=list(alpha),
                    stage_us=round(stage_us, 2), cell_updates_per_s=cells / (3 * stage_us * 1e-6),
                    fp64_ops_per_cell_stage=OPS[dyn], min_bytes_per_cell_stage=round(BYTES, 2),
                    fp64_ops_per_s=OPS[dyn] * cells / (stage_us * 1e-6),
@@ -215,14 +221,14 @@ def main():
             H = R.DEFAULT_HORIZON[dyn]
             rec['horizon'] = H
             rec['steps'] = math.ceil(H / dt)
-            rec['solve_ms'] = round(timed(lambda: R.solve(dyn, l, lo, hi, [H]), reps=1), 3)
-            V = R.solve(dyn, l, lo, hi, [H / 2, H])
+            rec['solve_ms'] = round(timed(lambda: R.solve(dyn, l, lo, hi, [H], game=game), reps=1), 3)
+            V = R.solve(dyn, l, lo, hi, [H / 2, H], game=game)
             rec['convergence_max_abs_V(H)-V(H/2)'] = float((V[1] - V[0]).abs().max())
             rec['V_range'] = [float(V[1].min()), float(V[1].max())]
         else:
             rec['steps'] = S
             rec['solve_ms'] = round(t1, 3)
-        if cells <= a.eager_max_cells:
+        if cells <= a.eager_max_cells and game == 'cooperative':
             eg = Eager(HO.Lattice(dyn, shape, lo, hi), alpha)
             ms = timed(lambda: eg.step(l, dt), reps=3)
             rec['eager_step_ms'] = round(ms, 3)

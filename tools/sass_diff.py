@@ -1,9 +1,11 @@
-"""Compare the SASS of two builds of a library kernel by kernel (cuobjdump -sass; no GPU needed).
+r"""Compare the SASS of two builds of a library kernel by kernel (cuobjdump -sass; no GPU needed).
 
-    python tools/sass_diff.py OLD.so NEW.so
+    python tools/sass_diff.py OLD.so NEW.so [--rename PATTERN REPLACEMENT]
 
 Prints, per kernel, whether its instructions are identical (encodings and offsets included), and lists the kernels
-only one side has. Exit code 1 when a kernel both sides have differs."""
+only one side has. Exit code 1 when a kernel both sides have differs. --rename applies re.sub(PATTERN, REPLACEMENT) to
+OLD's kernel names first, for a kernel whose mangled name gained a template argument (e.g. 'ELi(\d)EEEv' ->
+'ELi\1ELi0EEEv' for an added trailing int parameter)."""
 from __future__ import annotations
 
 import re
@@ -29,6 +31,10 @@ def kernels(path: str, cuobjdump: str = 'cuobjdump') -> dict:
 
 def main(argv) -> int:
     old, new = kernels(argv[0]), kernels(argv[1])
+    if len(argv) == 5 and argv[2] == '--rename':
+        old = {re.sub(argv[3], argv[4], k): v for k, v in old.items()}
+    elif len(argv) != 2:
+        sys.exit(__doc__)
     same = sorted(k for k in old if k in new and old[k] == new[k])
     changed = sorted(k for k in old if k in new and old[k] != new[k])
     removed = sorted(k for k in old if k not in new)
