@@ -34,8 +34,8 @@
  *   time         tau from 0; steps of dt = cfl / sum_i(alpha_i / spacing_i), the last one before each horizon clipped
  *                to land on it; Shu-Osher TVD-RK3.
  *
- * The airtaxi time-to-reach grid (DESIGN.md "Time-to-reach grid"; tests/hj_ttr_oracle.py restates it op for op) is the
- * same scheme on a reach problem, also declared:
+ * The airtaxi time-to-reach grid (DESIGN.md "Time-to-reach grid"; tests/hj_solve_oracle.py restates it op for op too)
+ * is the same scheme on a reach problem, also declared:
  *   state        [x, y, theta (periodic), v]: one airtaxi relative to its goal, position rotated into the goal's frame,
  *                heading minus the goal's heading, speed (the point the airtaxi reward looks up).
  *   Hamiltonian  x' = v cos theta, y' = v sin theta, theta' = w, v' = a; the controls MINIMISE:

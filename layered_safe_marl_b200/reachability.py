@@ -21,6 +21,7 @@ on a reach problem to the goal, with first-arrival times taken during the solve.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import math
 from typing import Optional, Sequence
@@ -59,6 +60,19 @@ def _problem(dyn: int, shape: Sequence[int], lo, hi, cfl: float) -> _lib.LsmHjPr
     return pr
 
 
+@contextlib.contextmanager
+def _on_device(lib, work_bytes: str, pr, values: torch.Tensor):
+    """On `values`' device: (`values` made contiguous, the work buffer `work_bytes` sizes for `pr`, the handle of
+    torch's current stream) for one solve."""
+    dev = values.device
+    with torch.cuda.device(dev):
+        nbytes = getattr(lib, work_bytes)(C.byref(pr))
+        if nbytes <= 0:
+            _lib.check(2, work_bytes, lib)
+        yield (values.contiguous(), torch.empty(nbytes, dtype=torch.uint8, device=dev),
+               torch.cuda.current_stream(dev).cuda_stream)
+
+
 def parse_game(game) -> int:
     """'cooperative' / 'adversarial' / 'constant' or its code 0 / 1 / 2 -> the code."""
     if isinstance(game, str):
@@ -78,10 +92,7 @@ def dissipation(dynamics, shape, lo, hi, cfl: float = 0.75, game='cooperative'):
     lib = _lib.load_hj()
     alpha = (C.c_double * 5)()
     dt = C.c_double()
-    if g == 0:
-        _lib.check(lib.lsm_hj_dissipation(C.byref(pr), alpha, C.byref(dt)), 'lsm_hj_dissipation', lib)
-    else:
-        _lib.check(lib.lsm_hj_game_dissipation(C.byref(pr), g, alpha, C.byref(dt)), 'lsm_hj_game_dissipation', lib)
+    _lib.check(lib.lsm_hj_game_dissipation(C.byref(pr), g, alpha, C.byref(dt)), 'lsm_hj_game_dissipation', lib)
     return np.array(alpha[:NDIM[dyn]], dtype=np.float64), float(dt.value)
 
 
@@ -99,21 +110,12 @@ def solve(dynamics, initial_values: torch.Tensor, lo, hi, horizons, cfl: float =
     if h.ndim != 1 or h.size == 0:
         raise ValueError("horizons must be a non-empty 1-D sequence")
     lib = _lib.load_hj()
-    dev = initial_values.device
-    with torch.cuda.device(dev):
-        init = initial_values.contiguous()
-        nbytes = lib.lsm_hj_work_bytes(C.byref(pr))
-        if nbytes <= 0:
-            _lib.check(2, 'lsm_hj_work_bytes', lib)
-        work = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        out = torch.empty((h.size,) + tuple(init.shape), dtype=torch.float64, device=dev)
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        args = (C.c_void_p(init.data_ptr()), h.ctypes.data_as(C.POINTER(C.c_double)), int(h.size),
-                C.c_void_p(out.data_ptr()), C.c_void_p(work.data_ptr()), C.c_void_p(stream))
-        if g == 0:
-            _lib.check(lib.lsm_hj_solve(C.byref(pr), *args), 'lsm_hj_solve', lib)
-        else:
-            _lib.check(lib.lsm_hj_game_solve(C.byref(pr), g, *args), 'lsm_hj_game_solve', lib)
+    with _on_device(lib, 'lsm_hj_work_bytes', pr, initial_values) as (init, work, stream):
+        out = torch.empty((h.size,) + tuple(init.shape), dtype=torch.float64, device=init.device)
+        rc = lib.lsm_hj_game_solve(C.byref(pr), g, C.c_void_p(init.data_ptr()), h.ctypes.data_as(C.POINTER(C.c_double)),
+                                   int(h.size), C.c_void_p(out.data_ptr()), C.c_void_p(work.data_ptr()),
+                                   C.c_void_p(stream))
+        _lib.check(rc, 'lsm_hj_game_solve', lib)
     return out
 
 
@@ -182,16 +184,9 @@ def solve_ttr(target: torch.Tensor, lo, hi, horizon: float, cfl: float = 0.75):
         raise TypeError("target must be a CUDA float64 tensor")
     pr = _ttr_problem(target.shape, lo, hi, cfl)
     lib = _lib.load_hj()
-    dev = target.device
-    with torch.cuda.device(dev):
-        l = target.contiguous()
-        nbytes = lib.lsm_hj_ttr_work_bytes(C.byref(pr))
-        if nbytes <= 0:
-            _lib.check(2, 'lsm_hj_ttr_work_bytes', lib)
-        work = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    with _on_device(lib, 'lsm_hj_ttr_work_bytes', pr, target) as (l, work, stream):
         ttr = torch.empty_like(l)
         V = torch.empty_like(l)
-        stream = torch.cuda.current_stream(dev).cuda_stream
         rc = lib.lsm_hj_ttr_solve(C.byref(pr), C.c_void_p(l.data_ptr()), float(horizon), C.c_void_p(ttr.data_ptr()),
                                   C.c_void_p(V.data_ptr()), C.c_void_p(work.data_ptr()), C.c_void_p(stream))
         _lib.check(rc, 'lsm_hj_ttr_solve', lib)

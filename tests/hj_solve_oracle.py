@@ -1,5 +1,5 @@
-"""The declared HJ reachability scheme in numpy, op for op (test infrastructure: the reference liblsm_b200_hj.so is
-checked against; DESIGN.md "HJ value functions").
+"""The declared HJ reachability scheme in numpy, op for op (test infrastructure: the reference every solve of
+liblsm_b200_hj.so is checked against; DESIGN.md "HJ value functions" and "Time-to-reach grid", include/lsm_b200_hj.h).
 
 It restates `hj_reachability`'s default "very_high" method (WENO5 upwind derivatives, global Lax-Friedrichs, TVD-RK3,
 `backwards_reachable_tube`) for the filter's relative dynamics (oracle/lsm_oracle.c apply_safety_filter), in float64:
@@ -11,14 +11,28 @@ It restates `hj_reachability`'s default "very_high" method (WENO5 upwind derivat
   alpha_j = d_j / (S_j + 1e-6)^2 with d = 0.1 / 0.6 / 0.3 and the result sum(alpha phi) / sum(alpha). Ghost nodes wrap
   on periodic dims; otherwise v[-j] = v[0] + sign(v[0]) |v[1] - v[0]| j and v[n-1+j] = v[n-1] + sign(v[n-1])
   |v[n-1] - v[n-2]| j.
-- H(x, p) = p . f(x) + sum_k a_k u*_k with a = p^T G and u*_k = a_k < 0 ? lo_k : hi_k, both agents' controls maximising
-  (float32-rounded boxes; the airtaxi speed saturation as written, each test restarting from the unsaturated boxes).
+- H(x, p) = p . f(x) + sum_k a_k u*_k with a = p^T G (float32-rounded boxes; the airtaxi speed saturation as written,
+  each test restarting from the unsaturated boxes). The controls split into the ego's and the other agent's: double
+  integrator [ax_e, ay_e | ax_o, ay_o] (k = 0, 1 | 2, 3); airtaxi [w_a, w_b, a_a, a_b] with k = 0, 2 the ego's and
+  k = 1, 3 the other's. The ego's controls maximise, u*_k = a_k < 0 ? lo_k : hi_k; the other agent's depend on the game
+  of lsm_hj_game_solve: 0 cooperative, maximise as well; 1 adversarial, minimise, u*_k = a_k < 0 ? hi_k : lo_k;
+  2 constant, held at 0, their terms dropped from H.
 - dV/dtau = min(0, H(x, (p- + p+)/2) + sum_i alpha_i (p+_i - p-_i) / 2). This is hj_reachability's backward solve:
   its Euler step with time_direction = -1 applies the Lax-Friedrichs flux to -H, which makes the dissipation enter
   with a plus sign in tau = -t (upwind: for dV/dtau = c V_x, c > 0 it gives c p+).
-- alpha_i = max over nodes |f_i| + sum_k max over nodes |G_ik| max(|lo_k|, |hi_k|) (unsaturated boxes);
-  dt = cfl / sum_i(alpha_i / spacing_i); h = min(dt, horizon - tau), tau set to the horizon when it is reached.
+- alpha_i = max over nodes |f_i| + sum_k max over nodes |G_ik| max(|lo_k|, |hi_k|) over the controls in play
+  (unsaturated boxes): all four in games 0 and 1, the ego's two in game 2; dt = cfl / sum_i(alpha_i / spacing_i);
+  h = min(dt, horizon - tau), tau set to the horizon when it is reached.
 - TVD-RK3: u1 = u + h L(u); u2 = 3/4 u + 1/4 (u1 + h L(u1)); u3 = 1/3 u + 2/3 (u2 + h L(u2)).
+
+The airtaxi time-to-reach solve (Lattice kind TTR) is the same scheme on a reach problem:
+- State [x, y, theta (periodic), v]: one airtaxi relative to its goal, in the goal's frame.
+- H(x, p) = p0 (v cos th) + p1 (v sin th) + sum_k a_k (a_k < 0 ? hi_k : lo_k) with a = (p2, p3): the controls
+  minimise. Boxes w in +-AT_W, a in [AT_AMIN, AT_AMAX]; v <= AT_VMIN gives a >= 0, v >= AT_VMAX gives a <= 0, each test
+  restarting from the unsaturated box.
+- alpha = [max |v cos th|, max |v sin th|, AT_W, max(|AT_AMIN|, |AT_AMAX|)] over the nodes.
+- First arrival: ttr = 0 where l <= 0, +inf elsewhere; after each RK3 step (tau0, h, start V0, end V1) a cell still at
+  +inf with V1 <= 0 takes tau0 + h * (V0 / (V0 - V1)).
 """
 from __future__ import annotations
 
@@ -30,7 +44,10 @@ DI_U = 0.5
 AT_W = float(np.float32(0.1))
 AT_AMIN, AT_AMAX = float(np.float32(-0.001)), float(np.float32(0.002))
 AT_VMIN, AT_VMAX = 60 * 0.514444 * 0.001, 175 * 0.514444 * 0.001
-PERIODIC = {0: (False,) * 4, 1: (False, False, True, False, False)}
+TTR = 2                 # the Lattice kind of the time-to-reach solve, next to dynamics 0 and 1
+PERIODIC = {0: (False,) * 4, 1: (False, False, True, False, False), TTR: (False, False, True, False)}
+COOPERATIVE, ADVERSARIAL, CONSTANT = 0, 1, 2
+GAMES = (COOPERATIVE, ADVERSARIAL, CONSTANT)
 
 
 def trig(theta):
@@ -49,6 +66,8 @@ def trig(theta):
 
 
 class Lattice:
+    """The lattice of dynamics 0 (double integrator), 1 (airtaxi) or TTR."""
+
     def __init__(self, dyn, shape, lo, hi):
         self.dyn, self.shape = int(dyn), tuple(int(s) for s in shape)
         self.periodic = PERIODIC[self.dyn]
@@ -59,7 +78,7 @@ class Lattice:
         self.coords = [lo[d] + self.spacing[d] * np.arange(n[d], dtype=np.float64) for d in range(len(n))]
         self.inv_dx = [1.0 / s for s in self.spacing]
         self.cth = self.sth = None
-        if self.dyn == 1:
+        if self.dyn != 0:
             self.cth, self.sth = trig(self.coords[2])
 
     def sub(self, starts, stops):
@@ -73,17 +92,23 @@ class Lattice:
         return s
 
 
-def dissipation(lat: Lattice, cfl: float = 0.75):
+def dissipation(lat: Lattice, cfl: float = 0.75, game: int = COOPERATIVE):
     c = lat.coords
     if lat.dyn == 0:
-        alpha = [np.max(np.abs(c[2])), np.max(np.abs(c[3])), DI_U + DI_U, DI_U + DI_U]
-    else:
+        u = DI_U if game == CONSTANT else DI_U + DI_U
+        alpha = [np.max(np.abs(c[2])), np.max(np.abs(c[3])), u, u]
+    elif lat.dyn == 1:
         va = c[3][None, :, None]
         vb = c[4][None, None, :]
         f0 = np.max(np.abs(-va + vb * lat.cth[:, None, None]))
         f1 = np.max(np.abs(vb * lat.sth[:, None, None]))
         a3 = max(abs(AT_AMIN), abs(AT_AMAX))
-        alpha = [f0 + AT_W * np.max(np.abs(c[1])), f1 + AT_W * np.max(np.abs(c[0])), AT_W + AT_W, a3, a3]
+        alpha = [f0 + AT_W * np.max(np.abs(c[1])), f1 + AT_W * np.max(np.abs(c[0])),
+                 AT_W if game == CONSTANT else AT_W + AT_W, a3, 0.0 if game == CONSTANT else a3]
+    else:
+        v = c[3][None, :]
+        alpha = [np.max(np.abs(v * lat.cth[:, None])), np.max(np.abs(v * lat.sth[:, None])), AT_W,
+                 max(abs(AT_AMIN), abs(AT_AMAX))]
     alpha = [float(a) for a in alpha]
     s = alpha[0] / lat.spacing[0]
     for d in range(1, len(alpha)):
@@ -138,35 +163,74 @@ def _bcast(vec, d, nd):
     return vec.reshape((1,) * d + (-1,) + (1,) * (nd - d - 1))
 
 
-def rate(lat: Lattice, u, alpha):
-    """L(u) = min(0, H(x, (p- + p+)/2) + sum_i alpha_i (p+_i - p-_i)/2)."""
-    nd = u.ndim
-    pl, pr = zip(*[derivs(u, d, lat.inv_dx[d], lat.periodic[d]) for d in range(nd)])
-    q = [(pl[d] + pr[d]) * 0.5 for d in range(nd)]
+def is_other(dyn, k):
+    """Whether control k of the avoid Hamiltonian is the other agent's."""
+    return k >= 2 if dyn == 0 else k % 2 == 1
+
+
+def _term(H, dyn, k, a, lo, hi, game):
+    if game == COOPERATIVE or not is_other(dyn, k):
+        return H + a * np.where(a < 0.0, lo, hi)
+    if game == ADVERSARIAL:
+        return H + a * np.where(a < 0.0, hi, lo)
+    return H
+
+
+def avoid_hamiltonian(lat: Lattice, q, game: int = COOPERATIVE):
+    """H_game(x, q) of dynamics 0 or 1 on the lattice, q = [q0 ..] arrays of its shape."""
+    nd = len(q)
     if lat.dyn == 0:
         vx, vy = _bcast(lat.coords[2], 2, nd), _bcast(lat.coords[3], 3, nd)
         H = q[0] * vx + q[1] * vy
-        for a in (q[2], q[3], -q[2], -q[3]):
-            H = H + a * np.where(a < 0.0, -DI_U, DI_U)
-    else:
-        x, y = _bcast(lat.coords[0], 0, nd), _bcast(lat.coords[1], 1, nd)
-        c, s = _bcast(lat.cth, 2, nd), _bcast(lat.sth, 2, nd)
-        va, vb = _bcast(lat.coords[3], 3, nd), _bcast(lat.coords[4], 4, nd)
-        f0 = -va + vb * c
-        f1 = vb * s
-        H = q[0] * f0 + q[1] * f1
-        a = [(q[0] * y + q[1] * (-x)) + q[2] * (-1.0), q[2], q[3], q[4]]
-        shp = (1, 1, 1, lat.shape[3], lat.shape[4])
-        va_b, vb_b = np.broadcast_to(va, shp), np.broadcast_to(vb, shp)
-        lo2 = np.full(shp, AT_AMIN); hi2 = np.full(shp, AT_AMAX); lo3 = np.full(shp, AT_AMIN); hi3 = np.full(shp, AT_AMAX)
-        for cond, which in ((va_b <= AT_VMIN, 'lo2'), (va_b >= AT_VMAX, 'hi2'), (vb_b <= AT_VMIN, 'lo3'), (vb_b >= AT_VMAX, 'hi3')):
-            for arr, val in ((lo2, AT_AMIN), (hi2, AT_AMAX), (lo3, AT_AMIN), (hi3, AT_AMAX)):
-                arr[cond] = val
-            {'lo2': lo2, 'hi2': hi2, 'lo3': lo3, 'hi3': hi3}[which][cond] = 0.0
-        lo = [-AT_W, -AT_W, lo2, lo3]
-        hi = [AT_W, AT_W, hi2, hi3]
-        for k in range(4):
-            H = H + a[k] * np.where(a[k] < 0.0, lo[k], hi[k])
+        for k, a in enumerate((q[2], q[3], -q[2], -q[3])):
+            H = _term(H, 0, k, a, -DI_U, DI_U, game)
+        return H
+    x, y = _bcast(lat.coords[0], 0, nd), _bcast(lat.coords[1], 1, nd)
+    c, s = _bcast(lat.cth, 2, nd), _bcast(lat.sth, 2, nd)
+    va, vb = _bcast(lat.coords[3], 3, nd), _bcast(lat.coords[4], 4, nd)
+    f0 = -va + vb * c
+    f1 = vb * s
+    H = q[0] * f0 + q[1] * f1
+    a = [(q[0] * y + q[1] * (-x)) + q[2] * (-1.0), q[2], q[3], q[4]]
+    # the speed saturation: each test restarts from the unsaturated boxes, so only the last one that holds applies
+    shp = (1, 1, 1, lat.shape[3], lat.shape[4])
+    va_b, vb_b = np.broadcast_to(va, shp), np.broadcast_to(vb, shp)
+    last = np.full(shp, -1)
+    for j, cond in enumerate((va_b <= AT_VMIN, va_b >= AT_VMAX, vb_b <= AT_VMIN, vb_b >= AT_VMAX)):
+        last = np.where(cond, j, last)
+    lo = [-AT_W, -AT_W, np.where(last == 0, 0.0, AT_AMIN), np.where(last == 2, 0.0, AT_AMIN)]
+    hi = [AT_W, AT_W, np.where(last == 1, 0.0, AT_AMAX), np.where(last == 3, 0.0, AT_AMAX)]
+    for k in range(4):
+        H = _term(H, 1, k, a[k], lo[k], hi[k], game)
+    return H
+
+
+def ttr_hamiltonian(lat: Lattice, q):
+    """H(x, q) of the time-to-reach solve on the lattice, q = [q0 .. q3] arrays of its shape."""
+    c, s = _bcast(lat.cth, 2, 4), _bcast(lat.sth, 2, 4)
+    v = _bcast(lat.coords[3], 3, 4)
+    f0 = v * c
+    f1 = v * s
+    H = q[0] * f0 + q[1] * f1
+    lo3 = np.full(v.shape, AT_AMIN); hi3 = np.full(v.shape, AT_AMAX)
+    for cond, which in ((v <= AT_VMIN, 'lo3'), (v >= AT_VMAX, 'hi3')):
+        lo3[cond] = AT_AMIN; hi3[cond] = AT_AMAX
+        {'lo3': lo3, 'hi3': hi3}[which][cond] = 0.0
+    a = [q[2], q[3]]
+    lo = [-AT_W, lo3]
+    hi = [AT_W, hi3]
+    for k in range(2):
+        H = H + a[k] * np.where(a[k] < 0.0, hi[k], lo[k])
+    return H
+
+
+def rate(lat: Lattice, u, alpha, game: int = COOPERATIVE):
+    """L(u) = min(0, H(x, (p- + p+)/2) + sum_i alpha_i (p+_i - p-_i)/2), H the TTR Hamiltonian or the avoid one of
+    `game`."""
+    nd = u.ndim
+    pl, pr = zip(*[derivs(u, d, lat.inv_dx[d], lat.periodic[d]) for d in range(nd)])
+    q = [(pl[d] + pr[d]) * 0.5 for d in range(nd)]
+    H = ttr_hamiltonian(lat, q) if lat.dyn == TTR else avoid_hamiltonian(lat, q, game)
     diss = alpha[0] * ((pr[0] - pl[0]) * 0.5)
     for d in range(1, nd):
         diss = diss + alpha[d] * ((pr[d] - pl[d]) * 0.5)
@@ -174,32 +238,55 @@ def rate(lat: Lattice, u, alpha):
     return np.where(hh < 0.0, hh, 0.0)
 
 
-def rk3_step(lat: Lattice, u, alpha, h):
-    u1 = u + h * rate(lat, u, alpha)
-    u2 = 0.75 * u + 0.25 * (u1 + h * rate(lat, u1, alpha))
-    return C13 * u + C23 * (u2 + h * rate(lat, u2, alpha))
+def rk3_step(lat: Lattice, u, alpha, h, game: int = COOPERATIVE):
+    u1 = u + h * rate(lat, u, alpha, game)
+    u2 = 0.75 * u + 0.25 * (u1 + h * rate(lat, u1, alpha, game))
+    return C13 * u + C23 * (u2 + h * rate(lat, u2, alpha, game))
 
 
-def solve(dyn, initial, lo, hi, horizons, cfl=0.75):
-    """V(tau) for each tau of `horizons`: float64 (K, *shape)."""
-    lat = Lattice(dyn, np.shape(initial), lo, hi)
-    alpha, dt = dissipation(lat, cfl)
+def arrive(ttr, u0, u3, tau0, h):
+    """The write-once first-arrival update after one step from u0 to u3 (in place on ttr)."""
+    hit = (u3 <= 0.0) & (ttr == np.inf)
+    with np.errstate(divide='ignore', invalid='ignore'):
+        t = tau0 + h * (u0 / (u0 - u3))
+    ttr[hit] = t[hit]
+
+
+def _solve(lat: Lattice, initial, horizons, cfl, game, ttr=None):
+    """V(tau) for each tau of `horizons`: float64 (K, *shape). With `ttr`, the arrival update after every step."""
+    alpha, dt = dissipation(lat, cfl, game)
     u = np.array(initial, dtype=np.float64)
     tau, out = 0.0, []
-    for target in horizons:
-        target = float(target)
-        while tau < target:
-            if target - tau <= dt:
-                h, tau = target - tau, target
+    for horizon in horizons:
+        horizon = float(horizon)
+        while tau < horizon:
+            tau0 = tau
+            if horizon - tau <= dt:
+                h, tau = horizon - tau, horizon
             else:
                 h, tau = dt, tau + dt
-            u = rk3_step(lat, u, alpha, h)
+            u3 = rk3_step(lat, u, alpha, h, game)
+            if ttr is not None:
+                arrive(ttr, u, u3, tau0, h)
+            u = u3
         out.append(u.copy())
     return np.stack(out)
 
 
-def step_at(lat: Lattice, u_block, starts, alpha, h):
+def solve(dyn, initial, lo, hi, horizons, cfl=0.75, game: int = COOPERATIVE):
+    """V(tau) of `game` for each tau of `horizons`: float64 (K, *shape)."""
+    return _solve(Lattice(dyn, np.shape(initial), lo, hi), initial, horizons, cfl, game)
+
+
+def solve_ttr(target, lo, hi, horizon, cfl=0.75):
+    """The time-to-reach solve: (ttr, V(horizon)), float64 arrays of the target's shape."""
+    ttr = np.where(np.asarray(target) <= 0.0, 0.0, np.inf)
+    V = _solve(Lattice(TTR, np.shape(target), lo, hi), target, [horizon], cfl, COOPERATIVE, ttr)[0]
+    return ttr, V
+
+
+def step_at(lat: Lattice, u_block, starts, alpha, h, game: int = COOPERATIVE):
     """One RK3 step evaluated at the centre of a block cut from the full lattice: exact when the block reaches 9 nodes
     past the centre in every dim or ends at the lattice's own boundary (three stages of a 3-node stencil)."""
     stops = [a + s for a, s in zip(starts, u_block.shape)]
-    return rk3_step(lat.sub(starts, stops), u_block, alpha, h)
+    return rk3_step(lat.sub(starts, stops), u_block, alpha, h, game)

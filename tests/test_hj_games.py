@@ -1,10 +1,9 @@
 """The adversarial and constant-control games of the HJ solver (lsm_hj_game_solve, reachability.solve(game=...))
-against their numpy restatement (tests/hj_game_oracle.py), closed forms, an independent Hamiltonian and trajectories.
+against their numpy restatement (tests/hj_solve_oracle.py), closed forms, an independent Hamiltonian and trajectories.
 
-CPU: the game oracle's game 0 is hj_solve_oracle bit for bit; lsm_hj_game_dissipation equals the oracle bit for bit;
-invalid games and arguments are refused with code 2; the oracle meets the double-integrator slab's closed form in
-every game.
-GPU: the kernel equals the game oracle bit for bit; game 0 is lsm_hj_solve bit for bit; the slabs on the default and a
+CPU: lsm_hj_game_dissipation equals the oracle bit for bit, and its game 0 lsm_hj_dissipation; invalid games and
+arguments are refused with code 2; the oracle meets the double-integrator slab's closed form in every game.
+GPU: the kernel equals the oracle bit for bit; game 0 is lsm_hj_solve bit for bit; the slabs on the default and a
 refined lattice; the Hamiltonian cell by cell; V_adversarial <= V_constant <= V_cooperative; the adversarial value is
 guaranteed along trajectories against any other agent; the grids through the environment and SafetyFilter, bit for bit
 with the C oracle; a side stream."""
@@ -21,7 +20,6 @@ sys.path.insert(0, os.path.join(REPO, 'oracle'))
 sys.path.insert(0, os.path.join(REPO, 'tests'))
 
 import _golden as G  # noqa: E402
-import hj_game_oracle as GO  # noqa: E402
 import hj_solve_oracle as HO  # noqa: E402
 import test_hj_game as TG  # noqa: E402
 from layered_safe_marl_b200 import _lib, hj_grid  # noqa: E402
@@ -40,25 +38,13 @@ def _problem(dyn, shape, lo, hi, cfl=0.75):
 # ----------------------------------------------------------------------------------------------------------------------
 # CPU
 # ----------------------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize('dyn,shape', [(0, (9, 11, 7, 5)), (1, (7, 5, 9, 4, 6))])
-def test_game_oracle_cooperative_is_the_solve_oracle_bit_for_bit(dyn, shape):
-    _, lo, hi = DI_LAT if dyn == 0 else AT_LAT
-    l = R.target(dyn, shape, lo, hi, 0.5 if dyn == 0 else 0.4572)
-    init = l + 0.05 * np.random.default_rng(3 + dyn).standard_normal(shape)
-    _, dt = HO.dissipation(HO.Lattice(dyn, shape, lo, hi))
-    horizons = [2.5 * dt, 6.0 * dt]
-    got = GO.solve(dyn, init, lo, hi, horizons, game=GO.COOPERATIVE)
-    want = HO.solve(dyn, init, lo, hi, horizons)
-    assert np.array_equal(got.view(np.int64), want.view(np.int64))
-
-
-@pytest.mark.parametrize('game', GO.GAMES)
+@pytest.mark.parametrize('game', HO.GAMES)
 @pytest.mark.parametrize('dyn,shape,cfl', [(0, DI_LAT[0], 0.75), (0, (9, 11, 7, 5), 0.5), (1, AT_LAT[0], 0.75),
                                            (1, (9, 9, 8, 5, 5), 0.5), (1, (7, 9, 5, 4, 6), 1.0)])
 def test_game_dissipation_equals_the_oracle_bit_for_bit(dyn, shape, cfl, game):
     lo, hi = (DI_LAT if dyn == 0 else AT_LAT)[1:]
     alpha, dt = R.dissipation(dyn, shape, lo, hi, cfl, game=game)
-    o_alpha, o_dt = GO.dissipation(HO.Lattice(dyn, shape, lo, hi), cfl, game)
+    o_alpha, o_dt = HO.dissipation(HO.Lattice(dyn, shape, lo, hi), cfl, game)
     assert np.array_equal(alpha, o_alpha) and dt == o_dt, (alpha, o_alpha, dt, o_dt)
     lib = _lib.load_hj()
     pr = _problem(dyn, shape, lo, hi, cfl)
@@ -101,7 +87,7 @@ def test_invalid_games_and_arguments_are_refused_with_code_2():
     cases = [bad(dynamics=2), bad(dynamics=-1), bad(shape=(0, 1)), bad(shape=(3, 0)), bad(lo=(1, 4.5)),
              bad(lo=(2, float('nan'))), bad(hi=(0, float('inf'))), bad(cfl=0.0), bad(cfl=1.5), bad(cfl=float('nan')),
              bad(cfl=-0.5)]
-    for game in GO.GAMES:
+    for game in HO.GAMES:
         for pr in cases:
             assert solve_rc(ctypes.byref(pr), game) == 2, lib.lsm_hj_last_error()
             assert lib.lsm_hj_game_dissipation(ctypes.byref(pr), game, a, ctypes.byref(dt)) == 2
@@ -140,11 +126,11 @@ def _slab(shape, game, lo=DI_LAT[1], hi=DI_LAT[2]):
     vx = lat.coords[2][None, None, :, None]
     dx0, dx2 = lat.spacing[0], lat.spacing[2]
     l = np.broadcast_to(np.abs(px) - SLAB_R, shape).copy()
-    if game == GO.ADVERSARIAL:      # kinks where |px| = |vx| tau and along vx = 0, where the closing test switches
+    if game == HO.ADVERSARIAL:      # kinks where |px| = |vx| tau and along vx = 0, where the closing test switches
         reach = np.abs(vx) * SLAB_T
         kink = (np.abs(np.abs(px) - reach) < 2 * dx0 + 2 * dx2 * SLAB_T) | (np.abs(vx) < 2 * dx2 - 1e-12)
     else:
-        A = 1.0 if game == GO.COOPERATIVE else 0.5
+        A = 1.0 if game == HO.COOPERATIVE else 0.5
         reach = vx ** 2 / (2 * A)
         kink = np.abs(np.abs(px) - reach) < 2 * dx0 + 2 * dx2 * np.abs(vx) / A
     exact = np.broadcast_to(np.maximum(np.abs(px) - (px * vx < 0) * reach, 0.0) - SLAB_R, shape)
@@ -163,7 +149,7 @@ SLAB_REFINED = {0: 1.27e-3, 1: 3.05e-2, 2: 2.72e-2}
 SLAB_MARGIN = 1.1
 
 
-@pytest.mark.parametrize('game', GO.GAMES)
+@pytest.mark.parametrize('game', HO.GAMES)
 def test_oracle_meets_the_slab_in_every_game(game):
     """On the default lattice's (px, vx) nodes and spacings: py has 3 nodes 0.225 m apart and vy 3 nodes 0.1 m/s apart
     up to 1 m/s, so alpha and the time step are the default lattice's, and the slab, constant along py and vy, gets the
@@ -171,9 +157,9 @@ def test_oracle_meets_the_slab_in_every_game(game):
     shape = (41, 3, 21, 3)
     lo = (DI_LAT[1][0], -0.225, DI_LAT[1][2], 0.8)
     hi = (DI_LAT[2][0], 0.225, DI_LAT[2][2], 1.0)
-    assert GO.dissipation(HO.Lattice(0, shape, lo, hi), 0.75, game)[1] == R.dissipation(0, *DI_LAT, game=game)[1]
+    assert HO.dissipation(HO.Lattice(0, shape, lo, hi), 0.75, game)[1] == R.dissipation(0, *DI_LAT, game=game)[1]
     l, exact, mask = _slab(shape, game, lo, hi)
-    V = GO.solve(0, l, lo, hi, [SLAB_T], game=game)[0]
+    V = HO.solve(0, l, lo, hi, [SLAB_T], game=game)[0]
     err = float(np.abs(V - exact)[mask].max())
     print(f"slab, {NAMES[game]}, horizon {SLAB_T} s: max |V - V*| = {err * 1e3:.2f} mm over {int(mask.sum())} cells")
     assert (V <= l + 4 * np.spacing(np.abs(l))).all()
@@ -207,7 +193,7 @@ def _h_ref(dyn, r, c, game, rng):
     lo, hi = TG._boxes(dyn, r)
     best = None
     for e in range(4):
-        if game == GO.ADVERSARIAL:
+        if game == HO.ADVERSARIAL:
             v = np.min([TG._rel_rate(dyn, ego, oth, _joint(dyn, lo, hi, e, o)) @ c for o in range(4)], axis=0)
         else:
             v = TG._rel_rate(dyn, ego, oth, _joint(dyn, lo, hi, e, None)) @ c
@@ -238,15 +224,15 @@ def _check_game_probe(dyn, shape, lo, hi, c, game, solve):
     return H, r
 
 
-@pytest.mark.parametrize('game', [GO.ADVERSARIAL, GO.CONSTANT])
+@pytest.mark.parametrize('game', [HO.ADVERSARIAL, HO.CONSTANT])
 @pytest.mark.parametrize('seed', [0, 1, 2, 3])
 @pytest.mark.parametrize('dyn', [0, 1])
 def test_oracle_game_hamiltonian_cell_by_cell(dyn, seed, game):
     c = TG._probe_c(dyn, seed)
     for shape, lo, hi in TG._probe_lattices()[dyn]:
         H, r = _check_game_probe(dyn, shape, lo, hi, c, game,
-                                 lambda u: GO.solve(dyn, u, lo, hi, [TG.PROBE_H], game=game)[0])
-        if dyn == 1 and game == GO.ADVERSARIAL:
+                                 lambda u: HO.solve(dyn, u, lo, hi, [TG.PROBE_H], game=game)[0])
+        if dyn == 1 and game == HO.ADVERSARIAL:
             TG._assert_saturation_cases(H, r)
 
 
@@ -269,7 +255,7 @@ def _assert_bits(got, want, what):
 
 
 @gpu
-@pytest.mark.parametrize('game', [GO.ADVERSARIAL, GO.CONSTANT])
+@pytest.mark.parametrize('game', [HO.ADVERSARIAL, HO.CONSTANT])
 @pytest.mark.parametrize('dyn,shape', [(0, (9, 11, 7, 5)), (0, (6, 6, 6, 6)), (0, (2, 3, 9, 3)), (1, (9, 9, 8, 5, 5)),
                                        (1, (7, 5, 9, 4, 6)), (1, (3, 2, 2, 3, 5)), (1, 'speed_bounds')])
 def test_game_solve_equals_the_oracle_bit_for_bit(dyn, shape, game):
@@ -286,13 +272,13 @@ def test_game_solve_equals_the_oracle_bit_for_bit(dyn, shape, game):
     horizons = [0.0] + [k * dt for k in steps]
     for init in (l, l + 0.05 * rng.standard_normal(shape)):
         got = R.solve(dyn, _cuda(init), lo, hi, horizons, game=game).cpu().numpy()
-        want = GO.solve(dyn, init, lo, hi, horizons, game=game)
+        want = HO.solve(dyn, init, lo, hi, horizons, game=game)
         _assert_bits(got[0], init, 'horizon 0')
         _assert_bits(got, want, f'{NAMES[game]} dyn={dyn} shape={shape}')
 
 
 @gpu
-@pytest.mark.parametrize('game', [GO.ADVERSARIAL, GO.CONSTANT])
+@pytest.mark.parametrize('game', [HO.ADVERSARIAL, HO.CONSTANT])
 @pytest.mark.parametrize('dyn', [0, 1])
 def test_game_solve_equals_the_oracle_on_the_default_lattice(dyn, game):
     shape, lo, hi = DI_LAT if dyn == 0 else AT_LAT
@@ -300,11 +286,11 @@ def test_game_solve_equals_the_oracle_on_the_default_lattice(dyn, game):
     _, dt = R.dissipation(dyn, shape, lo, hi, game=game)
     horizons = [dt, 1.5 * dt] if dyn == 0 else [dt]
     got = R.solve(dyn, _cuda(l), lo, hi, horizons, game=game).cpu().numpy()
-    _assert_bits(got, GO.solve(dyn, l, lo, hi, horizons, game=game), f'{NAMES[game]} dyn={dyn} default lattice')
+    _assert_bits(got, HO.solve(dyn, l, lo, hi, horizons, game=game), f'{NAMES[game]} dyn={dyn} default lattice')
 
 
-def _raw_game_solve(dyn, init, lo, hi, horizons, game):
-    """lsm_hj_game_solve called directly (reachability.solve sends game 0 to lsm_hj_solve)."""
+def _raw_solve(dyn, init, lo, hi, horizons, game=None):
+    """lsm_hj_game_solve, or lsm_hj_solve when game is None, called directly."""
     import torch
     lib = _lib.load_hj()
     pr = _problem(dyn, init.shape, lo, hi)
@@ -312,10 +298,12 @@ def _raw_game_solve(dyn, init, lo, hi, horizons, game):
     h = np.asarray(horizons, dtype=np.float64)
     out = torch.empty((h.size,) + tuple(init.shape), dtype=torch.float64, device='cuda')
     stream = torch.cuda.current_stream().cuda_stream
-    rc = lib.lsm_hj_game_solve(ctypes.byref(pr), game, ctypes.c_void_p(init.data_ptr()),
-                               h.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), int(h.size),
-                               ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(work.data_ptr()), ctypes.c_void_p(stream))
-    _lib.check(rc, 'lsm_hj_game_solve', lib)
+    args = (ctypes.c_void_p(init.data_ptr()), h.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), int(h.size),
+            ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(work.data_ptr()), ctypes.c_void_p(stream))
+    if game is None:
+        _lib.check(lib.lsm_hj_solve(ctypes.byref(pr), *args), 'lsm_hj_solve', lib)
+    else:
+        _lib.check(lib.lsm_hj_game_solve(ctypes.byref(pr), game, *args), 'lsm_hj_game_solve', lib)
     return out
 
 
@@ -325,13 +313,13 @@ def test_game_zero_is_the_cooperative_solve_bit_for_bit(dyn):
     shape, lo, hi = DI_LAT if dyn == 0 else AT_LAT
     l = _cuda(R.target(dyn, shape, lo, hi, 0.5 if dyn == 0 else 0.4572))
     H = R.DEFAULT_HORIZON[dyn]
-    want = R.solve(dyn, l, lo, hi, [H / 2, H])
-    got = _raw_game_solve(dyn, l, lo, hi, [H / 2, H], 0)
+    want = _raw_solve(dyn, l, lo, hi, [H / 2, H])
+    got = _raw_solve(dyn, l, lo, hi, [H / 2, H], 0)
     _assert_bits(got.cpu().numpy(), want.cpu().numpy(), f'dyn={dyn} game 0 against lsm_hj_solve')
 
 
 @gpu
-@pytest.mark.parametrize('game', GO.GAMES)
+@pytest.mark.parametrize('game', HO.GAMES)
 def test_slab_in_every_game_on_the_default_lattice_and_refined(game):
     errs = []
     for shape in (DI_LAT[0], (81, 5, 41, 3)):
@@ -347,7 +335,7 @@ def test_slab_in_every_game_on_the_default_lattice_and_refined(game):
 
 
 @gpu
-@pytest.mark.parametrize('game', [GO.ADVERSARIAL, GO.CONSTANT])
+@pytest.mark.parametrize('game', [HO.ADVERSARIAL, HO.CONSTANT])
 @pytest.mark.parametrize('seed', [0, 1, 2, 3])
 @pytest.mark.parametrize('dyn', [0, 1])
 def test_solver_game_hamiltonian_cell_by_cell(dyn, seed, game):
@@ -355,7 +343,7 @@ def test_solver_game_hamiltonian_cell_by_cell(dyn, seed, game):
     for i, (shape, lo, hi) in enumerate(TG._probe_lattices()[dyn] + [TG.ODD_LATTICES[dyn]]):
         H, r = _check_game_probe(dyn, shape, lo, hi, c, game,
                                  lambda u: R.solve(dyn, _cuda(u), lo, hi, [TG.PROBE_H], game=game)[0].cpu().numpy())
-        if dyn == 1 and i == 0 and game == GO.ADVERSARIAL:
+        if dyn == 1 and i == 0 and game == HO.ADVERSARIAL:
             TG._assert_saturation_cases(H, r)
 
 
@@ -381,7 +369,7 @@ def test_adversarial_below_constant_below_cooperative(dyn):
     shape, lo, hi = DI_LAT if dyn == 0 else AT_LAT
     l = _cuda(R.target(dyn, shape, lo, hi, 0.5 if dyn == 0 else 0.4572))
     H = R.DEFAULT_HORIZON[dyn]
-    V = {g: R.solve(dyn, l, lo, hi, [H], game=g)[0] for g in GO.GAMES}
+    V = {g: R.solve(dyn, l, lo, hi, [H], game=g)[0] for g in HO.GAMES}
     a = float((V[1] - V[2]).max())
     b = float((V[2] - V[0]).max())
     gaps = [float((V[0] - V[2]).max()), float((V[2] - V[1]).max())]
@@ -415,11 +403,11 @@ def test_the_adversarial_value_is_guaranteed_along_trajectories(dyn):
     g = TG.GAME[dyn]
     DEV = TG.DEV
     from layered_safe_marl_b200 import SafetyFilter
-    sf = SafetyFilter(g['name'], value_grid=_grid(dyn, GO.ADVERSARIAL))
+    sf = SafetyFilter(g['name'], value_grid=_grid(dyn, HO.ADVERSARIAL))
     ego, oth = TG._start_pairs(dyn, torch)
     N = ego.shape[0]
     V0 = sf.values(ego=ego, other=oth)[0]
-    Vc = SafetyFilter(g['name'], value_grid=_grid(dyn, GO.COOPERATIVE)).values(ego=ego, other=oth)[0]
+    Vc = SafetyFilter(g['name'], value_grid=_grid(dyn, HO.COOPERATIVE)).values(ego=ego, other=oth)[0]
     assert torch.isfinite(V0).all()
     corners = TG._t_corners(dyn, torch)
     # KI[e, o]: the joint corner with the ego at its corner e and the other agent at its corner o
@@ -476,7 +464,7 @@ def test_the_adversarial_value_is_guaranteed_along_trajectories(dyn):
 
 
 @gpu
-@pytest.mark.parametrize('game', [GO.ADVERSARIAL, GO.CONSTANT])
+@pytest.mark.parametrize('game', [HO.ADVERSARIAL, HO.CONSTANT])
 @pytest.mark.parametrize('case', ['cfg2', 'cfg3'])
 def test_game_grid_drives_the_env_bit_for_bit_with_the_oracle(case, game, monkeypatch):
     import test_cuda_parity as P
@@ -500,7 +488,7 @@ def test_game_grid_drives_the_env_bit_for_bit_with_the_oracle(case, game, monkey
 
 
 @gpu
-@pytest.mark.parametrize('game', [GO.ADVERSARIAL, GO.CONSTANT])
+@pytest.mark.parametrize('game', [HO.ADVERSARIAL, HO.CONSTANT])
 @pytest.mark.parametrize('dyn', [0, 1])
 def test_safety_filter_over_a_game_grid_equals_the_oracle(dyn, game):
     import test_safety_filter_op as F
@@ -515,7 +503,7 @@ def test_safety_filter_over_a_game_grid_equals_the_oracle(dyn, game):
 
 
 @gpu
-@pytest.mark.parametrize('game', [GO.ADVERSARIAL, GO.CONSTANT])
+@pytest.mark.parametrize('game', [HO.ADVERSARIAL, HO.CONSTANT])
 def test_game_solve_on_a_side_stream(game):
     import torch
     shape, lo, hi = AT_LAT

@@ -1,5 +1,5 @@
 """The airtaxi time-to-reach solve (liblsm_b200_hj.so lsm_hj_ttr_*, reachability.solve_ttr / ttr_grid) against the
-numpy restatement of its declared scheme (tests/hj_ttr_oracle.py) and against the game it solves.
+numpy restatement of its declared scheme (tests/hj_solve_oracle.py, Lattice kind TTR) and against the game it solves.
 
 CPU: the ctypes mirror of lsm_hj_ttr_problem; the library exports the TTR entry points and holds the TTR kernels; the
 dissipation coefficients and time step equal the oracle's bit for bit; every invalid argument is refused with code 2;
@@ -26,7 +26,7 @@ sys.path.insert(0, os.path.join(REPO, 'oracle'))
 sys.path.insert(0, os.path.join(REPO, 'tests'))
 
 import _golden as G  # noqa: E402
-import hj_ttr_oracle as TO  # noqa: E402
+import hj_solve_oracle as HO  # noqa: E402
 from layered_safe_marl_b200 import _build, _lib, hj_grid  # noqa: E402
 from layered_safe_marl_b200 import reachability as R  # noqa: E402
 from layered_safe_marl_b200.config import AirTaxiConfig as ATC  # noqa: E402
@@ -85,7 +85,7 @@ def test_ttr_kernels_are_built_for_sm100a_and_exported():
 ])
 def test_ttr_dissipation_equals_the_oracle_bit_for_bit(shape, lo, hi, cfl):
     alpha, dt = R.ttr_dissipation(shape, lo, hi, cfl)
-    o_alpha, o_dt = TO.dissipation(TO.Lattice(shape, lo, hi), cfl)
+    o_alpha, o_dt = HO.dissipation(HO.Lattice(HO.TTR, shape, lo, hi), cfl)
     assert np.array_equal(alpha, o_alpha) and dt == o_dt, (alpha, o_alpha, dt, o_dt)
     assert alpha[2] == W and alpha[3] == max(abs(AMIN), abs(AMAX))
 
@@ -180,7 +180,7 @@ def _ref_hamiltonian(r, c, rng):
 
 def _check_probe(oracle, c):
     shape, lo, hi = PROBE_LAT
-    lat = oracle.Lattice(shape, lo, hi)
+    lat = oracle.Lattice(oracle.TTR, shape, lo, hi)
     X = np.stack(np.meshgrid(*lat.coords, indexing='ij'), -1)
     u = X @ c + 0.3
     alpha, _ = oracle.dissipation(lat)
@@ -203,7 +203,7 @@ def _check_probe(oracle, c):
 def test_oracle_hamiltonian_is_the_unicycle_game(k):
     """One step of 1e-7 from u = c . x + b: (V - u) / h = min(0, H_ref) at every cell 3 nodes inside the lattice, where
     WENO5 returns the slope exactly and the dissipation vanishes."""
-    err, tol, neg = _check_probe(TO, np.array(PROBE_C[k]))
+    err, tol, neg = _check_probe(HO, np.array(PROBE_C[k]))
     print(f"c={PROBE_C[k]}: H_ref < 0 at {neg:.0%}, max |(V - u)/h - min(0, H_ref)| = {err:.3e} (tol {tol:.3e})")
     assert err <= tol
 
@@ -219,10 +219,10 @@ MUTATIONS = {
 @pytest.mark.parametrize('name', list(MUTATIONS))
 def test_a_mutated_oracle_fails_the_game_check(name):
     old, new = MUTATIONS[name]
-    src = open(TO.__file__).read()
+    src = open(HO.__file__).read()
     assert src.count(old) == 1, old
-    mod = types.ModuleType('hj_ttr_oracle_mutant')
-    exec(compile(src.replace(old, new), TO.__file__, 'exec'), mod.__dict__)
+    mod = types.ModuleType('hj_solve_oracle_mutant')
+    exec(compile(src.replace(old, new), HO.__file__, 'exec'), mod.__dict__)
     failed = 0
     for c in PROBE_C:
         err, tol, _ = _check_probe(mod, np.array(c))
@@ -265,7 +265,7 @@ def test_solve_ttr_equals_the_oracle_bit_for_bit(shape, cfl):
     for init in (l, l + 0.05 * rng.standard_normal(shape)):      # noise: every ghost sign and WENO branch
         for horizon in (0.0, 2.5 * dt, 7.3 * dt, 12.0 * dt):
             ttr, V = R.solve_ttr(_cuda(init), lo, hi, horizon, cfl)
-            want_t, want_v = TO.solve(init, lo, hi, horizon, cfl)
+            want_t, want_v = HO.solve_ttr(init, lo, hi, horizon, cfl)
             _assert_bits(ttr.cpu().numpy(), want_t, f'ttr {shape} cfl={cfl} horizon={horizon}')
             _assert_bits(V.cpu().numpy(), want_v, f'V {shape} cfl={cfl} horizon={horizon}')
             if horizon == 0.0:
@@ -281,7 +281,7 @@ def test_ttr_arrays_past_2_31_bytes_advance_one_step():
     shape, lo, hi = (401, 401, 24, 73), TTR_LAT[1], TTR_LAT[2]
     cells = int(np.prod(shape))
     assert cells * 8 > 2 ** 31
-    lat = TO.Lattice(shape, lo, hi)
+    lat = HO.Lattice(HO.TTR, shape, lo, hi)
     x = torch.as_tensor(lat.coords[0], device='cuda').view(-1, 1, 1, 1)
     y = torch.as_tensor(lat.coords[1], device='cuda').view(1, -1, 1, 1)
     th = torch.as_tensor(lat.coords[2], device='cuda').view(1, 1, -1, 1)
@@ -299,9 +299,9 @@ def test_ttr_arrays_past_2_31_bytes_advance_one_step():
         stops = [min(n, k + 10) for k, n in zip(c, shape)]
         starts[2], stops[2] = 0, shape[2]                        # the whole periodic dim
         block = init[tuple(slice(a, b) for a, b in zip(starts, stops))].cpu().numpy()
-        u3 = TO.step_at(lat, block, starts, alpha, dt)
+        u3 = HO.step_at(lat, block, starts, alpha, dt)
         t = np.where(block <= 0.0, 0.0, np.inf)
-        TO.arrive(t, block, u3, 0.0, dt)
+        HO.arrive(t, block, u3, 0.0, dt)
         at = tuple(k - a for k, a in zip(c, starts))
         for what, got, want in (('V', float(V[c]), u3[at]), ('ttr', float(ttr[c]), t[at])):
             assert np.float64(got).view(np.int64) == np.float64(want).view(np.int64), (what, c, got, want)
@@ -347,7 +347,7 @@ def _solved(shape=TTR_LAT[0], horizon=R.DEFAULT_TTR_HORIZON):
 def _row_error(shape):
     """Max |TTR - t*| on the y = 0, theta = 0 row over x in [-6, -0.8] and every speed node."""
     t = _solved(shape)
-    lat = TO.Lattice(shape, *TTR_LAT[1:])
+    lat = HO.Lattice(HO.TTR, shape, *TTR_LAT[1:])
     x, th, v = lat.coords[0], lat.coords[2], lat.coords[3]
     j, k = shape[1] // 2, int(np.argmin(np.abs(th)))
     assert lat.coords[1][j] == 0.0 and abs(th[k]) < 1e-12
@@ -379,7 +379,7 @@ def test_straight_line_closed_form_and_refinement():
 def test_no_cell_beats_the_no_turn_lower_bound():
     """No path to the goal disc is shorter than the straight line at full acceleration: TTR >= t*(max(0, d - r), v)."""
     t = _solved()
-    lat = TO.Lattice(*TTR_LAT)
+    lat = HO.Lattice(HO.TTR, *TTR_LAT)
     x, y, v = lat.coords[0], lat.coords[1], lat.coords[3]
     d = np.sqrt(x[:, None] ** 2 + y[None, :] ** 2)
     lb = _t_star(np.maximum(0.0, d - GOAL_R)[:, :, None, None], v[None, None, None, :])
@@ -494,7 +494,7 @@ def test_rollouts_attain_and_never_beat_the_ttr():
     heading outside the 45 deg cone, where the 0.4 km lattice cannot resolve the 0.35 km disc, and turn once more
     (+45 to +50 s, one turn being 2 pi / w = 63 s); the test allows that for at most 10 % of the starts."""
     t = _solved()
-    lat = TO.Lattice(*TTR_LAT)
+    lat = HO.Lattice(HO.TTR, *TTR_LAT)
     tt = np.where(np.isinf(t), R.DEFAULT_TTR_HORIZON, t)
     rng = np.random.default_rng(17)
     m = 96
@@ -526,7 +526,7 @@ def test_default_horizon_reaches_the_interior():
     H and 2H solves."""
     H = R.DEFAULT_TTR_HORIZON
     t1, t2 = _solved(horizon=H), _solved(horizon=2 * H)
-    lat = TO.Lattice(*TTR_LAT)
+    lat = HO.Lattice(HO.TTR, *TTR_LAT)
     x, y = lat.coords[0], lat.coords[1]
     inner = ((np.abs(x)[:, None] <= 8.0 - 2.0 + 1e-9) & (np.abs(y)[None, :] <= 8.0 - 2.0 + 1e-9))[:, :, None, None]
     inner = np.broadcast_to(inner, t1.shape)
